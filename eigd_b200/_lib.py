@@ -44,6 +44,8 @@ SIGNATURES = {
     "eigd_factor_destroy": (None, [c_ptr]),
     "eigd_factor_numeric": (c_int, [c_ptr, c_i64, c_ptr, c_ptr]),
     "eigd_factor_info": (c_int, [c_ptr, c_ptr]),
+    "eigd_factor_set_pivoting": (c_int, [c_ptr, c_int]),
+    "eigd_factor_pivot_counts": (c_int, [c_ptr, c_ptr]),
     "eigd_dmma_peak": (c_int, [c_int, c_int, c_ptr]),
     "eigd_factor_solve": (c_int, [c_ptr, c_ptr, c_i64, c_i64, c_ptr, c_i64, c_i64, c_int]),
     "eigd_factor_bytes": (c_i64, [c_ptr]),

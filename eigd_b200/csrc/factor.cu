@@ -8,7 +8,8 @@
 //            columns [0, ncols) hold L (unit diagonal implied, D on the diagonal), the
 //            trailing (f-ncols)^2 block is the contribution passed to the parent.
 //   linv   : explicit inverses of the 32x32 unit-lower diagonal blocks of every L11 (used by the
-//            panel solves of the factorisation).
+//            panel solves of the factorisation); with restricted Bunch-Kaufman pivoting the inverses of
+//            the dense diagonal blocks M (diag_factor_bk_kernel).
 //   xinv   : the full inverse X = L11^{-1} of every pivot block (recursive doubling from the
 //            32x32 inverses: X21 = -B^{-1} C A^{-1}).
 //   sfwd / sbwd : the solve panels S = [X ; -L21 X] (f x nc, column-major) and S^T (nc x f):
@@ -346,7 +347,173 @@ diag_factor_kernel(SymDev d, const int2* __restrict__ tasks, int kb, double* __r
   }
 }
 
-// rows below the pivot block: L_row = (F_row * Linv^T) * D^-1 ; one thread per row
+// Restricted Bunch-Kaufman variant of diag_factor_kernel (pivoting mode 1).  Bunch-Kaufman with alpha = (1 + sqrt 17) / 8,
+// the pivot search restricted to the rows and columns of this 32-column block, ties to the lowest index: 1x1 pivots,
+// 1x1 pivots with an interchange, or 2x2 pivots, which are rotated to diagonal form (Jacobi rotation) and eliminated
+// as two 1x1 pivots.  With R the product of the interchanges and rotations (orthogonal) and L unit lower,
+// R T R^T = L Lam L^T, i.e. T = M Lam M^T with M = R^T L, Lam diagonal.  Outputs as diag_factor_kernel: Li = M^-1 =
+// L^-1 R (dense), Lam in dval / dinv; the kernels after this one only use Li and Lam (see trsm_kernel,
+// inverse_init_kernel and the solve's tile bounds).  info[3] += 2x2 pivots, info[4] += interchanges.
+// Every warp takes the pivot decision redundantly from shared memory (warp reductions over the column / row,
+// lane 0's result broadcast: the decision is uniform), so a step costs a block barrier only where it writes.
+constexpr double BK_ALPHA = 0.6403882032022076;        // (1 + sqrt(17)) / 8
+
+__device__ __forceinline__ void warp_absmax(double& v, int& i) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const double v2 = __shfl_xor_sync(0xffffffffu, v, o);
+    const int i2 = __shfl_xor_sync(0xffffffffu, i, o);
+    if (v2 > v || (v2 == v && i2 < i)) { v = v2; i = i2; }
+  }
+  v = __shfl_sync(0xffffffffu, v, 0);
+  i = __shfl_sync(0xffffffffu, i, 0);
+}
+
+__global__ void __launch_bounds__(256)
+diag_factor_bk_kernel(SymDev d, const int2* __restrict__ tasks, int kb, double* __restrict__ fronts,
+                      double* __restrict__ linv, double* __restrict__ dval, double* __restrict__ dinv,
+                      const unsigned long long* __restrict__ amax_bits, double piv_tol,
+                      unsigned long long* __restrict__ info) {
+  __shared__ double T[NB][NB + 1];        // lower triangle; column j < current step holds d_j * L(:, j)
+  __shared__ double Li[NB][NB + 1];       // R during the elimination, L^-1 R afterwards
+  __shared__ double ds[NB];
+  int s = tasks[blockIdx.x].x;
+  int first = d.sn_first[s];
+  int nc = d.sn_first[s + 1] - first;
+  int64_t f = nc + (d.sn_rowptr[s + 1] - d.sn_rowptr[s]);
+  int j0 = kb * NB;
+  int bs = min(NB, nc - j0);
+  double* F = fronts + d.front_off[s];
+  const int tid = threadIdx.x, tx = tid & 31, ty = tid >> 5;
+  for (int c = ty; c < NB; c += 8) {
+    T[tx][c] = (tx < bs && c < bs && tx >= c) ? F[(j0 + tx) + (int64_t)(j0 + c) * f] : 0.0;
+    Li[tx][c] = (tx == c) ? 1.0 : 0.0;
+  }
+  const double thr = piv_tol * __longlong_as_double((long long)(*amax_bits));
+  int nneg = 0, npert = 0, nbad = 0, n2 = 0, nswap = 0;
+  auto at = [&](int i, int j) { return i >= j ? T[i][j] : T[j][i]; };
+  // symmetric interchange of positions p < q (both >= the current step): thread m < 32 swaps the pair of lower-triangle
+  // entries of index m, threads 32 .. 63 swap rows p, q of R
+  auto swap = [&](int p, int q) {
+    if (tid < 32) {
+      const int m = tid;
+      double *x = nullptr, *y = nullptr;
+      if (m < p) { x = &T[p][m]; y = &T[q][m]; }
+      else if (m == p) { x = &T[p][p]; y = &T[q][q]; }
+      else if (m < q) { x = &T[m][p]; y = &T[q][m]; }
+      else if (m > q) { x = &T[m][p]; y = &T[m][q]; }
+      if (x) { const double t = *x; *x = *y; *y = t; }
+    } else if (tid < 64) {
+      const int m = tid - 32;
+      const double t = Li[p][m]; Li[p][m] = Li[q][m]; Li[q][m] = t;
+    }
+  };
+  __syncthreads();
+  bool second = false;                    // step j is the second column of a rotated 2x2 pivot
+  for (int j = 0; j < bs; ++j) {
+    if (!second) {
+      const double akk = fabs(T[j][j]);
+      double cmax = (tx > j && tx < bs) ? fabs(T[tx][j]) : 0.0;
+      int imax = (tx > j && tx < bs) ? tx : NB;
+      warp_absmax(cmax, imax);
+      int piv = j;
+      if (imax < bs && !(akk >= BK_ALPHA * cmax)) {
+        double rmax = (tx >= j && tx < bs && tx != imax) ? fabs(at(imax, tx)) : 0.0;
+        int dummy = 0;
+        warp_absmax(rmax, dummy);
+        const double a = T[j][j], b = T[imax][j], c = T[imax][imax];
+        __syncthreads();                  // every warp has read the row of imax: the step may now write
+        if (akk >= BK_ALPHA * cmax * (cmax / rmax)) {
+        } else if (fabs(c) >= BK_ALPHA * rmax) {
+          piv = imax;
+        } else {
+          n2++;
+          if (imax != j + 1) { swap(j + 1, imax); nswap++; __syncthreads(); }
+          // Jacobi rotation J = [cs sn; -sn cs] with J^T [a b; b c] J = diag(a - t b, c + t b); rows / columns j, j + 1
+          // of the block and rows j, j + 1 of R and of L(:, < j) become J^T (x_j, x_j+1)
+          const double tau = (c - a) / (2.0 * b);
+          const double t = (tau >= 0.0 ? 1.0 : -1.0) / (fabs(tau) + sqrt(1.0 + tau * tau));
+          const double cs = 1.0 / sqrt(1.0 + t * t), sn = t * cs;
+          if (tid < 32) {
+            const int m = tid;
+            if (m < j) {
+              const double x = T[j][m], y = T[j + 1][m];
+              T[j][m] = cs * x - sn * y;
+              T[j + 1][m] = sn * x + cs * y;
+            } else if (m == j) {
+              T[j][j] = a - t * b;
+              T[j + 1][j + 1] = c + t * b;
+              T[j + 1][j] = 0.0;
+            } else if (m > j + 1) {
+              const double x = T[m][j], y = T[m][j + 1];
+              T[m][j] = cs * x - sn * y;
+              T[m][j + 1] = sn * x + cs * y;
+            }
+          } else if (tid < 64) {
+            const int m = tid - 32;
+            const double x = Li[j][m], y = Li[j + 1][m];
+            Li[j][m] = cs * x - sn * y;
+            Li[j + 1][m] = sn * x + cs * y;
+          }
+          __syncthreads();
+          second = true;
+        }
+      }
+      if (piv != j) { swap(j, piv); nswap++; __syncthreads(); }
+    } else {
+      second = false;
+    }
+    double dj = T[j][j];
+    if (!(dj == dj) || fabs(dj) > 1e300) { nbad++; dj = thr > 0.0 ? thr : 1.0; }
+    if (fabs(dj) < thr) { dj = (dj >= 0.0) ? thr : -thr; npert++; }
+    if (dj < 0.0) nneg++;
+    if (tid == 0) ds[j] = dj;
+    const double rd = 1.0 / dj;
+    if (tx > j) {
+      const double lij = T[tx][j] * rd;
+      for (int c = j + 1 + ((ty - (j + 1)) & 7); c <= tx; c += 8) T[tx][c] = fma(-lij, T[c][j], T[tx][c]);
+    }
+    __syncthreads();
+  }
+  for (int c = ty; c < bs; c += 8)
+    if (tx > c && tx < bs) T[tx][c] *= 1.0 / ds[c];
+  __syncthreads();
+  // Li <- L^-1 R: forward substitution on every column of R, column c by lanes 8c .. 8c+7 (as diag_factor_kernel)
+  {
+    const int c = tid >> 3, q = tid & 7;
+    const unsigned gmask = 0xffu << (8 * (c & 3));
+    for (int i = 1; i < bs; ++i) {
+      double sum = 0.0;
+      for (int k = q; k < i; k += 8) sum = fma(T[i][k], Li[k][c], sum);
+      sum += __shfl_xor_sync(gmask, sum, 1);
+      sum += __shfl_xor_sync(gmask, sum, 2);
+      sum += __shfl_xor_sync(gmask, sum, 4);
+      if (q == 0) Li[i][c] -= sum;
+      __syncwarp(gmask);
+    }
+  }
+  __syncthreads();
+  for (int c = ty; c < bs; c += 8)
+    if (tx < bs && tx > c) F[(j0 + tx) + (int64_t)(j0 + c) * f] = T[tx][c];
+  if (tid < bs) F[(j0 + tid) + (int64_t)(j0 + tid) * f] = ds[tid];
+  double* Lo = linv + d.linv_off[s] + (int64_t)kb * NB * NB;
+  for (int c = ty; c < NB; c += 8) Lo[tx + c * NB] = Li[tx][c];
+  if (tid < bs) {
+    dval[first + j0 + tid] = ds[tid];
+    dinv[first + j0 + tid] = 1.0 / ds[tid];
+  }
+  if (tid == 0) {
+    if (nneg) atomicAdd(&info[0], (unsigned long long)nneg);
+    if (npert) atomicAdd(&info[1], (unsigned long long)npert);
+    if (nbad) atomicAdd(&info[2], (unsigned long long)nbad);
+    if (n2) atomicAdd(&info[3], (unsigned long long)n2);
+    if (nswap) atomicAdd(&info[4], (unsigned long long)nswap);
+  }
+}
+
+// rows below the pivot block: L_row = (F_row * Linv^T) * D^-1 ; one thread per row.  DENSE (pivoted factor): Li is a
+// dense 32x32 block, otherwise unit lower triangular
+template <bool DENSE>
 __global__ void __launch_bounds__(TRSM_ROWS)
 trsm_kernel(SymDev d, const int2* __restrict__ tasks, int kb, double* __restrict__ fronts,
             const double* __restrict__ linv, const double* __restrict__ dinv) {
@@ -373,7 +540,7 @@ trsm_kernel(SymDev d, const int2* __restrict__ tasks, int kb, double* __restrict
   for (int c = 0; c < NB; ++c) {
     double sum = 0.0;
 #pragma unroll
-    for (int k = 0; k <= c; ++k) sum = fma(x[k], Li[c][k], sum);
+    for (int k = 0; k < (DENSE ? NB : c + 1); ++k) sum = fma(x[k], Li[c][k], sum);
     if (c < bs) F[(int64_t)c * f] = sum * di[c];
   }
 }
@@ -493,7 +660,11 @@ __device__ __forceinline__ void tile_gemm32(int K, FA fa, FB fb, double acc[4], 
   }
 }
 
-// X <- diag(linv blocks) (X was zeroed by a memset); one CTA per front
+// X <- diag(linv blocks) (X was zeroed by a memset); one CTA per front.  DENSE (pivoted factor): the whole 32x32 block
+// M^-1 of every pivot block, otherwise its lower triangle.  X = M11^-1 is then block lower triangular at 32-column
+// granularity; the doubling stages below (inverse_ca_kernel, inverse_bt_kernel) assume triangularity only at that
+// granularity -- their reduction bounds start / end at 32-column tile edges -- and so compute M11^-1 as written.
+template <bool DENSE>
 __global__ void __launch_bounds__(256)
 inverse_init_kernel(SymDev d, const int2* __restrict__ tasks, const double* __restrict__ linv, double* __restrict__ xinv) {
   int s = tasks[blockIdx.x].x;
@@ -505,7 +676,7 @@ inverse_init_kernel(SymDev d, const int2* __restrict__ tasks, const double* __re
     int kb = e / (NB * NB), r = e - kb * NB * NB;
     int i = r & 31, j = r >> 5;
     int gi = kb * NB + i, gj = kb * NB + j;
-    if (gi < nc && gj < nc && i >= j) X[gi + (int64_t)gj * nc] = Lo[e];
+    if (gi < nc && gj < nc && (DENSE || i >= j)) X[gi + (int64_t)gj * nc] = Lo[e];
   }
 }
 
@@ -747,7 +918,7 @@ extern "C" int eigd_factor_numeric(eigd_factor* f, int64_t nnz, const double* d_
   int64_t nfront = s->front_off[s->nsuper];
   EIGD_CUDA(cudaMemsetAsync(f->fronts, 0, (size_t)nfront * 8, g_eigd_stream));
   EIGD_CUDA(cudaMemsetAsync(f->amax, 0, 8, g_eigd_stream));
-  EIGD_CUDA(cudaMemsetAsync(f->info, 0, 32, g_eigd_stream));
+  EIGD_CUDA(cudaMemsetAsync(f->info, 0, f->pivoting ? 40 : 32, g_eigd_stream));
   EIGD_CUDA(cudaMemsetAsync(f->xinv, 0, (size_t)std::max<int64_t>(h->xinv_total, 1) * 8, g_eigd_stream));
   int g = (int)std::min<int64_t>((nnz + 255) / 256, 148 * 16);
   if (g < 1) g = 1;
@@ -767,10 +938,19 @@ extern "C" int eigd_factor_numeric(eigd_factor* f, int64_t nnz, const double* d_
     if (prof) cudaEventRecord(pe0, g_eigd_stream);
     switch (L.kind) {
       case 0: EIGD_LAUNCH(extend_add_kernel, L.count, 256, 0, h->d, t, f->fronts); break;
-      case 1: EIGD_LAUNCH(diag_factor_kernel, L.count, 256, 0, h->d, t, L.kb, f->fronts, f->linv, f->dval, f->dinv, f->amax, f->piv_tol, f->info); break;
-      case 2: EIGD_LAUNCH(trsm_kernel, L.count, TRSM_ROWS, 0, h->d, t, L.kb, f->fronts, f->linv, f->dinv); break;
+      case 1:
+        if (f->pivoting) EIGD_LAUNCH(diag_factor_bk_kernel, L.count, 256, 0, h->d, t, L.kb, f->fronts, f->linv, f->dval, f->dinv, f->amax, f->piv_tol, f->info);
+        else EIGD_LAUNCH(diag_factor_kernel, L.count, 256, 0, h->d, t, L.kb, f->fronts, f->linv, f->dval, f->dinv, f->amax, f->piv_tol, f->info);
+        break;
+      case 2:
+        if (f->pivoting) EIGD_LAUNCH(trsm_kernel<true>, L.count, TRSM_ROWS, 0, h->d, t, L.kb, f->fronts, f->linv, f->dinv);
+        else EIGD_LAUNCH(trsm_kernel<false>, L.count, TRSM_ROWS, 0, h->d, t, L.kb, f->fronts, f->linv, f->dinv);
+        break;
       case 3: EIGD_LAUNCH(trailing_update_kernel, L.count, 256, 0, h->d, t, L.kb, f->fronts, f->dval); break;
-      case 4: EIGD_LAUNCH(inverse_init_kernel, L.count, 256, 0, h->d, t, f->linv, f->xinv); break;
+      case 4:
+        if (f->pivoting) EIGD_LAUNCH(inverse_init_kernel<true>, L.count, 256, 0, h->d, t, f->linv, f->xinv);
+        else EIGD_LAUNCH(inverse_init_kernel<false>, L.count, 256, 0, h->d, t, f->linv, f->xinv);
+        break;
       case 5: EIGD_LAUNCH(inverse_ca_kernel, L.count, 256, 0, h->d, t, NB << L.kb, f->fronts, f->xinv, f->xtmp); break;
       case 6: EIGD_LAUNCH(inverse_bt_kernel, L.count, 256, 0, h->d, t, NB << L.kb, f->xinv, f->xtmp); break;
       case 7: EIGD_LAUNCH(panel_build_kernel, L.count, 256, 0, h->d, t, f->fronts, f->xinv, f->sfwd, f->sbwd); break;
@@ -842,6 +1022,23 @@ extern "C" int eigd_dmma_peak(int iters, int reps, double* tflops_out) {
   cudaEventDestroy(e1);
   cudaFree(sink);
   *tflops_out = best;
+  return 0;
+}
+
+extern "C" int eigd_factor_set_pivoting(eigd_factor* f, int mode) {
+  if (mode != 0 && mode != 1) { eigd_set_error("factor_set_pivoting: mode %d (0 static, 1 restricted Bunch-Kaufman)", mode); return 1; }
+  f->pivoting = mode;
+  return 0;
+}
+
+extern "C" int eigd_factor_pivot_counts(eigd_factor* f, int64_t* out2) {
+  out2[0] = out2[1] = 0;
+  if (!f->pivoting) return 0;
+  unsigned long long h[2];
+  EIGD_CUDA(cudaMemcpyAsync(h, f->info + 3, 16, cudaMemcpyDeviceToHost, g_eigd_stream));
+  EIGD_CUDA(cudaStreamSynchronize(g_eigd_stream));
+  out2[0] = (int64_t)h[0];
+  out2[1] = (int64_t)h[1];
   return 0;
 }
 

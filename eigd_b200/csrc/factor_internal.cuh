@@ -66,7 +66,8 @@ struct eigd_factor {
   SymDevHolder* h = nullptr;
   int max_rhs = 1;
   double* fronts = nullptr;   // f x f frontal matrices (factorisation workspace)
-  double* linv = nullptr;     // inverses of the 32x32 unit-lower diagonal blocks
+  double* linv = nullptr;     // inverses of the 32x32 unit-lower diagonal blocks (pivoted: of the dense blocks M, see
+                              // diag_factor_bk_kernel)
   double* xinv = nullptr;     // full inverse of every L11 (nc x nc, column-major)
   double* xtmp = nullptr;     // scratch of the same size (recursive-doubling products)
   double* sfwd = nullptr;     // solve panels S = [L11^-1 ; -L21 L11^-1], f x nc: column-major below the cut of the solve
@@ -85,6 +86,7 @@ struct eigd_factor {
   unsigned* cnt = nullptr;                // per-front completion counters of the solve (2 per supernode), monotone
   unsigned epoch = 0;                     // cooperative solve launches issued so far (host mirror)
   double piv_tol = 1e-11;
+  int pivoting = 0;                       // 0 static pivots, 1 restricted Bunch-Kaufman (eigd_factor_set_pivoting)
   int64_t bytes = 0;
   char* base = nullptr;
   bool owns = true;

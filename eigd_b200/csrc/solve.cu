@@ -84,6 +84,9 @@ struct SolveArgs {
                                   // phase, 16 slots per phase: 0 start, 1 waited, 2 product done, 3 reduced, 4 stored,
                                   // 5 signalled, 6 slot (record + panel slice) there, 7 end of tile, 8 top of the phase loop,
                                   // 9 dispatch
+  int blk_mask;                   // 31 for a factor with restricted Bunch-Kaufman pivoting, else 0: its pivot blocks of S are
+                                  // block lower triangular at 32-row granularity (dense 32 x 32 diagonal blocks), so the
+                                  // triangular skip bounds of a thin tile (TH < 32) are widened to the 32-row block
 };
 
 // vectors produced earlier in the same launch by other SMs are read through L2 (ld.global.cg): L1 is
@@ -269,7 +272,9 @@ __device__ __forceinline__ void tile_compute(const SolveArgs& a, int dir, bool u
   const int out = o0 + (lane % to);
   if (dir == 0) {
     // ---- forward: outputs are front rows; acc = S[row, 0:cend) w1 (+ the children's updates of the row)
-    const int cend = min(nc, o0 + to);                  // S is lower triangular inside the pivot rows
+    // S is lower triangular inside the pivot rows (a pivoted factor: at 32-row granularity; TH = 32 tiles start on a
+    // 32-row edge, thin tiles read on to the end of their 32-row block)
+    const int cend = min(nc, TH < 32 ? (o0 + to + a.blk_mask) & ~a.blk_mask : o0 + to);
     const int per = solve_slice_len(cend, ws);
     const int c0 = min(cend, slice * per), c1 = min(cend, c0 + per);
     const int th = min(to, f - o0);                     // rows of this row tile
@@ -302,10 +307,12 @@ __device__ __forceinline__ void tile_compute(const SolveArgs& a, int dir, bool u
       for (int r = 0; r < KT; ++r) acc[r] += cu[r];
     }
   } else {
-    // ---- backward: outputs are pivot columns; acc = S^T[col, o0:f) [z1 ; x2]
-    const int len = f - o0;
+    // ---- backward: outputs are pivot columns; acc = S^T[col, ob:f) [z1 ; x2], ob = o0 (pivoted factor, thin tile: the
+    // first row of o0's 32-row block)
+    const int ob = TH < 32 ? o0 & ~a.blk_mask : o0;
+    const int len = f - ob;
     const int per = solve_slice_len(len, ws);
-    const int i0 = min(f, o0 + slice * per), i1 = min(f, i0 + per);
+    const int i0 = min(f, ob + slice * per), i1 = min(f, i0 + per);
     const int tw = min(to, nc - o0);                    // pivot columns of this column tile
     const double* M = TILED ? a.sbwd + tr.soff + (int64_t)o0 * f + min(lane % to, tw - 1) : a.sbwd + tr.soff + min(out, nc - 1);
     warp_panel_product<KT, MCT, TH>(M, TILED ? tw : nc, i0, i1, lane, stage, acc, [&](int i, double* v) {
@@ -980,24 +987,26 @@ __device__ __forceinline__ bool mbar_test(unsigned long long* bar, unsigned pari
 }
 
 // the part of tile (tr, height th_) that warp `slice` of `ws` multiplies: first reduction index, count, leading dimension
-// (rows of a forward row tile / pivot columns of a backward column tile) and the offset of the run in sfwd / sbwd
+// (rows of a forward row tile / pivot columns of a backward column tile) and the offset of the run in sfwd / sbwd;
+// bm = SolveArgs::blk_mask (the reduction ranges of tile_compute)
 struct SliceDesc {
   int64_t off;
   int r0, len, ld;
 };
-__device__ __forceinline__ SliceDesc slice_of(const TileRec& tr, int dir, int th_, int slice, int ws) {
+__device__ __forceinline__ SliceDesc slice_of(const TileRec& tr, int dir, int th_, int slice, int ws, int bm) {
   const int nc = tr.nc, f = tr.nc + tr.nb, o0 = tr.tile * th_;
   SliceDesc s;
   if (dir == 0) {
-    const int cend = min(nc, o0 + th_);
+    const int cend = min(nc, (o0 + th_ + bm) & ~bm);
     const int per = solve_slice_len(cend, ws);
     s.r0 = min(cend, slice * per);
     s.len = min(cend, s.r0 + per) - s.r0;
     s.ld = min(th_, f - o0);
     s.off = tr.soff + (int64_t)o0 * nc + (int64_t)s.r0 * s.ld;
   } else {
-    const int per = solve_slice_len(f - o0, ws);
-    s.r0 = min(f, o0 + slice * per);
+    const int ob = o0 & ~bm;
+    const int per = solve_slice_len(f - ob, ws);
+    s.r0 = min(f, ob + slice * per);
     s.len = min(f, s.r0 + per) - s.r0;
     s.ld = min(th_, nc - o0);
     s.off = tr.soff + (int64_t)o0 * f + (int64_t)s.r0 * s.ld;
@@ -1062,7 +1071,7 @@ __device__ __forceinline__ void pipe_producer(const SolveArgs& a, char* pipe_bas
         r0 = __ldg(tp); r1 = __ldg(tp + 1); r2 = __ldg(tp + 2);
         r3 = __ldg(dp); r4 = __ldg(dp + 1);
         dir = ph.dir;
-        sd = slice_of(unpack_tile(r0, r1, r2), dir, (int)(ph.pad & 0xff), w % ph.ws, ph.ws);
+        sd = slice_of(unpack_tile(r0, r1, r2), dir, (int)(ph.pad & 0xff), w % ph.ws, ph.ws, a.blk_mask);
         bytes = (sd.len * sd.ld * 8 + 15) & ~15;
         loaded = true;
       }
@@ -1223,7 +1232,7 @@ __device__ __forceinline__ void level_phase_pipe(const SolveArgs& a, const Phase
       // the slice: in the warp's ring, or (larger than the ring, rare) where it lies in global memory -- same code,
       // generic loads
       const double* sbuf = reinterpret_cast<const double*>(sm.ring + max(sl.w, 0));
-      if (sl.w == -1) sbuf = (dir == 0 ? a.sfwd : a.sbwd) + slice_of(tr, dir, TH, slice, ws).off;
+      if (sl.w == -1) sbuf = (dir == 0 ? a.sfwd : a.sbwd) + slice_of(tr, dir, TH, slice, ws, a.blk_mask).off;
       tile_compute_smem<KT, TH>(a, dir, use_perm, tr, lane, slice, sl.x, sl.y, sl.z, sbuf, stage, acc, dw);
       __syncwarp();                 // every lane is done with the slot
       if (lane == 0) mbar_arrive(&sm.empty[cs.slot]);
@@ -1645,6 +1654,7 @@ extern "C" int eigd_factor_solve(eigd_factor* f, const double* B, int64_t brs, i
     a.xrs = xrs;
     a.xcs = xcs;
     a.k = kc;
+    a.blk_mask = f->pivoting ? 31 : 0;
     a.times = g_phase_times;
     a.trace = g_trace;
     a.skew = g_skew;

@@ -587,10 +587,19 @@ class PatternCache:
         return eid, ent[3], ent[4], True
 
 
-class Factor:
-    """Numeric LDL^T on the device for a fixed symbolic analysis."""
+PIVOTING_MODES = ("static", "bunch-kaufman")
 
-    def __init__(self, symbolic, max_rhs=32):
+
+class Factor:
+    """Numeric LDL^T on the device for a fixed symbolic analysis.
+
+    pivoting: "static" (no pivot search; a pivot below 1e-11 max|A| is perturbed to +-that threshold) or
+    "bunch-kaufman" (restricted Bunch-Kaufman 1x1 / 2x2 pivoting inside every 32-column pivot block, for indefinite
+    matrices with tiny or zero diagonal entries; pivots that are still tiny are perturbed and counted as well)."""
+
+    def __init__(self, symbolic, max_rhs=32, pivoting="static"):
+        if pivoting not in PIVOTING_MODES:
+            raise ValueError("pivoting must be one of %s, not %r" % (PIVOTING_MODES, pivoting))
         dev()
         self.sym = symbolic
         self.n = symbolic.n
@@ -605,6 +614,9 @@ class Factor:
               "factor_create_in")
         self.handle = h
         self.max_rhs = int(max_rhs)
+        self.pivoting = pivoting
+        if pivoting != "static":
+            check(lib.eigd_factor_set_pivoting(h, PIVOTING_MODES.index(pivoting)), "factor_set_pivoting")
 
     def __del__(self):
         try:
@@ -631,8 +643,12 @@ class Factor:
 
     def info(self):
         out = (ctypes.c_int64 * 3)()
-        check(_lib.load().eigd_factor_info(self.handle, ctypes.cast(out, ctypes.c_void_p)), "factor_info")
-        return {"negative_pivots": int(out[0]), "perturbed_pivots": int(out[1]), "non_finite": int(out[2])}
+        lib = _lib.load()
+        check(lib.eigd_factor_info(self.handle, ctypes.cast(out, ctypes.c_void_p)), "factor_info")
+        pc = (ctypes.c_int64 * 2)()
+        check(lib.eigd_factor_pivot_counts(self.handle, ctypes.cast(pc, ctypes.c_void_p)), "factor_pivot_counts")
+        return {"negative_pivots": int(out[0]), "perturbed_pivots": int(out[1]), "non_finite": int(out[2]),
+                "two_by_two_pivots": int(pc[0]), "interchanges": int(pc[1])}
 
     def nbytes(self):
         return int(_lib.load().eigd_factor_bytes(self.handle))

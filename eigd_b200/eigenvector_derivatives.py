@@ -102,11 +102,18 @@ class SpLuOperator:
 
     Extra keyword arguments (not in the reference): ``coords`` / ``dof_per_node`` enable geometric
     nested dissection, ``symbolic`` reuses an analysis, ``refine`` sets the number of iterative
-    refinement steps per solve (default: 1 if the factorisation met negative or perturbed pivots).
+    refinement steps per solve (default: 1 if the factorisation met negative or perturbed pivots),
+    ``pivoting`` chooses the pivot strategy of the LDL^T: ``"static"`` (default: no pivot search, a pivot below
+    1e-11 max|A| is perturbed to +-that threshold and the solves are refined) or ``"bunch-kaufman"`` (restricted
+    Bunch-Kaufman 1x1 / 2x2 pivoting inside every 32-column pivot block: for indefinite shifts with zero or tiny
+    diagonal entries, e.g. saddle-point operators or a shift close to an eigenvalue).  ``info`` reports the pivot
+    statistics either way; the probe / refinement policy is the same for both.
     """
 
     @_public
-    def __init__(self, mat, coords=None, dof_per_node=1, symbolic=None, refine=None, max_rhs=32):
+    def __init__(self, mat, coords=None, dof_per_node=1, symbolic=None, refine=None, max_rhs=32, pivoting="static"):
+        if pivoting not in D.PIVOTING_MODES:
+            raise ValueError("SpLuOperator: pivoting must be one of %s, not %r" % (D.PIVOTING_MODES, pivoting))
         self.tangent = None
         if isinstance(mat, D.CsrDevice):
             csr = mat
@@ -148,7 +155,7 @@ class SpLuOperator:
         elif isinstance(symbolic, D.Symbolic):
             symbolic = (symbolic, symbolic.assembly_map_device(csr.indptr, csr.indices))
         self.symbolic, self._amap = symbolic
-        self.lu = D.Factor(self.symbolic, max_rhs=max_rhs).numeric(csr.data, self._amap)
+        self.lu = D.Factor(self.symbolic, max_rhs=max_rhs, pivoting=pivoting).numeric(csr.data, self._amap)
         # The factorisation is now queued on the device.  Its pivot statistics (inertia, perturbed pivots) and the choice
         # of the refinement depth need a read-back, i.e. a wait for the whole factorisation: that is deferred to the first
         # use (``info`` / ``refine`` / the first solve), so that the caller's next host-side steps -- typically the

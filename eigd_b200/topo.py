@@ -412,13 +412,16 @@ class BucklingTopologyAnalysis:
     """examples/buckling.py ``TopologyAnalysis`` (:19-118): (K + BLF * G(u)) phi = 0 on the reduced dofs, with
     the fundamental path K_r u_r = f_r, shift-invert about ``sigma`` (mode="buckling": A = G_r, B = K_r,
     factor of K_r + sigma G_r, :548-640), and the gradient of an eigenvector functional including the
-    fundamental-path adjoint (:896-982).  Every vector of length n, 2*nnodes or nelems stays in HBM."""
+    fundamental-path adjoint (:896-982).  Every vector of length n, 2*nnodes or nelems stays in HBM.
+    ``pivoting`` (not in the reference) is the pivot strategy of the shifted factor K_r + sigma G_r (SpLuOperator);
+    the fundamental-path factor of K_r is SPD and always static."""
 
     def __init__(self, fltr, conn, X, bcs, forces={}, E=1.0, nu=0.3, ptype_K="simp", ptype_M="simp", ptype_G="simp",
                  rho0_K=1e-6, rho0_M=1e-9, rho0_G=1e-9, p=3.0, q=5.0, density=1.0, sigma=3.0, N=10, m=None,
                  solver_type="IRAM", tol=0.0, rtol=1e-10, eig_atol=1e-5, adjoint_method="shift-invert",
-                 adjoint_options=None, cost=1, deriv_type="tensor", seed=0):
+                 adjoint_options=None, cost=1, deriv_type="tensor", seed=0, pivoting="static"):
         self.fltr = fltr
+        self.pivoting = pivoting          # of the shifted factor K_r + sigma G_r (SpLuOperator); K_r alone is SPD
         self.seed = seed                  # IRAM start vector (deterministic: the eigensolve is replicated when sharded)
         self.conn, self.X = np.asarray(conn), np.asarray(X)
         self.prob = fe.BucklingQ4Problem(self.conn, self.X, bcs, forces, E=E, nu=nu, density=density, p=float(p),
@@ -460,7 +463,7 @@ class BucklingTopologyAnalysis:
         t1 = _now()
         self.profile["matrix assembly time"] = t1 - t0
         vals = D.axpby(1.0, Kr.data, float(self.sigma), Gr.data)          # K_r + sigma G_r on the shared pattern
-        self.factor = SpLuOperator(Kr.with_values(vals), symbolic=self.symbolic)
+        self.factor = SpLuOperator(Kr.with_values(vals), symbolic=self.symbolic, pivoting=self.pivoting)
         self.factor.count = 0
         self.Kr, self.Gr = Kr, Gr
         if self.solver_type == "IRAM":

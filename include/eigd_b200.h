@@ -125,6 +125,13 @@ int eigd_dmma_peak(int iters, int reps, double* tflops_out);
 int eigd_factor_numeric(eigd_factor* f, int64_t nnz, const double* d_vals, const int64_t* d_map);
 /* info[0] = #negative pivots (inertia), info[1] = #perturbed pivots, info[2] = #non-finite */
 int eigd_factor_info(eigd_factor* f, int64_t* info3);
+/* pivoting of the following eigd_factor_numeric calls: 0 = static (default; tiny pivots perturbed to +-1e-11 max|A|),
+ * 1 = restricted Bunch-Kaufman (1x1 / 1x1 interchanged / 2x2 pivots chosen inside every 32-column pivot block,
+ * 2x2 blocks rotated to diagonal form; tiny pivots still perturbed and counted).  Returns 1 for another mode. */
+int eigd_factor_set_pivoting(eigd_factor* f, int mode);
+/* out[0] = #2x2 pivots, out[1] = #row/column interchanges of the last restricted Bunch-Kaufman factorisation
+ * (0, 0 for a static one) */
+int eigd_factor_pivot_counts(eigd_factor* f, int64_t* out2);
 /* X = (L D L^T)^{-1} B in the original ordering; k columns, (rs, cs) strides; X may alias B */
 int eigd_factor_solve(eigd_factor* f, const double* d_B, int64_t brs, int64_t bcs,
                       double* d_X, int64_t xrs, int64_t xcs, int k);
