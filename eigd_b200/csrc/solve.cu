@@ -28,14 +28,10 @@
 #include "../../include/eigd_b200.h"
 
 #include <algorithm>
-#include <cstdlib>
 #include <vector>
 
 namespace {
 
-#ifndef EIGD_SUB_NW1
-#define EIGD_SUB_NW1 16
-#endif
 constexpr int MAX_PHASES_SMEM = 96;
 constexpr int MAX_SUB_LEVELS = 32;
 
@@ -69,12 +65,9 @@ struct SolveArgs {
   unsigned long long bar_base;
   unsigned* cnt;                  // completion counters: 2 * supernode + direction, monotone over the solves of a factor
   unsigned epoch;                 // number of this solve (1, 2, ...): counter c is complete at epoch * tiles(c)
-  int dbg;                        // developer ablation (EIGD_SOLVE_DBG): bit 0 no operand loads, bit 1 no panel copies, bit 2 no
-                                  // stores (subtree kernels); bit 3: the panel pipeline copies nothing, every tile of the
-                                  // level kernel reads its slice from global memory (the path of a slice larger than the ring)
   int p_begin, p_end;             // phases run by the cooperative kernel
   int ring_w;                     // bytes of shared-memory panel buffer per warp (front mode of the subtree phases)
-  int lring_w;                    // bytes of shared-memory panel ring per warp in the level kernel (0: no panel pipeline)
+  int lring_w;                    // bytes of shared-memory panel ring per warp in the level kernel (KT <= 2; 0 otherwise)
   int rec_cap;                    // tile records of a slot that fit in shared memory
   unsigned long long* times;      // developer profiling: %globaltimer of CTA 0 after every phase (NULL: off)
   unsigned long long* skew;       // developer profiling: %globaltimer of EVERY CTA's warp 0 in its first tile of every level
@@ -123,18 +116,50 @@ __device__ __forceinline__ void child_add(const SolveArgs& a, int64_t t, int64_t
 #pragma unroll
   for (int r = 0; r < KT; ++r)
     if (r < a.k) v[r] += __ldcg(p0 + (int64_t)r * a.sumf) + __ldcg(p1 + (int64_t)r * a.sumf);
-  if (link & LINK_HAS_OVF) {
-    const int o = __ldg(&a.ovf_row[t]);
-    if (o >= 0) {
-      const int cnt = __ldg(&a.ovf[o]);
-      const double* p2 = a.wbuf + 2 * a.slab_stride;
-      for (int q = 0; q < cnt; ++q) {
-        const int64_t src = __ldg(&a.ovf[o + 1 + q]);
+  if (link & LINK_HAS_OVF) ovf_add<KT>(a, t, v);
+}
+
+// v += w1 entry c of a front in the forward sweep: the right-hand side (gathered from B through perm in the first phase,
+// else the permuted copy) + the children's updates; v is zero on entry
+template <int KT>
+__device__ __forceinline__ void fwd_operand(const SolveArgs& a, bool use_perm, const TileRec& tr, int c, double* v) {
+  if (use_perm) {
+    const int64_t po = __ldg(&a.perm[tr.first + c]);
+    const double* bp = a.B + po * a.brs;
 #pragma unroll
-        for (int r = 0; r < KT; ++r)
-          if (r < a.k) v[r] += __ldcg(p2 + (int64_t)r * a.sumf + src);
-      }
-    }
+    for (int r = 0; r < KT; ++r)
+      if (r < a.k) v[r] = bp[(int64_t)r * a.bcs];
+  } else {
+    add_row<KT>(a.bperm, tr.first + c, a.k, v);
+  }
+  child_add<KT>(a, tr.w_off + c, tr.link, v);
+}
+
+// v += input entry i of a front in the backward sweep: z1 for a pivot row, the solution x2 (through sn_rows) below them
+template <int KT>
+__device__ __forceinline__ void bwd_operand(const SolveArgs& a, const TileRec& tr, int i, double* v) {
+  if (i < tr.nc) add_row<KT>(a.ybuf, tr.first + i, a.k, v);
+  else add_row<KT>(a.xperm, __ldg(&a.sn_rows[tr.row_off + i - tr.nc]), a.k, v);
+}
+
+// thin tile (TH < 32): the 32 / TH lane groups that shared the columns of every chunk add up their sums
+template <int KT, int TH>
+__device__ __forceinline__ void group_reduce(double* acc) {
+  if (TH < 32) {
+#pragma unroll
+    for (int o = TH; o < 32; o <<= 1)
+#pragma unroll
+      for (int r = 0; r < KT; ++r) acc[r] += __shfl_xor_sync(0xffffffffu, acc[r], o);
+  }
+}
+
+// permuted copy of the right-hand side for the later phases (coalesced writes, gathered reads); thread t of nt
+__device__ __forceinline__ void permute_rhs(const SolveArgs& a, int64_t t, int64_t nt) {
+  const int k = a.k;
+  for (int64_t e = t; e < (int64_t)a.n * k; e += nt) {
+    const int64_t i = e / k;
+    const int r = (int)(e - i * k);
+    a.bperm[e] = a.B[(int64_t)__ldg(&a.perm[i]) * a.brs + (int64_t)r * a.bcs];
   }
 }
 
@@ -172,6 +197,11 @@ struct DepWait {
   unsigned epoch;
   TileDep td;
   bool pending;
+  __device__ __forceinline__ void arm(int4 d0, int4 d1) {     // the tile's TileDep, read as two 16-byte words
+    td.self = d0.x; td.ndep = d0.y; td.d0 = d0.z; td.n0 = d0.w;
+    td.d1 = d1.x; td.n1 = d1.y; td.ovf = d1.z; td.pad = 0;
+    pending = td.ndep > 0;
+  }
   __device__ __forceinline__ static void spin(const unsigned* c, unsigned need) {
     unsigned v;
     do {
@@ -241,8 +271,8 @@ __device__ __forceinline__ void warp_panel_product(const double* __restrict__ M,
   }
 }
 
-// Grid-wide barrier, only for the rare in-kernel phases that are not synchronised by completion counters (a subtree
-// phase executed inside the cooperative kernel, the in-kernel copy of the permuted right-hand side).
+// Grid-wide barrier, only behind phase 0 of a plan without subtree phases: the later phases read the permuted copy of
+// the right-hand side that all CTAs write during phase 0, which no completion counter covers.
 // (the caller puts a CTA barrier -- of all its participating warps -- on both sides)
 __device__ __forceinline__ void grid_barrier_arrive_wait(unsigned long long* ctr, unsigned long long target) {
   if (threadIdx.x == 0) {
@@ -253,20 +283,17 @@ __device__ __forceinline__ void grid_barrier_arrive_wait(unsigned long long* ctr
     } while (v < target);
   }
 }
-__host__ __device__ inline bool barrier_between(const PhaseRec& a, const PhaseRec& b, int p) {
-  return a.ws == 0 || b.ws == 0 || p == 0;
-}
 
 // the products of one warp tile: slice `slice` of `ws` of the reduction dimension.
 // use_perm: the right-hand side is gathered from B through perm (first phase; later phases read the
 // permuted copy written during the first one)
-// TILED: the front's panels are stored tile-major with tile height TH (fronts above the cut, solve_plan.hpp)
+// TILED: the front's panels are stored tile-major with tile height TH (fronts above the cut, solve_plan.hpp); column-major
+// below the cut (the tile path of fronts_phase)
 template <int KT, int MC = DefaultMC<KT>::value, int TH = SOLVE_TILE, bool TILED = false, class WaitFn>
 __device__ __forceinline__ void tile_compute(const SolveArgs& a, int dir, bool use_perm, const TileRec& tr, int lane,
                                              int slice, int ws, double* stage, double* acc, WaitFn& wait) {
   constexpr int to = TH;
   constexpr int MCT = MC < TH ? MC : TH;               // loads in flight per lane and chunk: a chunk has TH columns per lane group
-  const int k = a.k;
   const int nc = tr.nc, f = tr.nc + tr.nb;
   const int o0 = tr.tile * to;
   const int out = o0 + (lane % to);
@@ -279,25 +306,10 @@ __device__ __forceinline__ void tile_compute(const SolveArgs& a, int dir, bool u
     const int c0 = min(cend, slice * per), c1 = min(cend, c0 + per);
     const int th = min(to, f - o0);                     // rows of this row tile
     const double* M = TILED ? a.sfwd + tr.soff + (int64_t)o0 * nc + min(lane % to, th - 1) : a.sfwd + tr.soff + min(out, f - 1);
-    warp_panel_product<KT, MCT, TH>(M, TILED ? th : f, c0, c1, lane, stage, acc, [&](int c, double* v) {
-      if (use_perm) {
-        const int64_t po = __ldg(&a.perm[tr.first + c]);
-        const double* bp = a.B + po * a.brs;
-#pragma unroll
-        for (int r = 0; r < KT; ++r)
-          if (r < k) v[r] = bp[(int64_t)r * a.bcs];
-      } else {
-        add_row<KT>(a.bperm, tr.first + c, k, v);
-      }
-      child_add<KT>(a, tr.w_off + c, tr.link, v);
-    }, wait);
+    warp_panel_product<KT, MCT, TH>(M, TILED ? th : f, c0, c1, lane, stage, acc,
+                                    [&](int c, double* v) { fwd_operand<KT>(a, use_perm, tr, c, v); }, wait);
     wait(lane);
-    if (TH < 32) {
-#pragma unroll
-      for (int o = TH; o < 32; o <<= 1)
-#pragma unroll
-        for (int r = 0; r < KT; ++r) acc[r] += __shfl_xor_sync(0xffffffffu, acc[r], o);
-    }
+    group_reduce<KT, TH>(acc);
     if (slice == 0 && lane < to && out >= nc && out < f) {
       double cu[KT];                                    // the children's updates of this output row
 #pragma unroll
@@ -315,55 +327,18 @@ __device__ __forceinline__ void tile_compute(const SolveArgs& a, int dir, bool u
     const int i0 = min(f, ob + slice * per), i1 = min(f, i0 + per);
     const int tw = min(to, nc - o0);                    // pivot columns of this column tile
     const double* M = TILED ? a.sbwd + tr.soff + (int64_t)o0 * f + min(lane % to, tw - 1) : a.sbwd + tr.soff + min(out, nc - 1);
-    warp_panel_product<KT, MCT, TH>(M, TILED ? tw : nc, i0, i1, lane, stage, acc, [&](int i, double* v) {
-      if (i < nc) add_row<KT>(a.ybuf, tr.first + i, k, v);
-      else add_row<KT>(a.xperm, __ldg(&a.sn_rows[tr.row_off + i - nc]), k, v);
-    }, wait);
+    warp_panel_product<KT, MCT, TH>(M, TILED ? tw : nc, i0, i1, lane, stage, acc,
+                                    [&](int i, double* v) { bwd_operand<KT>(a, tr, i, v); }, wait);
     wait(lane);
-    if (TH < 32) {
-#pragma unroll
-      for (int o = TH; o < 32; o <<= 1)
-#pragma unroll
-        for (int r = 0; r < KT; ++r) acc[r] += __shfl_xor_sync(0xffffffffu, acc[r], o);
-    }
+    group_reduce<KT, TH>(acc);
   }
 }
 
-template <int KT, int TH = SOLVE_TILE>
-__device__ __forceinline__ void tile_store(const SolveArgs& a, int dir, const TileRec& tr, int lane, const double* acc) {
-  const int k = a.k;
-  const int nc = tr.nc, f = tr.nc + tr.nb;
-  const int out = tr.tile * TH + lane;
-  if (TH < 32 && lane >= TH) return;
-  if (dir == 0) {
-    if (out < nc) {
-      const double di = __ldg(&a.dinv[tr.first + out]);
-      double* y = a.ybuf + (int64_t)(tr.first + out) * k;
-#pragma unroll
-      for (int r = 0; r < KT; ++r)
-        if (r < k) y[r] = di * acc[r];
-    } else if (out < f) {
-      const int slab = (int)((tr.link >> LINK_SLAB_SHIFT) & 0xff);
-      int64_t dst;                                            // row in the plane of the destination slab
-      if (slab < 2) dst = slab * a.slab_stride + (tr.link & LINK_WOFF_MASK) + __ldg(&a.rel[tr.row_off + out - nc]);
-      else dst = 2 * a.slab_stride + tr.w_off + out;
-      double* w = a.wbuf + dst;
-#pragma unroll
-      for (int r = 0; r < KT; ++r)
-        if (r < k) w[(int64_t)r * a.sumf] = acc[r];
-    }
-  } else if (out < nc) {
-    double* xp = a.xperm + (int64_t)(tr.first + out) * k;
-    double* xo = a.X + (int64_t)__ldg(&a.perm[tr.first + out]) * a.xrs;
-#pragma unroll
-    for (int r = 0; r < KT; ++r)
-      if (r < k) { xp[r] = acc[r]; xo[(int64_t)r * a.xcs] = acc[r]; }
-  }
-}
-
-// The index / scaling operands of tile_store, requested BEFORE the tile waits for its dependencies (level phases): the
-// D^-1 entry, the parent row position or the original index of the output then sit in registers when the sums are
-// ready, instead of adding a dependent look-up (an L2 or DRAM round trip) between the last FMA and the stores.
+// The stores of a tile's outputs: z1 = D^-1 y1 (forward, pivot rows), the update rows into the parent's slab (forward,
+// below the pivots), the solution into xperm and X (backward).  tile_store_request loads the index / scaling operands
+// (the D^-1 entry, the parent row position or the original index of the output); the pipelined level kernel requests
+// them BEFORE the tile waits for its dependencies, so that they sit in registers when the sums are ready instead of
+// adding a dependent look-up (an L2 or DRAM round trip) between the last FMA and the stores.
 struct StoreOps {
   double di;
   int64_t dst;
@@ -414,6 +389,11 @@ __device__ __forceinline__ void tile_store_with(const SolveArgs& a, int dir, con
     for (int r = 0; r < KT; ++r)
       if (r < k) { xp[r] = acc[r]; xo[(int64_t)r * a.xcs] = acc[r]; }
   }
+}
+
+template <int KT, int TH = SOLVE_TILE>
+__device__ __forceinline__ void tile_store(const SolveArgs& a, int dir, const TileRec& tr, int lane, const double* acc) {
+  tile_store_with<KT, TH>(a, dir, tr, lane, acc, tile_store_request<TH>(a, dir, tr, lane));
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -475,19 +455,6 @@ __device__ __forceinline__ void front_request(const SolveArgs& a, int dir, bool 
   const int k = a.k;
   const int nc = tr.nc, f = tr.nc + tr.nb;
   const bool kids = (tr.link & LINK_HAS_CHILDREN) != 0;
-  if (a.dbg & 1) {
-#pragma unroll
-    for (int r = 0; r < KT; ++r) o.b[r] = o.s0[r] = o.s1[r] = 1.0;
-#pragma unroll
-    for (int t = 0; t < FRONT_RT; ++t) {
-      o.auxd[t] = 1.0;
-      o.auxi[t] = 0;
-#pragma unroll
-      for (int r = 0; r < KT; ++r) o.u0[t][r] = o.u1[t][r] = 0.0;
-    }
-    o.perm0 = 0;
-    return;
-  }
   if (dir == 0) {
     const int64_t col = tr.first + min(lane, nc - 1);
     const double* bp = use_perm ? a.B + (int64_t)__ldg(&a.perm[col]) * a.brs : a.bperm + col * k;
@@ -547,22 +514,12 @@ __device__ __forceinline__ void front_compute(const SolveArgs& a, int dir, bool 
       } else {
 #pragma unroll
         for (int r = 0; r < KT; ++r) v[r] = 0.0;
-        if (lane < nc) {
-          if (use_perm) {
-            const double* bp = a.B + (int64_t)__ldg(&a.perm[tr.first + lane]) * a.brs;
-#pragma unroll
-            for (int r = 0; r < KT; ++r)
-              if (r < k) v[r] = bp[(int64_t)r * a.bcs];
-          } else {
-            add_row<KT>(a.bperm, tr.first + lane, k, v);
-          }
-          child_add<KT>(a, tr.w_off + lane, tr.link, v);
-        }
+        if (lane < nc) fwd_operand<KT>(a, use_perm, tr, lane, v);
       }
 #pragma unroll
       for (int r = 0; r < KT; ++r) stage[r * 32 + lane] = v[r];
       __syncwarp();
-      if (!(a.dbg & 2)) mbar_wait(bar, parity);
+      mbar_wait(bar, parity);
 #pragma unroll
       for (int t = 0; t < (PIPE ? FRONT_RT : FRONT_TILES_MAX); ++t) {
         if (t >= ntile) break;
@@ -586,8 +543,7 @@ __device__ __forceinline__ void front_compute(const SolveArgs& a, int dir, bool 
           for (int r = 0; r < KT; ++r) acc[r] += ops.u0[t][r] + ops.u1[t][r];
           if ((tr.link & LINK_HAS_OVF) && row >= nc && row < f) ovf_add<KT>(a, tr.w_off + row, acc);
           // store with the prefetched D^-1 / parent position (tile_store without its look-up)
-          if (a.dbg & 4) {
-          } else if (row < nc) {
+          if (row < nc) {
             double* y = a.ybuf + (int64_t)(tr.first + row) * k;
 #pragma unroll
             for (int r = 0; r < KT; ++r)
@@ -619,7 +575,7 @@ __device__ __forceinline__ void front_compute(const SolveArgs& a, int dir, bool 
           for (int r = 0; r < KT; ++r) vv[t][r] = (i < f && r < k) ? __ldcg(src + r) : 0.0;
         }
       }
-      if (!(a.dbg & 2)) mbar_wait(bar, parity);
+      mbar_wait(bar, parity);
       double acc[KT];
 #pragma unroll
       for (int r = 0; r < KT; ++r) acc[r] = 0.0;
@@ -636,11 +592,7 @@ __device__ __forceinline__ void front_compute(const SolveArgs& a, int dir, bool 
           double v[KT];
 #pragma unroll
           for (int r = 0; r < KT; ++r) v[r] = 0.0;
-          if (lane < nrow) {
-            const int i = cc + lane;
-            if (i < nc) add_row<KT>(a.ybuf, tr.first + i, k, v);
-            else add_row<KT>(a.xperm, __ldg(&a.sn_rows[tr.row_off + i - nc]), k, v);
-          }
+          if (lane < nrow) bwd_operand<KT>(a, tr, cc + lane, v);
 #pragma unroll
           for (int r = 0; r < KT; ++r) stage[r * 32 + lane] = v[r];
         }
@@ -655,7 +607,7 @@ __device__ __forceinline__ void front_compute(const SolveArgs& a, int dir, bool 
         __syncwarp();
       }
       if constexpr (PIPE) {
-        if (lane < nc && !(a.dbg & 4)) {
+        if (lane < nc) {
           double* xp = a.xperm + (int64_t)(tr.first + lane) * k;
           double* xo = a.X + (int64_t)ops.perm0 * a.xrs;
 #pragma unroll
@@ -674,9 +626,9 @@ constexpr int FRONT_DEPTH = 2;   // panel copies in flight per warp
 // Every front of this CTA's slot that belongs to this warp (front te = T0(level) + warp + 16 j), level by level
 // with a CTA barrier between levels.  The PANEL copies run ahead of the computation by up to FRONT_DEPTH fronts
 // and across level boundaries (panels do not depend on computed data): a FIFO of variable-size allocations in the
-// warp's ring buffer, one mbarrier per FIFO position.  The OPERANDS (right-hand side, child updates, D^-1, row
-// positions) are requested one front ahead into registers (KT <= 2).
-template <int KT, int NW, bool PIPE>
+// warp's ring buffer, one mbarrier per FIFO position.  PIPE: the OPERANDS (right-hand side, child updates, D^-1, row
+// positions) are requested one front ahead into registers.
+template <int KT, bool PIPE>
 __device__ __forceinline__ void fronts_phase(const SolveArgs& a, int dir, bool use_perm, int nl, const int* s_tab, int tb,
                                              int nrec, const int4* s_rec, int lane, int warp, double* stage, char* ring,
                                              int ring_w, unsigned long long* bars, int* s_q) {
@@ -719,14 +671,14 @@ __device__ __forceinline__ void fronts_phase(const SolveArgs& a, int dir, bool u
           if (o >= 0 && off < o + l && o < off + (int)b) clash = true;
         }
         if (clash) return;         // no room yet: try again after the next front has been consumed
-        if (lane == 0 && !(a.dbg & 2)) bulk_load(ring + off, panels + t.soff, b, &bars[e]);
+        if (lane == 0) bulk_load(ring + off, panels + t.soff, b, &bars[e]);
         last_end = off + (int)b;
       }
       __syncwarp();
       if (lane == 0) { s_q[2 * e] = off; s_q[2 * e + 1] = (int)b; }
       __syncwarp();
       ++qn;
-      pte += NW;
+      pte += SOLVE_WARPS;
       p_skip();
     }
   };
@@ -736,7 +688,7 @@ __device__ __forceinline__ void fronts_phase(const SolveArgs& a, int dir, bool u
   for (int ll = 0; ll < nl; ++ll) {
     const int l = level_of(ll);
     const int t0 = s_tab[l], t1 = s_tab[l + 1];
-    for (int te = t0 + warp; te < t1; te += NW) {
+    for (int te = t0 + warp; te < t1; te += SOLVE_WARPS) {
       TileRec tr = record(te);
       const int off = s_q[2 * qh];
       const unsigned parity = (par >> qh) & 1u;
@@ -746,8 +698,8 @@ __device__ __forceinline__ void fronts_phase(const SolveArgs& a, int dir, bool u
       bool nops_ready = false;
       if constexpr (PIPE) {
         // operands of this warp's next front of the SAME level (the next level's depend on this level's results)
-        if (te + NW < t1) {
-          const TileRec nt = record(te + NW);
+        if (te + SOLVE_WARPS < t1) {
+          const TileRec nt = record(te + SOLVE_WARPS);
           if (fits(nt, (unsigned)solve_panel_doubles(nt.nc + nt.nb, nt.nc) * 8u)) {
             front_request<KT>(a, dir, use_perm, nt, lane, nops);
             nops_ready = true;
@@ -788,17 +740,18 @@ __device__ __forceinline__ void fronts_phase(const SolveArgs& a, int dir, bool u
 
 // A subtree phase in FRONT MODE as its own (ordinary, non-cooperative) launch: one CTA per slot.  The forward one
 // is the first thing a solve does, the backward one the last, so stream order replaces the grid barrier; the kernel
-// gets its own register / shared-memory budget (panel ring) and the level kernel keeps its L1.
-template <int KT, int NW, bool PIPE>
-__global__ void __launch_bounds__(NW * 32, 1) subtree_kernel(SolveArgs a, int p) {
+// gets its own register / shared-memory budget (panel ring) and the level kernel keeps its L1.  The operands of the next
+// front are prefetched into registers for k = 1 only: wider ones do not fit the 128-register budget of a 16-warp CTA.
+template <int KT>
+__global__ void __launch_bounds__(SOLVE_WARPS * 32, 1) subtree_kernel(SolveArgs a, int p) {
   extern __shared__ double smem[];
   __shared__ int s_tab[MAX_SUB_LEVELS];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   double* stage = smem + warp * (32 * KT);                 // [KT][32] per warp
-  char* ring_all = reinterpret_cast<char*>(smem + NW * 32 * KT);
-  unsigned long long* mbar_all = reinterpret_cast<unsigned long long*>(ring_all + (size_t)NW * a.ring_w);
-  int* s_q = reinterpret_cast<int*>(mbar_all + FRONT_DEPTH * NW) + 2 * FRONT_DEPTH * warp;
-  int4* s_rec = reinterpret_cast<int4*>(mbar_all + 2 * FRONT_DEPTH * NW);
+  char* ring_all = reinterpret_cast<char*>(smem + SOLVE_WARPS * 32 * KT);
+  unsigned long long* mbar_all = reinterpret_cast<unsigned long long*>(ring_all + (size_t)SOLVE_WARPS * a.ring_w);
+  int* s_q = reinterpret_cast<int*>(mbar_all + FRONT_DEPTH * SOLVE_WARPS) + 2 * FRONT_DEPTH * warp;
+  int4* s_rec = reinterpret_cast<int4*>(mbar_all + 2 * FRONT_DEPTH * SOLVE_WARPS);
   unsigned long long* bars = mbar_all + FRONT_DEPTH * warp;
   if (lane < FRONT_DEPTH) mbar_init(&bars[lane], 1);
   asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -821,18 +774,10 @@ __global__ void __launch_bounds__(NW * 32, 1) subtree_kernel(SolveArgs a, int p)
       for (int e = threadIdx.x; e < 3 * nrec; e += blockDim.x) s_rec[e] = __ldg(src + e);
     }
     __syncthreads();
-    fronts_phase<KT, NW, PIPE>(a, dir, use_perm, nl, s_tab, tb, nrec, s_rec, lane, warp, stage, ring_all + (size_t)warp * a.ring_w,
-                     a.ring_w, bars, s_q);
+    fronts_phase<KT, KT == 1>(a, dir, use_perm, nl, s_tab, tb, nrec, s_rec, lane, warp, stage,
+                              ring_all + (size_t)warp * a.ring_w, a.ring_w, bars, s_q);
   }
-  if (use_perm) {
-    // permuted copy of the right-hand side for the level phases (coalesced writes, gathered reads)
-    const int k = a.k;
-    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < (int64_t)a.n * k; e += (int64_t)gridDim.x * blockDim.x) {
-      const int64_t i = e / k;
-      const int r = (int)(e - i * k);
-      a.bperm[e] = a.B[(int64_t)__ldg(&a.perm[i]) * a.brs + (int64_t)r * a.bcs];
-    }
-  }
+  if (use_perm) permute_rhs(a, (int64_t)blockIdx.x * blockDim.x + threadIdx.x, (int64_t)gridDim.x * blockDim.x);
   if (a.times && blockIdx.x == 0 && threadIdx.x == 0) {
     unsigned long long t;
     asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
@@ -840,10 +785,40 @@ __global__ void __launch_bounds__(NW * 32, 1) subtree_kernel(SolveArgs a, int p)
   }
 }
 
-// One level phase: the tiles (height TH) of one level of the tree in one direction, CTA-strided; ws warps share a tile
-// and split its reduction dimension.  A tile waits for the completion counters of the fronts it reads from and
+// The partial sums of the ws warps that share a tile meet in shared memory (cta_sync: the CTA barrier of the warps that
+// share tiles); the slice-0 warp (lead) adds them in a FIXED order (bitwise reproducible), for KT <= 2 in four
+// independent chains at a time so that the shared-memory latencies overlap
+template <int KT, class SyncFn>
+__device__ __forceinline__ void reduce_slices(double* acc, double* part, int warp, int lane, int ws, bool lead,
+                                              SyncFn cta_sync) {
+#pragma unroll
+  for (int r = 0; r < KT; ++r) part[(warp * KT + r) * 32 + lane] = acc[r];
+  cta_sync();
+  if (lead && KT > 2) {
+    for (int s = 1; s < ws; ++s)
+#pragma unroll
+      for (int r = 0; r < KT; ++r) acc[r] += part[((warp + s) * KT + r) * 32 + lane];
+  }
+  if (lead && KT <= 2) {
+#pragma unroll
+    for (int r = 0; r < KT; ++r) {
+      double p0 = 0.0, p1 = 0.0, p2 = 0.0, p3 = 0.0;
+      for (int s = 1; s < ws; s += 4) {
+        p0 += part[((warp + s) * KT + r) * 32 + lane];
+        if (s + 1 < ws) p1 += part[((warp + s + 1) * KT + r) * 32 + lane];
+        if (s + 2 < ws) p2 += part[((warp + s + 2) * KT + r) * 32 + lane];
+        if (s + 3 < ws) p3 += part[((warp + s + 3) * KT + r) * 32 + lane];
+      }
+      acc[r] += (p0 + p1) + (p2 + p3);
+    }
+  }
+}
+
+// One level phase of the 16-warp level kernel (KT > 2): the tiles (height TH) of one level of the tree in one direction,
+// CTA-strided; ws warps share a tile and split its reduction dimension.  Every tile reads its slice of the tile-major
+// panel straight from global memory.  A tile waits for the completion counters of the fronts it reads from and
 // increments its own front's counter when its outputs are stored (no grid barrier).
-template <int KT, int TH, bool TILED>
+template <int KT, int TH>
 __device__ __forceinline__ void level_phase(const SolveArgs& a, const PhaseRec& ph, int p, bool use_perm, int lane, int warp,
                                             double* stage, double* part, bool have_next, int4 (*s_next)[5]) {
   const int64_t tile_off = ph.tile_off;
@@ -857,18 +832,8 @@ __device__ __forceinline__ void level_phase(const SolveArgs& a, const PhaseRec& 
     double acc[KT];
 #pragma unroll
     for (int r = 0; r < KT; ++r) acc[r] = 0.0;
-    TileRec tr;
-    tr.first = tr.nc = tr.nb = tr.tile = 0;
-    tr.soff = tr.w_off = tr.row_off = tr.link = 0;
-    DepWait dw;
-    dw.cnt = a.cnt;
-    dw.ovf = a.dep_ovf;
-    dw.epoch = a.epoch;
-    dw.pending = false;
-    dw.td.self = 0;
-    StoreOps sto;
-    sto.di = 0.0;
-    sto.dst = 0;
+    TileRec tr{};
+    DepWait dw{a.cnt, a.dep_ovf, a.epoch, TileDep{}, false};
     if (have) {
       int4 d0, d1;
       if (have_next && ct == (int)blockIdx.x) {
@@ -881,49 +846,21 @@ __device__ __forceinline__ void level_phase(const SolveArgs& a, const PhaseRec& 
         d0 = __ldg(q);
         d1 = __ldg(q + 1);
       }
-      dw.td.self = d0.x; dw.td.ndep = d0.y; dw.td.d0 = d0.z; dw.td.n0 = d0.w;
-      dw.td.d1 = d1.x; dw.td.n1 = d1.y; dw.td.ovf = d1.z; dw.td.pad = 0;
-      dw.pending = dw.td.ndep > 0;
-      if (KT <= 2 && slice == 0) sto = tile_store_request<TH>(a, dir, tr, lane);      // (costs registers: single / pair solves only)
+      dw.arm(d0, d1);
       const bool tr_on = a.trace && blockIdx.x == 0 && ct == 0 && threadIdx.x == 0;
       if (tr_on) a.trace[16 * p + 0] = clock64();
       if (a.trace) {              // trace build of the chain: wait first so that the segments separate
         dw(lane);
         if (tr_on) a.trace[16 * p + 1] = clock64();
       }
-      tile_compute<KT, DefaultMC<KT>::value, TH, TILED>(a, dir, use_perm, tr, lane, slice, ws, stage, acc, dw);
+      tile_compute<KT, DefaultMC<KT>::value, TH, true>(a, dir, use_perm, tr, lane, slice, ws, stage, acc, dw);
       if (tr_on) a.trace[16 * p + 2] = clock64();
     }
-    if (ws > 1) {
-      // partial sums of the ws slices meet in shared memory; the slice-0 warp adds them in a FIXED order (bitwise
-      // reproducible), four independent chains at a time so that the shared-memory latencies overlap
-#pragma unroll
-      for (int r = 0; r < KT; ++r) part[(warp * KT + r) * 32 + lane] = acc[r];
-      __syncthreads();
-      if (have && slice == 0 && KT > 2) {
-        for (int s = 1; s < ws; ++s)
-#pragma unroll
-          for (int r = 0; r < KT; ++r) acc[r] += part[((warp + s) * KT + r) * 32 + lane];
-      }
-      if (have && slice == 0 && KT <= 2) {
-#pragma unroll
-        for (int r = 0; r < KT; ++r) {
-          double p0 = 0.0, p1 = 0.0, p2 = 0.0, p3 = 0.0;
-          for (int s = 1; s < ws; s += 4) {
-            p0 += part[((warp + s) * KT + r) * 32 + lane];
-            if (s + 1 < ws) p1 += part[((warp + s + 1) * KT + r) * 32 + lane];
-            if (s + 2 < ws) p2 += part[((warp + s + 2) * KT + r) * 32 + lane];
-            if (s + 3 < ws) p3 += part[((warp + s + 3) * KT + r) * 32 + lane];
-          }
-          acc[r] += (p0 + p1) + (p2 + p3);
-        }
-      }
-    }
+    if (ws > 1) reduce_slices<KT>(acc, part, warp, lane, ws, have && slice == 0, [] { __syncthreads(); });
     const bool tr_on2 = a.trace && blockIdx.x == 0 && ct == 0 && threadIdx.x == 0;
     if (tr_on2) a.trace[16 * p + 3] = clock64();
     if (have && slice == 0) {
-      if (KT <= 2) tile_store_with<KT, TH>(a, dir, tr, lane, acc, sto);
-      else tile_store<KT, TH>(a, dir, tr, lane, acc);
+      tile_store<KT, TH>(a, dir, tr, lane, acc);
       if (tr_on2) a.trace[16 * p + 4] = clock64();
       signal_done(a.cnt + dw.td.self);
       if (tr_on2) a.trace[16 * p + 5] = clock64();
@@ -931,7 +868,6 @@ __device__ __forceinline__ void level_phase(const SolveArgs& a, const PhaseRec& 
     if (ws > 1) __syncthreads();
   }
 }
-
 
 // ---------------------------------------------------------------------------------------------------------
 // ASYNCHRONOUS PANEL PIPELINE of the level phases: a warp-specialised producer / consumer kernel.
@@ -1014,9 +950,8 @@ __device__ __forceinline__ SliceDesc slice_of(const TileRec& tr, int dir, int th
   return s;
 }
 
-// tile of consumer warp w in (phase ph, CTA-tile index ct), or -1
+// tile of consumer warp w in (level phase ph, CTA-tile index ct), or -1
 __device__ __forceinline__ int pipe_tile_of(const PhaseRec& ph, int ct, int w) {
-  if (ph.ws <= 0) return -1;
   const int tpc = SOLVE_WARPS / ph.ws;
   const int te = ct * tpc + w / ph.ws;
   return te < ph.ntiles ? te : -1;
@@ -1071,14 +1006,14 @@ __device__ __forceinline__ void pipe_producer(const SolveArgs& a, char* pipe_bas
         r0 = __ldg(tp); r1 = __ldg(tp + 1); r2 = __ldg(tp + 2);
         r3 = __ldg(dp); r4 = __ldg(dp + 1);
         dir = ph.dir;
-        sd = slice_of(unpack_tile(r0, r1, r2), dir, (int)(ph.pad & 0xff), w % ph.ws, ph.ws, a.blk_mask);
+        sd = slice_of(unpack_tile(r0, r1, r2), dir, (int)ph.pad, w % ph.ws, ph.ws, a.blk_mask);
         bytes = (sd.len * sd.ld * 8 + 15) & ~15;
         loaded = true;
       }
       int off;
       bool clash = false;
       if (bytes == 0) off = -2;                                 // empty slice: nothing to copy
-      else if (bytes > a.lring_w || (a.dbg & 8)) off = -1;      // larger than the ring: the tile reads it from global memory
+      else if (bytes > a.lring_w) off = -1;      // larger than the ring: the tile reads it from global memory
       else {
         off = (last_end + 127) & ~127;
         if (off + bytes > a.lring_w) off = 0;
@@ -1116,7 +1051,6 @@ __device__ __forceinline__ void tile_compute_smem(const SolveArgs& a, int dir, b
                                                   int slice, int sr0, int slen, int sld, const double* sbuf, double* stage,
                                                   double* acc, WaitFn& wait) {
   constexpr int nks = 32 / TH;
-  const int k = a.k;
   const int nc = tr.nc, f = tr.nc + tr.nb;
   const int o0 = tr.tile * TH;
   const int g = lane / TH;
@@ -1131,21 +1065,8 @@ __device__ __forceinline__ void tile_compute_smem(const SolveArgs& a, int dir, b
     wait(lane);
     if (lane < ncol) {
       const int c = sr0 + cc + lane;
-      if (dir == 0) {
-        if (use_perm) {
-          const int64_t po = __ldg(&a.perm[tr.first + c]);
-          const double* bp = a.B + po * a.brs;
-#pragma unroll
-          for (int r = 0; r < KT; ++r)
-            if (r < k) v[r] = bp[(int64_t)r * a.bcs];
-        } else {
-          add_row<KT>(a.bperm, tr.first + c, k, v);
-        }
-        child_add<KT>(a, tr.w_off + c, tr.link, v);
-      } else {
-        if (c < nc) add_row<KT>(a.ybuf, tr.first + c, k, v);
-        else add_row<KT>(a.xperm, __ldg(&a.sn_rows[tr.row_off + c - nc]), k, v);
-      }
+      if (dir == 0) fwd_operand<KT>(a, use_perm, tr, c, v);
+      else bwd_operand<KT>(a, tr, c, v);
     }
     // forward: the children's updates of this output row go straight into the sum (requested together with the operands;
     // slice 0 always has a first chunk: its range starts at column 0)
@@ -1165,12 +1086,7 @@ __device__ __forceinline__ void tile_compute_smem(const SolveArgs& a, int dir, b
     __syncwarp();
   }
   wait(lane);
-  if (TH < 32) {
-#pragma unroll
-    for (int o = TH; o < 32; o <<= 1)
-#pragma unroll
-      for (int r = 0; r < KT; ++r) acc[r] += __shfl_xor_sync(0xffffffffu, acc[r], o);
-  }
+  group_reduce<KT, TH>(acc);
 }
 
 struct ConsumerState {
@@ -1178,8 +1094,8 @@ struct ConsumerState {
   unsigned par;      // parity of that slot's barriers
 };
 
-// One level phase on the consumer side of the panel pipeline: as level_phase, but the tile's record, dependencies and
-// slice descriptor come from the warp's current slot and the panel slice from its shared-memory ring.
+// One level phase on the consumer side of the panel pipeline (KT <= 2): as level_phase, but the tile's record,
+// dependencies and slice descriptor come from the warp's current slot and the panel slice from its shared-memory ring.
 template <int KT, int TH>
 __device__ __forceinline__ void level_phase_pipe(const SolveArgs& a, const PhaseRec& ph, int p, bool use_perm, int lane, int warp,
                                                  double* stage, double* part, ConsumerState& cs, const PipeSmem& sm) {
@@ -1195,18 +1111,9 @@ __device__ __forceinline__ void level_phase_pipe(const SolveArgs& a, const Phase
     double acc[KT];
 #pragma unroll
     for (int r = 0; r < KT; ++r) acc[r] = 0.0;
-    TileRec tr;
-    tr.first = tr.nc = tr.nb = tr.tile = 0;
-    tr.soff = tr.w_off = tr.row_off = tr.link = 0;
-    DepWait dw;
-    dw.cnt = a.cnt;
-    dw.ovf = a.dep_ovf;
-    dw.epoch = a.epoch;
-    dw.pending = false;
-    dw.td.self = 0;
-    StoreOps sto;
-    sto.di = 0.0;
-    sto.dst = 0;
+    TileRec tr{};
+    DepWait dw{a.cnt, a.dep_ovf, a.epoch, TileDep{}, false};
+    StoreOps sto{};
     const bool tr_on = a.trace && blockIdx.x == 0 && ct == (int)blockIdx.x && threadIdx.x == 0;
     const bool sk_on = a.skew && threadIdx.x == 0 && ct == (int)blockIdx.x && have;
     unsigned long long* sk = a.skew + ((size_t)p * gridDim.x + blockIdx.x) * 4;
@@ -1217,11 +1124,9 @@ __device__ __forceinline__ void level_phase_pipe(const SolveArgs& a, const Phase
       mbar_wait(&sm.full[cs.slot], cs.par);                 // record written, panel slice landed
       const int4* r = sm.rec + cs.slot * PIPE_REC_INT4;
       tr = unpack_tile(r[0], r[1], r[2]);
-      const int4 d0 = r[3], d1 = r[4], sl = r[5];
-      dw.td.self = d0.x; dw.td.ndep = d0.y; dw.td.d0 = d0.z; dw.td.n0 = d0.w;
-      dw.td.d1 = d1.x; dw.td.n1 = d1.y; dw.td.ovf = d1.z; dw.td.pad = 0;
-      dw.pending = dw.td.ndep > 0;
-      if (KT <= 2 && slice == 0) sto = tile_store_request<TH>(a, dir, tr, lane);
+      const int4 sl = r[5];
+      dw.arm(r[3], r[4]);
+      if (slice == 0) sto = tile_store_request<TH>(a, dir, tr, lane);
       if (a.trace || a.skew) {      // trace builds of the chain: wait first so that the segments separate
         if (tr_on) a.trace[16 * p + 6] = clock64();
         if (sk_on) sk[1] = gtime();
@@ -1239,33 +1144,10 @@ __device__ __forceinline__ void level_phase_pipe(const SolveArgs& a, const Phase
       if (++cs.slot == PIPE_DEPTH) { cs.slot = 0; cs.par ^= 1u; }
       if (tr_on) a.trace[16 * p + 2] = clock64();
     }
-    if (ws > 1) {
-#pragma unroll
-      for (int r = 0; r < KT; ++r) part[(warp * KT + r) * 32 + lane] = acc[r];
-      consumer_sync();
-      if (have && slice == 0 && KT > 2) {
-        for (int s = 1; s < ws; ++s)
-#pragma unroll
-          for (int r = 0; r < KT; ++r) acc[r] += part[((warp + s) * KT + r) * 32 + lane];
-      }
-      if (have && slice == 0 && KT <= 2) {
-#pragma unroll
-        for (int r = 0; r < KT; ++r) {
-          double p0 = 0.0, p1 = 0.0, p2 = 0.0, p3 = 0.0;
-          for (int s = 1; s < ws; s += 4) {
-            p0 += part[((warp + s) * KT + r) * 32 + lane];
-            if (s + 1 < ws) p1 += part[((warp + s + 1) * KT + r) * 32 + lane];
-            if (s + 2 < ws) p2 += part[((warp + s + 2) * KT + r) * 32 + lane];
-            if (s + 3 < ws) p3 += part[((warp + s + 3) * KT + r) * 32 + lane];
-          }
-          acc[r] += (p0 + p1) + (p2 + p3);
-        }
-      }
-    }
+    if (ws > 1) reduce_slices<KT>(acc, part, warp, lane, ws, have && slice == 0, [] { consumer_sync(); });
     if (tr_on) a.trace[16 * p + 3] = clock64();
     if (have && slice == 0) {
-      if (KT <= 2) tile_store_with<KT, TH>(a, dir, tr, lane, acc, sto);
-      else tile_store<KT, TH>(a, dir, tr, lane, acc);
+      tile_store_with<KT, TH>(a, dir, tr, lane, acc, sto);
       if (tr_on) a.trace[16 * p + 4] = clock64();
       signal_done(a.cnt + dw.td.self);
       if (tr_on) a.trace[16 * p + 5] = clock64();
@@ -1281,13 +1163,16 @@ __device__ __forceinline__ void level_phase_pipe(const SolveArgs& a, const Phase
 // walks its share in that order, and a tile spins only on the completion counters of the fronts it reads from
 // (TileDep).  A dependency always lies earlier in the global order and all CTAs are co-resident (cooperative
 // launch), so the earliest unfinished tile can always run: no deadlock.
-template <int KT, bool PIPE>
-__global__ void __launch_bounds__(PIPE ? PIPE_THREADS : SOLVE_WARPS * 32, 1) solve_kernel(SolveArgs a) {
+// The one- and two-column solves of the eigensolver run the producer / consumer form (17 warps at 96 registers: the
+// tiles keep no panel entries in registers; measured 228 -> 218 us and 296 -> 285 us at C2); that is too few
+// registers for wider tiles (k = 4: 306 -> 330 us), which run 16 warps that read the tile-major panels themselves.
+template <int KT>
+__global__ void __launch_bounds__(KT <= 2 ? PIPE_THREADS : SOLVE_WARPS * 32, 1) solve_kernel(SolveArgs a) {
+  constexpr bool pipe = KT <= 2;      // panel pipeline (producer warp + shared-memory rings)
   extern __shared__ double smem[];
   __shared__ PhaseRec s_phase[MAX_PHASES_SMEM];
-  __shared__ int4 s_next[PIPE ? 1 : SOLVE_WARPS][5];       // first tile record + dependencies of the next phase, per warp
+  __shared__ int4 s_next[pipe ? 1 : SOLVE_WARPS][5];       // first tile record + dependencies of the next phase, per warp
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  constexpr bool pipe = PIPE;         // tile-major panels + panel pipeline (a.lring_w > 0), or the column-major form
   constexpr int NT = SOLVE_WARPS * 32;                      // consumer threads (the whole CTA without the pipeline)
   double* stage = smem + (warp % SOLVE_WARPS) * (32 * KT);  // [KT][32] per warp
   double* part = smem + SOLVE_WARPS * 32 * KT;              // [SOLVE_WARPS][KT][32] partial sums
@@ -1330,72 +1215,34 @@ __global__ void __launch_bounds__(PIPE ? PIPE_THREADS : SOLVE_WARPS * 32, 1) sol
   for (int p = a.p_begin; p < a.p_end; ++p) {
     if (a.trace && blockIdx.x == 0 && threadIdx.x == 0) a.trace[16 * p + 8] = clock64();
     const PhaseRec ph = p < MAX_PHASES_SMEM ? s_phase[p] : a.phases[p];
-    const int64_t tile_off = ph.tile_off;
-    const int dir = ph.dir, ws = ph.ws, ntiles = ph.ntiles;
     const bool use_perm = (p == 0);
     // request this warp's first tile record of the NEXT phase now (static schedule): the load completes
     // behind this phase's work instead of in front of the next phase's
-    bool nxt_have = false, bar_after = false;
+    bool nxt_have = false;
     int4 nxt = make_int4(0, 0, 0, 0);
-    if (p + 1 < a.p_end) {
+    if (!pipe && p + 1 < a.p_end) {
       const PhaseRec nx = (p + 1) < MAX_PHASES_SMEM ? s_phase[p + 1] : a.phases[p + 1];
-      bar_after = barrier_between(ph, nx, p);
-      if (nx.ws > 0 && !pipe) {
-        const int te = (int)blockIdx.x * (SOLVE_WARPS / nx.ws) + warp / nx.ws;
-        if (te < nx.ntiles) {
-          nxt_have = true;
-          if (lane < 3) nxt = __ldg(reinterpret_cast<const int4*>(a.tiles + nx.tile_off + te) + lane);
-          else if (lane < 5) nxt = __ldg(reinterpret_cast<const int4*>(a.deps + nx.tile_off + te) + (lane - 3));
-        }
+      const int te = (int)blockIdx.x * (SOLVE_WARPS / nx.ws) + warp / nx.ws;
+      if (te < nx.ntiles) {
+        nxt_have = true;
+        if (lane < 3) nxt = __ldg(reinterpret_cast<const int4*>(a.tiles + nx.tile_off + te) + lane);
+        else if (lane < 5) nxt = __ldg(reinterpret_cast<const int4*>(a.deps + nx.tile_off + te) + (lane - 3));
       }
     }
-    if (p == 0 && a.p_end > 1) {
-      // permuted copy of the right-hand side for the later phases (coalesced writes, gathered reads)
-      const int k = a.k;
-      for (int64_t e = (int64_t)blockIdx.x * NT + threadIdx.x; e < (int64_t)a.n * k; e += (int64_t)gridDim.x * NT) {
-        const int64_t i = e / k;
-        const int r = (int)(e - i * k);
-        a.bperm[e] = a.B[(int64_t)__ldg(&a.perm[i]) * a.brs + (int64_t)r * a.bcs];
-      }
-    }
-    if (ws == 0) {
-      // ---- subtree phase: every slot walks the local levels of its own subtrees; only CTA barriers
-      const int nl = ntiles, nslots = ph.level;
-      for (int slot = blockIdx.x; slot < nslots; slot += gridDim.x) {
-        const int* tab = a.sub_ptr + tile_off + (int64_t)slot * (nl + 1);
-        for (int ll = 0; ll < nl; ++ll) {
-          const int l = dir == 0 ? ll : nl - 1 - ll;
-          const int t0 = __ldg(&tab[l]), t1 = __ldg(&tab[l + 1]);
-          for (int te = t0 + warp; te < t1; te += SOLVE_WARPS) {
-            const TileRec tr = load_tile(a.tiles + te);
-            double acc[KT];
-#pragma unroll
-            for (int r = 0; r < KT; ++r) acc[r] = 0.0;
-            NoWait nw;
-            tile_compute<KT>(a, dir, use_perm, tr, lane, 0, 1, stage, acc, nw);
-            tile_store<KT>(a, dir, tr, lane, acc);
-          }
-          cta_sync();           // CTA-scope ordering: the level's results are visible to the whole slot
-        }
-      }
-    } else if constexpr (pipe) {
-      const int th_ = (int)(ph.pad & 0xff);
+    // without subtree phases, phase 0 gathers B through perm itself and writes the permuted copy that the later phases
+    // read; the grid barrier behind it makes the copy complete for them
+    const bool bar_after = p == 0 && a.p_end > 1;
+    if (bar_after) permute_rhs(a, (int64_t)blockIdx.x * NT + threadIdx.x, (int64_t)gridDim.x * NT);
+    const int th_ = (int)ph.pad;
+    if constexpr (pipe) {
       if (a.trace && blockIdx.x == 0 && threadIdx.x == 0) a.trace[16 * p + 9] = clock64();
       if (th_ == 8) level_phase_pipe<KT, 8>(a, ph, p, use_perm, lane, warp, stage, part, cs, sm);
       else if (th_ == 16) level_phase_pipe<KT, 16>(a, ph, p, use_perm, lane, warp, stage, part, cs, sm);
       else level_phase_pipe<KT, SOLVE_TILE>(a, ph, p, use_perm, lane, warp, stage, part, cs, sm);
     } else {
-      // the tiles read their panel entries themselves: column-major panels, or (SOLVE_TILED) the tile-major ones
-      const int th_ = (int)(ph.pad & 0xff);
-      if (ph.pad & SOLVE_TILED) {
-        if (th_ == 8) level_phase<KT, 8, true>(a, ph, p, use_perm, lane, warp, stage, part, have_next, s_next);
-        else if (th_ == 16) level_phase<KT, 16, true>(a, ph, p, use_perm, lane, warp, stage, part, have_next, s_next);
-        else level_phase<KT, SOLVE_TILE, true>(a, ph, p, use_perm, lane, warp, stage, part, have_next, s_next);
-      } else {
-        if (th_ == 8) level_phase<KT, 8, false>(a, ph, p, use_perm, lane, warp, stage, part, have_next, s_next);
-        else if (th_ == 16) level_phase<KT, 16, false>(a, ph, p, use_perm, lane, warp, stage, part, have_next, s_next);
-        else level_phase<KT, SOLVE_TILE, false>(a, ph, p, use_perm, lane, warp, stage, part, have_next, s_next);
-      }
+      if (th_ == 8) level_phase<KT, 8>(a, ph, p, use_perm, lane, warp, stage, part, have_next, s_next);
+      else if (th_ == 16) level_phase<KT, 16>(a, ph, p, use_perm, lane, warp, stage, part, have_next, s_next);
+      else level_phase<KT, SOLVE_TILE>(a, ph, p, use_perm, lane, warp, stage, part, have_next, s_next);
     }
     if constexpr (!pipe) {
       // ---- hand the prefetched first tile record of the next phase to the whole warp
@@ -1428,20 +1275,12 @@ int upload_vec(SymDevHolder* h, const std::vector<T>& v, T** out) {
   return 0;
 }
 
-// launch shape of the subtree kernel per right-hand-side count: warps per CTA and whether the operands of the
-// next front are prefetched into registers (needs the 128-register budget of a 16-warp CTA)
-template <int KT>
-struct SubCfg {
-  static constexpr int NW = KT == 1 ? EIGD_SUB_NW1 : 16;
-  static constexpr bool PIPE = KT == 1 && NW == 16;
-};
-
 struct KernelCfg {
   bool ready = false;
   int grid = 0;
-  size_t smem = 0;      // cooperative level kernel: staging + partial sums
-  size_t smem_pipe = 0; // ... + panel rings, mbarriers, slice FIFOs and record slots of the panel pipeline
-  int lring_w = 0;      // panel ring bytes per warp in the level kernel
+  size_t smem = 0;      // cooperative level kernel: staging + partial sums (+ for KT <= 2 the panel rings, mbarriers
+                        // and record slots of the panel pipeline)
+  int lring_w = 0;      // panel ring bytes per warp in the level kernel (KT <= 2)
   size_t smem_sub = 0;  // subtree kernel: staging + panel ring + mbarriers + front records
   int ring_w = 0;       // panel ring bytes per warp
   int rec_cap = 0;      // front records staged in shared memory
@@ -1455,25 +1294,26 @@ int configure(int slot) {
   if (c.ready) return 0;
   const size_t stage_b = (size_t)SOLVE_WARPS * 32 * KT * 8;
   c.smem = 2 * stage_b;
-  {
+  if (KT <= 2) {
     // panel pipeline of the level kernel: what is left of the 227 KB per CTA after the staging / partial-sum arrays,
     // the kernel's static shared memory (phase records, first-tile records) and the pipeline's own bookkeeping
     cudaFuncAttributes fa;
-    EIGD_CUDA(cudaFuncGetAttributes(&fa, solve_kernel<KT, true>));
+    EIGD_CUDA(cudaFuncGetAttributes(&fa, solve_kernel<KT>));
     const size_t misc = pipe_smem_misc();
     const size_t budget = 227 * 1024 - fa.sharedSizeBytes - 1024;
     size_t ring = budget > c.smem + misc ? (budget - c.smem - misc) / SOLVE_WARPS : 0;
     ring = std::min<size_t>(ring, 16384) / 256 * 256;
-    c.lring_w = ring >= 2048 ? (int)ring : 0;
-    c.smem_pipe = c.lring_w ? c.smem + (size_t)SOLVE_WARPS * c.lring_w + misc : c.smem;
+    if (ring < 2048) { eigd_set_error("solve: the panel rings of the level kernel do not fit in shared memory"); return 5; }
+    c.lring_w = (int)ring;
+    c.smem += (size_t)SOLVE_WARPS * c.lring_w + misc;
   }
-  EIGD_CUDA(cudaFuncSetAttribute(solve_kernel<KT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c.smem_pipe));
-  EIGD_CUDA(cudaFuncSetAttribute(solve_kernel<KT, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c.smem));
+  EIGD_CUDA(cudaFuncSetAttribute(solve_kernel<KT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c.smem));
   int occ = 0;
-  EIGD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, solve_kernel<KT, true>, PIPE_THREADS, c.smem_pipe));
+  EIGD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, solve_kernel<KT>, KT <= 2 ? PIPE_THREADS : SOLVE_WARPS * 32,
+                                                          c.smem));
   if (occ < 1) { eigd_set_error("solve: kernel does not fit on an SM"); return 5; }
   // subtree kernel: staging [NW][KT][32] | panel ring | mbarriers + copy queue | front records; 227 KB per CTA on sm_100a
-  constexpr int NW = SubCfg<KT>::NW;
+  constexpr int NW = SOLVE_WARPS;
   const size_t stage_s = (size_t)NW * 32 * KT * 8;
   const size_t budget = 227 * 1024 - 1024;
   c.rec_cap = KT <= 4 ? 512 : 256;
@@ -1481,8 +1321,7 @@ int configure(int slot) {
   ring = std::min<size_t>(ring, 10240) / 256 * 256;
   c.ring_w = (int)ring;
   c.smem_sub = stage_s + ring * NW + 2 * FRONT_DEPTH * NW * 8 + (size_t)c.rec_cap * 48;
-  EIGD_CUDA(cudaFuncSetAttribute(subtree_kernel<KT, NW, SubCfg<KT>::PIPE>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 (int)c.smem_sub));
+  EIGD_CUDA(cudaFuncSetAttribute(subtree_kernel<KT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c.smem_sub));
   c.grid = g_num_sms;
   c.ready = true;
   return 0;
@@ -1500,45 +1339,32 @@ int launch_solve(int slot, eigd_factor* f, SolveArgs& a) {
   a.deps = f->h->solve.deps;
   a.dep_ovf = f->h->solve.dep_ovf;
   a.ring_w = c.ring_w;
-  a.lring_w = 0;
+  a.lring_w = c.lring_w;
   a.rec_cap = c.rec_cap;
-  // subtree phases in front mode run as their own launches in front of / behind the cooperative level kernel
-  const bool sub_first = np >= 1 && hp[0].ws == 0 && hp[0].pad == 0;
-  const bool sub_last = np >= 2 && hp[np - 1].ws == 0 && hp[np - 1].pad == 0;
-  a.p_begin = sub_first ? 1 : 0;
-  a.p_end = sub_last ? np - 1 : np;
+  // the subtree phases (a plan with a cut: the first and the last phase) run as their own launches in front of / behind
+  // the cooperative level kernel
+  const bool sub = np >= 2 && hp[0].ws == 0;
+  a.p_begin = sub ? 1 : 0;
+  a.p_end = sub ? np - 1 : np;
   a.bar_base = f->bar_base;
   a.epoch = 0;
-  if (sub_first) {
-    subtree_kernel<KT, SubCfg<KT>::NW, SubCfg<KT>::PIPE><<<hp[0].level, SubCfg<KT>::NW * 32, c.smem_sub, g_eigd_stream>>>(a, 0);
+  if (sub) {
+    subtree_kernel<KT><<<hp[0].level, SOLVE_WARPS * 32, c.smem_sub, g_eigd_stream>>>(a, 0);
     EIGD_CUDA(cudaGetLastError());
     ++g_eigd_launches;
   }
   if (a.p_end > a.p_begin) {
     a.epoch = ++f->epoch;            // one epoch per cooperative launch: the completion counters never reset
-    int nbar = 0;
-    for (int p = a.p_begin; p + 1 < a.p_end; ++p) nbar += barrier_between(hp[p], hp[p + 1], p) ? 1 : 0;
-    // tile-major panels (SOLVE_TILED in the level phases' records) <=> the level kernel runs its panel pipeline
-    bool tiled = false;
-    for (int p = a.p_begin; p < a.p_end; ++p) tiled = tiled || (hp[p].ws > 0 && (hp[p].pad & SOLVE_TILED));
-    // the producer / consumer form runs 17 warps per CTA at 96 registers: right for the one- and two-column solves of
-    // the eigensolver (the tiles keep no panel entries in registers; measured 228 -> 218 us and 296 -> 285 us at C2), too
-    // few for wider ones (k = 4: 306 -> 330 us), which keep the 16-warp form and read the tile-major panels themselves
-    // (EIGD_SOLVE_PIPE_KMAX: developer override)
-    static int pipe_kmax = -1;
-    if (pipe_kmax < 0) { const char* e = getenv("EIGD_SOLVE_PIPE_KMAX"); pipe_kmax = e ? atoi(e) : 2; }
-    tiled = tiled && c.lring_w > 0 && KT <= pipe_kmax;
-    a.lring_w = tiled ? c.lring_w : 0;
+    // the one grid barrier: behind phase 0 of a plan without subtree phases (solve_kernel)
+    const int nbar = a.p_begin == 0 && a.p_end > 1 ? 1 : 0;
     void* params[] = {(void*)&a};
-    EIGD_CUDA(cudaLaunchCooperativeKernel(tiled ? (void*)solve_kernel<KT, true> : (void*)solve_kernel<KT, false>, dim3(c.grid),
-                                          dim3(tiled ? PIPE_THREADS : SOLVE_WARPS * 32), params, tiled ? c.smem_pipe : c.smem,
-                                          g_eigd_stream));
+    EIGD_CUDA(cudaLaunchCooperativeKernel((void*)solve_kernel<KT>, dim3(c.grid), dim3(KT <= 2 ? PIPE_THREADS : SOLVE_WARPS * 32),
+                                          params, c.smem, g_eigd_stream));
     ++g_eigd_launches;
     f->bar_base += (unsigned long long)nbar * (unsigned long long)c.grid;
   }
-  if (sub_last) {
-    subtree_kernel<KT, SubCfg<KT>::NW, SubCfg<KT>::PIPE><<<hp[np - 1].level, SubCfg<KT>::NW * 32, c.smem_sub, g_eigd_stream>>>(a,
-                                                                                                                      np - 1);
+  if (sub) {
+    subtree_kernel<KT><<<hp[np - 1].level, SOLVE_WARPS * 32, c.smem_sub, g_eigd_stream>>>(a, np - 1);
     EIGD_CUDA(cudaGetLastError());
     ++g_eigd_launches;
   }
@@ -1658,11 +1484,6 @@ extern "C" int eigd_factor_solve(eigd_factor* f, const double* B, int64_t brs, i
     a.times = g_phase_times;
     a.trace = g_trace;
     a.skew = g_skew;
-    {
-      static int dbg = -1;
-      if (dbg < 0) { const char* e = getenv("EIGD_SOLVE_DBG"); dbg = e ? atoi(e) : 0; }
-      a.dbg = dbg;
-    }
     int rc;
     SolveTiming tm;
     if (g_timing_on) {

@@ -4,7 +4,6 @@
 #include "solve_plan.hpp"
 
 #include <algorithm>
-#include <cstdlib>
 #include <functional>
 #include <queue>
 
@@ -117,7 +116,6 @@ void build_solve_plan_host(const eigd_symbolic* S, int target_warps, int nslots,
   P.nslots = nslots;
   P.sub_ptr.clear();
   P.sub_slot.assign(ns, -1);
-  if (const char* e = getenv("EIGD_SOLVE_CUT")) cut_req = atoi(e);     // developer override (tuning runs)
   if (cut_req >= S->nlevels - 1) cut_req = S->nlevels - 2;
   if (cut_req >= 0 && nslots > 0) {
     assign_subtrees(S, cut_req, nslots, P.sub_slot);
@@ -139,26 +137,20 @@ void build_solve_plan_host(const eigd_symbolic* S, int target_warps, int nslots,
     }
   }
   const int cut = P.cut_level, nl = cut + 1;
-  // front mode (default): ONE record per front in the subtree phases -- a warp brings the front's whole panel
-  // into shared memory with one bulk copy and runs all its row tiles from there; EIGD_SOLVE_FRONTS=0 keeps the
-  // one-record-per-tile form (developer comparison runs)
-  bool front_mode = true;
-  if (const char* e = getenv("EIGD_SOLVE_FRONTS")) front_mode = atoi(e) != 0;
+  // ONE record per front in the subtree phases (front mode): a warp brings the front's whole panel into shared memory
+  // with one bulk copy and runs all its row tiles from there
   auto subtree_phase = [&](int dir) {
     // tiles ordered by (slot, level); table entry [slot * (nl + 1) + l] = first tile of local level l
     std::vector<std::vector<int>> bucket((size_t)nslots * nl);
     for (int k = 0; k < ns; ++k)
       if (S->sn_level[k] <= cut) bucket[(size_t)P.sub_slot[k] * nl + S->sn_level[k]].push_back(k);
-    PhaseRec ph{dir, 0, nl, nslots, (int64_t)P.sub_ptr.size(), front_mode ? 0 : SOLVE_TILE};
+    PhaseRec ph{dir, 0, nl, nslots, (int64_t)P.sub_ptr.size(), 0};
     for (int s = 0; s < nslots; ++s) {
       for (int l = 0; l < nl; ++l) {
         P.sub_ptr.push_back((int)P.tiles.size());
         for (int k : bucket[(size_t)s * nl + l]) {
-          int outs = dir == 0 ? sn_fsize(S, k) : sn_ncols(S, k);
-          for (int t = 0; t * SOLVE_TILE < outs && (t == 0 || !front_mode); ++t) {
-            P.tiles.push_back(rec(k, t));
-            P.deps.push_back(TileDep{0, 0, 0, 0, 0, 0, 0, 0});
-          }
+          P.tiles.push_back(rec(k, 0));
+          P.deps.push_back(TileDep{0, 0, 0, 0, 0, 0, 0, 0});
         }
       }
       P.sub_ptr.push_back((int)P.tiles.size());
@@ -170,9 +162,7 @@ void build_solve_plan_host(const eigd_symbolic* S, int target_warps, int nslots,
   // SMs would idle while a few of them stream 64 - 128 KB panel slices each (the upper levels: one to a few dozen wide
   // fronts).  With per-front completion counters instead of grid barriers a finer tiling costs no extra synchronisation.
   // (Round 1 measured a variable tile height as slower -- with a grid barrier per level and the tile-serial overheads of
-  // that kernel; EIGD_SOLVE_THIN=0 restores 32 everywhere for comparison runs.)
-  bool thin = true;
-  if (const char* e = getenv("EIGD_SOLVE_THIN")) thin = atoi(e) != 0;
+  // that kernel.)
   auto count_tiles = [&](int dir, int l, int to) {
     int64_t nt = 0;
     for (int q = S->level_ptr[l]; q < S->level_ptr[l + 1]; ++q) {
@@ -183,24 +173,20 @@ void build_solve_plan_host(const eigd_symbolic* S, int target_warps, int nslots,
   };
   const int ncta = std::max(1, target_warps / SOLVE_WARPS);
   std::vector<int> height(2 * (size_t)S->nlevels, SOLVE_TILE);      // [dir * nlevels + level]
-  for (int dir = 0; dir < 2 && thin; ++dir)
+  for (int dir = 0; dir < 2; ++dir)
     for (int l = cut + 1; l < S->nlevels; ++l) {
       int to = SOLVE_TILE;
       while (to > 8 && count_tiles(dir, l, to / 2) <= ncta) to /= 2;
       height[(size_t)dir * S->nlevels + l] = to;
     }
-  // tile-major panels + the asynchronous shared-memory panel pipeline of the level kernel (EIGD_SOLVE_PIPE=0: column-major
-  // panels read straight from global memory, the round-1 / early round-2 form, kept for comparison runs)
-  bool tiled = true;
-  if (const char* e = getenv("EIGD_SOLVE_PIPE")) tiled = atoi(e) != 0;
+  // the panels of the fronts above the cut are stored tile-major in their level's tile height (solve_plan.hpp)
   P.th_fwd.assign(ns, 0);
   P.th_bwd.assign(ns, 0);
-  if (tiled)
-    for (int k = 0; k < ns; ++k)
-      if (S->sn_level[k] > cut) {
-        P.th_fwd[k] = height[(size_t)0 * S->nlevels + S->sn_level[k]];
-        P.th_bwd[k] = height[(size_t)1 * S->nlevels + S->sn_level[k]];
-      }
+  for (int k = 0; k < ns; ++k)
+    if (S->sn_level[k] > cut) {
+      P.th_fwd[k] = height[(size_t)0 * S->nlevels + S->sn_level[k]];
+      P.th_bwd[k] = height[(size_t)1 * S->nlevels + S->sn_level[k]];
+    }
   auto level_phase = [&](int dir, int l) {
     int redmax = 1;
     const int to = height[(size_t)dir * S->nlevels + l];
@@ -210,7 +196,7 @@ void build_solve_plan_host(const eigd_symbolic* S, int target_warps, int nslots,
     }
     const int64_t nt = count_tiles(dir, l, to);
     const int ws = pick_ws((int)nt, redmax, target_warps);
-    PhaseRec ph{dir, ws, 0, l, (int64_t)P.tiles.size(), to | (tiled ? SOLVE_TILED : 0)};
+    PhaseRec ph{dir, ws, 0, l, (int64_t)P.tiles.size(), to};
     // tiles of front k in direction d, in the tile height of ITS level's phase (completion-counter targets)
     auto ntile = [&](int k, int d) {
       const int tk = S->sn_level[k] > cut ? height[(size_t)d * S->nlevels + S->sn_level[k]] : SOLVE_TILE;

@@ -35,7 +35,7 @@ EIGD_HD inline int64_t solve_panel_doubles(int f, int nc) { return ((int64_t)f *
 // of a tile-major panel (below) starts on a 16-byte boundary -- the unit of a bulk copy into shared memory.
 EIGD_HD inline int solve_slice_len(int len, int ws) { return (((len + ws - 1) / ws) + 1) & ~1; }
 
-// TILE-MAJOR solve panels of the fronts ABOVE the cut (level phases; PhaseRec::pad carries SOLVE_TILED).  With tile
+// TILE-MAJOR solve panels of the fronts ABOVE the cut (level phases; PhaseRec::pad is the tile height).  With tile
 // height TH (outputs per warp tile: 32, 16 or 8, chosen per level and direction) the f x nc panel S of a front is
 // stored tile by tile: row tile t (rows t TH ... , th = min(TH, f - t TH) of them) occupies th * nc doubles from
 // offset t TH nc, element (row r, column c) at c * th + (r - t TH).  S^T (nc x f) likewise by column tiles: tile t
@@ -43,7 +43,6 @@ EIGD_HD inline int solve_slice_len(int len, int ws) { return (((len + ws - 1) / 
 // The part of a tile that one warp multiplies -- a contiguous range of the reduction dimension -- is then ONE
 // contiguous run of doubles, which the level kernel brings into shared memory with one bulk copy, ahead of time.
 // Fronts below the cut keep plain column-major panels (the subtree kernels copy whole fronts).
-constexpr int64_t SOLVE_TILED = 0x100;   // flag in PhaseRec::pad next to the tile height (low byte)
 
 // One warp tile: 32 consecutive outputs of one front.  Everything the warp needs about the front
 // travels in this one 48-byte record; the forward sweep needs no further index look-up before it
@@ -87,8 +86,8 @@ static_assert(sizeof(TileDep) == 32, "TileDep is read as two 16-byte words");
 struct PhaseRec {
   int dir, ws, ntiles, level;     // dir 0 forward, 1 backward
   int64_t tile_off;
-  int64_t pad;                    // level phase: tile height (= SOLVE_TILE); subtree phase: SOLVE_TILE = one record
-                                  // per 32-output tile, 0 = FRONT MODE, one record per front (tile field 0)
+  int64_t pad;                    // level phase: tile height (32, 16 or 8); subtree phase: 0 (one record per front,
+                                  // tile field 0)
 };
 static_assert(sizeof(PhaseRec) == 32, "PhaseRec layout");
 

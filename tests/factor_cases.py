@@ -12,6 +12,8 @@ negative eigenvalues when it is known without an eigensolve (None otherwise).
     below the pivot block (partial extend-add, TRSM and trailing-update tiles).
   * grid_case: finite-element grid patterns with 1, 2, 3 or 6 DOF per node, under several supernode caps and with or
     without relaxed amalgamation.
+  * block_diagonal_case: disjoint dense blocks, whose solve plan has level-phase panel slices larger than the
+    shared-memory ring of the pipelined level kernel.
   * kron_case: a shifted Kronecker-sum Laplacian whose spectrum is known in closed form, so that the number of
     eigenvalues below the shift (the inertia of the shifted factor) is exact at 50 000 DOF."""
 import numpy as np
@@ -129,6 +131,23 @@ def bordered_case(blocks, border, kind="spd", seed=0):
         raise ValueError(kind)
     name = "bordered-%s-%s+%d" % (kind, "/".join(map(str, blocks)), border)
     return Case(name, csr_from_dense(M, mask), opts=BORDERED_OPTS, nneg=nneg)
+
+
+def block_diagonal_case(nblocks=400, w=96, seed=0):
+    """nblocks disjoint dense SPD w x w blocks: one w-wide supernode each, all on one level of the tree and no subtree
+    phases.  With w = 96 the level has 3 * nblocks 32-output tiles per direction, enough to give every warp of 148 SMs a
+    tile of its own (ws = 1), so each front's widest tile multiplies a 96 x 32 panel slice of 24 576 bytes, larger than
+    the 16 KB shared-memory ring of the pipelined level kernel: those tiles read their slice from global memory."""
+    rng = np.random.default_rng(seed + nblocks + 7 * w)
+    blocks = []
+    for _ in range(nblocks):
+        M = rng.uniform(-1.0, 1.0, (w, w))
+        M = (M + M.T) * 0.5
+        M[np.diag_indices(w)] = np.abs(M).sum(axis=1) + 0.1
+        blocks.append(M)
+    A = sp.block_diag(blocks, format="csr")
+    A.sort_indices()
+    return Case("block-diagonal-%dx%d" % (nblocks, w), A, nneg=0)
 
 
 def grid_matrix(nx, ny, dof, seed):

@@ -14,6 +14,7 @@ import scipy.sparse.linalg as spla
 from eigd_b200 import _lib, fe
 from eigd_b200.device import Symbolic
 import multifrontal_oracle as mo
+import factor_cases as fc
 
 MASK48 = (1 << 48) - 1
 
@@ -100,9 +101,9 @@ def emulate(plan, S, sym_arr, dinv, b, shuffle=None):
     height = {}                        # tile index -> tile height of its level phase (PhaseRec.pad)
     for d, ws, ntiles, level, tile_off, _to in plan["phases"]:
         if ws > 0:
-            assert int(_to) & 0xff in (8, 16, 32)          # low byte: tile height; 0x100: tile-major panel storage
+            assert int(_to) in (8, 16, 32)
             for te in range(tile_off, tile_off + ntiles):
-                height[int(te)] = int(_to) & 0xff
+                height[int(te)] = int(_to)
 
     def run_level_tile(te, d):
         selfc, deps = tile_deps(plan, te)
@@ -122,24 +123,23 @@ def emulate(plan, S, sym_arr, dinv, b, shuffle=None):
 
     for d, ws, ntiles, level, tile_off, _to in plan["phases"]:
         if ws == 0 and pending:
-            drain()                    # the kernel puts a grid barrier in front of an in-kernel subtree phase
+            drain()                    # the backward subtree launch follows the level kernel in stream order
         if ws == 0:
+            assert _to == 0
             nl, nslots = int(ntiles), int(level)
             for slot in range(nslots):
                 tab = plan["sub_ptr"][tile_off + slot * (nl + 1): tile_off + (slot + 1) * (nl + 1)]
                 for ll in range(nl):
                     l = ll if d == 0 else nl - 1 - ll
                     for te in range(tab[l], tab[l + 1]):
-                        if _to == 0:              # front mode: one record per front, the kernel runs all its tiles
-                            first, nc, nb, tile = (int(v) for v in tiles[te][:4])
-                            assert tile == 0
-                            outs = nc + nb if d == 0 else nc
-                            for t in range((outs + 31) // 32):
-                                rec = tiles[te].copy()
-                                rec[3] = t
-                                do_tile(int(d), rec)
-                        else:
-                            do_tile(int(d), tiles[te])
+                        # one record per front, the subtree kernel runs all its tiles
+                        first, nc, nb, tile = (int(v) for v in tiles[te][:4])
+                        assert tile == 0
+                        outs = nc + nb if d == 0 else nc
+                        for t in range((outs + 31) // 32):
+                            rec = tiles[te].copy()
+                            rec[3] = t
+                            do_tile(int(d), rec)
         else:
             for te in range(tile_off, tile_off + ntiles):
                 if shuffle is None:
@@ -176,6 +176,10 @@ def build_case(nx, ny, dof, use_coords):
     return A, sym, arr, orc, S
 
 
+# the plan arguments of the device solve on a B200: 148 SMs x 16 warps, 148 CTA slots, automatic cut
+PRODUCTION = (148 * 16, 148, -2)
+
+
 @pytest.mark.parametrize("nx,ny,dof,use_coords", [(22, 17, 1, True), (14, 11, 2, True), (19, 13, 1, False)])
 def test_plan_emulation_matches_scipy(nx, ny, dof, use_coords):
     A, sym, arr, orc, S = build_case(nx, ny, dof, use_coords)
@@ -186,7 +190,7 @@ def test_plan_emulation_matches_scipy(nx, ny, dof, use_coords):
     ntiles_b = sum(-(-(S[f].shape[1]) // 32) for f in S)
     nlevels = len(arr["level_ptr"]) - 1
     seen_cut = set()
-    for target_warps, nslots, cut in [(64, 4, -1), (64, 4, -2), (2368, 148, -2), (32, 3, 1), (32, 5, 2), (16, 2, nlevels)]:
+    for target_warps, nslots, cut in [(64, 4, -1), (64, 4, -2), PRODUCTION, (32, 3, 1), (32, 5, 2), (16, 2, nlevels)]:
         plan = plan_arrays(sym, target_warps, nslots, cut)
         x, done = emulate(plan, S, arr, orc.dinv, b)
         assert np.abs(x - x_ref).max() <= 1e-10 * np.abs(x_ref).max(), (target_warps, nslots, cut)
@@ -197,8 +201,12 @@ def test_plan_emulation_matches_scipy(nx, ny, dof, use_coords):
         # the level keeps the full height; thinner tiles only add to the count)
         assert len([1 for k in done if k[0] == 0]) >= ntiles_f
         assert len([1 for k in done if k[0] == 1]) >= ntiles_b
-        if int((plan["phases"][:, 5][plan["phases"][:, 1] > 0] & 0xff).min(initial=32)) == 32:
+        if int(plan["phases"][:, 5][plan["phases"][:, 1] > 0].min(initial=32)) == 32:
             assert len([1 for k in done if k[0] == 0]) == ntiles_f and len([1 for k in done if k[0] == 1]) == ntiles_b
+        if (target_warps, nslots, cut) == PRODUCTION:
+            ph = plan["phases"]
+            assert (ph[ph[:, 1] == 0, 5] == 0).all()                        # subtree phases: one record per front
+            assert np.isin(ph[ph[:, 1] > 0, 5], (8, 16, 32)).all()          # level phases: the tile height
         cutl = int(plan["meta"][0])
         seen_cut.add(cutl)
         if cutl >= 0:
@@ -221,3 +229,37 @@ def test_child_slabs_are_consistent():
         kids = [c for c in range(ns) if par[c] == p]
         assert [int(slab[c]) for c in kids] == [min(i, 2) for i in range(len(kids))]
     assert all(int(slab[k]) == 255 for k in range(ns) if par[k] < 0)
+
+
+RING_CAP = 16384        # the largest panel ring per warp of the pipelined level kernel (solve.cu, configure)
+
+
+def slice_bytes(rec, d, th, ws, bm=0):
+    """Bytes of the tile-major panel slice each of the ws warps of level-phase tile rec multiplies (slice_of, solve.cu)."""
+    first, nc, nb, tile = (int(v) for v in rec[:4])
+    f, o0 = nc + nb, tile * th
+    if d == 0:
+        lo, hi, ld = 0, min(nc, (o0 + th + bm) & ~bm), min(th, f - o0)
+    else:
+        lo, hi, ld = o0 & ~bm, f, min(th, nc - o0)
+    per = ((-(-(hi - lo) // ws)) + 1) & ~1                            # solve_slice_len
+    out = []
+    for s in range(ws):
+        r0 = min(hi, lo + s * per)
+        out.append((min(hi, r0 + per) - r0) * ld * 8)
+    return out
+
+
+def test_block_diagonal_slices_exceed_the_ring():
+    """The block-diagonal case of the device tests is there to make level-phase tiles read a panel slice larger than
+    the pipelined kernel's ring from global memory, in both sweeps; no grid case does."""
+    c = fc.block_diagonal_case()
+    sym = Symbolic(c.A.indptr, c.A.indices, c.n, coords=c.coords, dof_per_node=c.dof, opts=c.opts)
+    plan = plan_arrays(sym, *PRODUCTION)
+    big = {0: 0, 1: 0}
+    for d, ws, ntiles, level, tile_off, th in plan["phases"]:
+        if ws == 0:
+            continue
+        for te in range(tile_off, tile_off + ntiles):
+            big[int(d)] += sum(b > RING_CAP for b in slice_bytes(plan["tiles"][te], int(d), int(th), int(ws)))
+    assert big[0] > 0 and big[1] > 0, big
