@@ -405,7 +405,8 @@ __device__ __forceinline__ void tile_store(const SolveArgs& a, int dir, const Ti
 // shared-memory buffer with ONE bulk copy (cp.async.bulk, completion on an mbarrier), the next front's panel is
 // requested before the current one is consumed (two half-buffers), the operand vector is gathered once per
 // front instead of once per tile, and all row tiles run out of shared memory.  Fronts that do not fit (panel
-// larger than the warp's buffer, or more than 32 pivot columns) take the tile path below, record by record.
+// larger than FRONT_PANEL_MAX, or more than 32 pivot columns; for k >= 2 in the backward sweep also a panel and
+// operand block larger than the warp's buffer) take the tile path below, record by record.
 __device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(unsigned long long* bar, int count) {
   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
@@ -426,58 +427,56 @@ __device__ __forceinline__ void mbar_wait(unsigned long long* bar, unsigned pari
   } while (!ok);
 }
 
-struct FrontRing {
-  char* base;                  // this warp's buffer: two half-buffers of `half` bytes
-  int half;
-  unsigned long long* bar;     // two mbarriers, one per half (a front larger than `half` uses both halves and bar[0])
-  unsigned uses[2];            // completed copies per barrier (parity of the next wait)
-};
+// per-lane asynchronous copies into shared memory (LDGSTS): they hold no register while in flight, and each lane
+// has its own source address, so they serve the gathers through perm, rel and sn_rows as well
+__device__ __forceinline__ void cp_async8(void* dst, const void* src) {
+  asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(smem_u32(dst)), "l"(src) : "memory");
+}
+__device__ __forceinline__ void cp_async4(void* dst, const void* src) {
+  asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(smem_u32(dst)), "l"(src) : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+template <int N>
+__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
-constexpr int FRONT_TILES_MAX = 8;   // row tiles / row chunks of a front in front mode (non-pipelined form): f <= 256
-constexpr int FRONT_RT = 3;    // row tiles (forward) / row chunks (backward) a pipelined front may have: f <= 96
+constexpr int FRONT_TILES_MAX = 8;   // row tiles / row chunks of a front in front mode (k >= 2): f <= 256
+constexpr int FRONT_RT = 3;    // row tiles (forward) / row chunks (backward) of a front in the k = 1 pipeline: f <= 96
+// Largest panel that takes front mode.  Not the ring size: the forward front path adds the children's updates of a row
+// before its products, the tile path after them, so moving this bound would change the bits of the result.
+constexpr int FRONT_PANEL_MAX = 10240;
 
-// Operands of one front, REQUESTED one front ahead (software pipeline in registers, KT <= 2): by the time the
+// Operands of one front, REQUESTED one front ahead (software pipeline in registers, k = 1): by the time the
 // front is processed its loads have landed, so a front costs no exposed memory round trip in the forward sweep
 // and one (index -> value) in the backward sweep.
-template <int KT>
 struct FrontOps {
-  double b[KT], s0[KT], s1[KT];            // forward: w1 entry of lane c = b + (s0 + s1)
-  double u0[FRONT_RT][KT], u1[FRONT_RT][KT];   // forward: children's updates of row t*32 + lane
-  double auxd[FRONT_RT];                   // forward: D^-1 of pivot row t*32 + lane
-  int auxi[FRONT_RT];                      // forward: position of update row t*32 + lane in the parent; backward:
-                                           // row index of input entry t*32 + lane (auxi[t]) ...
-  int perm0;                               // ... backward: original index of pivot column `lane`
+  double b, s0, s1;                  // forward: w1 entry of lane c = b + (s0 + s1)
+  double u0[FRONT_RT], u1[FRONT_RT];   // forward: children's updates of row t*32 + lane
+  double auxd[FRONT_RT];             // forward: D^-1 of pivot row t*32 + lane
+  int auxi[FRONT_RT];                // forward: position of update row t*32 + lane in the parent; backward:
+                                     // row index of input entry t*32 + lane (auxi[t]) ...
+  int perm0;                         // ... backward: original index of pivot column `lane`
 };
 
-template <int KT>
 __device__ __forceinline__ void front_request(const SolveArgs& a, int dir, bool use_perm, const TileRec& tr, int lane,
-                                              FrontOps<KT>& o) {
-  const int k = a.k;
+                                              FrontOps& o) {
   const int nc = tr.nc, f = tr.nc + tr.nb;
   const bool kids = (tr.link & LINK_HAS_CHILDREN) != 0;
   if (dir == 0) {
     const int64_t col = tr.first + min(lane, nc - 1);
-    const double* bp = use_perm ? a.B + (int64_t)__ldg(&a.perm[col]) * a.brs : a.bperm + col * k;
-    const int64_t bs = use_perm ? a.bcs : 1;
+    const double* bp = use_perm ? a.B + (int64_t)__ldg(&a.perm[col]) * a.brs : a.bperm + col;
     const double* w0 = a.wbuf + tr.w_off + lane;
-#pragma unroll
-    for (int r = 0; r < KT; ++r) {
-      const bool ok = r < k && lane < nc;
-      o.b[r] = ok ? __ldcg(bp + r * bs) : 0.0;
-      o.s0[r] = (ok && kids) ? __ldcg(w0 + (int64_t)r * a.sumf) : 0.0;
-      o.s1[r] = (ok && kids) ? __ldcg(w0 + a.slab_stride + (int64_t)r * a.sumf) : 0.0;
-    }
+    const bool ok = lane < nc;
+    o.b = ok ? __ldcg(bp) : 0.0;
+    o.s0 = (ok && kids) ? __ldcg(w0) : 0.0;
+    o.s1 = (ok && kids) ? __ldcg(w0 + a.slab_stride) : 0.0;
 #pragma unroll
     for (int t = 0; t < FRONT_RT; ++t) {
       const int row = t * SOLVE_TILE + lane;
       o.auxd[t] = row < nc ? __ldg(&a.dinv[tr.first + row]) : 0.0;
       o.auxi[t] = (row >= nc && row < f) ? __ldg(&a.rel[tr.row_off + row - nc]) : 0;
-#pragma unroll
-      for (int r = 0; r < KT; ++r) {
-        const bool ok = r < k && kids && row >= nc && row < f;
-        o.u0[t][r] = ok ? __ldcg(w0 + t * SOLVE_TILE + (int64_t)r * a.sumf) : 0.0;
-        o.u1[t][r] = ok ? __ldcg(w0 + t * SOLVE_TILE + a.slab_stride + (int64_t)r * a.sumf) : 0.0;
-      }
+      const bool upd = kids && row >= nc && row < f;
+      o.u0[t] = upd ? __ldcg(w0 + t * SOLVE_TILE) : 0.0;
+      o.u1[t] = upd ? __ldcg(w0 + t * SOLVE_TILE + a.slab_stride) : 0.0;
     }
   } else {
     o.perm0 = lane < nc ? __ldg(&a.perm[tr.first + lane]) : 0;
@@ -489,136 +488,275 @@ __device__ __forceinline__ void front_request(const SolveArgs& a, int dir, bool 
   }
 }
 
-// one front out of shared memory (buf = its panel, copy completion on `bar`); ops = its prefetched operands (PIPE)
-template <int KT, bool PIPE>
-__device__ __forceinline__ void front_compute(const SolveArgs& a, int dir, bool use_perm, TileRec tr, const double* buf,
-                                              unsigned long long* bar, unsigned parity, const FrontOps<PIPE ? KT : 1>& ops,
-                                              int lane, double* stage) {
-  const int k = a.k;
+// one front of a one-column solve out of shared memory (buf = its panel, copy completion on `bar`), with the operands
+// prefetched into registers
+__device__ __forceinline__ void front_compute_k1(const SolveArgs& a, int dir, const TileRec& tr, const double* buf,
+                                                 unsigned long long* bar, unsigned parity, const FrontOps& ops, int lane,
+                                                 double* stage) {
   const int nc = tr.nc, f = tr.nc + tr.nb;
-    const int ntile = (f + SOLVE_TILE - 1) / SOLVE_TILE;
-    if (dir == 0) {
-      // ---- forward: w1 (nc <= 32 entries) gathered once, then every row tile of S w1 out of shared memory
-      double v[KT];
-      if constexpr (PIPE) {
+  const int ntile = (f + SOLVE_TILE - 1) / SOLVE_TILE;
+  if (dir == 0) {
+    // ---- forward: w1 (nc <= 32 entries) staged once, then every row tile of S w1 out of shared memory
+    double v = ops.b + (ops.s0 + ops.s1);
+    if ((tr.link & LINK_HAS_OVF) && lane < nc) {
+      double z = 0.0;
+      ovf_add<1>(a, tr.w_off + lane, &z);
+      v += z;
+    }
+    stage[lane] = v;
+    __syncwarp();
+    mbar_wait(bar, parity);
 #pragma unroll
-        for (int r = 0; r < KT; ++r) v[r] = ops.b[r] + (ops.s0[r] + ops.s1[r]);
-        if ((tr.link & LINK_HAS_OVF) && lane < nc) {
-          double z[KT];
-#pragma unroll
-          for (int r = 0; r < KT; ++r) z[r] = 0.0;
-          ovf_add<KT>(a, tr.w_off + lane, z);
-#pragma unroll
-          for (int r = 0; r < KT; ++r) v[r] += z[r];
-        }
-      } else {
-#pragma unroll
-        for (int r = 0; r < KT; ++r) v[r] = 0.0;
-        if (lane < nc) fwd_operand<KT>(a, use_perm, tr, lane, v);
-      }
-#pragma unroll
-      for (int r = 0; r < KT; ++r) stage[r * 32 + lane] = v[r];
-      __syncwarp();
-      mbar_wait(bar, parity);
-#pragma unroll
-      for (int t = 0; t < (PIPE ? FRONT_RT : FRONT_TILES_MAX); ++t) {
-        if (t >= ntile) break;
-        const int row = t * SOLVE_TILE + lane;
-        double acc[KT];
-#pragma unroll
-        for (int r = 0; r < KT; ++r) acc[r] = 0.0;
-        if constexpr (!PIPE) {
-          if (row >= nc && row < f) child_add<KT>(a, tr.w_off + row, tr.link, acc);
-        }
-        const int cend = min(nc, (t + 1) * SOLVE_TILE);
-        const double* col = buf + min(row, f - 1);
+    for (int t = 0; t < FRONT_RT; ++t) {
+      if (t >= ntile) break;
+      const int row = t * SOLVE_TILE + lane;
+      double acc = 0.0;
+      const int cend = min(nc, (t + 1) * SOLVE_TILE);
+      const double* col = buf + min(row, f - 1);
 #pragma unroll 4
-        for (int c = 0; c < cend; ++c) {
-          const double m = col[c * f];
-#pragma unroll
-          for (int r = 0; r < KT; ++r) acc[r] = fma(m, stage[r * 32 + c], acc[r]);
-        }
-        if constexpr (PIPE) {
-#pragma unroll
-          for (int r = 0; r < KT; ++r) acc[r] += ops.u0[t][r] + ops.u1[t][r];
-          if ((tr.link & LINK_HAS_OVF) && row >= nc && row < f) ovf_add<KT>(a, tr.w_off + row, acc);
-          // store with the prefetched D^-1 / parent position (tile_store without its look-up)
-          if (row < nc) {
-            double* y = a.ybuf + (int64_t)(tr.first + row) * k;
-#pragma unroll
-            for (int r = 0; r < KT; ++r)
-              if (r < k) y[r] = ops.auxd[t] * acc[r];
-          } else if (row < f) {
-            const int sl = (int)((tr.link >> LINK_SLAB_SHIFT) & 0xff);
-            const int64_t dst = sl < 2 ? sl * a.slab_stride + (tr.link & LINK_WOFF_MASK) + ops.auxi[t]
-                                       : 2 * a.slab_stride + tr.w_off + row;
-            double* w = a.wbuf + dst;
-#pragma unroll
-            for (int r = 0; r < KT; ++r)
-              if (r < k) w[(int64_t)r * a.sumf] = acc[r];
-          }
-        } else {
-          tr.tile = t;
-          tile_store<KT>(a, 0, tr, lane, acc);
-        }
-      }
-    } else {
-      // ---- backward: x1 = S^T [z1 ; x2], lane = pivot column (nc <= 32), front rows streamed in chunks of 32
-      double vv[PIPE ? FRONT_RT : 1][KT];
-      if constexpr (PIPE) {
-        // all chunks' values are requested at once (their indices arrived with the previous front)
-#pragma unroll
-        for (int t = 0; t < FRONT_RT; ++t) {
-          const int i = t * SOLVE_TILE + lane;
-          const double* src = (i < nc ? a.ybuf : a.xperm) + (int64_t)ops.auxi[t] * k;
-#pragma unroll
-          for (int r = 0; r < KT; ++r) vv[t][r] = (i < f && r < k) ? __ldcg(src + r) : 0.0;
-        }
-      }
-      mbar_wait(bar, parity);
-      double acc[KT];
-#pragma unroll
-      for (int r = 0; r < KT; ++r) acc[r] = 0.0;
-      const double* colp = buf + min(lane, nc - 1);
-#pragma unroll
-      for (int t = 0; t < (PIPE ? FRONT_RT : FRONT_TILES_MAX); ++t) {
-        const int cc = t * SOLVE_TILE;
-        if (cc >= f) break;
-        const int nrow = min(32, f - cc);
-        if constexpr (PIPE) {
-#pragma unroll
-          for (int r = 0; r < KT; ++r) stage[r * 32 + lane] = vv[t][r];
-        } else {
-          double v[KT];
-#pragma unroll
-          for (int r = 0; r < KT; ++r) v[r] = 0.0;
-          if (lane < nrow) bwd_operand<KT>(a, tr, cc + lane, v);
-#pragma unroll
-          for (int r = 0; r < KT; ++r) stage[r * 32 + lane] = v[r];
-        }
-        __syncwarp();
-        const double* rowp = colp + cc * nc;
-#pragma unroll 4
-        for (int j = 0; j < nrow; ++j) {
-          const double m = rowp[j * nc];
-#pragma unroll
-          for (int r = 0; r < KT; ++r) acc[r] = fma(m, stage[r * 32 + j], acc[r]);
-        }
-        __syncwarp();
-      }
-      if constexpr (PIPE) {
-        if (lane < nc) {
-          double* xp = a.xperm + (int64_t)(tr.first + lane) * k;
-          double* xo = a.X + (int64_t)ops.perm0 * a.xrs;
-#pragma unroll
-          for (int r = 0; r < KT; ++r)
-            if (r < k) { xp[r] = acc[r]; xo[(int64_t)r * a.xcs] = acc[r]; }
-        }
-      } else {
-        tr.tile = 0;
-        tile_store<KT>(a, 1, tr, lane, acc);
+      for (int c = 0; c < cend; ++c) acc = fma(col[c * f], stage[c], acc);
+      acc += ops.u0[t] + ops.u1[t];
+      if ((tr.link & LINK_HAS_OVF) && row >= nc && row < f) ovf_add<1>(a, tr.w_off + row, &acc);
+      // store with the prefetched D^-1 / parent position (tile_store without its look-up)
+      if (row < nc) {
+        a.ybuf[tr.first + row] = ops.auxd[t] * acc;
+      } else if (row < f) {
+        const int sl = (int)((tr.link >> LINK_SLAB_SHIFT) & 0xff);
+        const int64_t dst = sl < 2 ? sl * a.slab_stride + (tr.link & LINK_WOFF_MASK) + ops.auxi[t]
+                                   : 2 * a.slab_stride + tr.w_off + row;
+        a.wbuf[dst] = acc;
       }
     }
+  } else {
+    // ---- backward: x1 = S^T [z1 ; x2], lane = pivot column (nc <= 32), front rows streamed in chunks of 32; all
+    // chunks' values are requested at once (their indices arrived with the previous front)
+    double vv[FRONT_RT];
+#pragma unroll
+    for (int t = 0; t < FRONT_RT; ++t) {
+      const int i = t * SOLVE_TILE + lane;
+      vv[t] = i < f ? __ldcg((i < nc ? a.ybuf : a.xperm) + ops.auxi[t]) : 0.0;
+    }
+    mbar_wait(bar, parity);
+    double acc = 0.0;
+    const double* colp = buf + min(lane, nc - 1);
+#pragma unroll
+    for (int t = 0; t < FRONT_RT; ++t) {
+      const int cc = t * SOLVE_TILE;
+      if (cc >= f) break;
+      const int nrow = min(32, f - cc);
+      stage[lane] = vv[t];
+      __syncwarp();
+      const double* rowp = colp + cc * nc;
+#pragma unroll 4
+      for (int j = 0; j < nrow; ++j) acc = fma(rowp[j * nc], stage[j], acc);
+      __syncwarp();
+    }
+    if (lane < nc) {
+      a.xperm[tr.first + lane] = acc;
+      a.X[(int64_t)ops.perm0 * a.xrs] = acc;
+    }
+  }
+}
+
+// ---- OPERAND STAGING of a multi-column front (KT >= 2).  The operands travel in shared memory, in the warp's ring
+// right behind the front's panel (same allocation), requested one front ahead with per-lane cp.async:
+//   forward : b [nc][k] (right-hand side of the pivot rows) | s0, s1 [k][f] (slabs 0 and 1 of every row; fronts with
+//             children only) | D^-1 [nc] | rel [nb] (int, parent positions of the update rows)
+//   backward: v [f][KT] (the input [z1 ; x2], gathered at the front's start through the indices) | sn_rows [nb] (int)
+//             | perm [nc] (int)
+// The request is split in two: the early part goes out before the current front is computed; the late part needs an
+// index loaded by the early part (forward, first phase: B through perm) and closes the front's copy group.
+// The forward sweep stages its operands at KT = 2 only.  C2 on a B200 (forward subtree phase, CTA-0 timestamps, staging
+// in every forward front that fits): k = 2 55.6 -> 52.4 us, but k = 4 69.7 -> 71.9 us and k = 10 135.1 -> 144.1 us;
+// there the direct loads stay (profiles/r3_subtree_staging.txt).
+template <int KT>
+constexpr bool FWD_STAGE = KT == 2;
+
+__host__ __device__ __forceinline__ int front_ops_doubles(const TileRec& t, int dir, int k, int kt) {
+  const int nc = t.nc, nb = t.nb, f = nc + nb;
+  if (dir == 0) return k * nc + ((t.link & LINK_HAS_CHILDREN) ? 2 * k * f : 0) + nc + (nb + 1) / 2;
+  return f * kt + (nb + nc + 1) / 2;
+}
+
+template <int KT>
+__device__ __forceinline__ int front_ops_early(const SolveArgs& a, int dir, bool use_perm, const TileRec& tr, int lane,
+                                               double* ops) {
+  if (dir != 0 || !FWD_STAGE<KT>) return 0;
+  const int k = a.k;
+  const int nc = tr.nc, f = tr.nc + tr.nb;
+  if (!use_perm)
+    for (int e = lane; e < nc * k; e += 32) cp_async8(ops + e, a.bperm + (int64_t)tr.first * k + e);
+  double* d = ops + k * nc;
+  if (tr.link & LINK_HAS_CHILDREN) {
+    for (int r = 0; r < k; ++r)
+      for (int row = lane; row < f; row += 32) {
+        const double* s = a.wbuf + tr.w_off + row + (int64_t)r * a.sumf;
+        cp_async8(d + r * f + row, s);
+        cp_async8(d + (k + r) * f + row, s + a.slab_stride);
+      }
+    d += 2 * k * f;
+  }
+  if (lane < nc) cp_async8(d + lane, a.dinv + tr.first + lane);
+  int* rel = reinterpret_cast<int*>(d + nc);
+  for (int i = lane; i < tr.nb; i += 32) cp_async4(rel + i, a.rel + tr.row_off + i);
+  return (use_perm && lane < nc) ? __ldg(&a.perm[tr.first + lane]) : 0;
+}
+
+template <int KT>
+__device__ __forceinline__ void front_ops_late(const SolveArgs& a, int dir, bool use_perm, const TileRec& tr, int lane,
+                                               double* ops, int po) {
+  const int nc = tr.nc, f = tr.nc + tr.nb;
+  if (dir == 0) {
+    if (FWD_STAGE<KT> && use_perm && lane < nc) {
+      const double* bp = a.B + (int64_t)po * a.brs;
+#pragma unroll
+      for (int r = 0; r < KT; ++r)
+        if (r < a.k) cp_async8(ops + lane * a.k + r, bp + (int64_t)r * a.bcs);
+    }
+  } else {
+    int* idx = reinterpret_cast<int*>(ops + f * KT);
+    for (int i = lane; i < tr.nb; i += 32) cp_async4(idx + i, a.sn_rows + tr.row_off + i);
+    if (lane < nc) cp_async4(idx + tr.nb + lane, a.perm + tr.first + lane);
+  }
+  cp_async_commit();
+}
+
+// acc[0:KT) = fma(m, s[0:KT), acc) with 16-byte shared loads, two right-hand sides each (s 16-byte aligned)
+template <int KT>
+__device__ __forceinline__ void fma_row(double m, const double* s, double* acc) {
+  static_assert(KT % 2 == 0, "the paired operand layout needs an even KT");
+  const double2* s2 = reinterpret_cast<const double2*>(s);
+#pragma unroll
+  for (int r = 0; r < KT / 2; ++r) {
+    const double2 q = s2[r];
+    acc[2 * r] = fma(m, q.x, acc[2 * r]);
+    acc[2 * r + 1] = fma(m, q.y, acc[2 * r + 1]);
+  }
+}
+
+// forward sweep of one front of a multi-column solve out of shared memory (buf = its panel, copy completion on `bar`).
+// ops = its staged operand block, or NULL (it did not fit in the ring): the operands are then loaded directly, in the
+// same summation order.  next_late() issues the late part of the next front's request once w1 is staged.
+template <int KT, class NextFn>
+__device__ __forceinline__ void front_forward(const SolveArgs& a, bool use_perm, const TileRec& tr, const double* buf,
+                                              unsigned long long* bar, unsigned parity, const double* ops, int lane,
+                                              double* stage, NextFn next_late) {
+  const int k = a.k;
+  const int nc = tr.nc, f = tr.nc + tr.nb;
+  const bool kids = (tr.link & LINK_HAS_CHILDREN) != 0;
+  const double* s0 = nullptr;    // the staged slabs, D^-1 and parent positions
+  const double* dv = nullptr;
+  const int* rel = nullptr;
+  if (ops) {
+    s0 = ops + k * nc;
+    dv = s0 + (kids ? 2 * k * f : 0);
+    rel = reinterpret_cast<const int*>(dv + nc);
+    cp_async_wait<0>();           // this front's copy group (the next front's early part is not committed yet)
+    __syncwarp();
+  }
+  // w1 entry of lane c: b + (s0 + s1) (+ overflow); stage[c][KT]
+  double v[KT];
+#pragma unroll
+  for (int r = 0; r < KT; ++r) v[r] = 0.0;
+  if (lane < nc) {
+    if (ops) {
+#pragma unroll
+      for (int r = 0; r < KT; ++r)
+        if (r < k) {
+          const double b = ops[lane * k + r];
+          v[r] = use_perm ? b : v[r] + b;
+          if (kids) v[r] += s0[r * f + lane] + s0[(k + r) * f + lane];
+        }
+      if (tr.link & LINK_HAS_OVF) ovf_add<KT>(a, tr.w_off + lane, v);
+    } else {
+      fwd_operand<KT>(a, use_perm, tr, lane, v);
+    }
+  }
+#pragma unroll
+  for (int r = 0; r < KT; ++r) stage[lane * KT + r] = v[r];
+  __syncwarp();
+  next_late();
+  mbar_wait(bar, parity);
+  const int ntile = (f + SOLVE_TILE - 1) / SOLVE_TILE;
+#pragma unroll 1
+  for (int t = 0; t < FRONT_TILES_MAX; ++t) {
+    if (t >= ntile) break;
+    const int row = t * SOLVE_TILE + lane;
+    double acc[KT];
+#pragma unroll
+    for (int r = 0; r < KT; ++r) acc[r] = 0.0;
+    if (row >= nc && row < f) {
+      if (!ops) {
+        child_add<KT>(a, tr.w_off + row, tr.link, acc);
+      } else if (kids) {
+#pragma unroll
+        for (int r = 0; r < KT; ++r)
+          if (r < k) acc[r] += s0[r * f + row] + s0[(k + r) * f + row];
+        if (tr.link & LINK_HAS_OVF) ovf_add<KT>(a, tr.w_off + row, acc);
+      }
+    }
+    const int cend = min(nc, (t + 1) * SOLVE_TILE);
+    const double* col = buf + min(row, f - 1);
+#pragma unroll 4
+    for (int c = 0; c < cend; ++c) fma_row<KT>(col[c * f], stage + c * KT, acc);
+    if (!ops) {
+      TileRec tt = tr;
+      tt.tile = t;
+      tile_store<KT>(a, 0, tt, lane, acc);
+    } else if (row < nc) {
+      double* y = a.ybuf + (int64_t)(tr.first + row) * k;
+      const double di = dv[row];
+#pragma unroll
+      for (int r = 0; r < KT; ++r)
+        if (r < k) y[r] = di * acc[r];
+    } else if (row < f) {
+      const int sl = (int)((tr.link >> LINK_SLAB_SHIFT) & 0xff);
+      const int64_t dst = sl < 2 ? sl * a.slab_stride + (tr.link & LINK_WOFF_MASK) + rel[row - nc]
+                                 : 2 * a.slab_stride + tr.w_off + row;
+      double* w = a.wbuf + dst;
+#pragma unroll
+      for (int r = 0; r < KT; ++r)
+        if (r < k) w[(int64_t)r * a.sumf] = acc[r];
+    }
+  }
+}
+
+// backward sweep of one front of a multi-column solve: x1 = S^T [z1 ; x2], lane = pivot column (nc <= 32).  The
+// indices arrived with the previous front; the values go into v[f][KT] with one gather, while the next front's
+// indices are requested, and the product runs over all f rows out of shared memory.
+template <int KT, class NextFn>
+__device__ __forceinline__ void front_backward(const SolveArgs& a, const TileRec& tr, const double* buf,
+                                               unsigned long long* bar, unsigned parity, double* ops, int lane,
+                                               NextFn next_late) {
+  const int k = a.k;
+  const int nc = tr.nc, f = tr.nc + tr.nb;
+  const int* idx = reinterpret_cast<const int*>(ops + f * KT);
+  cp_async_wait<0>();
+  __syncwarp();
+  for (int i = lane; i < f; i += 32) {
+    const double* src = i < nc ? a.ybuf + (int64_t)(tr.first + i) * k : a.xperm + (int64_t)idx[i - nc] * k;
+#pragma unroll
+    for (int r = 0; r < KT; ++r)
+      if (r < k) cp_async8(ops + i * KT + r, src + r);
+  }
+  cp_async_commit();
+  next_late();
+  cp_async_wait<1>();             // the gather (the next front's indices may stay in flight)
+  __syncwarp();
+  mbar_wait(bar, parity);
+  double acc[KT];
+#pragma unroll
+  for (int r = 0; r < KT; ++r) acc[r] = 0.0;
+  const double* colp = buf + min(lane, nc - 1);
+#pragma unroll 4
+  for (int j = 0; j < f; ++j) fma_row<KT>(colp[j * nc], ops + j * KT, acc);
+  if (lane < nc) {
+    double* xp = a.xperm + (int64_t)(tr.first + lane) * k;
+    double* xo = a.X + (int64_t)idx[tr.nb + lane] * a.xrs;
+#pragma unroll
+    for (int r = 0; r < KT; ++r)
+      if (r < k) { xp[r] = acc[r]; xo[(int64_t)r * a.xcs] = acc[r]; }
+  }
 }
 
 constexpr int FRONT_DEPTH = 2;   // panel copies in flight per warp
@@ -626,21 +764,23 @@ constexpr int FRONT_DEPTH = 2;   // panel copies in flight per warp
 // Every front of this CTA's slot that belongs to this warp (front te = T0(level) + warp + 16 j), level by level
 // with a CTA barrier between levels.  The PANEL copies run ahead of the computation by up to FRONT_DEPTH fronts
 // and across level boundaries (panels do not depend on computed data): a FIFO of variable-size allocations in the
-// warp's ring buffer, one mbarrier per FIFO position.  PIPE: the OPERANDS (right-hand side, child updates, D^-1, row
-// positions) are requested one front ahead into registers.
-template <int KT, bool PIPE>
+// warp's ring buffer, one mbarrier per FIFO position.  The OPERANDS (right-hand side, child updates, D^-1, row
+// positions; backward: row indices) are requested one front ahead, for the warp's next front of the SAME level only
+// (the next level's depend on this level's results): into registers for k = 1 (FrontOps), into the front's ring
+// allocation behind its panel in the backward sweep of k >= 2 and the forward sweep of k = 2 (FWD_STAGE).
+template <int KT>
 __device__ __forceinline__ void fronts_phase(const SolveArgs& a, int dir, bool use_perm, int nl, const int* s_tab, int tb,
                                              int nrec, const int4* s_rec, int lane, int warp, double* stage, char* ring,
                                              int ring_w, unsigned long long* bars, int* s_q) {
-  // the backward sweep of a multi-column solve is faster on the tile path (measured: k = 10, 95 vs 103 us at C2)
-  const bool front_ok = dir == 0 || KT == 1;
+  constexpr bool K1 = KT == 1;
   const double* panels = dir == 0 ? a.sfwd : a.sbwd;
   auto record = [&](int te) {
     const int q = te - tb;
     return q < nrec ? unpack_tile(s_rec[3 * q], s_rec[3 * q + 1], s_rec[3 * q + 2]) : load_tile(a.tiles + te);
   };
-  auto fits = [&](const TileRec& t, unsigned b) {
-    return front_ok && t.nc <= 32 && (int)b <= ring_w && t.nc + t.nb <= (PIPE ? FRONT_RT : FRONT_TILES_MAX) * SOLVE_TILE;
+  auto panel_bytes = [](const TileRec& t) { return (int)solve_panel_doubles(t.nc + t.nb, t.nc) * 8; };
+  auto fits = [&](const TileRec& t, int b) {
+    return t.nc <= 32 && b <= min(ring_w, FRONT_PANEL_MAX) && t.nc + t.nb <= (K1 ? FRONT_RT : FRONT_TILES_MAX) * SOLVE_TILE;
   };
   auto level_of = [&](int ll) { return dir == 0 ? ll : nl - 1 - ll; };
   // producer cursor (pl, pte): next front whose panel copy has not been requested yet
@@ -652,38 +792,56 @@ __device__ __forceinline__ void fronts_phase(const SolveArgs& a, int dir, bool u
     }
   };
   p_skip();
-  int qh = 0, qn = 0;             // FIFO head position and occupancy; entry e: s_q[2e] = offset (-1: no copy), s_q[2e+1] = bytes
+  // FIFO head position and occupancy; entry e: s_q[2e] = offset (-1: tile path), s_q[2e+1] = bytes allocated (more than
+  // the panel: the operand block follows it)
+  int qh = 0, qn = 0;
   unsigned par = 0;               // parity bit per FIFO position
   int last_end = 0;               // end of the newest allocation
   auto produce = [&]() {
     while (qn < FRONT_DEPTH && pl < nl) {
       const TileRec t = record(pte);
-      const unsigned b = (unsigned)solve_panel_doubles(t.nc + t.nb, t.nc) * 8u;
+      const int b = panel_bytes(t);
       const int e = (qh + qn) % FRONT_DEPTH;
-      int off = -1;
+      int off = -1, len = b;
       if (fits(t, b)) {
+        if (!K1 && (dir == 1 || FWD_STAGE<KT>)) {
+          // staged operands.  A forward front whose operands do not fit loads them directly, a backward one takes the
+          // tile path (both paths of the backward sweep sum in the same order).
+          const int ob = b + front_ops_doubles(t, dir, a.k, KT) * 8;
+          if (ob <= ring_w) len = ob;
+          else if (dir) len = -1;
+        }
+      } else {
+        len = -1;
+      }
+      if (len >= 0) {
         off = (last_end + 127) & ~127;
-        if (off + (int)b > ring_w) off = 0;
+        if (off + len > ring_w) off = 0;
         bool clash = false;
         for (int i = 0; i < qn; ++i) {
           const int ei = (qh + i) % FRONT_DEPTH;
           const int o = s_q[2 * ei], l = s_q[2 * ei + 1];
-          if (o >= 0 && off < o + l && o < off + (int)b) clash = true;
+          if (o >= 0 && off < o + l && o < off + len) clash = true;
         }
         if (clash) return;         // no room yet: try again after the next front has been consumed
-        if (lane == 0) bulk_load(ring + off, panels + t.soff, b, &bars[e]);
-        last_end = off + (int)b;
+        if (lane == 0) bulk_load(ring + off, panels + t.soff, (unsigned)b, &bars[e]);
+        last_end = off + len;
       }
       __syncwarp();
-      if (lane == 0) { s_q[2 * e] = off; s_q[2 * e + 1] = (int)b; }
+      if (lane == 0) { s_q[2 * e] = off; s_q[2 * e + 1] = len; }
       __syncwarp();
       ++qn;
       pte += SOLVE_WARPS;
       p_skip();
     }
   };
+  // operand block of FIFO entry e holding front t, or NULL
+  auto ops_of = [&](int e, const TileRec& t) -> double* {
+    const int o = s_q[2 * e], b = panel_bytes(t);
+    return (o >= 0 && s_q[2 * e + 1] > b) ? reinterpret_cast<double*>(ring + o + b) : nullptr;
+  };
   produce();
-  FrontOps<PIPE ? KT : 1> ops, nops;
+  FrontOps ops, nops;
   bool ops_ready = false;
   for (int ll = 0; ll < nl; ++ll) {
     const int l = level_of(ll);
@@ -692,22 +850,38 @@ __device__ __forceinline__ void fronts_phase(const SolveArgs& a, int dir, bool u
       TileRec tr = record(te);
       const int off = s_q[2 * qh];
       const unsigned parity = (par >> qh) & 1u;
-      if constexpr (PIPE) {
-        if (off >= 0 && !ops_ready) front_request<KT>(a, dir, use_perm, tr, lane, ops);
-      }
+      double* cur = nullptr;      // k >= 2: this front's staged operands
       bool nops_ready = false;
-      if constexpr (PIPE) {
+      if constexpr (K1) {
+        if (off >= 0 && !ops_ready) front_request(a, dir, use_perm, tr, lane, ops);
         // operands of this warp's next front of the SAME level (the next level's depend on this level's results)
         if (te + SOLVE_WARPS < t1) {
           const TileRec nt = record(te + SOLVE_WARPS);
-          if (fits(nt, (unsigned)solve_panel_doubles(nt.nc + nt.nb, nt.nc) * 8u)) {
-            front_request<KT>(a, dir, use_perm, nt, lane, nops);
+          if (fits(nt, panel_bytes(nt))) {
+            front_request(a, dir, use_perm, nt, lane, nops);
             nops_ready = true;
           }
         }
+      } else {
+        cur = ops_of(qh, tr);
+        if (cur && !ops_ready) front_ops_late<KT>(a, dir, use_perm, tr, lane, cur, front_ops_early<KT>(a, dir, use_perm, tr, lane, cur));
       }
+      // k >= 2: the next front of the same level, if its FIFO entry already holds an operand block
+      double* nxt = nullptr;
+      int npo = 0;
+      if (!K1 && te + SOLVE_WARPS < t1 && qn >= 2) {
+        const TileRec nt = record(te + SOLVE_WARPS);
+        nxt = ops_of((qh + 1) % FRONT_DEPTH, nt);
+        if (nxt) npo = front_ops_early<KT>(a, dir, use_perm, nt, lane, nxt);
+      }
+      auto next_late = [&]() {      // (the record is read again: it would hold 12 registers across the front)
+        if (nxt) front_ops_late<KT>(a, dir, use_perm, record(te + SOLVE_WARPS), lane, nxt, npo);
+        else cp_async_commit();   // an empty group: front_backward waits for all but the newest
+      };
       if (off < 0) {
-        // ---- tile path (global loads), every 32-output tile of the front
+        // ---- tile path (global loads), every 32-output tile of the front.  Panel loads in flight per lane: 8, 16 at
+        // KT = 4, what the register budget left by the staged front paths allows.  Spill stores (ptxas, sm_100a) at
+        // KT = 4 / 6 / 8 / 10: 20 / 0 / 24 / 20 bytes with 8, 8 / 16 / 20 / 92 with 16
         const int nc = tr.nc, f = tr.nc + tr.nb;
         const int ntile = ((dir == 0 ? f : nc) + SOLVE_TILE - 1) / SOLVE_TILE;
         for (int t = 0; t < ntile; ++t) {
@@ -716,21 +890,27 @@ __device__ __forceinline__ void fronts_phase(const SolveArgs& a, int dir, bool u
 #pragma unroll
           for (int r = 0; r < KT; ++r) acc[r] = 0.0;
           NoWait nw;
-          tile_compute<KT, (KT <= 2 ? 8 : DefaultMC<KT>::value)>(a, dir, use_perm, tr, lane, 0, 1, stage, acc, nw);
+          tile_compute<KT, (KT == 4 ? DefaultMC<KT>::value : 8)>(a, dir, use_perm, tr, lane, 0, 1, stage, acc, nw);
           tile_store<KT>(a, dir, tr, lane, acc);
         }
+        if constexpr (!K1) next_late();
       } else {
-        front_compute<KT, PIPE>(a, dir, use_perm, tr, reinterpret_cast<const double*>(ring + off), &bars[qh], parity, ops,
-                                lane, stage);
+        const double* buf = reinterpret_cast<const double*>(ring + off);
+        if constexpr (K1) front_compute_k1(a, dir, tr, buf, &bars[qh], parity, ops, lane, stage);
+        else if (dir == 0) front_forward<KT>(a, use_perm, tr, buf, &bars[qh], parity, FWD_STAGE<KT> ? cur : nullptr, lane, stage,
+                                             next_late);
+        else front_backward<KT>(a, tr, buf, &bars[qh], parity, cur, lane, next_late);
         par ^= 1u << qh;
       }
       __syncwarp();               // every lane is done with the allocation before it can be reused
       qh = (qh + 1) % FRONT_DEPTH;
       --qn;
       produce();
-      if constexpr (PIPE) {
+      if constexpr (K1) {
         ops = nops;
         ops_ready = nops_ready;
+      } else {
+        ops_ready = nxt != nullptr;
       }
     }
     ops_ready = false;
@@ -741,13 +921,14 @@ __device__ __forceinline__ void fronts_phase(const SolveArgs& a, int dir, bool u
 // A subtree phase in FRONT MODE as its own (ordinary, non-cooperative) launch: one CTA per slot.  The forward one
 // is the first thing a solve does, the backward one the last, so stream order replaces the grid barrier; the kernel
 // gets its own register / shared-memory budget (panel ring) and the level kernel keeps its L1.  The operands of the next
-// front are prefetched into registers for k = 1 only: wider ones do not fit the 128-register budget of a 16-warp CTA.
+// front are prefetched into registers for k = 1 and into the panel ring (cp.async) for k >= 2 (forward sweep: k = 2
+// only): wider operands do not fit the 128-register budget of a 16-warp CTA.
 template <int KT>
 __global__ void __launch_bounds__(SOLVE_WARPS * 32, 1) subtree_kernel(SolveArgs a, int p) {
-  extern __shared__ double smem[];
+  extern __shared__ __align__(16) double smem[];
   __shared__ int s_tab[MAX_SUB_LEVELS];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  double* stage = smem + warp * (32 * KT);                 // [KT][32] per warp
+  double* stage = smem + warp * (32 * KT);                 // [KT][32] (tile path) or [32][KT] (front mode) per warp
   char* ring_all = reinterpret_cast<char*>(smem + SOLVE_WARPS * 32 * KT);
   unsigned long long* mbar_all = reinterpret_cast<unsigned long long*>(ring_all + (size_t)SOLVE_WARPS * a.ring_w);
   int* s_q = reinterpret_cast<int*>(mbar_all + FRONT_DEPTH * SOLVE_WARPS) + 2 * FRONT_DEPTH * warp;
@@ -774,8 +955,8 @@ __global__ void __launch_bounds__(SOLVE_WARPS * 32, 1) subtree_kernel(SolveArgs 
       for (int e = threadIdx.x; e < 3 * nrec; e += blockDim.x) s_rec[e] = __ldg(src + e);
     }
     __syncthreads();
-    fronts_phase<KT, KT == 1>(a, dir, use_perm, nl, s_tab, tb, nrec, s_rec, lane, warp, stage,
-                              ring_all + (size_t)warp * a.ring_w, a.ring_w, bars, s_q);
+    fronts_phase<KT>(a, dir, use_perm, nl, s_tab, tb, nrec, s_rec, lane, warp, stage,
+                     ring_all + (size_t)warp * a.ring_w, a.ring_w, bars, s_q);
   }
   if (use_perm) permute_rhs(a, (int64_t)blockIdx.x * blockDim.x + threadIdx.x, (int64_t)gridDim.x * blockDim.x);
   if (a.times && blockIdx.x == 0 && threadIdx.x == 0) {
@@ -1318,7 +1499,7 @@ int configure(int slot) {
   const size_t budget = 227 * 1024 - 1024;
   c.rec_cap = KT <= 4 ? 512 : 256;
   size_t ring = (budget - stage_s - 2 * FRONT_DEPTH * NW * 8 - (size_t)c.rec_cap * 48) / NW;
-  ring = std::min<size_t>(ring, 10240) / 256 * 256;
+  ring = std::min<size_t>(ring, 16384) / 256 * 256;   // the launches that stage no operands use FRONT_PANEL_MAX of it
   c.ring_w = (int)ring;
   c.smem_sub = stage_s + ring * NW + 2 * FRONT_DEPTH * NW * 8 + (size_t)c.rec_cap * 48;
   EIGD_CUDA(cudaFuncSetAttribute(subtree_kernel<KT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c.smem_sub));
@@ -1338,7 +1519,6 @@ int launch_solve(int slot, eigd_factor* f, SolveArgs& a) {
   a.cnt = f->cnt;
   a.deps = f->h->solve.deps;
   a.dep_ovf = f->h->solve.dep_ovf;
-  a.ring_w = c.ring_w;
   a.lring_w = c.lring_w;
   a.rec_cap = c.rec_cap;
   // the subtree phases (a plan with a cut: the first and the last phase) run as their own launches in front of / behind
@@ -1348,11 +1528,18 @@ int launch_solve(int slot, eigd_factor* f, SolveArgs& a) {
   a.p_end = sub ? np - 1 : np;
   a.bar_base = f->bar_base;
   a.epoch = 0;
-  if (sub) {
-    subtree_kernel<KT><<<hp[0].level, SOLVE_WARPS * 32, c.smem_sub, g_eigd_stream>>>(a, 0);
+  // a subtree launch that stages operands in its ring (the backward one for KT >= 2, the forward one for KT = 2) gets the
+  // whole ring; the others only hold panels, which FRONT_PANEL_MAX bounds, and leave the rest of the SM's shared memory
+  // to L1
+  auto subtree_launch = [&](int p, bool staged) -> int {
+    a.ring_w = staged ? c.ring_w : std::min(c.ring_w, FRONT_PANEL_MAX);
+    const size_t smem = c.smem_sub - (size_t)SOLVE_WARPS * (c.ring_w - a.ring_w);
+    subtree_kernel<KT><<<hp[p].level, SOLVE_WARPS * 32, smem, g_eigd_stream>>>(a, p);
     EIGD_CUDA(cudaGetLastError());
     ++g_eigd_launches;
-  }
+    return 0;
+  };
+  if (sub && (rc = subtree_launch(0, FWD_STAGE<KT>))) return rc;
   if (a.p_end > a.p_begin) {
     a.epoch = ++f->epoch;            // one epoch per cooperative launch: the completion counters never reset
     // the one grid barrier: behind phase 0 of a plan without subtree phases (solve_kernel)
@@ -1363,11 +1550,7 @@ int launch_solve(int slot, eigd_factor* f, SolveArgs& a) {
     ++g_eigd_launches;
     f->bar_base += (unsigned long long)nbar * (unsigned long long)c.grid;
   }
-  if (sub) {
-    subtree_kernel<KT><<<hp[np - 1].level, SOLVE_WARPS * 32, c.smem_sub, g_eigd_stream>>>(a, np - 1);
-    EIGD_CUDA(cudaGetLastError());
-    ++g_eigd_launches;
-  }
+  if (sub && (rc = subtree_launch(np - 1, KT >= 2))) return rc;
   return 0;
 }
 
