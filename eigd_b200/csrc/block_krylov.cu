@@ -17,159 +17,25 @@
 //     BW  = B W,  G = W^T BW = R1^T R1,  W <- W R1^-1, BW <- BW R1^-1      (Cholesky QR ...
 //     G2  = W^T BW = R2^T R2,  W <- W R2^-1, BW <- BW R2^-1                 ... twice: orthonormal to rounding)
 //     V[m : m+P] = W, BV[m : m+P] = BW;  A_j = (H1 + H2)[j : j+P] (diagonal block), R_j = R2 R1 (sub-diagonal block)
-// The small P x P factorisations run in one warp on the device (no host round trip inside a cycle).
+// Everything after the solve is ONE cooperative launch per step (block_step_kernel: CTAs own 1024-element chunks of n,
+// software grid barriers only where a dot product crosses CTAs, bitwise-reproducible fixed-order sums); the small
+// P x P factorisations run in one thread of every CTA (no host round trip inside a cycle).
 //
 // Storage as in krylov.cu: V and BV are (ncv + P) x n row-major (one vector per row, leading dimension ld).
 #include "common.cuh"
 #include "../../include/eigd_b200.h"
 
-#include <cstdlib>
+#include <algorithm>
 
 namespace {
 
 constexpr int BK_THREADS = 256;
+constexpr int BK_WARPS = BK_THREADS / 32;
 constexpr int BK_EPT = 4;                        // elements per thread and chunk
 constexpr int BK_CHUNK = BK_THREADS * BK_EPT;
-constexpr int BK_ROWS = 4;                       // basis rows in flight per thread
 constexpr int BK_JMAX = 128;                     // basis vectors per launch
 constexpr int BK_PMAX = 4;
-
-__device__ unsigned int g_block_ticket = 0;
-
-// out[a * P + c] = sum_i Vb[a][i] * W[c][i]  (a < j rows of the basis, c < P new vectors, W rows at W + c * ldw).
-// CTA-strided chunks of 1024 elements: the P vectors' entries live in registers, BK_ROWS basis rows are streamed at a
-// time; per-warp partial sums accumulate in shared memory, per-CTA partials go to `partial`, the last CTA to finish
-// (ticket) adds them in a fixed order -- bitwise reproducible, one launch.
-template <int P>
-__device__ void block_chol(const double* __restrict__ G, double* __restrict__ Rinv, double* __restrict__ Racc, int pass);
-
-// chol_pass >= 0 (Gram-matrix call, j == P): the last CTA also factors the P x P result (block_chol) -- one launch less
-// per Cholesky-QR pass.
-template <int P>
-__global__ void __launch_bounds__(BK_THREADS)
-block_dots_kernel(int64_t n, int j, const double* __restrict__ Vb, int64_t ldv, const double* __restrict__ W, int64_t ldw,
-                  double* __restrict__ partial, double* __restrict__ out, unsigned int* __restrict__ ticket, int chol_pass,
-                  double* __restrict__ Rinv, double* __restrict__ Racc) {
-  extern __shared__ double red[];                // [BK_THREADS / 32][j * P]
-  __shared__ bool last;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int JP = j * P;
-  for (int e = tid; e < (BK_THREADS / 32) * JP; e += BK_THREADS) red[e] = 0.0;
-  __syncthreads();
-  double* myred = red + warp * JP;
-  for (int64_t c0 = (int64_t)blockIdx.x * BK_CHUNK; c0 < n; c0 += (int64_t)gridDim.x * BK_CHUNK) {
-    const int64_t i0 = c0 + tid;
-    double wv[P][BK_EPT];
-#pragma unroll
-    for (int c = 0; c < P; ++c)
-#pragma unroll
-      for (int q = 0; q < BK_EPT; ++q) {
-        const int64_t i = i0 + (int64_t)q * BK_THREADS;
-        wv[c][q] = (i < n) ? W[(int64_t)c * ldw + i] : 0.0;
-      }
-    for (int a0 = 0; a0 < j; a0 += BK_ROWS) {
-      double v[BK_ROWS][BK_EPT];
-#pragma unroll
-      for (int r = 0; r < BK_ROWS; ++r) {
-        const double* row = Vb + (int64_t)min(a0 + r, j - 1) * ldv;
-#pragma unroll
-        for (int q = 0; q < BK_EPT; ++q) {
-          const int64_t i = i0 + (int64_t)q * BK_THREADS;
-          v[r][q] = (i < n) ? __ldg(row + i) : 0.0;
-        }
-      }
-#pragma unroll
-      for (int r = 0; r < BK_ROWS; ++r)
-#pragma unroll
-        for (int c = 0; c < P; ++c) {
-          double s = 0.0;
-#pragma unroll
-          for (int q = 0; q < BK_EPT; ++q) s = fma(v[r][q], wv[c][q], s);
-          s = warp_sum(s);
-          if (lane == 0 && a0 + r < j) myred[(a0 + r) * P + c] += s;
-        }
-    }
-  }
-  __syncthreads();
-  for (int e = tid; e < JP; e += BK_THREADS) {
-    double s = 0.0;
-#pragma unroll
-    for (int g = 0; g < BK_THREADS / 32; ++g) s += red[g * JP + e];
-    partial[(int64_t)blockIdx.x * JP + e] = s;
-  }
-  __threadfence();
-  __syncthreads();
-  if (tid == 0) last = (atomicAdd(ticket, 1u) == gridDim.x - 1);
-  __syncthreads();
-  if (!last) return;
-  __threadfence();
-  const int ncta = gridDim.x;
-  for (int e = warp; e < JP; e += BK_THREADS / 32) {      // one warp per output, lanes stride over the CTAs
-    double s = 0.0;
-    for (int c = lane; c < ncta; c += 32) s += __ldcg(partial + (int64_t)c * JP + e);
-    s = warp_sum(s);
-    if (lane == 0) out[e] = s;
-  }
-  if (tid == 0) *ticket = 0u;
-  if (chol_pass >= 0) {
-    __syncthreads();
-    if (tid == 0) block_chol<P>(out, Rinv, Racc, chol_pass);
-  }
-}
-
-// W[c][i] += sign * sum_a H[a * P + c] * Vb[a][i]
-// H1 / Aout / jblk (second Gram-Schmidt pass only, else NULL): CTA 0 also writes the diagonal block of the projected
-// operator, Aout = (H1 + H)[jblk : jblk + P].
-template <int P>
-__global__ void __launch_bounds__(BK_THREADS)
-block_axpy_kernel(int64_t n, int j, const double* __restrict__ Vb, int64_t ldv, const double* __restrict__ H, double sign,
-                  double* __restrict__ W, int64_t ldw, const double* __restrict__ H1, double* __restrict__ Aout, int jblk) {
-  extern __shared__ double hs[];                 // [j * P]
-  const int tid = threadIdx.x;
-  if (Aout && blockIdx.x == 0 && tid < P * P) Aout[tid] = H1[jblk * P + tid] + H[jblk * P + tid];
-  for (int e = tid; e < j * P; e += BK_THREADS) hs[e] = sign * H[e];
-  __syncthreads();
-  for (int64_t c0 = (int64_t)blockIdx.x * BK_CHUNK; c0 < n; c0 += (int64_t)gridDim.x * BK_CHUNK) {
-    const int64_t i0 = c0 + tid;
-    double acc[P][BK_EPT];
-#pragma unroll
-    for (int c = 0; c < P; ++c)
-#pragma unroll
-      for (int q = 0; q < BK_EPT; ++q) {
-        const int64_t i = i0 + (int64_t)q * BK_THREADS;
-        acc[c][q] = (i < n) ? W[(int64_t)c * ldw + i] : 0.0;
-      }
-    for (int a0 = 0; a0 < j; a0 += BK_ROWS) {
-      double v[BK_ROWS][BK_EPT];
-#pragma unroll
-      for (int r = 0; r < BK_ROWS; ++r) {
-        const double* row = Vb + (int64_t)min(a0 + r, j - 1) * ldv;
-#pragma unroll
-        for (int q = 0; q < BK_EPT; ++q) {
-          const int64_t i = i0 + (int64_t)q * BK_THREADS;
-          v[r][q] = (i < n) ? __ldg(row + i) : 0.0;
-        }
-      }
-#pragma unroll
-      for (int r = 0; r < BK_ROWS; ++r) {
-        if (a0 + r >= j) break;
-#pragma unroll
-        for (int c = 0; c < P; ++c) {
-          const double h = hs[(a0 + r) * P + c];
-#pragma unroll
-          for (int q = 0; q < BK_EPT; ++q) acc[c][q] = fma(h, v[r][q], acc[c][q]);
-        }
-      }
-    }
-#pragma unroll
-    for (int c = 0; c < P; ++c)
-#pragma unroll
-      for (int q = 0; q < BK_EPT; ++q) {
-        const int64_t i = i0 + (int64_t)q * BK_THREADS;
-        if (i < n) W[(int64_t)c * ldw + i] = acc[c][q];
-      }
-  }
-}
+constexpr int BK_RMAX = BK_JMAX + BK_PMAX;       // basis rows a Gram-Schmidt pass can see
 
 // Cholesky G = R^T R of the P x P Gram matrix (row-major G[a * P + c]); writes the inverse Rinv (upper triangular,
 // row-major) for the scaling kernel and accumulates Racc <- R * Racc (Racc = identity on the first pass: pass 0).
@@ -232,25 +98,324 @@ __device__ void block_chol(const double* __restrict__ G, double* __restrict__ Ri
     for (int c = 0; c < P; ++c) Racc[a * P + c] = A[a][c] + bad;
 }
 
-// W <- W Rinv, BW <- BW Rinv (Rinv upper triangular, row-major); vectors are rows (W + c * ld)
+// ---- one block step as one cooperative launch ------------------------------------------------------------------
+// Every dot product keeps the summation order of the separate dots / reduce kernels this launch replaced, so the
+// results do not depend on the grid: a pass over J basis rows has the virtual grid gv = min(ceil(n / 1024), cap(J P));
+// virtual CTA v adds its chunks v, v + gv, ... (per thread a 4-term fma chain, warp_sum, per warp in chunk order),
+// then its 8 warps in order into partial[v]; an output is the lane-strided sum over the gv partials, then warp_sum.
+// A CTA runs the virtual CTAs blockIdx.x, blockIdx.x + gridDim.x, ...  Axpy, scaling and B W are per element or per
+// row and keep their own order (basis rows ascending, CSR order), whatever CTA computes them.
+struct StepArgs {
+  int64_t n, ld;
+  const double* V;            // basis V[0:m] and BV[0:m] (rows, leading dimension ld)
+  const double* BV;
+  double* W;                  // the new block V[m : m+P] (on entry: the solve's output) and BV[m : m+P]
+  double* BW;
+  int m, lo, j;               // local pass against rows lo .. m-1, full pass against 0 .. m-1; A_j = rows j .. j+P-1
+  int gs;                     // 0: start block (B W and the Cholesky QR only)
+  int split;                  // the two partial-sum regions overlap: one barrier more between reading and rewriting
+  int gv1, gv2, gvg;          // virtual grids of the local pass, the full pass and the P x P Gram matrices
+  double* part_a;             // partial sums of the local pass and of the first Gram matrix
+  double* part_b;             // partial sums of the full pass and of the second Gram matrix
+  double *H1, *H2, *Aout, *Rout, *scratch;
+  const int *bp, *bi;
+  const double* bv;
+  unsigned long long* ctr;
+  unsigned long long base;
+};
+
+// this thread's elements i0 + q * 256 of the P rows W[c * ld + i] (zero past n)
 template <int P>
-__global__ void __launch_bounds__(256)
-block_scale_kernel(int64_t n, const double* __restrict__ Rinv, double* __restrict__ W, double* __restrict__ BW, int64_t ld) {
-  __shared__ double x[P * P];
-  if (threadIdx.x < P * P) x[threadIdx.x] = Rinv[threadIdx.x];
-  __syncthreads();
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-    double w[P], b[P];
+__device__ __forceinline__ void load_block(double (&w)[P][BK_EPT], const double* W, int64_t ld, int64_t i0, int64_t n) {
 #pragma unroll
-    for (int c = 0; c < P; ++c) { w[c] = W[(int64_t)c * ld + i]; b[c] = BW[(int64_t)c * ld + i]; }
+  for (int c = 0; c < P; ++c)
+#pragma unroll
+    for (int q = 0; q < BK_EPT; ++q) {
+      const int64_t i = i0 + (int64_t)q * BK_THREADS;
+      w[c][q] = (i < n) ? __ldcg(W + (int64_t)c * ld + i) : 0.0;
+    }
+}
+
+template <int P>
+__device__ __forceinline__ void store_block(const double (&w)[P][BK_EPT], double* W, int64_t ld, int64_t i0, int64_t n) {
+#pragma unroll
+  for (int c = 0; c < P; ++c)
+#pragma unroll
+    for (int q = 0; q < BK_EPT; ++q) {
+      const int64_t i = i0 + (int64_t)q * BK_THREADS;
+      if (i < n) W[(int64_t)c * ld + i] = w[c][q];
+    }
+}
+
+template <int R>
+__device__ __forceinline__ void load_rows(double (&v)[R][BK_EPT], const double* __restrict__ Vb, int64_t ld, int a0,
+                                          int rows, int64_t i0, int64_t n) {
+#pragma unroll
+  for (int r = 0; r < R; ++r) {
+    const double* row = Vb + (int64_t)(a0 + r) * ld;
+    const bool ok = a0 + r < rows;
+#pragma unroll
+    for (int q = 0; q < BK_EPT; ++q) {
+      const int64_t i = i0 + (int64_t)q * BK_THREADS;
+      v[r][q] = (ok && i < n) ? __ldg(row + i) : 0.0;
+    }
+  }
+}
+
+// f(v, a0) on this thread's elements of the rows a0 .. a0 + R - 1 of Vb[0:rows], ascending; the loads of the next
+// group are issued before f runs on the current one (with one group per trip every trip waited for its own round trip)
+template <int R, class F>
+__device__ __forceinline__ void sweep_rows(const double* __restrict__ Vb, int64_t ld, int rows, int64_t i0, int64_t n, F&& f) {
+  double va[R][BK_EPT], vb[R][BK_EPT];
+  load_rows<R>(va, Vb, ld, 0, rows, i0, n);
+  for (int a0 = 0; a0 < rows; a0 += 2 * R) {
+    const int a1 = a0 + R;
+    if (a1 < rows) load_rows<R>(vb, Vb, ld, a1, rows, i0, n);
+    f(va, a0);
+    if (a1 >= rows) break;
+    if (a1 + R < rows) load_rows<R>(va, Vb, ld, a1 + R, rows, i0, n);
+    f(vb, a1);
+  }
+}
+
+// myred[(a0 + r) * P + c] += warp_sum(sum_q v[r][q] w[c][q]) for the rows a0 + r < rows
+template <int R, int P>
+__device__ __forceinline__ void dot_rows(const double (&v)[R][BK_EPT], const double (&w)[P][BK_EPT], int a0, int rows,
+                                         double* myred) {
+#pragma unroll
+  for (int r = 0; r < R; ++r) {
+    if (a0 + r >= rows) break;
+#pragma unroll
+    for (int c = 0; c < P; ++c) {
+      double s = 0.0;
+#pragma unroll
+      for (int q = 0; q < BK_EPT; ++q) s = fma(v[r][q], w[c][q], s);
+      s = warp_sum(s);
+      if ((threadIdx.x & 31) == 0) myred[(a0 + r) * P + c] += s;
+    }
+  }
+}
+
+// w[c][q] += hs[(a0 + r) * P + c] * v[r][q] for the rows a0 + r < rows (hs holds -H)
+template <int R, int P>
+__device__ __forceinline__ void axpy_rows(const double (&v)[R][BK_EPT], double (&w)[P][BK_EPT], int a0, int rows,
+                                          const double* hs) {
+#pragma unroll
+  for (int r = 0; r < R; ++r) {
+    if (a0 + r >= rows) break;
+#pragma unroll
+    for (int c = 0; c < P; ++c) {
+      const double h = hs[(a0 + r) * P + c];
+#pragma unroll
+      for (int q = 0; q < BK_EPT; ++q) w[c][q] = fma(h, v[r][q], w[c][q]);
+    }
+  }
+}
+
+// W <- W Rinv, BW <- BW Rinv (x = Rinv, upper triangular, row-major)
+template <int P>
+__device__ __forceinline__ void scale_block(double (&w)[P][BK_EPT], double (&b)[P][BK_EPT], const double* x) {
+#pragma unroll
+  for (int q = 0; q < BK_EPT; ++q)
 #pragma unroll
     for (int c = P - 1; c >= 0; --c) {
       double sw = 0.0, sb = 0.0;
 #pragma unroll
-      for (int t = 0; t <= c; ++t) { sw = fma(w[t], x[t * P + c], sw); sb = fma(b[t], x[t * P + c], sb); }
-      W[(int64_t)c * ld + i] = sw;
-      BW[(int64_t)c * ld + i] = sb;
+      for (int t = 0; t <= c; ++t) { sw = fma(w[t][q], x[t * P + c], sw); sb = fma(b[t][q], x[t * P + c], sb); }
+      w[c][q] = sw;
+      b[c][q] = sb;
     }
+}
+
+// b = B W on this thread's rows of the chunk (W of every row from global memory).  The four rows run in lock step,
+// two entries each per trip (all index loads, then all gathers); per row and column the products are added in CSR
+// order, as in spmm_kernel.
+template <int P>
+__device__ __forceinline__ void spmm_rows(double (&b)[P][BK_EPT], const int* __restrict__ bp, const int* __restrict__ bi,
+                                          const double* __restrict__ bv, const double* W, int64_t ld, int64_t i0, int64_t n) {
+  constexpr int U = 2;
+  int p[BK_EPT], e[BK_EPT];
+#pragma unroll
+  for (int q = 0; q < BK_EPT; ++q) {
+    const int64_t i = i0 + (int64_t)q * BK_THREADS;
+    p[q] = i < n ? bp[i] : 0;
+    e[q] = i < n ? bp[i + 1] : 0;
+#pragma unroll
+    for (int c = 0; c < P; ++c) b[c][q] = 0.0;
+  }
+  for (int t = 0;; t += U) {
+    int idx[BK_EPT][U];
+    double val[BK_EPT][U], x[BK_EPT][U][P];
+#pragma unroll
+    for (int q = 0; q < BK_EPT; ++q)
+#pragma unroll
+      for (int u = 0; u < U; ++u) {
+        const int pp = p[q] + t + u;
+        idx[q][u] = pp < e[q] ? bi[pp] : 0;
+        val[q][u] = pp < e[q] ? bv[pp] : 0.0;
+      }
+#pragma unroll
+    for (int q = 0; q < BK_EPT; ++q)
+#pragma unroll
+      for (int u = 0; u < U; ++u)
+#pragma unroll
+        for (int c = 0; c < P; ++c) x[q][u][c] = p[q] + t + u < e[q] ? __ldcg(W + (int64_t)c * ld + idx[q][u]) : 0.0;
+    bool more = false;
+#pragma unroll
+    for (int q = 0; q < BK_EPT; ++q) {
+#pragma unroll
+      for (int u = 0; u < U; ++u)
+        if (p[q] + t + u < e[q])
+#pragma unroll
+          for (int c = 0; c < P; ++c) b[c][q] = fma(val[q][u], x[q][u][c], b[c][q]);
+      more |= p[q] + t + U < e[q];
+    }
+    if (!more) break;
+  }
+#pragma unroll
+  for (int q = 0; q < BK_EPT; ++q)
+#pragma unroll
+    for (int c = 0; c < P; ++c) b[c][q] = fma(1.0, b[c][q], 0.0);       // Y = alpha acc + 0 of spmm_kernel
+}
+
+// The partial sums of one pass (see above): chunk(i0, myred) adds a chunk's dot products into this warp's row of red.
+template <class F>
+__device__ __forceinline__ void pass_partials(int gv, int64_t nch, int JP, double* red, double* partial, F&& chunk) {
+  const int tid = threadIdx.x;
+  for (int v = blockIdx.x; v < gv; v += gridDim.x) {
+    for (int e = tid; e < BK_WARPS * JP; e += BK_THREADS) red[e] = 0.0;
+    __syncthreads();
+    for (int64_t ch = v; ch < nch; ch += gv) chunk(ch * BK_CHUNK + tid, red + (tid >> 5) * JP);
+    __syncthreads();
+    for (int e = tid; e < JP; e += BK_THREADS) {
+      double s = 0.0;
+#pragma unroll
+      for (int g = 0; g < BK_WARPS; ++g) s += red[g * JP + e];
+      partial[(int64_t)v * JP + e] = s;
+    }
+    __syncthreads();
+  }
+}
+
+// output e of a pass (after a grid barrier): lanes stride over the gv partials, then warp_sum
+__device__ __forceinline__ double reduce_partial(const double* partial, int gv, int JP, int e) {
+  double s = 0.0;
+  for (int c = threadIdx.x & 31; c < gv; c += 32) s += __ldcg(partial + (int64_t)c * JP + e);
+  return warp_sum(s);
+}
+
+// every CTA reduces all JP outputs: hs[e] = sign * out[e], and out[e] to global memory when g is set
+__device__ __forceinline__ void reduce_all(const double* partial, int gv, int JP, double sign, double* hs, double* g) {
+  for (int e = threadIdx.x >> 5; e < JP; e += BK_WARPS) {
+    const double s = reduce_partial(partial, gv, JP, e);
+    if ((threadIdx.x & 31) == 0) {
+      hs[e] = sign * s;
+      if (g) g[e] = s;
+    }
+  }
+  __syncthreads();
+}
+
+// One block step after the P-column solve ('|' is a grid barrier):
+//   1. partial sums of H1 = BV[lo:m] W                                                                   |
+//   2. H1; W -= V[lo:m]^T H1 and, in the same sweep over the chunk, partial sums of H2 = BV[0:m] W       |
+//      H2, one warp per output across the grid                                                          |
+//   3. W -= V[0:m]^T H2 -> V[m : m+P]; A_j = (H1 + H2)[j : j+P]                                          |
+//   4. BW = B W -> BV[m : m+P]; partial sums of G1 = BW^T W                                              |
+//   5. R1 from G1 (every CTA); W, BW <- W, BW R1^-1; partial sums of G2                                 |
+//   6. R2 from G2; W, BW <- W, BW R2^-1; R_j = R2 R1
+// The start block runs stages 4 to 6.  W and BW are re-read from L2 in each stage (they are written by other CTAs'
+// stages; 2 P n doubles), V[0:m] and BV[0:m] stream from HBM once per pass.
+template <int P>
+__global__ void __launch_bounds__(BK_THREADS, 2) block_step_kernel(StepArgs a) {
+  __shared__ double red[BK_WARPS * BK_RMAX * P];
+  __shared__ double hs[BK_RMAX * P];
+  __shared__ double rinv[P * P], racc[P * P];
+  const int tid = threadIdx.x;
+  const int64_t n = a.n, ld = a.ld;
+  const int64_t nch = (n + BK_CHUNK - 1) / BK_CHUNK;
+  unsigned long long target = a.base;
+  auto grid_barrier = [&]() {
+    target += gridDim.x;
+    coop_grid_barrier(a.ctr, target);
+  };
+  constexpr int R = P <= 2 ? 4 : 2;           // basis rows per load group (see sweep_rows): registers of 2 CTAs per SM
+  using Rows = double[R][BK_EPT];
+  if (a.gs) {
+    const int J1 = a.m - a.lo, J2 = a.m;
+    const double* Vlo = a.V + (int64_t)a.lo * ld;
+    const double* BVlo = a.BV + (int64_t)a.lo * ld;
+    pass_partials(a.gv1, nch, J1 * P, red, a.part_a, [&](int64_t i0, double* myred) {
+      double w[P][BK_EPT];
+      load_block<P>(w, a.W, ld, i0, n);
+      sweep_rows<R>(BVlo, ld, J1, i0, n, [&](const Rows& v, int a0) { dot_rows<R, P>(v, w, a0, J1, myred); });
+    });
+    grid_barrier();
+    reduce_all(a.part_a, a.gv1, J1 * P, -1.0, hs, blockIdx.x == 0 ? a.H1 : nullptr);
+    if (a.split) grid_barrier();
+    pass_partials(a.gv2, nch, J2 * P, red, a.part_b, [&](int64_t i0, double* myred) {
+      double w[P][BK_EPT];
+      load_block<P>(w, a.W, ld, i0, n);
+      sweep_rows<R>(Vlo, ld, J1, i0, n, [&](const Rows& v, int a0) { axpy_rows<R, P>(v, w, a0, J1, hs); });
+      store_block<P>(w, a.W, ld, i0, n);
+      sweep_rows<R>(a.BV, ld, J2, i0, n, [&](const Rows& v, int a0) { dot_rows<R, P>(v, w, a0, J2, myred); });
+    });
+    grid_barrier();
+    for (int e = blockIdx.x * BK_WARPS + (tid >> 5); e < J2 * P; e += gridDim.x * BK_WARPS) {
+      const double s = reduce_partial(a.part_b, a.gv2, J2 * P, e);
+      if ((tid & 31) == 0) a.H2[e] = s;
+    }
+    grid_barrier();
+    for (int e = tid; e < J2 * P; e += BK_THREADS) hs[e] = -1.0 * __ldcg(a.H2 + e);
+    if (blockIdx.x == 0 && tid < P * P) a.Aout[tid] = __ldcg(a.H1 + (a.j - a.lo) * P + tid) + __ldcg(a.H2 + a.j * P + tid);
+    __syncthreads();
+    for (int64_t ch = blockIdx.x; ch < nch; ch += gridDim.x) {
+      const int64_t i0 = ch * BK_CHUNK + tid;
+      double w[P][BK_EPT];
+      load_block<P>(w, a.W, ld, i0, n);
+      sweep_rows<R>(a.V, ld, J2, i0, n, [&](const Rows& v, int a0) { axpy_rows<R, P>(v, w, a0, J2, hs); });
+      store_block<P>(w, a.W, ld, i0, n);
+    }
+    grid_barrier();
+  }
+  pass_partials(a.gvg, nch, P * P, red, a.part_a, [&](int64_t i0, double* myred) {
+    double w[P][BK_EPT], b[P][BK_EPT];
+    spmm_rows<P>(b, a.bp, a.bi, a.bv, a.W, ld, i0, n);
+    store_block<P>(b, a.BW, ld, i0, n);
+    load_block<P>(w, a.W, ld, i0, n);
+    dot_rows<P, P>(b, w, 0, P, myred);
+  });
+  grid_barrier();
+  reduce_all(a.part_a, a.gvg, P * P, 1.0, hs, blockIdx.x == 0 ? a.scratch : nullptr);
+  if (tid == 0) block_chol<P>(hs, rinv, racc, 0);
+  __syncthreads();
+  if (blockIdx.x == 0 && tid < P * P) a.scratch[P * P + tid] = rinv[tid];
+  if (a.split) grid_barrier();
+  pass_partials(a.gvg, nch, P * P, red, a.part_b, [&](int64_t i0, double* myred) {
+    double w[P][BK_EPT], b[P][BK_EPT];
+    load_block<P>(w, a.W, ld, i0, n);
+    load_block<P>(b, a.BW, ld, i0, n);
+    scale_block<P>(w, b, rinv);
+    store_block<P>(w, a.W, ld, i0, n);
+    store_block<P>(b, a.BW, ld, i0, n);
+    dot_rows<P, P>(b, w, 0, P, myred);
+  });
+  grid_barrier();
+  reduce_all(a.part_b, a.gvg, P * P, 1.0, hs, blockIdx.x == 0 ? a.scratch : nullptr);
+  if (tid == 0) block_chol<P>(hs, rinv, racc, 1);
+  __syncthreads();
+  if (blockIdx.x == 0 && tid < P * P) {
+    a.scratch[P * P + tid] = rinv[tid];
+    a.Rout[tid] = racc[tid];
+  }
+  for (int64_t ch = blockIdx.x; ch < nch; ch += gridDim.x) {
+    const int64_t i0 = ch * BK_CHUNK + tid;
+    double w[P][BK_EPT], b[P][BK_EPT];
+    load_block<P>(w, a.W, ld, i0, n);
+    load_block<P>(b, a.BW, ld, i0, n);
+    scale_block<P>(w, b, rinv);
+    store_block<P>(w, a.W, ld, i0, n);
+    store_block<P>(b, a.BW, ld, i0, n);
   }
 }
 
@@ -275,43 +440,41 @@ inline int ew_grid(int64_t n) {
   return (int)(g < 1 ? 1 : (g > 148 * 8 ? 148 * 8 : g));
 }
 
+// Launches block_step_kernel<P> for a (its grid, virtual grids, partial-sum regions and barrier base are set here).
+// work: the eigd_gemm_tn_workspace buffer, which bounds every virtual grid (gv x outputs must fit) as it bounded the
+// grids of the separate dots kernels.
 template <int P>
-int dots(int64_t n, int j, const double* Vb, int64_t ldv, const double* W, int64_t ldw, double* out, double* work,
-         int chol_pass = -1, double* Rinv = nullptr, double* Racc = nullptr) {
-  unsigned int* ticket = nullptr;
-  EIGD_CUDA(cudaGetSymbolAddress((void**)&ticket, g_block_ticket));
-  int64_t want = (n + BK_CHUNK - 1) / BK_CHUNK;
-  const int64_t cap = eigd_gemm_tn_workspace(32, 32) / ((int64_t)j * P);     // partial[grid][j * P] must fit the workspace
-  int grid = (int)(want < cap ? want : cap);
-  if (grid < 1) { eigd_set_error("block_dots: workspace too small"); return 8; }
-  const size_t smem = (size_t)(BK_THREADS / 32) * j * P * sizeof(double);
-  EIGD_LAUNCH(block_dots_kernel<P>, grid, BK_THREADS, smem, n, j, Vb, ldv, W, ldw, work, out, ticket, chol_pass, Rinv, Racc);
-  EIGD_CHECK_LAUNCH();
-  return 0;
-}
-
-template <int P>
-int axpy(int64_t n, int j, const double* Vb, int64_t ldv, const double* H, double sign, double* W, int64_t ldw,
-         const double* H1 = nullptr, double* Aout = nullptr, int jblk = 0) {
-  int64_t want = (n + BK_CHUNK - 1) / BK_CHUNK;
-  int grid = (int)(want < 148 * 16 ? want : 148 * 16);
-  EIGD_LAUNCH(block_axpy_kernel<P>, grid, BK_THREADS, (size_t)j * P * sizeof(double), n, j, Vb, ldv, H, sign, W, ldw, H1, Aout, jblk);
-  EIGD_CHECK_LAUNCH();
-  return 0;
-}
-
-// Cholesky QR (twice) of the P vectors W in the B inner product; BW = B W on entry and on exit; Racc <- R2 R1.
-// scratch: 2 * P * P doubles (Gram matrix, inverse factor)
-template <int P>
-int cholqr2(int64_t n, double* W, double* BW, int64_t ld, double* Racc, double* scratch, double* work) {
-  double* G = scratch;
-  double* Rinv = scratch + P * P;
+int block_step(StepArgs a, double* work) {
+  static int max_grid = 0;
   int rc;
-  for (int pass = 0; pass < 2; ++pass) {
-    if ((rc = dots<P>(n, P, BW, ld, W, ld, G, work, pass, Rinv, Racc))) return rc;   // G = BW^T W, factored by the last CTA
-    EIGD_LAUNCH(block_scale_kernel<P>, ew_grid(n), 256, 0, n, Rinv, W, BW, ld);
-    EIGD_CHECK_LAUNCH();
+  unsigned long long *ctr = nullptr, *base = nullptr;
+  if ((rc = coop_counter(&ctr, &base)) || (rc = coop_max_grid(block_step_kernel<P>, 1 << 20, 1 << 30, &max_grid))) return rc;
+  const int64_t ws = eigd_gemm_tn_workspace(32, 32);
+  const int64_t nch = (a.n + BK_CHUNK - 1) / BK_CHUNK;
+  auto vgrid = [&](int J) {
+    const int64_t cap = ws / ((int64_t)J * P);
+    return (int)(nch < cap ? nch : cap);
+  };
+  a.gvg = vgrid(P);
+  int64_t size_a = (int64_t)a.gvg * P * P, size_b = size_a;
+  if (a.gs) {
+    a.gv1 = vgrid(a.m - a.lo);
+    a.gv2 = vgrid(a.m);
+    if (a.gv2 < 1) { eigd_set_error("block_lanczos: workspace too small"); return 8; }
+    size_a = std::max(size_a, (int64_t)a.gv1 * (a.m - a.lo) * P);
+    size_b = std::max(size_b, (int64_t)a.gv2 * a.m * P);
   }
+  a.part_b = work;
+  a.part_a = work + (ws - size_a);
+  a.split = size_a + size_b > ws;
+  a.ctr = ctr;
+  a.base = *base;
+  const int grid = (int)(nch < max_grid ? nch : max_grid);
+  void* params[] = {(void*)&a};
+  EIGD_CUDA(cudaLaunchCooperativeKernel((void*)block_step_kernel<P>, dim3(grid), dim3(BK_THREADS), params, 0, g_eigd_stream));
+  ++g_eigd_launches;
+  const int barriers = (a.gs ? 6 : 2) + a.split * (a.gs ? 2 : 1);
+  *base += (unsigned long long)barriers * (unsigned long long)grid;
   return 0;
 }
 
@@ -321,12 +484,9 @@ int extend(eigd_factor* f, int refine, int n, const int* mp, const int* mi, cons
            double* H1, double* H2, double* scratch, double* work, double* work2) {
   int rc;
   int step = 0;
-  static int local_first = -1;          // EIGD_LANCZOS_LOCAL=0: two full passes (developer comparison runs)
-  if (local_first < 0) { const char* e = getenv("EIGD_LANCZOS_LOCAL"); local_first = e ? atoi(e) : 1; }
   for (int j = j0, m = m0; j < ncv; j += P, m += P, ++step) {
     const double* bvj = BV + (int64_t)j * ld;
     double* W = V + (int64_t)m * ld;
-    double* BW = BV + (int64_t)m * ld;
     // W = OP V_j = factor^{-1} (B V_j): the P vectors are rows (stride ld between vectors, 1 inside)
     if ((rc = eigd_factor_solve(f, bvj, 1, ld, W, 1, ld, P))) return rc;
     for (int it = 0; it < refine; ++it) {                        // X += F (B V_j - mat X)
@@ -343,26 +503,27 @@ int extend(eigd_factor* f, int refine, int n, const int* mp, const int* mi, cons
     // block being expanded and its predecessor (block three-term recurrence), or the whole basis in the first step
     // after a thick restart (the locked Ritz vectors: the arrow) -- then one FULL classical pass against V[0:m].  The
     // local pass takes out the large components (where the cancellation is), the full pass the O(eps)-relative ones
-    // left along the older vectors: full reorthogonalisation at half the basis traffic of two full passes.
-    const int lo = (step == 0 || local_first == 0) ? 0 : (j - P > 0 ? j - P : 0);
-    if ((rc = dots<P>(n, m - lo, BV + (int64_t)lo * ld, ld, W, ld, H1, work))) return rc;
-    if ((rc = axpy<P>(n, m - lo, V + (int64_t)lo * ld, ld, H1, -1.0, W, ld))) return rc;
-    if ((rc = dots<P>(n, m, BV, ld, W, ld, H2, work))) return rc;
-    // diagonal block A_j = (H1 + H2)[j : j + P]; H1 holds rows lo .. m-1
-    if ((rc = axpy<P>(n, m, V, ld, H2, -1.0, W, ld, H1 - (int64_t)lo * P, Ablk + (int64_t)step * P * P, j))) return rc;
-    // BW = B W, then orthonormalise the block
-    if ((rc = eigd_csr_spmm(n, bp, bi, bv, W, 1, ld, BW, 1, ld, P, 1.0, 0.0))) return rc;
-    if ((rc = cholqr2<P>(n, W, BW, ld, Rblk + (int64_t)step * P * P, scratch, work))) return rc;
+    // left along the older vectors: full reorthogonalisation at half the basis traffic of two full passes.  Then
+    // BW = B W and the Cholesky QR (twice) of the block, all in one launch.
+    StepArgs a{};
+    a.n = n; a.ld = ld; a.V = V; a.BV = BV; a.W = W; a.BW = BV + (int64_t)m * ld;
+    a.m = m; a.lo = step == 0 ? 0 : (j - P > 0 ? j - P : 0); a.j = j; a.gs = 1;
+    a.H1 = H1; a.H2 = H2; a.Aout = Ablk + (int64_t)step * P * P; a.Rout = Rblk + (int64_t)step * P * P; a.scratch = scratch;
+    a.bp = bp; a.bi = bi; a.bv = bv;
+    if ((rc = block_step<P>(a, work))) return rc;
   }
   return 0;
 }
 
+// scratch: 3 P x P (Gram matrix, inverse factor, R = R2 R1)
 template <int P>
 int start_block(int n, const int* bp, const int* bi, const double* bv, double* V, double* BV, int64_t ld, double* scratch,
                 double* work) {
-  int rc;
-  if ((rc = eigd_csr_spmm(n, bp, bi, bv, V, 1, ld, BV, 1, ld, P, 1.0, 0.0))) return rc;
-  return cholqr2<P>(n, V, BV, ld, scratch + 2 * P * P, scratch, work);
+  StepArgs a{};
+  a.n = n; a.ld = ld; a.V = V; a.BV = BV; a.W = V; a.BW = BV; a.gs = 0;
+  a.Rout = scratch + 2 * P * P; a.scratch = scratch;
+  a.bp = bp; a.bi = bi; a.bv = bv;
+  return block_step<P>(a, work);
 }
 
 }  // namespace

@@ -41,3 +41,36 @@ __device__ __forceinline__ double warp_sum(double v) {
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
   return v;
 }
+
+// ---- cooperative kernels with a software grid barrier (dense.cu mgs_sweep, block_krylov.cu block_step) ----
+// All of them share one monotonic arrival counter: every CTA adds 1 per barrier, so a launch on G CTAs with b
+// barriers adds b * G, and the next launch (stream-ordered) waits for targets counted from the new base.
+__device__ __forceinline__ void coop_grid_barrier(unsigned long long* ctr, unsigned long long target) {
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    unsigned long long v;
+    asm volatile("red.release.gpu.global.add.u64 [%0], 1;" ::"l"(ctr) : "memory");
+    do {
+      asm volatile("ld.acquire.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(ctr) : "memory");
+    } while (v < target);
+  }
+  __syncthreads();
+}
+
+// The counter of the current device (allocated and zeroed on first use) and the arrivals enqueued so far; the caller
+// adds its launch's barriers x grid to *base after the launch.  Defined in dense.cu.
+int coop_counter(unsigned long long** ctr, unsigned long long** base);
+
+// Largest co-resident grid of a 256-thread kernel: SMs x min(occupancy, per_sm), at most cap; computed once (*max_grid)
+template <class Kernel>
+static int coop_max_grid(Kernel kernel, int per_sm, int cap, int* max_grid) {
+  if (*max_grid > 0) return 0;
+  int dev = 0, sms = 0, occ = 0;
+  EIGD_CUDA(cudaGetDevice(&dev));
+  EIGD_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+  EIGD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, 256, 0));
+  if (occ < 1) { eigd_set_error("cooperative kernel does not fit on an SM"); return 7; }
+  int g = sms * (occ < per_sm ? occ : per_sm);
+  *max_grid = g > cap ? cap : g;
+  return 0;
+}

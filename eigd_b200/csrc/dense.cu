@@ -550,18 +550,6 @@ struct MgsArgs {
   double* H[MGS_MAX];
 };
 
-__device__ __forceinline__ void mgs_grid_barrier(unsigned long long* ctr, unsigned long long target) {
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    unsigned long long v;
-    asm volatile("red.release.gpu.global.add.u64 [%0], 1;" ::"l"(ctr) : "memory");
-    do {
-      asm volatile("ld.acquire.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(ctr) : "memory");
-    } while (v < target);
-  }
-  __syncthreads();
-}
-
 __global__ void __launch_bounds__(256)
 mgs_sweep_kernel(int64_t n, int k, int j, MgsArgs a, double* __restrict__ w, double* __restrict__ partial,
                  unsigned long long* ctr, unsigned long long base) {
@@ -598,7 +586,7 @@ mgs_sweep_kernel(int64_t n, int k, int j, MgsArgs a, double* __restrict__ w, dou
       for (int g = 0; g < RG; ++g) s += red[g * k + threadIdx.x];
       mine[threadIdx.x] = s;
     }
-    mgs_grid_barrier(ctr, base + (unsigned long long)(t + 1) * (unsigned long long)G);
+    coop_grid_barrier(ctr, base + (unsigned long long)(t + 1) * (unsigned long long)G);
     const double* all = partial + (int64_t)(t & 1) * G * k;
     double s = 0.0;
     if (on)
@@ -645,34 +633,21 @@ mgs_sweep_kernel(int64_t n, int k, int j, MgsArgs a, double* __restrict__ w, dou
   }
 }
 
-static unsigned long long* g_mgs_ctr = nullptr;
-static unsigned long long g_mgs_base = 0;
-static int g_mgs_dev = -1;
+static unsigned long long* g_coop_ctr = nullptr;
+static unsigned long long g_coop_base = 0;
+static int g_coop_dev = -1;
 
-// the monotonic arrival counter of the cooperative kernels of this file (stream-ordered launches: every launch adds
-// exactly barriers x grid arrivals, so the next launch starts from a known base)
-static int coop_counter_ready() {
+int coop_counter(unsigned long long** ctr, unsigned long long** base) {
   int dev = 0;
   EIGD_CUDA(cudaGetDevice(&dev));
-  if (dev != g_mgs_dev) {
-    EIGD_CUDA(cudaMalloc(&g_mgs_ctr, sizeof(unsigned long long)));
-    EIGD_CUDA(cudaMemsetAsync(g_mgs_ctr, 0, sizeof(unsigned long long), g_eigd_stream));
-    g_mgs_base = 0;
-    g_mgs_dev = dev;
+  if (dev != g_coop_dev) {
+    EIGD_CUDA(cudaMalloc(&g_coop_ctr, sizeof(unsigned long long)));
+    EIGD_CUDA(cudaMemsetAsync(g_coop_ctr, 0, sizeof(unsigned long long), g_eigd_stream));
+    g_coop_base = 0;
+    g_coop_dev = dev;
   }
-  return 0;
-}
-
-template <class Kernel>
-static int coop_max_grid(Kernel kernel, int per_sm, int cap, int* max_grid) {
-  if (*max_grid > 0) return 0;
-  int dev = 0, sms = 0, occ = 0;
-  EIGD_CUDA(cudaGetDevice(&dev));
-  EIGD_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-  EIGD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, 256, 0));
-  if (occ < 1) { eigd_set_error("cooperative kernel does not fit on an SM"); return 7; }
-  int g = sms * (occ < per_sm ? occ : per_sm);
-  *max_grid = g > cap ? cap : g;
+  *ctr = g_coop_ctr;
+  *base = &g_coop_base;
   return 0;
 }
 
@@ -685,7 +660,8 @@ extern "C" int eigd_mgs_sweep(int64_t n, int k, int j, const double* const* W, d
   int rc;
   // the two halves of the partial-sum buffer (2 x grid x k doubles) live in the reduction workspace
   const int cap = (int)(eigd_gemm_tn_workspace(TN_KMAX, TN_KMAX) / (2 * MGS_KMAX));
-  if ((rc = coop_counter_ready()) || (rc = coop_max_grid(mgs_sweep_kernel, per_sm, cap, &max_grid))) return rc;
+  unsigned long long *ctr = nullptr, *base = nullptr;
+  if ((rc = coop_counter(&ctr, &base)) || (rc = coop_max_grid(mgs_sweep_kernel, per_sm, cap, &max_grid))) return rc;
   const int RG = 256 / k;
   int64_t want = (n + (int64_t)RG * 4 - 1) / ((int64_t)RG * 4);
   int grid = (int)(want < 1 ? 1 : (want > max_grid ? max_grid : want));
@@ -695,11 +671,11 @@ extern "C" int eigd_mgs_sweep(int64_t n, int k, int j, const double* const* W, d
     for (int t = 0; t < jj; ++t) { a.W[t] = W[j0 + t]; a.H[t] = H[j0 + t]; }
     for (int t = jj; t < MGS_MAX; ++t) { a.W[t] = nullptr; a.H[t] = nullptr; }
     int64_t n_ = n; int k_ = k, jj_ = jj;
-    unsigned long long base = g_mgs_base;
-    void* params[] = {(void*)&n_, (void*)&k_, (void*)&jj_, (void*)&a, (void*)&d_w, (void*)&d_work, (void*)&g_mgs_ctr, (void*)&base};
+    unsigned long long base0 = *base;
+    void* params[] = {(void*)&n_, (void*)&k_, (void*)&jj_, (void*)&a, (void*)&d_w, (void*)&d_work, (void*)&ctr, (void*)&base0};
     EIGD_CUDA(cudaLaunchCooperativeKernel((void*)mgs_sweep_kernel, dim3(grid), dim3(256), params, 0, g_eigd_stream));
     ++g_eigd_launches;
-    g_mgs_base += (unsigned long long)jj * (unsigned long long)grid;
+    *base += (unsigned long long)jj * (unsigned long long)grid;
   }
   return 0;
 }
