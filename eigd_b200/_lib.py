@@ -48,6 +48,8 @@ SIGNATURES = {
     "eigd_factor_pivot_counts": (c_int, [c_ptr, c_ptr]),
     "eigd_dmma_peak": (c_int, [c_int, c_int, c_ptr]),
     "eigd_factor_solve": (c_int, [c_ptr, c_ptr, c_i64, c_i64, c_ptr, c_i64, c_i64, c_int]),
+    "eigd_factor_set_refinement": (c_int, [c_ptr, c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_int]),
+    "eigd_factor_apply": (c_int, [c_ptr, c_ptr, c_i64, c_i64, c_ptr, c_i64, c_i64, c_int]),
     "eigd_factor_bytes": (c_i64, [c_ptr]),
     "eigd_solve_timing_begin": (c_int, []),
     "eigd_solve_timing_end": (c_int, [c_ptr, c_ptr]),
@@ -55,13 +57,13 @@ SIGNATURES = {
     "eigd_solve_set_trace": (c_int, [c_ptr]),
     "eigd_solve_set_skew": (c_int, [c_ptr]),
     "eigd_solve_num_phases": (c_int, [c_ptr]),
-    "eigd_lanczos_extend": (c_int, [c_ptr, c_int, c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_int,
-                                    c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_int, c_ptr, c_ptr]),
+    "eigd_lanczos_extend": (c_int, [c_ptr, c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_int, c_int, c_ptr, c_ptr, c_ptr,
+                                    c_ptr, c_int, c_ptr]),
     "eigd_stored_assemble": (c_int, [c_i64, c_ptr, c_ptr, c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr]),
     "eigd_stored_quadform": (c_int, [c_int, c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_int, c_i64, c_ptr]),
     "eigd_segment_sum": (c_int, [c_int, c_ptr, c_ptr, c_ptr, c_dbl, c_ptr]),
-    "eigd_block_lanczos_extend": (c_int, [c_ptr, c_int, c_int, c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64,
-                                          c_int, c_int, c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr]),
+    "eigd_block_lanczos_extend": (c_int, [c_ptr, c_int, c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_int, c_int, c_int,
+                                          c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr]),
     "eigd_block_lanczos_start": (c_int, [c_int, c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_ptr, c_ptr]),
     "eigd_q4_assemble": (c_int, [c_int, c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_ptr, c_ptr]),
     "eigd_q4_quadforms": (c_int, [c_int, c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_int, c_int, c_ptr, c_ptr, c_dbl, c_dbl, c_ptr]),

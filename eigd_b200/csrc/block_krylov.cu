@@ -10,7 +10,7 @@
 //
 // One call runs the block steps of a restart cycle without returning to the host.  Per step (m = basis vectors so far,
 // j = first vector of the block being expanded):
-//     W   = factor^{-1} BV[j : j+P]                      (one P-column solve, + refinement steps)
+//     W   = factor^{-1} BV[j : j+P]                      (one P-column eigd_factor_apply)
 //     H1  = BV[lo:m] W, W -= V[lo:m]^T H1                (local Gram-Schmidt pass in the B inner product: lo = j - P, the two
 //                                                         blocks of the three-term recurrence; lo = 0 after a restart)
 //     H2  = BV[0:m] W,  W -= V[0:m]^T H2                 (unconditional full pass: full reorthogonalisation)
@@ -419,27 +419,6 @@ __global__ void __launch_bounds__(BK_THREADS, 2) block_step_kernel(StepArgs a) {
   }
 }
 
-// r = b - r for P strided vectors; x += dx
-__global__ void block_sub_from_kernel(int64_t n, int P, const double* __restrict__ b, int64_t ldb, double* __restrict__ r, int64_t ldr) {
-  for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n * P; e += (int64_t)gridDim.x * blockDim.x) {
-    const int c = (int)(e / n);
-    const int64_t i = e - (int64_t)c * n;
-    r[(int64_t)c * ldr + i] = b[(int64_t)c * ldb + i] - r[(int64_t)c * ldr + i];
-  }
-}
-__global__ void block_add_to_kernel(int64_t n, int P, const double* __restrict__ dx, int64_t ldd, double* __restrict__ x, int64_t ldx) {
-  for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n * P; e += (int64_t)gridDim.x * blockDim.x) {
-    const int c = (int)(e / n);
-    const int64_t i = e - (int64_t)c * n;
-    x[(int64_t)c * ldx + i] += dx[(int64_t)c * ldd + i];
-  }
-}
-
-inline int ew_grid(int64_t n) {
-  int64_t g = (n + 255) / 256;
-  return (int)(g < 1 ? 1 : (g > 148 * 8 ? 148 * 8 : g));
-}
-
 // Launches block_step_kernel<P> for a (its grid, virtual grids, partial-sum regions and barrier base are set here).
 // work: the eigd_gemm_tn_workspace buffer, which bounds every virtual grid (gv x outputs must fit) as it bounded the
 // grids of the separate dots kernels.
@@ -479,26 +458,15 @@ int block_step(StepArgs a, double* work) {
 }
 
 template <int P>
-int extend(eigd_factor* f, int refine, int n, const int* mp, const int* mi, const double* mv, const int* bp, const int* bi,
-           const double* bv, double* V, double* BV, int64_t ld, int j0, int m0, int ncv, double* Ablk, double* Rblk,
-           double* H1, double* H2, double* scratch, double* work, double* work2) {
+int extend(eigd_factor* f, int n, const int* bp, const int* bi, const double* bv, double* V, double* BV, int64_t ld, int j0,
+           int m0, int ncv, double* Ablk, double* Rblk, double* H1, double* H2, double* scratch, double* work) {
   int rc;
   int step = 0;
   for (int j = j0, m = m0; j < ncv; j += P, m += P, ++step) {
     const double* bvj = BV + (int64_t)j * ld;
     double* W = V + (int64_t)m * ld;
     // W = OP V_j = factor^{-1} (B V_j): the P vectors are rows (stride ld between vectors, 1 inside)
-    if ((rc = eigd_factor_solve(f, bvj, 1, ld, W, 1, ld, P))) return rc;
-    for (int it = 0; it < refine; ++it) {                        // X += F (B V_j - mat X)
-      double* r = work2;
-      double* dx = work2 + (int64_t)P * n;
-      if ((rc = eigd_csr_spmm(n, mp, mi, mv, W, 1, ld, r, 1, n, P, 1.0, 0.0))) return rc;
-      EIGD_LAUNCH(block_sub_from_kernel, ew_grid((int64_t)n * P), 256, 0, (int64_t)n, P, bvj, ld, r, (int64_t)n);
-      EIGD_CHECK_LAUNCH();
-      if ((rc = eigd_factor_solve(f, r, 1, n, dx, 1, n, P))) return rc;
-      EIGD_LAUNCH(block_add_to_kernel, ew_grid((int64_t)n * P), 256, 0, (int64_t)n, P, dx, (int64_t)n, W, ld);
-      EIGD_CHECK_LAUNCH();
-    }
+    if ((rc = eigd_factor_apply(f, bvj, 1, ld, W, 1, ld, P))) return rc;
     // Gram-Schmidt in the B inner product: a LOCAL pass against the vectors W is coupled to in exact arithmetic -- the
     // block being expanded and its predecessor (block three-term recurrence), or the whole basis in the first step
     // after a thick restart (the locked Ritz vectors: the arrow) -- then one FULL classical pass against V[0:m].  The
@@ -528,19 +496,17 @@ int start_block(int n, const int* bp, const int* bi, const double* bv, double* V
 
 }  // namespace
 
-extern "C" int eigd_block_lanczos_extend(eigd_factor* f, int refine, int n, int P, const int* d_mat_indptr,
-                                         const int* d_mat_indices, const double* d_mat_vals, const int* d_b_indptr,
-                                         const int* d_b_indices, const double* d_b_vals, double* d_V, double* d_BV, int64_t ld,
-                                         int j0, int m0, int ncv, double* d_Ablk, double* d_Rblk, double* d_H1, double* d_H2,
-                                         double* d_scratch, double* d_work, double* d_work2) {
+extern "C" int eigd_block_lanczos_extend(eigd_factor* f, int n, int P, const int* d_b_indptr, const int* d_b_indices,
+                                         const double* d_b_vals, double* d_V, double* d_BV, int64_t ld, int j0, int m0, int ncv,
+                                         double* d_Ablk, double* d_Rblk, double* d_H1, double* d_H2, double* d_scratch,
+                                         double* d_work) {
   if (j0 >= ncv) return 0;
   if ((ncv - j0) % P != 0 || m0 < j0 + P) { eigd_set_error("block_lanczos_extend: the cycle does not end on a block boundary"); return 7; }
   if (m0 + (ncv - j0) > BK_JMAX + BK_PMAX) { eigd_set_error("block_lanczos_extend: basis too large"); return 7; }
-  if (refine > 0 && (!d_mat_indptr || !d_work2)) { eigd_set_error("block_lanczos_extend: refinement needs the shifted matrix and 2 P n doubles of work"); return 7; }
   switch (P) {
-    case 2: return extend<2>(f, refine, n, d_mat_indptr, d_mat_indices, d_mat_vals, d_b_indptr, d_b_indices, d_b_vals, d_V, d_BV, ld, j0, m0, ncv, d_Ablk, d_Rblk, d_H1, d_H2, d_scratch, d_work, d_work2);
-    case 3: return extend<3>(f, refine, n, d_mat_indptr, d_mat_indices, d_mat_vals, d_b_indptr, d_b_indices, d_b_vals, d_V, d_BV, ld, j0, m0, ncv, d_Ablk, d_Rblk, d_H1, d_H2, d_scratch, d_work, d_work2);
-    case 4: return extend<4>(f, refine, n, d_mat_indptr, d_mat_indices, d_mat_vals, d_b_indptr, d_b_indices, d_b_vals, d_V, d_BV, ld, j0, m0, ncv, d_Ablk, d_Rblk, d_H1, d_H2, d_scratch, d_work, d_work2);
+    case 2: return extend<2>(f, n, d_b_indptr, d_b_indices, d_b_vals, d_V, d_BV, ld, j0, m0, ncv, d_Ablk, d_Rblk, d_H1, d_H2, d_scratch, d_work);
+    case 3: return extend<3>(f, n, d_b_indptr, d_b_indices, d_b_vals, d_V, d_BV, ld, j0, m0, ncv, d_Ablk, d_Rblk, d_H1, d_H2, d_scratch, d_work);
+    case 4: return extend<4>(f, n, d_b_indptr, d_b_indices, d_b_vals, d_V, d_BV, ld, j0, m0, ncv, d_Ablk, d_Rblk, d_H1, d_H2, d_scratch, d_work);
     default: eigd_set_error("block_lanczos_extend: block size must be 2, 3 or 4"); return 7;
   }
 }

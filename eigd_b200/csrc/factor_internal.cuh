@@ -87,6 +87,12 @@ struct eigd_factor {
   unsigned epoch = 0;                     // cooperative solve launches issued so far (host mirror)
   double piv_tol = 1e-11;
   int pivoting = 0;                       // 0 static pivots, 1 restricted Bunch-Kaufman (eigd_factor_set_pivoting)
+  struct {                                // iterative refinement of eigd_factor_apply (eigd_factor_set_refinement)
+    int steps, cols;                      // depth; right-hand sides the scratch holds
+    const int *indptr, *indices;          // the caller's device CSR of the factorised matrix
+    const double* vals;
+    double* work;                         // the caller's scratch, 2 x n x cols doubles
+  } refine = {};
   int64_t bytes = 0;
   char* base = nullptr;
   bool owns = true;

@@ -31,14 +31,6 @@ __global__ void lanczos_finish_kernel(int64_t n, const double* __restrict__ w, c
   }
 }
 
-// r = b - r (residual of the refinement step), x += dx
-__global__ void sub_from_kernel(int64_t n, const double* __restrict__ b, double* __restrict__ r) {
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) r[i] = b[i] - r[i];
-}
-__global__ void add_to_kernel(int64_t n, const double* __restrict__ dx, double* __restrict__ x) {
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) x[i] += dx[i];
-}
-
 inline int ew_grid(int64_t n) {
   int64_t g = (n + 255) / 256;
   return (int)(g < 1 ? 1 : (g > 148 * 8 ? 148 * 8 : g));
@@ -46,28 +38,15 @@ inline int ew_grid(int64_t n) {
 
 }  // namespace
 
-extern "C" int eigd_lanczos_extend(eigd_factor* f, int refine, int n, const int* d_mat_indptr, const int* d_mat_indices,
-                                   const double* d_mat_vals, const int* d_b_indptr, const int* d_b_indices,
+extern "C" int eigd_lanczos_extend(eigd_factor* f, int n, const int* d_b_indptr, const int* d_b_indices,
                                    const double* d_b_vals, double* d_V, double* d_BV, int64_t ld, int j0, int j1,
-                                   double* d_w, double* d_h, double* d_g, double* d_ab, int ldab, double* d_work,
-                                   double* d_work2) {
+                                   double* d_w, double* d_h, double* d_g, double* d_ab, int ldab, double* d_work) {
   if (j1 <= j0) return 0;
-  if (refine > 0 && (!d_mat_indptr || !d_work2)) { eigd_set_error("lanczos_extend: refinement needs the shifted matrix and 2n doubles of work"); return 7; }
   int rc;
   for (int j = j0; j < j1; ++j) {
     const double* bvj = d_BV + (int64_t)j * ld;
     // w = OP v_j = (A - sigma B)^{-1} (B v_j)
-    if ((rc = eigd_factor_solve(f, bvj, 1, 1, d_w, 1, 1, 1))) return rc;
-    for (int it = 0; it < refine; ++it) {                      // x += F (b - mat x)
-      double* r = d_work2;
-      double* dx = d_work2 + n;
-      if ((rc = eigd_csr_spmm(n, d_mat_indptr, d_mat_indices, d_mat_vals, d_w, 1, 1, r, 1, 1, 1, 1.0, 0.0))) return rc;
-      EIGD_LAUNCH(sub_from_kernel, ew_grid(n), 256, 0, (int64_t)n, bvj, r);
-      EIGD_CHECK_LAUNCH();
-      if ((rc = eigd_factor_solve(f, r, 1, 1, dx, 1, 1, 1))) return rc;
-      EIGD_LAUNCH(add_to_kernel, ew_grid(n), 256, 0, (int64_t)n, dx, d_w);
-      EIGD_CHECK_LAUNCH();
-    }
+    if ((rc = eigd_factor_apply(f, bvj, 1, 1, d_w, 1, 1, 1))) return rc;
     // classical Gram-Schmidt against v_0 .. v_j in the B inner product, second pass unconditional (DGKS)
     if ((rc = eigd_basis_dots(n, j + 1, d_BV, ld, d_w, d_h, d_work))) return rc;
     if ((rc = eigd_basis_axpy(n, j + 1, d_V, ld, d_h, 1, -1.0, d_w))) return rc;

@@ -1554,6 +1554,17 @@ int launch_solve(int slot, eigd_factor* f, SolveArgs& a) {
   return 0;
 }
 
+// Y = X + s Y on n x k strided operands, s = -1 (residual b - r) or +1 (update dx + x): one rounding per element, so the
+// results are fl(b - r) and fl(x + dx)
+__global__ void refine_xpsy_kernel(int64_t n, int k, const double* __restrict__ X, int64_t xrs, int64_t xcs, double s,
+                                   double* __restrict__ Y, int64_t yrs, int64_t ycs) {
+  for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n * k; e += (int64_t)gridDim.x * blockDim.x) {
+    int64_t i; int c;
+    if (ycs == 1) { i = e / k; c = (int)(e - i * k); } else { c = (int)(e / n); i = e - (int64_t)c * n; }
+    Y[i * yrs + c * ycs] = X[i * xrs + c * xcs] + s * Y[i * yrs + c * ycs];
+  }
+}
+
 }  // namespace
 
 int build_solve_plan_dev(eigd_symbolic* S, SymDevHolder* h) {
@@ -1688,6 +1699,45 @@ extern "C" int eigd_factor_solve(eigd_factor* f, const double* B, int64_t brs, i
       EIGD_CUDA(cudaEventRecord(tm.e1, g_eigd_stream));
       g_timings.push_back(tm);
     }
+  }
+  return 0;
+}
+
+// ---- iterative refinement x += F (b - A x) against the matrix registered with eigd_factor_set_refinement ----------
+extern "C" int eigd_factor_set_refinement(eigd_factor* f, int steps, const int* d_indptr, const int* d_indices,
+                                          const double* d_vals, double* d_work, int work_cols) {
+  if (steps < 0 || work_cols < 0 || (steps > 0 && (!d_indptr || !d_indices || !d_vals)) || (work_cols > 0 && !d_work)) {
+    eigd_set_error("factor_set_refinement: a refinement depth needs the matrix, a scratch width needs the scratch");
+    return 7;
+  }
+  f->refine = {steps, work_cols, d_indptr, d_indices, d_vals, d_work};
+  return 0;
+}
+
+extern "C" int eigd_factor_apply(eigd_factor* f, const double* B, int64_t brs, int64_t bcs, double* X, int64_t xrs,
+                                 int64_t xcs, int k) {
+  const auto& r = f->refine;
+  if (r.steps == 0 || k < 1) return eigd_factor_solve(f, B, brs, bcs, X, xrs, xcs, k);
+  if (k > r.cols) { eigd_set_error("factor_apply: %d right-hand sides, but the refinement scratch holds %d", k, r.cols); return 7; }
+  const int n = f->sym->n;
+  // the residual R (and the copy of B) are laid out like X, so that every element-wise pass is coalesced on both sides
+  const int64_t rrs = xcs == 1 ? k : 1, rcs = xcs == 1 ? 1 : n;
+  double* R = r.work;
+  const int g = (int)std::min<int64_t>(((int64_t)n * k + 255) / 256, 148 * 8);     // grid of the element-wise passes
+  int rc;
+  if (X == B) {                                           // the solve overwrites B, which every residual needs
+    if ((rc = eigd_copy2d(n, k, B, brs, bcs, R + (int64_t)n * k, rrs, rcs))) return rc;
+    B = R + (int64_t)n * k, brs = rrs, bcs = rcs;
+  }
+  if ((rc = eigd_factor_solve(f, B, brs, bcs, X, xrs, xcs, k))) return rc;
+  for (int it = 0; it < r.steps; ++it) {
+    // k == 1 stays a one-column product (spmv_kernel): its summation order differs from the multi-column kernel's
+    if ((rc = eigd_csr_spmm(n, r.indptr, r.indices, r.vals, X, xrs, xcs, R, rrs, rcs, k, 1.0, 0.0))) return rc;
+    EIGD_LAUNCH(refine_xpsy_kernel, g, 256, 0, (int64_t)n, k, B, brs, bcs, -1.0, R, rrs, rcs);     // R = B - A X
+    EIGD_CHECK_LAUNCH();
+    if ((rc = eigd_factor_solve(f, R, rrs, rcs, R, rrs, rcs, k))) return rc;                    // dX = F R, in place
+    EIGD_LAUNCH(refine_xpsy_kernel, g, 256, 0, (int64_t)n, k, R, rrs, rcs, 1.0, X, xrs, xcs);      // X = dX + X
+    EIGD_CHECK_LAUNCH();
   }
   return 0;
 }

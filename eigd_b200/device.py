@@ -615,6 +615,7 @@ class Factor:
         self.handle = h
         self.max_rhs = int(max_rhs)
         self.pivoting = pivoting
+        self.refine, self._refine_mat, self._refine_work, self._refine_cols = 0, None, None, 0
         if pivoting != "static":
             check(lib.eigd_factor_set_pivoting(h, PIVOTING_MODES.index(pivoting)), "factor_set_pivoting")
 
@@ -653,42 +654,57 @@ class Factor:
     def nbytes(self):
         return int(_lib.load().eigd_factor_bytes(self.handle))
 
-    def solve(self, B, out=None):
-        """out = (L D L^T)^{-1} B for a (n,) or (n, k) device tensor; out may alias B."""
+    def set_refinement(self, steps, mat, k=1):
+        """The refined solves (``solve(refined=True)``, the Lanczos extends) add ``steps`` rounds of iterative refinement
+        x += F(b - mat x), ``mat`` the CsrDevice this factor factorised; the scratch they need, 2 n k doubles owned
+        here, grows to the widest k asked for."""
+        if steps and k > self._refine_cols:
+            self._refine_work, self._refine_cols = torch.empty(2 * self.n * k, dtype=F64, device=dev()), k
+        self.refine, self._refine_mat = int(steps), mat
+        check(_lib.load().eigd_factor_set_refinement(self.handle, self.refine, _ptr(mat.indptr), _ptr(mat.indices),
+                                                     _ptr(mat.data), _ptr(self._refine_work), self._refine_cols),
+              "factor_set_refinement")
+
+    def solve(self, B, out=None, refined=False):
+        """out = (L D L^T)^{-1} B for a (n,) or (n, k) device tensor; out may alias B.  refined: followed by the
+        refinement steps of ``set_refinement``."""
         B2 = _as2d(_chk(B, "B"))
         if B2.shape[0] != self.n:
             raise ValueError("dimension mismatch in solve")
         if out is None:
             out = torch.empty_like(B)
         X2 = _as2d(_chk(out, "out"))
+        k = B2.shape[1]
+        steps = self.refine if refined else 0
+        if steps and k > self._refine_cols:
+            self.set_refinement(steps, self._refine_mat, k)
+        name = "eigd_factor_apply" if refined else "eigd_factor_solve"
         tok = Timeline.begin("solve")
         l0 = launch_count() if tok else 0
-        check(_lib.load().eigd_factor_solve(self.handle, _ptr(B2), B2.stride(0), B2.stride(1), _ptr(X2), X2.stride(0),
-                                            X2.stride(1), B2.shape[1]), "factor_solve")
-        if tok:
-            Timeline.end(tok, self.solve_bytes(B2.shape[1]), launch_count() - l0)
+        check(getattr(_lib.load(), name)(self.handle, _ptr(B2), B2.stride(0), B2.stride(1), _ptr(X2), X2.stride(0),
+                                         X2.stride(1), k), name)
+        if tok:                             # steps + 1 sweeps and steps SpMMs with the factorised matrix (as CsrDevice.spmm)
+            spmm = self._refine_mat.nnz * 12 + (self.n + 1) * 4 + 2 * self.n * k * 8 if steps else 0
+            Timeline.end(tok, (steps + 1) * self.solve_bytes(k) + steps * spmm, launch_count() - l0)
         return out
 
 
 def lanczos_extend(op, Bip, Vt, BVt, j0, j1, w, h, g, ab):
     """Steps j0 .. j1-1 of the shift-and-invert Lanczos recurrence on the device (csrc/krylov.cu).
 
-    op: SpLuOperator (factor + shifted matrix for refinement); Bip: CsrDevice of the inner product;
+    op: SpLuOperator (its factor applies the refinement it registered); Bip: CsrDevice of the inner product;
     Vt, BVt: (ncv + 1, n) row-major bases; w: (n,); h, g: (ncv + 1,); ab: (2, ncv + 1) [alpha; beta^2]."""
     n = Vt.shape[1]
     for t in (Vt, BVt, w, h, g, ab):
         _chk(t)
     if not (Vt.is_contiguous() and BVt.is_contiguous() and ab.is_contiguous() and w.is_contiguous()):
         raise ValueError("lanczos_extend needs contiguous row-major bases")
-    refine = int(getattr(op, "refine", 0))
-    work2 = empty(2 * n) if refine else None
-    mat = op.mat
+    op.lu.set_refinement(op.refine, op.mat, 1)    # reading op.refine settles the depth; scratch for one column
     tok = Timeline.begin("lanczos")
     l0 = launch_count() if tok else 0
-    check(_lib.load().eigd_lanczos_extend(op.lu.handle, refine, n, _ptr(mat.indptr), _ptr(mat.indices), _ptr(mat.data),
-                                          _ptr(Bip.indptr), _ptr(Bip.indices), _ptr(Bip.data), _ptr(Vt), _ptr(BVt),
-                                          Vt.stride(0), int(j0), int(j1), _ptr(w), _ptr(h), _ptr(g), _ptr(ab),
-                                          ab.stride(0), _ptr(_State.work), _ptr(work2)), "lanczos_extend")
+    check(_lib.load().eigd_lanczos_extend(op.lu.handle, n, _ptr(Bip.indptr), _ptr(Bip.indices), _ptr(Bip.data), _ptr(Vt),
+                                          _ptr(BVt), Vt.stride(0), int(j0), int(j1), _ptr(w), _ptr(h), _ptr(g), _ptr(ab),
+                                          ab.stride(0), _ptr(_State.work)), "lanczos_extend")
     nsteps = int(j1) - int(j0)
     op.count += nsteps                      # one operator application per step, as SpLuOperator counts them
     if tok:
@@ -712,15 +728,12 @@ def block_lanczos_extend(op, Bip, Vt, BVt, P, j0, m0, ncv, Ablk, Rblk, H1, H2, s
         _chk(t)
     if not (Vt.is_contiguous() and BVt.is_contiguous()):
         raise ValueError("block_lanczos_extend needs contiguous row-major bases")
-    refine = int(getattr(op, "refine", 0))
-    work2 = empty(2 * P * n) if refine else None
-    mat = op.mat
+    op.lu.set_refinement(op.refine, op.mat, P)    # reading op.refine settles the depth; scratch for P columns
     tok = Timeline.begin("lanczos")
     l0 = launch_count() if tok else 0
-    check(_lib.load().eigd_block_lanczos_extend(op.lu.handle, refine, n, int(P), _ptr(mat.indptr), _ptr(mat.indices), _ptr(mat.data),
-                                                _ptr(Bip.indptr), _ptr(Bip.indices), _ptr(Bip.data), _ptr(Vt), _ptr(BVt),
-                                                Vt.stride(0), int(j0), int(m0), int(ncv), _ptr(Ablk), _ptr(Rblk), _ptr(H1), _ptr(H2),
-                                                _ptr(scratch), _ptr(_State.work), _ptr(work2)), "block_lanczos_extend")
+    check(_lib.load().eigd_block_lanczos_extend(op.lu.handle, n, int(P), _ptr(Bip.indptr), _ptr(Bip.indices), _ptr(Bip.data),
+                                                _ptr(Vt), _ptr(BVt), Vt.stride(0), int(j0), int(m0), int(ncv), _ptr(Ablk), _ptr(Rblk),
+                                                _ptr(H1), _ptr(H2), _ptr(scratch), _ptr(_State.work)), "block_lanczos_extend")
     op.count += int(ncv) - int(j0)          # one operator application per new basis vector, as SpLuOperator counts columns
     if tok:
         Timeline.end(tok, 0, launch_count() - l0)

@@ -166,7 +166,7 @@ class SpLuOperator:
     def _finish(self):
         if self._state is not None:
             return
-        self._state = {"info": None, "refine": 0, "probe": None, "probe_refined": None}
+        self._state = {"info": None, "probe": None, "probe_refined": None}
         st = self._state
         st["info"] = info = self.lu.info()
         if info["non_finite"]:
@@ -185,19 +185,19 @@ class SpLuOperator:
                 refine = 0 if st["probe"] < 1e-13 else 1
             else:
                 refine = 0
-        st["refine"] = int(refine)
-        if st["refine"] and (info["perturbed_pivots"] or info["negative_pivots"]):
+        self.lu.set_refinement(refine, self.mat)
+        if self.lu.refine and (info["perturbed_pivots"] or info["negative_pivots"]):
             # static pivoting is only as good as the refined solve it leaves behind: measure that, iterate the
             # refinement to tolerance if one step is not enough, and say so loudly if it cannot be reached
             # (a shift that sits on an eigenvalue; the reference's partially pivoted LU would lose accuracy there too)
             st["probe_refined"] = self._probe_residual(refined=True)
-            while st["probe_refined"] > 1e-10 and st["refine"] < 4:
-                st["refine"] += 1
+            while st["probe_refined"] > 1e-10 and self.lu.refine < 4:
+                self.lu.set_refinement(self.lu.refine + 1, self.mat)
                 st["probe_refined"] = self._probe_residual(refined=True)
             if not st["probe_refined"] <= 1e-8:
                 warnings.warn("SpLuOperator: the LDL^T factorisation of the shifted matrix is inaccurate (relative residual "
                               "%.1e after %d refinement steps, %d perturbed and %d negative pivots); move the shift away "
-                              "from the spectrum" % (st["probe_refined"], st["refine"], info["perturbed_pivots"],
+                              "from the spectrum" % (st["probe_refined"], self.lu.refine, info["perturbed_pivots"],
                                                      info["negative_pivots"]))
 
     @property
@@ -208,12 +208,12 @@ class SpLuOperator:
     @property
     def refine(self):
         self._finish()
-        return self._state["refine"]
+        return self.lu.refine
 
     @refine.setter
     def refine(self, value):
         self._finish()
-        self._state["refine"] = int(value)
+        self.lu.set_refinement(value, self.mat)
 
     @property
     def probe(self):
@@ -245,21 +245,9 @@ class SpLuOperator:
     # -- device entry point used by every solver in this package --------------------------------
     def solve_dev(self, Bd, out=None):
         """X = mat^{-1} B for a device (n,) or (n, k) tensor; counts k solves (reference :19-22)."""
-        k = 1 if Bd.dim() == 1 else Bd.shape[1]
-        self.count += k
-        if out is not None and out.data_ptr() == Bd.data_ptr() and self.refine:
-            Bd = Bd.clone()
-        X = self.lu.solve(Bd, out=out)
-        for _ in range(self.refine):                 # iterative refinement: x += F(b - mat x)
-            R = self.mat.spmm(X)
-            Bc = _contig(Bd)
-            D.axpby(1.0, Bc.reshape(-1), -1.0, R.reshape(-1), out=R.reshape(-1))
-            dX = self.lu.solve(R)
-            if X.is_contiguous():
-                D.axpby(1.0, X.reshape(-1), 1.0, dX.reshape(-1), out=X.reshape(-1))
-            else:
-                D.col_axpy(X, small_to_dev(np.ones(k)), dX, sign=1.0)
-        return X
+        self._finish()                               # settles the refinement depth the factor applies
+        self.count += 1 if Bd.dim() == 1 else Bd.shape[1]
+        return self.lu.solve(Bd, out=out, refined=True)
 
     @_public
     def _apply(self, x):

@@ -135,6 +135,15 @@ int eigd_factor_pivot_counts(eigd_factor* f, int64_t* out2);
 /* X = (L D L^T)^{-1} B in the original ordering; k columns, (rs, cs) strides; X may alias B */
 int eigd_factor_solve(eigd_factor* f, const double* d_B, int64_t brs, int64_t bcs,
                       double* d_X, int64_t xrs, int64_t xcs, int k);
+/* iterative refinement of eigd_factor_apply: `steps` rounds of x += F (b - A x) against the device CSR A (the
+ * factorised matrix; may be NULL when steps == 0), with d_work >= 2 * n * work_cols doubles of scratch (may be NULL when
+ * work_cols == 0).  Both stay owned by the caller and must outlive their registration.  A new factor has steps = 0. */
+int eigd_factor_set_refinement(eigd_factor* f, int steps, const int* d_indptr, const int* d_indices, const double* d_vals,
+                               double* d_work, int work_cols);
+/* X = A^{-1} B as the operator applies it: eigd_factor_solve followed by the registered refinement steps, over all k
+ * columns; X may alias B.  Fails when the refinement depth is not 0 and k exceeds the registered work_cols. */
+int eigd_factor_apply(eigd_factor* f, const double* d_B, int64_t brs, int64_t bcs,
+                      double* d_X, int64_t xrs, int64_t xcs, int k);
 /* live timing of every solve launch between begin and end (CUDA events on the launching stream, used by
  * bench.py for the roofline of the dominant kernel): calls_by_k / ms_by_k have 33 entries, index = number
  * of right-hand sides of the launch */
@@ -155,17 +164,14 @@ int64_t eigd_factor_bytes(const eigd_factor* f);
 /* ---- device-resident Lanczos recurrence: replaces the reverse-communication loop around ARPACK dsaupd
  *      (eigd/arpack.py:438-442) and the step body of BasicLanczos.solve
  *      (eigd/eigenvector_derivatives.py:1496-1545).  Runs steps j0 .. j1-1 without returning to the host:
- *      w = factor^{-1} BV[j] (refine steps of iterative refinement against the shifted matrix `mat`, which
- *      may be NULL when refine == 0), two classical Gram-Schmidt passes against V[0..j] in the B inner
+ *      w = factor^{-1} BV[j] (eigd_factor_apply: the refinement registered with the factor, whose
+ *      scratch must hold one column), two classical Gram-Schmidt passes against V[0..j] in the B inner
  *      product, BV[j+1] = B w, beta_j^2 = w . B w, V[j+1] = w / beta_j, BV[j+1] /= beta_j.
  *      V, BV: (ncv + 1) x n row-major with leading dimension ld; w, h, g: n, ncv + 1, ncv + 1 doubles;
- *      ab: 2 x ldab, row 0 <- alpha_j, row 1 <- beta_j^2; work >= eigd_gemm_tn_workspace() doubles;
- *      work2: 2n doubles (refinement only). ------------------------------------------------------------ */
-int eigd_lanczos_extend(eigd_factor* f, int refine, int n, const int* d_mat_indptr, const int* d_mat_indices,
-                        const double* d_mat_vals, const int* d_b_indptr, const int* d_b_indices,
+ *      ab: 2 x ldab, row 0 <- alpha_j, row 1 <- beta_j^2; work >= eigd_gemm_tn_workspace() doubles. ------- */
+int eigd_lanczos_extend(eigd_factor* f, int n, const int* d_b_indptr, const int* d_b_indices,
                         const double* d_b_vals, double* d_V, double* d_BV, int64_t ld, int j0, int j1,
-                        double* d_w, double* d_h, double* d_g, double* d_ab, int ldab, double* d_work,
-                        double* d_work2);
+                        double* d_w, double* d_h, double* d_g, double* d_ab, int ldab, double* d_work);
 
 /* ---- operators on stored unit element matrices (csrc/stored_fe.cu): the CRM-like shell driver, replacing what TACS
  *      does on the host in reference examples/crm.py:122-142 (assembleMatType) and :331-355 (addMatDVSensInnerProduct,
@@ -187,12 +193,12 @@ int eigd_segment_sum(int nseg, const int* d_seg_ptr, const int* d_perm, const do
  *      ld) holding m0 >= j0 + P B-orthonormal vectors on entry and ncv + P on exit.  Per step s the P x P diagonal
  *      block (H1 + H2)[j : j + P] goes to Ablk[s] and the sub-diagonal block R (W = V_new R) to Rblk[s] (row-major);
  *      a rank-deficient block (breakdown) is flagged by NaNs in Rblk.  H1, H2: (ncv + P) * P doubles; scratch: 3 P^2;
- *      work >= eigd_gemm_tn_workspace(); work2: 2 P n doubles (refinement only). ------------------------------ */
-int eigd_block_lanczos_extend(eigd_factor* f, int refine, int n, int P, const int* d_mat_indptr, const int* d_mat_indices,
-                              const double* d_mat_vals, const int* d_b_indptr, const int* d_b_indices,
+ *      work >= eigd_gemm_tn_workspace().  The P-column solves are eigd_factor_apply: the refinement
+ *      registered with the factor, whose scratch must hold P columns. -------------------------------------------- */
+int eigd_block_lanczos_extend(eigd_factor* f, int n, int P, const int* d_b_indptr, const int* d_b_indices,
                               const double* d_b_vals, double* d_V, double* d_BV, int64_t ld, int j0, int m0, int ncv,
                               double* d_Ablk, double* d_Rblk, double* d_H1, double* d_H2, double* d_scratch,
-                              double* d_work, double* d_work2);
+                              double* d_work);
 /* B-orthonormalise the P start vectors V[0:P] (rows) in place and set BV[0:P] = B V[0:P]; scratch: 3 P^2 doubles */
 int eigd_block_lanczos_start(int n, int P, const int* d_b_indptr, const int* d_b_indices, const double* d_b_vals,
                              double* d_V, double* d_BV, int64_t ld, double* d_scratch, double* d_work);
