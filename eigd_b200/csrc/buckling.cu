@@ -11,48 +11,10 @@
 //   reduce_vector / full_vector                       examples/buckling.py:499-518
 //   Be, Te, detJ                                      examples/fe_utils.py:58-98
 #include "common.cuh"
+#include "q4_element.cuh"
 #include "../../include/eigd_b200.h"
 
 namespace {
-
-struct Geo {
-  double Nx[4][4], Ny[4][4], detJ[4];  // [gauss point][node]
-};
-
-__device__ __forceinline__ void geometry(const int* __restrict__ conn, const double* __restrict__ xy, int e, int nd[4], Geo& g) {
-  const double gp = 0.57735026918962576451;
-  double xe[4], ye[4];
-#pragma unroll
-  for (int a = 0; a < 4; ++a) {
-    nd[a] = conn[e * 4 + a];
-    xe[a] = xy[2 * nd[a]];
-    ye[a] = xy[2 * nd[a] + 1];
-  }
-#pragma unroll
-  for (int q = 0; q < 4; ++q) {
-    // index = 2*j + i with xi = pts[i], eta = pts[j] (examples/buckling.py:266-273)
-    double xi = (q & 1) ? gp : -gp;
-    double eta = (q & 2) ? gp : -gp;
-    double Nxi[4] = {-0.25 * (1.0 - eta), 0.25 * (1.0 - eta), 0.25 * (1.0 + eta), -0.25 * (1.0 + eta)};
-    double Neta[4] = {-0.25 * (1.0 - xi), -0.25 * (1.0 + xi), 0.25 * (1.0 + xi), 0.25 * (1.0 - xi)};
-    double J00 = 0, J10 = 0, J01 = 0, J11 = 0;
-#pragma unroll
-    for (int a = 0; a < 4; ++a) {
-      J00 = fma(xe[a], Nxi[a], J00);
-      J10 = fma(ye[a], Nxi[a], J10);
-      J01 = fma(xe[a], Neta[a], J01);
-      J11 = fma(ye[a], Neta[a], J11);
-    }
-    double det = J00 * J11 - J01 * J10;
-    double i00 = J11 / det, i01 = -J01 / det, i10 = -J10 / det, i11 = J00 / det;
-#pragma unroll
-    for (int a = 0; a < 4; ++a) {
-      g.Nx[q][a] = i00 * Nxi[a] + i10 * Neta[a];
-      g.Ny[q][a] = i01 * Nxi[a] + i11 * Neta[a];
-    }
-    g.detJ[q] = det;
-  }
-}
 
 // sdet[e][q][i] = detJ_q * ks[e] * (C0 Be(q) u_e)_i : the weights of Te in the element stress stiffness
 __global__ void __launch_bounds__(128)
@@ -60,30 +22,24 @@ q4_stress_kernel(int nelems, const int* __restrict__ conn, const double* __restr
                  const double* __restrict__ ks, const double* __restrict__ u, double* __restrict__ sdet) {
   int e = blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= nelems) return;
-  int nd[4];
-  Geo g;
-  geometry(conn, xy, e, nd, g);
+  const Q4Nodes el = q4_gather(conn, xy, e);
+  const Q4Geom g = q4_geometry(el);
   double ue[8];
 #pragma unroll
   for (int a = 0; a < 4; ++a) {
-    ue[2 * a] = u[2 * nd[a]];
-    ue[2 * a + 1] = u[2 * nd[a] + 1];
+    ue[2 * a] = u[2 * el.nd[a]];
+    ue[2 * a + 1] = u[2 * el.nd[a] + 1];
   }
-  const double c00 = cmat[0], c01 = cmat[1], c02 = cmat[2], c11 = cmat[3], c12 = cmat[4], c22 = cmat[5];
+  const Q4C0 c0 = q4_c0_load(cmat);
   const double s = ks[e];
 #pragma unroll
   for (int q = 0; q < 4; ++q) {
-    double ex = 0, ey = 0, gxy = 0;
-#pragma unroll
-    for (int a = 0; a < 4; ++a) {
-      ex = fma(g.Nx[q][a], ue[2 * a], ex);
-      ey = fma(g.Ny[q][a], ue[2 * a + 1], ey);
-      gxy = fma(g.Ny[q][a], ue[2 * a], fma(g.Nx[q][a], ue[2 * a + 1], gxy));
-    }
+    double eps[3], sig[3];
+    q4_strain(g.Nx[q], g.Ny[q], ue, eps);
+    q4_c0_mul(c0, eps, sig);
     const double w = g.detJ[q] * s;
-    sdet[(e * 4 + q) * 3 + 0] = w * (c00 * ex + c01 * ey + c02 * gxy);
-    sdet[(e * 4 + q) * 3 + 1] = w * (c01 * ex + c11 * ey + c12 * gxy);
-    sdet[(e * 4 + q) * 3 + 2] = w * (c02 * ex + c12 * ey + c22 * gxy);
+#pragma unroll
+    for (int i = 0; i < 3; ++i) sdet[(e * 4 + q) * 3 + i] = w * sig[i];
   }
 }
 
@@ -101,21 +57,15 @@ __global__ void q4_assemble_geometric_kernel(int64_t nnz, const int64_t* __restr
     int ab = (int)(s - (int64_t)e * 64);
     int a = ab >> 3, b = ab & 7;
     if ((a & 1) != (b & 1)) continue;
-    int na = a >> 1, nb = b >> 1;
-    int nd[4];
-    Geo g;
-    geometry(conn, xy, e, nd, g);
+    const Q4Nodes el = q4_gather(conn, xy, e);
     double ge = 0.0;
 #pragma unroll
     for (int q = 0; q < 4; ++q) {
       const double* sd = sdet + ((int64_t)e * 4 + q) * 3;
-      // select the two nodes without dynamic register indexing
-      double nxa = 0, nya = 0, nxb = 0, nyb = 0;
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        if (i == na) { nxa = g.Nx[q][i]; nya = g.Ny[q][i]; }
-        if (i == nb) { nxb = g.Nx[q][i]; nyb = g.Ny[q][i]; }
-      }
+      double N[4], Nx[4], Ny[4], na, nxa, nya, nb, nxb, nyb;
+      q4_point(el, q, N, Nx, Ny);
+      q4_node(a >> 1, N, Nx, Ny, na, nxa, nya);
+      q4_node(b >> 1, N, Nx, Ny, nb, nxb, nyb);
       ge += sd[0] * nxa * nxb + sd[1] * nya * nyb + sd[2] * (nxa * nyb + nya * nxb);
     }
     gv += ge;
@@ -137,9 +87,8 @@ q4_gderiv_kernel(int nelems, const int* __restrict__ conn, const double* __restr
   int e = (int)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) / G);
   const bool valid = e < nelems;
   if (!valid) e = nelems - 1;
-  int nd[4];
-  Geo g;
-  geometry(conn, xy, e, nd, g);
+  const Q4Nodes el = q4_gather(conn, xy, e);
+  const Q4Geom g = q4_geometry(el);
   double dfds[4][3];
 #pragma unroll
   for (int q = 0; q < 4; ++q) dfds[q][0] = dfds[q][1] = dfds[q][2] = 0.0;
@@ -147,7 +96,7 @@ q4_gderiv_kernel(int nelems, const int* __restrict__ conn, const double* __restr
     double w[8], v[8];
 #pragma unroll
     for (int a = 0; a < 4; ++a) {
-      int64_t o = (int64_t)(2 * nd[a]) * ldw + k;
+      int64_t o = (int64_t)(2 * el.nd[a]) * ldw + k;
       w[2 * a] = W[o];
       w[2 * a + 1] = W[o + ldw];
       v[2 * a] = V[o];
@@ -179,32 +128,30 @@ q4_gderiv_kernel(int nelems, const int* __restrict__ conn, const double* __restr
       for (int o = G >> 1; o > 0; o >>= 1) dfds[q][i] += __shfl_xor_sync(0xffffffffu, dfds[q][i], o, G);
     }
   if (!valid || lane != 0) return;
-  const double c00 = cmat[0], c01 = cmat[1], c02 = cmat[2], c11 = cmat[3], c12 = cmat[4], c22 = cmat[5];
+  const Q4C0 c0 = q4_c0_load(cmat);
   double ue[8];
 #pragma unroll
   for (int a = 0; a < 4; ++a) {
-    ue[2 * a] = u[2 * nd[a]];
-    ue[2 * a + 1] = u[2 * nd[a] + 1];
+    ue[2 * a] = u[2 * el.nd[a]];
+    ue[2 * a + 1] = u[2 * el.nd[a] + 1];
   }
   double drho = 0.0;
   double de[8] = {0, 0, 0, 0, 0, 0, 0, 0};
 #pragma unroll
   for (int q = 0; q < 4; ++q) {
-    const double f0 = g.detJ[q] * dfds[q][0], f1 = g.detJ[q] * dfds[q][1], f2 = g.detJ[q] * dfds[q][2];
-    const double t0 = c00 * f0 + c01 * f1 + c02 * f2;
-    const double t1 = c01 * f0 + c11 * f1 + c12 * f2;
-    const double t2 = c02 * f0 + c12 * f1 + c22 * f2;
-    double ex = 0, ey = 0, gxy = 0;
+    const double f[3] = {g.detJ[q] * dfds[q][0], g.detJ[q] * dfds[q][1], g.detJ[q] * dfds[q][2]};
+    double t[3], eps[3];
+    q4_c0_mul(c0, f, t);
+    q4_strain(g.Nx[q], g.Ny[q], ue, eps);
 #pragma unroll
-    for (int a = 0; a < 4; ++a) {
-      ex = fma(g.Nx[q][a], ue[2 * a], ex);
-      ey = fma(g.Ny[q][a], ue[2 * a + 1], ey);
-      gxy = fma(g.Ny[q][a], ue[2 * a], fma(g.Nx[q][a], ue[2 * a + 1], gxy));
-      // Be columns: dof u -> [Nx, 0, Ny], dof v -> [0, Ny, Nx]
-      de[2 * a] += g.Nx[q][a] * t0 + g.Ny[q][a] * t2;
-      de[2 * a + 1] += g.Ny[q][a] * t1 + g.Nx[q][a] * t2;
-    }
-    drho += t0 * ex + t1 * ey + t2 * gxy;
+    for (int a = 0; a < 4; ++a)
+#pragma unroll
+      for (int d = 0; d < 2; ++d) {
+        double b[3];
+        q4_strain_rows(d, g.Nx[q][a], g.Ny[q][a], b);
+        de[2 * a + d] += b[d] * t[d] + b[2] * t[2];  // Be^T t without the zero row 1 - d
+      }
+    drho += t[0] * eps[0] + t[1] * eps[1] + t[2] * eps[2];
   }
   if (out_rho) out_rho[e] += sx * dks[e] * drho;
   if (due) {

@@ -6,47 +6,12 @@
 //   thermal      examples/thermal.py:126-148 (K), :150-190 (dK), :192-214 (M), :216-246 (dM)
 //   plane stress examples/natural_frequency.py:134-160 (K), :162-203 (dK), :205-236 (M), :238-284 (dM)
 //   node scatter examples/thermal.py:612-615, examples/natural_frequency.py:509-512
-// Shape functions / Jacobian follow examples/fe_utils.py:4-16, 26-44 (2x2 Gauss, +-1/sqrt(3)).
+// Shape functions, Jacobian and strain: q4_element.cuh.
 #include "common.cuh"
+#include "q4_element.cuh"
 #include "../../include/eigd_b200.h"
 
 namespace {
-
-struct Q4Geom {
-  double Nx[4][4], Ny[4][4], N[4][4], detJ[4];  // [gauss point][node]
-};
-
-__device__ __forceinline__ void q4_geometry(const double xe[4], const double ye[4], Q4Geom& g) {
-  const double gp = 0.57735026918962576451;
-#pragma unroll
-  for (int q = 0; q < 4; ++q) {
-    // index = 2*j + i with xi = pts[i], eta = pts[j] (thermal.py:117); sums do not depend on it
-    double xi = (q & 1) ? gp : -gp;
-    double eta = (q & 2) ? gp : -gp;
-    double Nxi[4] = {-0.25 * (1.0 - eta), 0.25 * (1.0 - eta), 0.25 * (1.0 + eta), -0.25 * (1.0 + eta)};
-    double Neta[4] = {-0.25 * (1.0 - xi), -0.25 * (1.0 + xi), 0.25 * (1.0 + xi), 0.25 * (1.0 - xi)};
-    g.N[q][0] = 0.25 * (1.0 - xi) * (1.0 - eta);
-    g.N[q][1] = 0.25 * (1.0 + xi) * (1.0 - eta);
-    g.N[q][2] = 0.25 * (1.0 + xi) * (1.0 + eta);
-    g.N[q][3] = 0.25 * (1.0 - xi) * (1.0 + eta);
-    double J00 = 0, J10 = 0, J01 = 0, J11 = 0;
-#pragma unroll
-    for (int a = 0; a < 4; ++a) {
-      J00 = fma(xe[a], Nxi[a], J00);
-      J10 = fma(ye[a], Nxi[a], J10);
-      J01 = fma(xe[a], Neta[a], J01);
-      J11 = fma(ye[a], Neta[a], J11);
-    }
-    double det = J00 * J11 - J01 * J10;
-    double i00 = J11 / det, i01 = -J01 / det, i10 = -J10 / det, i11 = J00 / det;
-#pragma unroll
-    for (int a = 0; a < 4; ++a) {
-      g.Nx[q][a] = i00 * Nxi[a] + i10 * Neta[a];
-      g.Ny[q][a] = i01 * Nxi[a] + i11 * Neta[a];
-    }
-    g.detJ[q] = det;
-  }
-}
 
 // G lanes per element; lane l handles modes l, l+G, ...
 template <int KIND, int G>
@@ -59,23 +24,16 @@ q4_quadforms_kernel(int nelems, const int* __restrict__ conn, const double* __re
   int e = (int)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) / G);
   const bool valid = e < nelems;
   if (!valid) e = nelems - 1;  // keep the whole warp converged for the shuffles
-  int nd[4];
-  double xe[4], ye[4];
-#pragma unroll
-  for (int a = 0; a < 4; ++a) {
-    nd[a] = conn[e * 4 + a];
-    xe[a] = xy[2 * nd[a]];
-    ye[a] = xy[2 * nd[a] + 1];
-  }
-  Q4Geom g;
-  q4_geometry(xe, ye, g);
+  const Q4Nodes el = q4_gather(conn, xy, e);
+  const Q4Geom g = q4_geometry(el);
+  const Q4C0 c0 = KIND == 1 ? q4_c0_load(cmat) : Q4C0{};  // cmat may be NULL for kind 0
   double sumK = 0.0, sumM = 0.0;
   for (int k = lane; k < N; k += G) {
     if (KIND == 0) {
       double wa[4], wb[4], v[4];
 #pragma unroll
       for (int a = 0; a < 4; ++a) {
-        int64_t o = (int64_t)nd[a] * ldw + k;
+        int64_t o = (int64_t)el.nd[a] * ldw + k;
         v[a] = V[o];
         wa[a] = WA ? WA[o] : 0.0;
         wb[a] = WB ? WB[o] : 0.0;
@@ -99,7 +57,7 @@ q4_quadforms_kernel(int nelems, const int* __restrict__ conn, const double* __re
       double wa[8], wb[8], v[8];
 #pragma unroll
       for (int a = 0; a < 4; ++a) {
-        int64_t o = (int64_t)(2 * nd[a]) * ldw + k;
+        int64_t o = (int64_t)(2 * el.nd[a]) * ldw + k;
         v[2 * a] = V[o];
         v[2 * a + 1] = V[o + ldw];
         wa[2 * a] = WA ? WA[o] : 0.0;
@@ -107,27 +65,20 @@ q4_quadforms_kernel(int nelems, const int* __restrict__ conn, const double* __re
         wb[2 * a] = WB ? WB[o] : 0.0;
         wb[2 * a + 1] = WB ? WB[o + ldw] : 0.0;
       }
-      const double c00 = cmat[0], c01 = cmat[1], c02 = cmat[2], c11 = cmat[3], c12 = cmat[4], c22 = cmat[5];
 #pragma unroll
       for (int q = 0; q < 4; ++q) {
-        double ew[3] = {0, 0, 0}, ev[3] = {0, 0, 0}, hw[2] = {0, 0}, hv[2] = {0, 0};
+        double ew[3], ev[3], s[3], hw[2] = {0, 0}, hv[2] = {0, 0};
+        q4_strain(g.Nx[q], g.Ny[q], wa, ew);
+        q4_strain(g.Nx[q], g.Ny[q], v, ev);
 #pragma unroll
         for (int a = 0; a < 4; ++a) {
-          ew[0] = fma(g.Nx[q][a], wa[2 * a], ew[0]);
-          ew[1] = fma(g.Ny[q][a], wa[2 * a + 1], ew[1]);
-          ew[2] = fma(g.Ny[q][a], wa[2 * a], fma(g.Nx[q][a], wa[2 * a + 1], ew[2]));
-          ev[0] = fma(g.Nx[q][a], v[2 * a], ev[0]);
-          ev[1] = fma(g.Ny[q][a], v[2 * a + 1], ev[1]);
-          ev[2] = fma(g.Ny[q][a], v[2 * a], fma(g.Nx[q][a], v[2 * a + 1], ev[2]));
           hw[0] = fma(g.N[q][a], wb[2 * a], hw[0]);
           hw[1] = fma(g.N[q][a], wb[2 * a + 1], hw[1]);
           hv[0] = fma(g.N[q][a], v[2 * a], hv[0]);
           hv[1] = fma(g.N[q][a], v[2 * a + 1], hv[1]);
         }
-        double s0 = c00 * ev[0] + c01 * ev[1] + c02 * ev[2];
-        double s1 = c01 * ev[0] + c11 * ev[1] + c12 * ev[2];
-        double s2 = c02 * ev[0] + c12 * ev[1] + c22 * ev[2];
-        sumK = fma(g.detJ[q], ew[0] * s0 + ew[1] * s1 + ew[2] * s2, sumK);
+        q4_c0_mul(c0, ev, s);
+        sumK = fma(g.detJ[q], ew[0] * s[0] + ew[1] * s[1] + ew[2] * s[2], sumK);
         sumM = fma(g.detJ[q], hw[0] * hv[0] + hw[1] * hv[1], sumM);
       }
     }
@@ -155,55 +106,33 @@ __global__ void q4_assemble_kernel(int64_t nnz, const int64_t* __restrict__ src_
   int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (p >= nnz) return;
   constexpr int NE = (KIND == 0) ? 4 : 8;
-  const double gp = 0.57735026918962576451;
+  const Q4C0 c0 = KIND == 1 ? q4_c0_load(cmat) : Q4C0{};  // cmat may be NULL for kind 0
   double kv = 0.0, mv = 0.0;
   for (int64_t q = src_ptr[p]; q < src_ptr[p + 1]; ++q) {
     int64_t s = src[q];
     int e = (int)(s / (NE * NE));
     int ab = (int)(s - (int64_t)e * NE * NE);
     int a = ab / NE, b = ab - a * NE;
-    double xe[4], ye[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      int nd = conn[e * 4 + i];
-      xe[i] = xy[2 * nd];
-      ye[i] = xy[2 * nd + 1];
-    }
+    const int ia = KIND == 0 ? a : a >> 1, ib = KIND == 0 ? b : b >> 1;  // element nodes of dofs a, b
+    const Q4Nodes el = q4_gather(conn, xy, e);
     double ke = 0.0, me = 0.0;
 #pragma unroll
     for (int g = 0; g < 4; ++g) {
-      double xi = (g & 1) ? gp : -gp, eta = (g & 2) ? gp : -gp;
-      double Nxi[4] = {-0.25 * (1.0 - eta), 0.25 * (1.0 - eta), 0.25 * (1.0 + eta), -0.25 * (1.0 + eta)};
-      double Neta[4] = {-0.25 * (1.0 - xi), -0.25 * (1.0 + xi), 0.25 * (1.0 + xi), 0.25 * (1.0 - xi)};
-      double Nn[4] = {0.25 * (1.0 - xi) * (1.0 - eta), 0.25 * (1.0 + xi) * (1.0 - eta),
-                      0.25 * (1.0 + xi) * (1.0 + eta), 0.25 * (1.0 - xi) * (1.0 + eta)};
-      double J00 = 0, J10 = 0, J01 = 0, J11 = 0;
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        J00 = fma(xe[i], Nxi[i], J00);
-        J10 = fma(ye[i], Nxi[i], J10);
-        J01 = fma(xe[i], Neta[i], J01);
-        J11 = fma(ye[i], Neta[i], J11);
-      }
-      double det = J00 * J11 - J01 * J10;
-      double i00 = J11 / det, i01 = -J01 / det, i10 = -J10 / det, i11 = J00 / det;
+      double N[4], Nx[4], Ny[4], na, nxa, nya, nb, nxb, nyb;
+      const double det = q4_point(el, g, N, Nx, Ny);
+      q4_node(ia, N, Nx, Ny, na, nxa, nya);
+      q4_node(ib, N, Nx, Ny, nb, nxb, nyb);
       if (KIND == 0) {
-        double nxa = i00 * Nxi[a] + i10 * Neta[a], nya = i01 * Nxi[a] + i11 * Neta[a];
-        double nxb = i00 * Nxi[b] + i10 * Neta[b], nyb = i01 * Nxi[b] + i11 * Neta[b];
         ke = fma(det, nxa * nxb + nya * nyb, ke);
-        me = fma(det, Nn[a] * Nn[b], me);
+        me = fma(det, na * nb, me);
       } else {
-        int na = a >> 1, ca = a & 1, nb = b >> 1, cb = b & 1;
-        double nxa = i00 * Nxi[na] + i10 * Neta[na], nya = i01 * Nxi[na] + i11 * Neta[na];
-        double nxb = i00 * Nxi[nb] + i10 * Neta[nb], nyb = i01 * Nxi[nb] + i11 * Neta[nb];
-        // columns of Be: dof u -> [Nx, 0, Ny], dof v -> [0, Ny, Nx]
-        double ba[3] = {ca ? 0.0 : nxa, ca ? nya : 0.0, ca ? nxa : nya};
-        double bb[3] = {cb ? 0.0 : nxb, cb ? nyb : 0.0, cb ? nxb : nyb};
-        double t0 = cmat[0] * bb[0] + cmat[1] * bb[1] + cmat[2] * bb[2];
-        double t1 = cmat[1] * bb[0] + cmat[3] * bb[1] + cmat[4] * bb[2];
-        double t2 = cmat[2] * bb[0] + cmat[4] * bb[1] + cmat[5] * bb[2];
-        ke = fma(det, ba[0] * t0 + ba[1] * t1 + ba[2] * t2, ke);
-        if (ca == cb) me = fma(det, Nn[na] * Nn[nb], me);
+        const int ca = a & 1, cb = b & 1;
+        double ba[3], bb[3], t[3];
+        q4_strain_rows(ca, nxa, nya, ba);
+        q4_strain_rows(cb, nxb, nyb, bb);
+        q4_c0_mul(c0, bb, t);
+        ke = fma(det, ba[0] * t[0] + ba[1] * t[1] + ba[2] * t[2], ke);
+        if (ca == cb) me = fma(det, na * nb, me);
       }
     }
     kv = fma(ks[e], ke, kv);
