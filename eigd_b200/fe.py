@@ -22,6 +22,7 @@ import torch
 from . import _lib
 from . import device as D
 from ._hostdev import is_dev, to_dev, to_host, like_input
+from .device import _ptr
 
 
 def grid_mesh(nx, ny, Lx=1.0, Ly=1.0):
@@ -81,25 +82,26 @@ def node_adjacency(conn, nnodes):
     return np.cumsum(nptr).astype(np.int32), e[order].astype(np.int32)
 
 
-def _ptr(t):
-    return ctypes.c_void_p(t.data_ptr()) if t is not None else None
-
-
-class _Half:
-    """One of the two reference callbacks ``dAdx(w, v)`` / ``dBdx(w, v)``."""
+class _SensitivityCallback:
+    """A reference sensitivity callback such as ``dAdx(w, v)``: ``which`` of the operators of ``parent``, called with
+    host or device operands; subclasses give its device form ``device_call(W, V)``."""
 
     def __init__(self, parent, which):
         self.parent, self.which = parent, which
-        self.fused_with = None
+
+    def __call__(self, w, v):
+        return like_input(self.device_call(to_dev(w), to_dev(v)), w)
+
+
+class _Half(_SensitivityCallback):
+    """One of the two reference callbacks ``dAdx(w, v)`` / ``dBdx(w, v)``."""
+
+    fused_with = None       # the other half: add_eig_total_derivative then evaluates both in one fused call
 
     def device_call(self, W, V):
         if self.which == "A":
             return self.parent.device_call_fused(W, None, V, 1.0, 0.0)
         return self.parent.device_call_fused(None, W, V, 0.0, 1.0)
-
-    def __call__(self, w, v):
-        out = self.device_call(to_dev(w), to_dev(v))
-        return like_input(out, w)
 
 
 class Q4Problem:
@@ -254,12 +256,8 @@ def reduced_structure(indptr, indices, src_ptr, src, reduced, ndof):
     return r_indptr, r_indices, r_src_ptr, src[pos]
 
 
-class _BucklingCallback:
+class _BucklingCallback(_SensitivityCallback):
     """dAdu / dAdx / dBdx of examples/buckling.py:924-979 as device operators on REDUCED (n_r, N) operands."""
-
-    def __init__(self, parent, which):
-        self.parent, self.which = parent, which
-        self.fused_with = None
 
     def device_call(self, Wr, Vr):
         pr = self.parent
@@ -276,9 +274,6 @@ class _BucklingCallback:
         else:                                                                     # dKdx
             D.q4_quadforms(1, pr.conn_d, pr.xy_d, pr.cmat6_d, W2, None, V2, pr.base.dk_d, pr.base.dm_d, 1.0, 0.0, out)
         return out
-
-    def __call__(self, w, v):
-        return like_input(self.device_call(to_dev(w), to_dev(v)), w)
 
 
 class BucklingQ4Problem:

@@ -19,21 +19,16 @@ The unit matrices E1, E3, F1, F3 are computed once on the host (vectorised numpy
 sensitivities w^T (dK/dt_c) v per component with one warp per element and a warp-shuffle segmented reduction
 (``eigd_stored_quadform``, ``eigd_segment_sum``).
 """
-import ctypes
-import time
-
 import numpy as np
 import torch
 
 from . import _lib
 from . import device as D
 from . import fe
-from ._hostdev import to_dev, to_host, like_input, small_to_dev
-from .eigenvector_derivatives import IRAM, BasicLanczos, SpLuOperator, add_eig_total_derivative
-
-
-def _ptr(t):
-    return ctypes.c_void_p(t.data_ptr()) if t is not None else None
+from ._hostdev import to_dev, to_host, small_to_dev
+from .device import _ptr
+from .eigenvector_derivatives import SpLuOperator, add_eig_total_derivative
+from .topo import _EigenAnalysis, _now
 
 
 # ------------------------------------------------------------------------------------------
@@ -119,17 +114,11 @@ def shell_unit_matrices(conn, X, E=73.1e9, nu=0.33, rho=2780.0, kshear=5.0 / 6.0
 # ------------------------------------------------------------------------------------------
 # device operators
 # ------------------------------------------------------------------------------------------
-class _ShellCallback:
+class _ShellCallback(fe._SensitivityCallback):
     """``dAdx(w, v)`` / ``dBdx(w, v)`` of crm.py:331-355: one value per design variable (component thickness)."""
-
-    def __init__(self, parent, which):
-        self.parent, self.which = parent, which
 
     def device_call(self, W, V):
         return self.parent._sensitivity(self.which, W, V)
-
-    def __call__(self, w, v):
-        return like_input(self.device_call(to_dev(w), to_dev(v)), w)
 
 
 class ShellProblem:
@@ -220,28 +209,15 @@ class ShellProblem:
         return out
 
 
-def _now():
-    torch.cuda.synchronize()
-    return time.perf_counter()
-
-
-class ShellModalAnalysis:
+class ShellModalAnalysis(_EigenAnalysis):
     """The ``CRM`` driver of examples/crm.py (:19-376) on the synthetic shell: same method names, same ``profile`` keys,
     modal-compliance objective with f[1::6] = 1 (:267-293), per-mode "vector" total derivative (:357-370)."""
 
     def __init__(self, prob, N=10, m=None, omega0=10.0, solver_type="IRAM", tol=1e-14, rtol=1e-10, eig_atol=1e-5,
                  adjoint_method="sibk", adjoint_options=None, deriv_type="vector", seed=0):
-        self.prob = prob
-        self.N, self.m, self.omega0 = N, m, omega0
-        self.solver_type, self.tol, self.rtol, self.eig_atol = solver_type, tol, rtol, eig_atol
-        self.adjoint_method = "sibk" if adjoint_method == "shift-invert" else adjoint_method
-        self.adjoint_options = dict(adjoint_options or {})
-        self.deriv_type = deriv_type
-        self.seed = seed
+        super().__init__(prob, N, m, solver_type, tol, rtol, eig_atol, adjoint_method, adjoint_options, deriv_type, seed)
+        self.omega0 = omega0
         self.x = np.ones(prob.ncomp)                       # crm.py: t = 0.01, scale 100
-        self.symbolic = None
-        self.sharding = None
-        self.profile = {}
         f = np.zeros(prob.ndof_full)
         f[1::6] = 1.0
         self.fr_d = to_dev(f[prob.reduced])
@@ -263,33 +239,12 @@ class ShellModalAnalysis:
         sigma = self.omega0 ** 2
         self.sigma = sigma
         vals = D.axpby(1.0, self.Kr.data, -float(sigma), self.Mr.data)
-        if self.symbolic is None:
-            ts = _now()
-            coords, dofpn = p.dof_coords()
-            sym = D.Symbolic(p.indptr, p.indices, p.ndof, coords=coords, dof_per_node=dofpn)
-            self.symbolic = (sym, sym.assembly_map_device(self.Kr.indptr, self.Kr.indices))
-            self.profile["symbolic analysis time"] = _now() - ts
-            t1 = _now()
+        if self._symbolic_once(self.Kr) is not None:
+            t1 = _now()                                    # the eigensolve time excludes the analysis
         self.factor = SpLuOperator(self.Kr.with_values(vals), symbolic=self.symbolic)
-        self.factor.count = 0
-        if self.solver_type == "IRAM":
-            if self.m is None:
-                self.m = max(2 * self.N + 1, 60)
-            self.eig_solver = IRAM(N=self.N, m=self.m, eig_atol=self.eig_atol)
-            self.eig_solver.seed = self.seed
-        else:
-            if self.m is None:
-                self.m = max(3 * self.N + 1, 60)
-            self.eig_solver = BasicLanczos(N=self.N, m=self.m, eig_atol=self.eig_atol, tol=self.tol)
-        self.eig_solver.sharding = self.sharding
-        self.lam, _ = self.eig_solver.solve(self.Kr, self.Mr, self.factor, sigma)
-        self.lam = np.asarray(self.lam)
+        self._new_eig_solver(self.N)
+        self.lam = np.asarray(self._eigensolve(self.Kr, self.Mr, sigma, t1))
         self.Q = self.eig_solver._Phi_d
-        t2 = _now()
-        self.profile["eigenvalue solve time"] = t2 - t1
-        self.profile["solve preconditioner count"] = self.factor.count
-        self.profile["m"] = self.m
-        self.profile["eig_solver.m"] = str(self.eig_solver.m)
 
     def initialize_adjoint(self):
         self.Qb = D.zeros(self.prob.ndof, self.N)
@@ -306,18 +261,11 @@ class ShellModalAnalysis:
         D.gemm_nn(self.fr_d.unsqueeze(1), small_to_dev((2.0 * compb * val / self.lam)[None, :]), self.Qb, alpha=1.0, beta=1.0)
         self.lamb -= compb * (val * val) / self.lam ** 2
 
-    def finalize_adjoint(self):
-        res_list = []
-        self.factor.count = 0
-        t0 = _now()
-        psi, corr_data = self.eig_solver.solve_adjoint(self.Qb, rtol=self.rtol, method=self.adjoint_method,
-                                                       callback=res_list.append, **self.adjoint_options)
-        t1 = _now()
+    def _eigenvector_seeds(self):
+        return self.Qb
+
+    def _total_derivative(self, psi, corr_data):
         self.psi = psi
-        self.profile["adjoint preconditioner count"] = self.factor.count
-        self.profile["adjoint solution time"] = t1 - t0
-        self.profile["adjoint residuals"] = res_list
-        self.profile["adjoint correction data"] = corr_data
         grad = D.zeros(self.prob.ncomp)
         shard = self.sharding
         if shard is not None and shard.world > 1 and self.deriv_type == "vector":
@@ -326,12 +274,6 @@ class ShellModalAnalysis:
         else:
             self.grad = add_eig_total_derivative(self.lam, self.Q, self.lamb, self.Qb, psi, self.prob.dAdx, self.prob.dBdx, grad,
                                                  adj_corr_data=corr_data, deriv_type=self.deriv_type)
-        t2 = _now()
-        self.profile["total derivative time"] = t2 - t1
-
-    def time_to_gradient(self):
-        p = self.profile
-        return p["eigenvalue solve time"] + p["adjoint solution time"] + p["total derivative time"]
 
 
 def _sharded_vector_derivative(model, psi, corr_data, shard):

@@ -28,7 +28,90 @@ def _now():
     return time.perf_counter()
 
 
-class _Q4Analysis:
+class _EigenAnalysis:
+    """Forward and reverse pipeline shared by the model drivers.
+
+    A driver's forward pass assembles its pencil, analyses the pattern with ``_symbolic_once``, factors the shifted
+    matrix into ``self.factor`` and runs ``_new_eig_solver`` and ``_eigensolve``.  Its reverse pass is
+    ``finalize_adjoint`` here, with the driver's eigenvector seeds (``_eigenvector_seeds``) and total derivative
+    (``_total_derivative``)."""
+
+    def __init__(self, prob, N, m, solver_type, tol, rtol, eig_atol, adjoint_method, adjoint_options, deriv_type, seed):
+        self.prob = prob
+        self.N, self.m = N, m
+        self.solver_type, self.tol, self.rtol, self.eig_atol = solver_type, tol, rtol, eig_atol
+        if adjoint_method == "shift-invert":          # the examples' historical alias (thermal.py:37)
+            adjoint_method = "sibk"
+        self.adjoint_method = adjoint_method
+        self.adjoint_options = dict(adjoint_options or {})
+        self.deriv_type = deriv_type
+        self.seed = seed              # IRAM start vector (deterministic: the eigensolve is replicated when sharded)
+        self.Q = self.lam = None
+        self.symbolic = None
+        self.sharding = None          # dist.ModeSharding for the per-mode adjoint / element-range shards
+        self.profile = {}
+
+    # ---- forward ------------------------------------------------------------------------------
+    def _symbolic_once(self, K):
+        """Symbolic analysis of the pattern of ``self.prob``'s system matrix K, once per sparsity pattern.  Returns its
+        time, or None when the analysis of an earlier call is reused."""
+        if self.symbolic is not None:
+            return None
+        ts = _now()
+        coords, dofpn = self.prob.dof_coords()
+        sym = D.Symbolic(self.prob.indptr, self.prob.indices, K.shape[0], coords=coords, dof_per_node=dofpn)
+        self.symbolic = (sym, sym.assembly_map_device(K.indptr, K.indices))
+        self.profile["symbolic analysis time"] = dt = _now() - ts
+        return dt
+
+    def _new_eig_solver(self, N, iram=None, lanczos=None):
+        """``self.eig_solver`` for N modes: IRAM or BasicLanczos by ``solver_type``, with the driver's own extra arguments
+        of each (``iram``, ``lanczos``).  ``self.m`` gets its default on the first call and keeps it."""
+        if self.solver_type == "IRAM":
+            if self.m is None:
+                self.m = max(2 * N + 1, 60)
+            self.eig_solver = IRAM(N=N, m=self.m, eig_atol=self.eig_atol, **(iram or {}))
+            self.eig_solver.seed = self.seed
+        else:
+            if self.m is None:
+                self.m = max(3 * N + 1, 60)
+            self.eig_solver = BasicLanczos(N=N, m=self.m, eig_atol=self.eig_atol, tol=self.tol, **(lanczos or {}))
+
+    def _eigensolve(self, A, B, sigma, t1):
+        """``self.eig_solver`` on the pencil (A, B) about ``sigma`` with ``self.factor``; the eigenvalue solve time runs
+        from ``t1``.  Returns the eigenvalues."""
+        self.factor.count = 0
+        self.eig_solver.sharding = self.sharding
+        lam, _ = self.eig_solver.solve(A, B, self.factor, sigma)
+        t2 = _now()
+        self.profile["solve preconditioner count"] = self.factor.count
+        self.profile["eigenvalue solve time"] = t2 - t1
+        self.profile["m"] = self.m
+        self.profile["eig_solver.m"] = str(self.eig_solver.m)
+        return lam
+
+    # ---- reverse ------------------------------------------------------------------------------
+    def finalize_adjoint(self):
+        res_list = []
+        self.factor.count = 0
+        t0 = _now()
+        psi, corr_data = self.eig_solver.solve_adjoint(self._eigenvector_seeds(), rtol=self.rtol, method=self.adjoint_method,
+                                                       callback=res_list.append, **self.adjoint_options)
+        t1 = _now()
+        self.profile["adjoint preconditioner count"] = self.factor.count
+        self.profile["adjoint solution time"] = t1 - t0
+        self.profile["adjoint residuals"] = res_list
+        self.profile["adjoint iterations"] = len(res_list)
+        self.profile["adjoint correction data"] = corr_data
+        self._total_derivative(psi, corr_data)
+        self.profile["total derivative time"] = _now() - t1
+
+    def time_to_gradient(self):
+        p = self.profile
+        return p["eigenvalue solve time"] + p["adjoint solution time"] + p["total derivative time"]
+
+
+class _Q4Analysis(_EigenAnalysis):
     kind = "thermal"
     nrigid = 0            # leading modes computed but dropped (rigid-body modes of the free structure)
 
@@ -36,22 +119,13 @@ class _Q4Analysis:
                  eig_atol=1e-5, adjoint_method="sibk", adjoint_options=None, deriv_type="tensor", seed=0, **material):
         self.fltr = fltr
         self.conn, self.X = np.asarray(conn), np.asarray(X)
-        self.prob = fe.Q4Problem(self.conn, self.X, self.kind, **material)
+        super().__init__(fe.Q4Problem(self.conn, self.X, self.kind, **material), N, m, solver_type, tol, rtol, eig_atol,
+                         adjoint_method, adjoint_options, deriv_type, seed)
         self.nelems, self.nnodes, self.nvars = self.prob.nelems, self.prob.nnodes, self.prob.ndof
-        self.sigma, self.N, self.m, self.Ntarget = sigma, N, m, Ntarget
-        self.solver_type, self.tol, self.rtol, self.eig_atol = solver_type, tol, rtol, eig_atol
-        if adjoint_method == "shift-invert":          # the examples' historical alias (thermal.py:37)
-            adjoint_method = "sibk"
-        self.adjoint_method = adjoint_method
-        self.adjoint_options = dict(adjoint_options or {})
-        self.deriv_type = deriv_type
-        self.seed = seed
+        self.sigma, self.Ntarget = sigma, Ntarget
         self.x = 0.95 * np.ones(self.fltr.num_design_vars)      # thermal.py:71, natural_frequency.py:75
-        self.Q = self.lam = None
-        self.symbolic = None
-        self.sharding = None          # dist.ModeSharding for the per-mode adjoint / element-range shards
-        self.profile = {"nnodes": self.nnodes, "nelems": self.nelems, "solver_type": solver_type,
-                        "adjoint_method": adjoint_method, "N": N}
+        self.profile.update(nnodes=self.nnodes, nelems=self.nelems, solver_type=solver_type,
+                            adjoint_method=self.adjoint_method, N=N)
 
     # ---- forward ------------------------------------------------------------------------------
     def solve_eigenvalue_problem(self, store=False):
@@ -59,36 +133,14 @@ class _Q4Analysis:
         K, M = self.prob.assemble()
         t1 = _now()
         self.profile["matrix assembly time"] = t1 - t0
-        vals = D.axpby(1.0, K.data, -float(self.sigma), M.data)           # K - sigma M on the shared pattern
-        shifted = K.with_values(vals)
-        coords, dofpn = self.prob.dof_coords()
-        if self.symbolic is None:                                         # once per sparsity pattern
-            ts = _now()
-            sym = D.Symbolic(self.prob.indptr, self.prob.indices, self.nvars, coords=coords, dof_per_node=dofpn)
-            self.symbolic = (sym, sym.assembly_map_device(K.indptr, K.indices))
-            self.profile["symbolic analysis time"] = _now() - ts
-            t1 = _now()
+        shifted = K.with_values(D.axpby(1.0, K.data, -float(self.sigma), M.data))    # K - sigma M on the shared pattern
+        if self._symbolic_once(K) is not None:
+            t1 = _now()                                                   # the eigensolve time excludes the analysis
         self.factor = SpLuOperator(shifted, symbolic=self.symbolic)
         self.K, self.M = K, M
-        self.factor.count = 0
-        ncomp = self.N + self.nrigid
-        if self.solver_type == "IRAM":
-            if self.m is None:
-                self.m = max(2 * ncomp + 1, 60)
-            self.eig_solver = IRAM(N=ncomp, m=self.m, eig_atol=self.eig_atol, tol=self.tol)
-            self.eig_solver.seed = self.seed
-        else:
-            if self.m is None:
-                self.m = max(3 * ncomp + 1, 60)
-            self.eig_solver = BasicLanczos(N=ncomp, m=self.m, eig_atol=self.eig_atol, tol=self.tol, Ntarget=self.Ntarget)
-        self.eig_solver.sharding = self.sharding
+        self._new_eig_solver(self.N + self.nrigid, iram=dict(tol=self.tol), lanczos=dict(Ntarget=self.Ntarget))
         self.prob.sharding = self.sharding
-        lam, _ = self.eig_solver.solve(K, M, self.factor, self.sigma)
-        t2 = _now()
-        self.profile["solve preconditioner count"] = self.factor.count
-        self.profile["eigenvalue solve time"] = t2 - t1
-        self.profile["m"] = self.m
-        self.profile["eig_solver.m"] = str(self.eig_solver.m)
+        lam = self._eigensolve(K, M, self.sigma, t1)
         self.lam0 = np.asarray(lam)
         self.Q0 = self.eig_solver._Phi_d                                   # (n, N + nrigid) device
         return self.lam0[self.nrigid:], self.Q0[:, self.nrigid:]
@@ -120,19 +172,13 @@ class _Q4Analysis:
         self.rhoE = self.prob.set_density(rho=self.rho)
         K, M = self.prob.assemble()
         Kt, Mt = self.prob.assemble_tangent(rho_t)
-        coords, dofpn = self.prob.dof_coords()
-        if self.symbolic is None:
-            sym = D.Symbolic(self.prob.indptr, self.prob.indices, self.nvars, coords=coords, dof_per_node=dofpn)
-            self.symbolic = (sym, sym.assembly_map_device(K.indptr, K.indices))
+        self._symbolic_once(K)
         shifted = K.with_values(D.axpby(1.0, K.data, -float(self.sigma), M.data))
         self.factor = SpLuOperator(shifted, symbolic=self.symbolic)
         self.factor.tangent = K.with_values(D.axpby(1.0, Kt.data, -float(self.sigma), Mt.data))
         self.factor.dtype = np.dtype(np.complex128)
         self.K, self.M = K, M
-        ncomp = self.N + self.nrigid
-        if self.m is None:
-            self.m = max(3 * ncomp + 1, 60)
-        self.eig_solver = BasicLanczos(N=ncomp, m=self.m, eig_atol=self.eig_atol, tol=self.tol, Ntarget=self.Ntarget)
+        self._new_eig_solver(self.N + self.nrigid, lanczos=dict(Ntarget=self.Ntarget))
         lam, Phi = self.eig_solver.solve((K, Kt), (M, Mt), self.factor, self.sigma)
         self.lam0, self.Q0 = np.asarray(lam), np.asarray(Phi)               # complex host arrays
         self.lam, self.Q = self.lam0[self.nrigid:], self.Q0[:, self.nrigid:]
@@ -147,20 +193,12 @@ class _Q4Analysis:
         self.Qb = self.Q0b[:, self.nrigid:]
 
     # ---- reverse ------------------------------------------------------------------------------
-    def finalize_adjoint(self):
-        res_list = []
-        self.factor.count = 0
-        t0 = _now()
-        psi0, corr_data = self.eig_solver.solve_adjoint(self.Q0b, rtol=self.rtol, method=self.adjoint_method,
-                                                        callback=res_list.append, **self.adjoint_options)
-        t1 = _now()
+    def _eigenvector_seeds(self):
+        return self.Q0b
+
+    def _total_derivative(self, psi0, corr_data):
         self.psi0 = psi0
         self.psi = psi0[:, self.nrigid:]
-        self.profile["adjoint preconditioner count"] = self.factor.count
-        self.profile["adjoint solution time"] = t1 - t0
-        self.profile["adjoint residuals"] = res_list
-        self.profile["adjoint iterations"] = len(res_list)
-        self.profile["adjoint correction data"] = corr_data
         nr = self.nrigid
         if nr:                                                            # natural_frequency.py:484-494
             data0 = {}
@@ -176,13 +214,6 @@ class _Q4Analysis:
         rhob = self.prob.scatter_to_nodes(self.rhoEb)
         g = self.fltr.apply_gradient(rhob, self.x_d)
         D.axpby(1.0, self.xb, 1.0, g, out=self.xb)
-        t2 = _now()
-        self.profile["total derivative time"] = t2 - t1
-        return
-
-    def time_to_gradient(self):
-        p = self.profile
-        return p["eigenvalue solve time"] + p["adjoint solution time"] + p["total derivative time"]
 
 
 class ThermalTopologyAnalysis(_Q4Analysis):
@@ -408,7 +439,7 @@ def make_natural_frequency_model(nx=128, ny=64, Lx=1.0, Ly=1.0, rfact=4.0, N=10,
 # ------------------------------------------------------------------------------------------
 # linearised buckling -- examples/buckling.py
 # ------------------------------------------------------------------------------------------
-class BucklingTopologyAnalysis:
+class BucklingTopologyAnalysis(_EigenAnalysis):
     """examples/buckling.py ``TopologyAnalysis`` (:19-118): (K + BLF * G(u)) phi = 0 on the reduced dofs, with
     the fundamental path K_r u_r = f_r, shift-invert about ``sigma`` (mode="buckling": A = G_r, B = K_r,
     factor of K_r + sigma G_r, :548-640), and the gradient of an eigenvector functional including the
@@ -422,40 +453,24 @@ class BucklingTopologyAnalysis:
                  adjoint_options=None, cost=1, deriv_type="tensor", seed=0, pivoting="static"):
         self.fltr = fltr
         self.pivoting = pivoting          # of the shifted factor K_r + sigma G_r (SpLuOperator); K_r alone is SPD
-        self.seed = seed                  # IRAM start vector (deterministic: the eigensolve is replicated when sharded)
         self.conn, self.X = np.asarray(conn), np.asarray(X)
-        self.prob = fe.BucklingQ4Problem(self.conn, self.X, bcs, forces, E=E, nu=nu, density=density, p=float(p),
-                                         q=float(q), rho0_K=rho0_K, rho0_G=rho0_G, ptype_K=ptype_K.lower(),
-                                         ptype_G=ptype_G.lower())
+        prob = fe.BucklingQ4Problem(self.conn, self.X, bcs, forces, E=E, nu=nu, density=density, p=float(p), q=float(q),
+                                    rho0_K=rho0_K, rho0_G=rho0_G, ptype_K=ptype_K.lower(), ptype_G=ptype_G.lower())
+        super().__init__(prob, N, m, solver_type, tol, rtol, eig_atol, adjoint_method, adjoint_options, deriv_type, seed)
         self.nelems, self.nnodes, self.nvars = self.prob.nelems, self.prob.nnodes, self.prob.ndof
         self.reduced, self.f = self.prob.reduced, self.prob.f
         self.E, self.nu, self.p, self.q, self.density = E, nu, p, q, density
         self.rho0_K, self.rho0_G = rho0_K, rho0_G
-        self.sigma, self.N, self.m = sigma, N, m
-        self.solver_type, self.tol, self.rtol, self.eig_atol = solver_type, tol, rtol, eig_atol
-        if adjoint_method == "shift-invert":
-            adjoint_method = "sibk"
-        self.adjoint_method = adjoint_method
-        self.adjoint_options = dict(adjoint_options or {})
-        self.cost, self.deriv_type = cost, deriv_type
+        self.sigma, self.cost = sigma, cost
         self.x = 0.5 * np.ones(self.fltr.num_design_vars)                 # buckling.py:81
-        self.symbolic = None
-        self.sharding = None
-        self.Q = self.lam = None
-        self.profile = {"nnodes": self.nnodes, "nelems": self.nelems, "solver_type": solver_type,
-                        "adjoint_method": adjoint_method, "N": N}
+        self.profile.update(nnodes=self.nnodes, nelems=self.nelems, solver_type=solver_type,
+                            adjoint_method=self.adjoint_method, N=N)
 
     # ---- forward (:548-640, 811-838) ----------------------------------------------------------------
     def solve_eigenvalue_problem(self, store=False):
         t0 = _now()
         Kr = self.prob.assemble_K()
-        if self.symbolic is None:                                         # once per sparsity pattern
-            ts = _now()
-            coords, dofpn = self.prob.dof_coords()
-            sym = D.Symbolic(self.prob.indptr, self.prob.indices, self.prob.nred, coords=coords, dof_per_node=dofpn)
-            self.symbolic = (sym, sym.assembly_map_device(Kr.indptr, Kr.indices))
-            self.profile["symbolic analysis time"] = _now() - ts
-            t0 += self.profile["symbolic analysis time"]
+        t0 += self._symbolic_once(Kr) or 0.0                              # the assembly time excludes the analysis
         self.Kfact = SpLuOperator(Kr, symbolic=self.symbolic, max_rhs=1)  # fundamental path K_r u_r = f_r
         ur = self.Kfact.solve_dev(self.prob.fr_d)
         self.u_d = self.prob.set_displacement(ur)
@@ -464,26 +479,12 @@ class BucklingTopologyAnalysis:
         self.profile["matrix assembly time"] = t1 - t0
         vals = D.axpby(1.0, Kr.data, float(self.sigma), Gr.data)          # K_r + sigma G_r on the shared pattern
         self.factor = SpLuOperator(Kr.with_values(vals), symbolic=self.symbolic, pivoting=self.pivoting)
-        self.factor.count = 0
         self.Kr, self.Gr = Kr, Gr
+        self._new_eig_solver(self.N, iram=dict(mode="buckling"), lanczos=dict(mode="buckling"))
         if self.solver_type == "IRAM":
-            if self.m is None:
-                self.m = max(2 * self.N + 1, 60)
-            self.eig_solver = IRAM(N=self.N, m=self.m, eig_atol=self.eig_atol, mode="buckling")
-            self.eig_solver.seed = self.seed
             self.eig_solver.reference_pairing = getattr(self, "reference_pairing", False)
             self.eig_solver.block_size = getattr(self, "block_size", None)
-        else:
-            if self.m is None:
-                self.m = max(3 * self.N + 1, 60)
-            self.eig_solver = BasicLanczos(N=self.N, m=self.m, eig_atol=self.eig_atol, tol=self.tol, mode="buckling")
-        self.eig_solver.sharding = self.sharding
-        mu, _ = self.eig_solver.solve(Gr, Kr, self.factor, self.sigma)
-        t2 = _now()
-        self.profile["solve preconditioner count"] = self.factor.count
-        self.profile["eigenvalue solve time"] = t2 - t1
-        self.profile["m"] = self.m
-        self.profile["eig_solver.m"] = str(self.eig_solver.m)
+        mu = self._eigensolve(Gr, Kr, self.sigma, t1)
         self.BLF = np.asarray(mu)[: self.N]
         self.Qr = self.eig_solver._Phi_d                                   # (n_r, N) device
         return self.BLF, self.Qr
@@ -583,19 +584,11 @@ class BucklingTopologyAnalysis:
         return like_input(g, self.x)
 
     # ---- reverse (:866-982) -------------------------------------------------------------------------
-    def finalize_adjoint(self):
-        res_list = []
-        self.factor.count = 0
-        t0 = _now()
-        psir, corr_data = self.eig_solver.solve_adjoint(self.Qrb, rtol=self.rtol, method=self.adjoint_method,
-                                                        callback=res_list.append, **self.adjoint_options)
-        t1 = _now()
+    def _eigenvector_seeds(self):
+        return self.Qrb
+
+    def _total_derivative(self, psir, corr_data):
         self.psir = psir
-        self.profile["adjoint preconditioner count"] = self.factor.count
-        self.profile["adjoint solution time"] = t1 - t0
-        self.profile["adjoint residuals"] = res_list
-        self.profile["adjoint iterations"] = len(res_list)
-        self.profile["adjoint correction data"] = corr_data
         pr = self.prob
         # d/du of the eigen-terms: dfdu0 = sum_i w_i^T (dG/du) phi_i  (dB/du = 0: K does not depend on u)
         dfdu0 = D.zeros(self.nvars)
@@ -611,13 +604,6 @@ class BucklingTopologyAnalysis:
         self.rhob = pr.scatter_to_nodes(self.rhoEb)
         g = self.fltr.apply_gradient(self.rhob, self.x_d)
         D.axpby(1.0, self.xb, 1.0, g, out=self.xb)
-        t2 = _now()
-        self.profile["total derivative time"] = t2 - t1
-        return
-
-    def time_to_gradient(self):
-        p = self.profile
-        return p["eigenvalue solve time"] + p["adjoint solution time"] + p["total derivative time"]
 
 
 def domain_compressed_column(nx=64, ny=128, Lx=1.0, Ly=2.0, shear_force=False):
