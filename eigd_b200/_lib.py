@@ -60,14 +60,16 @@ SIGNATURES = {
     "eigd_lanczos_extend": (c_int, [c_ptr, c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_int, c_int, c_ptr, c_ptr, c_ptr,
                                     c_ptr, c_int, c_ptr]),
     "eigd_stored_assemble": (c_int, [c_i64, c_ptr, c_ptr, c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr]),
-    "eigd_stored_quadform": (c_int, [c_int, c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_int, c_i64, c_ptr]),
+    "eigd_stored_quadform": (c_int, [c_int, c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_int, c_i64, c_ptr, c_ptr,
+                                     c_ptr, c_ptr, c_dbl, c_dbl]),
     "eigd_segment_sum": (c_int, [c_int, c_ptr, c_ptr, c_ptr, c_dbl, c_ptr]),
     "eigd_block_lanczos_extend": (c_int, [c_ptr, c_int, c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_int, c_int, c_int,
                                           c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr]),
     "eigd_block_lanczos_start": (c_int, [c_int, c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_ptr, c_ptr]),
     "eigd_q4_assemble": (c_int, [c_int, c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_ptr, c_ptr]),
     "eigd_q4_quadforms": (c_int, [c_int, c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_int, c_int, c_ptr, c_ptr, c_dbl, c_dbl, c_ptr]),
-    "eigd_q4_material": (c_int, [c_int, c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr]),
+    "eigd_q4_material": (c_int, [c_int, c_int, c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr]),
+    "eigd_h8_element_matrices": (c_int, [c_int, c_ptr, c_ptr, c_dbl, c_dbl, c_dbl, c_ptr, c_ptr]),
     "eigd_node_gather": (c_int, [c_int, c_ptr, c_ptr, c_ptr, c_dbl, c_ptr]),
     "eigd_filter_project": (c_int, [c_int, c_dbl, c_dbl, c_ptr, c_ptr, c_ptr]),
     "eigd_q4_stress": (c_int, [c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr]),

@@ -214,13 +214,14 @@ extern "C" int eigd_filter_project(int n, double beta, double eta, const double*
 }
 
 // ---- element density and material interpolation ----------------------------------------------
-// rhoE[e] = 1/4 sum_a rho[conn[e, a]]          (examples/thermal.py:348-353, natural_frequency.py:399-404)
+// rhoE[e] = 1/npe sum_a rho[conn[e, a]]        (examples/thermal.py:348-353, natural_frequency.py:399-404)
+//   npe = 4 (Q4) or 8 (H8) nodes per element
 // law 0 (thermal.py:132,198,175-188,236-244): ks = k0((1-b) r^p + b), ms = c0((1-b) r + b)
 // law 1 (natural_frequency.py:140-143,219-220 "simp"): ks = r^p + r0, ms = c0 r
 // law 2 (RAMP, natural_frequency.py:142-143): ks = r/(1+q(1-r)) + r0, ms = c0 r
 // par = {p or q, k0, c0, b or r0}
 namespace {
-__global__ void q4_material_kernel(int law, int nelems, const int* __restrict__ conn, const double* __restrict__ rho,
+__global__ void q4_material_kernel(int law, int nelems, int npe, const int* __restrict__ conn, const double* __restrict__ rho,
                                    double p0, double k0, double c0, double b, double* __restrict__ rhoE,
                                    double* __restrict__ ks, double* __restrict__ ms, double* __restrict__ dk,
                                    double* __restrict__ dm) {
@@ -228,7 +229,11 @@ __global__ void q4_material_kernel(int law, int nelems, const int* __restrict__ 
   if (e >= nelems) return;
   double r;
   if (conn) {
-    r = 0.25 * (rho[conn[4 * e]] + rho[conn[4 * e + 1]] + rho[conn[4 * e + 2]] + rho[conn[4 * e + 3]]);
+    const int* c = conn + (int64_t)npe * e;
+    if (npe == 4)
+      r = 0.25 * (rho[c[0]] + rho[c[1]] + rho[c[2]] + rho[c[3]]);
+    else
+      r = 0.125 * (rho[c[0]] + rho[c[1]] + rho[c[2]] + rho[c[3]] + rho[c[4]] + rho[c[5]] + rho[c[6]] + rho[c[7]]);
     if (rhoE) rhoE[e] = r;
   } else {
     r = rho[e];
@@ -258,11 +263,12 @@ __global__ void q4_material_kernel(int law, int nelems, const int* __restrict__ 
 }
 }  // namespace
 
-extern "C" int eigd_q4_material(int law, int nelems, const int* d_conn, const double* d_rho, const double* par4,
+extern "C" int eigd_q4_material(int law, int nelems, int npe, const int* d_conn, const double* d_rho, const double* par4,
                                 double* d_rhoE, double* d_ks, double* d_ms, double* d_dk, double* d_dm) {
   if (nelems <= 0) return 0;
   if (law < 0 || law > 2) { eigd_set_error("q4_material: unknown law %d", law); return 1; }
-  EIGD_LAUNCH(q4_material_kernel, (nelems + 255) / 256, 256, 0, law, nelems, d_conn, d_rho, par4[0], par4[1], par4[2],
+  if (npe != 4 && npe != 8) { eigd_set_error("q4_material: %d nodes per element (4: Q4, 8: H8)", npe); return 1; }
+  EIGD_LAUNCH(q4_material_kernel, (nelems + 255) / 256, 256, 0, law, nelems, npe, d_conn, d_rho, par4[0], par4[1], par4[2],
               par4[3], d_rhoE, d_ks, d_ms, d_dk, d_dm);
   EIGD_CHECK_LAUNCH();
   return 0;

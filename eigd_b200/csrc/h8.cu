@@ -1,0 +1,78 @@
+// Unit element matrices of the trilinear hexahedron (H8), computed once per mesh and kept in HBM: the per-design
+// assembly and sensitivities of the 3-D solid then run on the stored-matrix kernels of stored_fe.cu, which read each
+// 24 x 24 matrix once instead of evaluating 8 Jacobians for each of its 576 entries.
+//
+//   K0_e = sum_q detJ B^T C B                      (isotropic elasticity, E and nu)
+//   M0_e = density sum_q detJ (N N^T (x) I_3)      (consistent mass)
+//
+// dof order node-major (u_x, u_y, u_z), as fe.element_dofs(conn, 3).  Element: h8_element.cuh.
+#include "common.cuh"
+#include "h8_element.cuh"
+#include "../../include/eigd_b200.h"
+
+namespace {
+
+// One warp per element.  Lane b < 24 owns column b (node b / 3, component b % 3) of both matrices; lane l works on
+// node l & 7 of the shape-function and Jacobian routine, and the values of node a are read from lane a by shuffles.
+// K0 and M0 are stored row-major, row a written by lanes 0..23 at once (coalesced).
+__global__ void __launch_bounds__(256)
+h8_element_matrices_kernel(int nelems, const int* __restrict__ conn, const double* __restrict__ X, H8C c, double density,
+                           double* __restrict__ K0, double* __restrict__ M0) {
+  const int lane = threadIdx.x & 31;
+  const int64_t e = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  if (e >= nelems) return;  // whole warps only: blockDim is a multiple of 32
+  const int a = lane & 7;
+  const H8Node nd = h8_gather(conn, X, e, a);
+  const int bn = lane < 24 ? lane / 3 : 0, cb = lane < 24 ? lane % 3 : 0;
+  double kc[24], mc[8];
+#pragma unroll
+  for (int i = 0; i < 24; ++i) kc[i] = 0.0;
+#pragma unroll
+  for (int i = 0; i < 8; ++i) mc[i] = 0.0;
+#pragma unroll 1
+  for (int q = 0; q < 8; ++q) {
+    double N, Nx, Ny, Nz;
+    const double det = h8_point(nd, a, q, N, Nx, Ny, Nz);
+    const double nb = __shfl_sync(0xffffffffu, N, bn), nxb = __shfl_sync(0xffffffffu, Nx, bn);
+    const double nyb = __shfl_sync(0xffffffffu, Ny, bn), nzb = __shfl_sync(0xffffffffu, Nz, bn);
+    double bb[6], s[6];
+    h8_strain_rows(cb, nxb, nyb, nzb, bb);
+    h8_c_mul(c, bb, s);
+#pragma unroll
+    for (int an = 0; an < 8; ++an) {
+      const double na = __shfl_sync(0xffffffffu, N, an), nxa = __shfl_sync(0xffffffffu, Nx, an);
+      const double nya = __shfl_sync(0xffffffffu, Ny, an), nza = __shfl_sync(0xffffffffu, Nz, an);
+#pragma unroll
+      for (int ca = 0; ca < 3; ++ca) {
+        double ba[6];
+        h8_strain_rows(ca, nxa, nya, nza, ba);
+        double t = 0.0;
+#pragma unroll
+        for (int i = 0; i < 6; ++i) t = fma(ba[i], s[i], t);
+        kc[3 * an + ca] = fma(det, t, kc[3 * an + ca]);
+      }
+      mc[an] = fma(det, na * nb, mc[an]);
+    }
+  }
+  if (lane >= 24) return;
+  double* k = K0 + e * 576 + lane;
+  double* m = M0 + e * 576 + lane;
+#pragma unroll
+  for (int r = 0; r < 24; ++r) {
+    k[r * 24] = kc[r];
+    m[r * 24] = (r % 3 == cb) ? density * mc[r / 3] : 0.0;
+  }
+}
+
+}  // namespace
+
+extern "C" int eigd_h8_element_matrices(int nelems, const int* d_conn, const double* d_X, double E, double nu, double density,
+                                        double* d_K0, double* d_M0) {
+  if (nelems <= 0) return 0;
+  if (!(nu > -1.0 && nu < 0.5)) { eigd_set_error("h8_element_matrices: Poisson ratio %g outside (-1, 0.5)", nu); return 1; }
+  const H8C c = {E * nu / ((1.0 + nu) * (1.0 - 2.0 * nu)), E / (2.0 * (1.0 + nu))};
+  const int grid = (int)(((int64_t)nelems * 32 + 255) / 256);
+  EIGD_LAUNCH(h8_element_matrices_kernel, grid, 256, 0, nelems, d_conn, d_X, c, density, d_K0, d_M0);
+  EIGD_CHECK_LAUNCH();
+  return 0;
+}

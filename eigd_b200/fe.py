@@ -1,4 +1,4 @@
-"""Device-side finite-element operators for the Q4 problems of the reference examples.
+"""Device-side finite-element operators for the Q4 problems of the reference examples and the H8 solid.
 
 Host part (numpy, runs once per mesh): mesh numbering, DOF maps, the CSR pattern of K/M and the
 integer assembly maps (element, a, b) -> CSR non-zero, node -> element adjacency, the conic
@@ -37,6 +37,22 @@ def grid_mesh(nx, ny, Lx=1.0, Ly=1.0):
     conn[:, 1] = nodes[1:, :-1].T.ravel()
     conn[:, 2] = nodes[1:, 1:].T.ravel()
     conn[:, 3] = nodes[:-1, 1:].T.ravel()
+    return conn, X
+
+
+def hex_mesh(nx, ny, nz, Lx=1.0, Ly=1.0, Lz=1.0):
+    """Structured H8 mesh extending the numbering of ``grid_mesh``: node(i, j, k) = (i*(ny+1) + j)*(nz+1) + k,
+    element e = i + nx*(j + ny*k); nodes 0-3 counter-clockwise (seen from +z) on the element's bottom face, 4-7 above
+    them, so that detJ > 0.  Returns conn (nelems, 8) and X (nnodes, 3)."""
+    nodes = np.arange((nx + 1) * (ny + 1) * (nz + 1), dtype=np.int64).reshape(nx + 1, ny + 1, nz + 1)
+    grid = np.meshgrid(np.linspace(0, Lx, nx + 1), np.linspace(0, Ly, ny + 1), np.linspace(0, Lz, nz + 1), indexing="ij")
+    X = np.stack([g.ravel() for g in grid], axis=1)
+    corners = [(0, 0), (1, 0), (1, 1), (0, 1)]              # (di, dj) counter-clockwise
+    conn = np.empty((nx * ny * nz, 8), dtype=np.int64)
+    for dk in (0, 1):
+        for a, (di, dj) in enumerate(corners):
+            c = nodes[di:di + nx, dj:dj + ny, dk:dk + nz]
+            conn[:, 4 * dk + a] = c.transpose(2, 1, 0).ravel()      # i fastest, then j, then k
     return conn, X
 
 
@@ -104,7 +120,36 @@ class _Half(_SensitivityCallback):
         return self.parent.device_call_fused(None, W, V, 0.0, 1.0)
 
 
-class Q4Problem:
+class _ElementMaterial:
+    """Nodal density -> element density (the mean over the element's ``npe`` nodes) and the penalised material factors
+    ks, ms and their derivatives dk, dm (eigd_q4_material), for the problems with one density per element."""
+
+    npe = 4
+
+    def set_density(self, rho=None, rhoE=None):
+        """Nodal density rho (filtered design) -> element density + material factors, or set the
+        element densities directly."""
+        lib = _lib.load()
+        if rhoE is not None:
+            self.rhoE_d.copy_(to_dev(rhoE))
+            _lib.check(lib.eigd_q4_material(self.law, self.nelems, self.npe, None, _ptr(self.rhoE_d), self._par_c, None,
+                                            _ptr(self.ks_d), _ptr(self.ms_d), _ptr(self.dk_d), _ptr(self.dm_d)), "q4_material")
+        else:
+            rho_d = to_dev(rho)
+            _lib.check(lib.eigd_q4_material(self.law, self.nelems, self.npe, _ptr(self.conn_d), _ptr(rho_d), self._par_c,
+                                            _ptr(self.rhoE_d), _ptr(self.ks_d), _ptr(self.ms_d), _ptr(self.dk_d),
+                                            _ptr(self.dm_d)), "q4_material")
+        return self.rhoE_d
+
+    def _element_mean(self, rho_t):
+        """Element mean of the nodal vector ``rho_t`` (the material outputs of this call are scratch)."""
+        rhoEt, s1, s2, s3, s4 = (D.empty(self.nelems) for _ in range(5))
+        _lib.check(_lib.load().eigd_q4_material(self.law, self.nelems, self.npe, _ptr(self.conn_d), _ptr(to_dev(rho_t)),
+                                                self._par_c, _ptr(rhoEt), _ptr(s1), _ptr(s2), _ptr(s3), _ptr(s4)), "q4_material")
+        return rhoEt
+
+
+class Q4Problem(_ElementMaterial):
     """Thermal (1 DOF/node) or plane-stress (2 DOF/node) Q4 model with its operators in HBM.
 
     kind "thermal": K_e = kappa(rho_e) sum_q detJ Be^T Be, M_e = c(rho_e) sum_q detJ N N^T
@@ -160,31 +205,12 @@ class Q4Problem:
         self.dAdx, self.dBdx = _Half(self, "A"), _Half(self, "B")
         self.dAdx.fused_with, self.dBdx.fused_with = self.dBdx, self.dAdx
 
-    # ---- material -----------------------------------------------------------------------------
-    def set_density(self, rho=None, rhoE=None):
-        """Nodal density rho (filtered design) -> element density + material factors, or set the
-        element densities directly."""
-        lib = _lib.load()
-        if rhoE is not None:
-            self.rhoE_d.copy_(to_dev(rhoE))
-            _lib.check(lib.eigd_q4_material(self.law, self.nelems, None, _ptr(self.rhoE_d), self._par_c, None,
-                                            _ptr(self.ks_d), _ptr(self.ms_d), _ptr(self.dk_d), _ptr(self.dm_d)), "q4_material")
-        else:
-            rho_d = to_dev(rho)
-            _lib.check(lib.eigd_q4_material(self.law, self.nelems, _ptr(self.conn_d), _ptr(rho_d), self._par_c,
-                                            _ptr(self.rhoE_d), _ptr(self.ks_d), _ptr(self.ms_d), _ptr(self.dk_d),
-                                            _ptr(self.dm_d)), "q4_material")
-        return self.rhoE_d
-
+    # ---- material (set_density: _ElementMaterial) -----------------------------------------------
     def assemble_tangent(self, rho_t):
         """Directional derivative of (K, M) along the nodal density direction ``rho_t`` (device, (nnodes,)), on the same
         pattern: the assembly kernel with the material factors replaced by (dk/drho_e) rho_e', (dm/drho_e) rho_e'.
         Used by the dual-number (complex-step) mode of the drivers."""
-        lib = _lib.load()
-        rhoEt, s1, s2, s3, s4 = (D.empty(self.nelems) for _ in range(5))
-        # element mean of the nodal direction (the material outputs of this call are scratch)
-        _lib.check(lib.eigd_q4_material(self.law, self.nelems, _ptr(self.conn_d), _ptr(to_dev(rho_t)), self._par_c, _ptr(rhoEt),
-                                        _ptr(s1), _ptr(s2), _ptr(s3), _ptr(s4)), "q4_material")
+        rhoEt = self._element_mean(rho_t)
         kt, mt = self.dk_d * rhoEt, self.dm_d * rhoEt
         Kv, Mv = D.empty(self.nnz), D.empty(self.nnz)
         D.q4_assemble(self.kid, self.conn_d, self.xy_d, kt, mt, self.cmat6_d, self.src_ptr_d, self.src_d, self.nnz, Kv, Mv)
@@ -230,6 +256,127 @@ class Q4Problem:
 
     def scatter_to_nodes(self, evals, scale=0.25):
         """rho_b[v] = scale * sum_{e ni v} evals[e] (examples/thermal.py:612-615)."""
+        ev = to_dev(evals)
+        out = D.empty(self.nnodes)
+        D.node_gather(self.nptr_d, self.nelem_d, ev, scale, out)
+        return like_input(out, evals)
+
+
+def _cols(t):
+    """(n,) or (n, N) device operand -> contiguous (n, N)."""
+    if t is None:
+        return None
+    t = t if t.dim() == 2 else t.unsqueeze(1)
+    return t if t.is_contiguous() else t.contiguous()
+
+
+class H8Problem(_ElementMaterial):
+    """Free 3-D isotropic solid on trilinear hexahedra (3 DOF/node) with its operators in HBM.
+
+    K_e = s(rho_e) K0_e, M_e = rho_e M0_e with s = rho^p + rho0_K (SIMP) or rho/(1+q(1-rho)) + rho0_K (RAMP), the laws
+    of the plane-stress ``Q4Problem``; rho_e is the mean of the 8 nodal densities.  The unit matrices
+    K0_e = sum_q detJ B^T C B and M0_e = density sum_q detJ (N N^T (x) I_3) (2x2x2 Gauss) are computed once per mesh on
+    the device (eigd_h8_element_matrices, 9.2 KB per element) and stay resident; per design, assembly and the
+    sensitivities are the stored-matrix kernels (eigd_stored_assemble, eigd_stored_quadform)."""
+
+    npe = 8
+    NE = 24
+
+    def __init__(self, conn, X, E=1.0, nu=0.3, density=1.0, p=3.0, rho0_K=1e-6, ptype_K="simp", q=5.0):
+        dev = D.dev()
+        self.conn = np.asarray(conn, dtype=np.int64)
+        self.X = np.asarray(X, dtype=np.float64)
+        if self.conn.ndim != 2 or self.conn.shape[1] != 8 or self.X.ndim != 2 or self.X.shape[1] != 3:
+            raise ValueError("H8Problem needs conn (nelems, 8) and X (nnodes, 3)")
+        self.nelems = self.conn.shape[0]
+        self.nnodes = self.X.shape[0]
+        self.dof = 3
+        self.ndof = 3 * self.nnodes
+        self.var = element_dofs(self.conn, 3)
+        self.indptr, self.indices, src_ptr, src = assembly_structure(self.var, self.ndof)
+        self.nnz = len(self.indices)
+        nptr, nelem = node_adjacency(self.conn, self.nnodes)
+        if ptype_K == "simp":
+            self.law, self.par = 1, np.array([p, 1.0, 1.0, rho0_K])
+        elif ptype_K == "ramp":
+            self.law, self.par = 2, np.array([q, 1.0, 1.0, rho0_K])
+        else:
+            raise ValueError("unknown ptype_K %r" % ptype_K)
+        self._par_c = (ctypes.c_double * 4)(*[float(v) for v in self.par])
+        # ---- device mirrors -------------------------------------------------------------
+        self.conn_d = torch.as_tensor(self.conn.astype(np.int32), device=dev)
+        self.X_d = to_dev(np.ascontiguousarray(self.X))
+        self.dofmap_d = torch.as_tensor(self.var.astype(np.int32), device=dev)
+        self.indptr_d = torch.as_tensor(self.indptr, device=dev)
+        self.indices_d = torch.as_tensor(self.indices, device=dev)
+        self.src_ptr_d = torch.as_tensor(src_ptr, device=dev)
+        self.src_d = torch.as_tensor(src, device=dev)
+        del src_ptr, src
+        self.nptr_d = torch.as_tensor(nptr, device=dev)
+        self.nelem_d = torch.as_tensor(nelem, device=dev)
+        ne2 = self.NE * self.NE
+        self.K0_d, self.M0_d = D.empty(self.nelems * ne2), D.empty(self.nelems * ne2)
+        _lib.check(_lib.load().eigd_h8_element_matrices(self.nelems, _ptr(self.conn_d), _ptr(self.X_d), float(E), float(nu),
+                                                        float(density), _ptr(self.K0_d), _ptr(self.M0_d)), "h8_element_matrices")
+        self.rhoE_d = D.empty(self.nelems)
+        self.ks_d, self.ms_d = D.empty(self.nelems), D.empty(self.nelems)
+        self.dk_d, self.dm_d = D.empty(self.nelems), D.empty(self.nelems)
+        self.sharding = None          # dist.ModeSharding: element-range shards of the df/dx reduction
+        self.dAdx, self.dBdx = _Half(self, "A"), _Half(self, "B")
+        self.dAdx.fused_with, self.dBdx.fused_with = self.dBdx, self.dAdx
+
+    def _assemble(self, ck, cm):
+        Kv, Mv = D.empty(self.nnz), D.empty(self.nnz)
+        _lib.check(_lib.load().eigd_stored_assemble(self.nnz, _ptr(self.src_ptr_d), _ptr(self.src_d), self.NE, _ptr(self.K0_d),
+                                                    None, _ptr(ck), None, _ptr(Kv), _ptr(self.M0_d), None, _ptr(cm), None,
+                                                    _ptr(Mv)), "stored_assemble")
+        shape = (self.ndof, self.ndof)
+        return (D.CsrDevice(self.indptr_d, self.indices_d, Kv, shape), D.CsrDevice(self.indptr_d, self.indices_d, Mv, shape))
+
+    def assemble(self):
+        """K(rho), M(rho) as CsrDevice sharing one pattern."""
+        return self._assemble(self.ks_d, self.ms_d)
+
+    def assemble_tangent(self, rho_t):
+        """Directional derivative of (K, M) along the nodal density direction ``rho_t`` (device, (nnodes,)): the same
+        assembly with the coefficients (dk/drho_e) rho_e', (dm/drho_e) rho_e'.  Used by the dual-number mode of the
+        drivers."""
+        rhoEt = self._element_mean(rho_t)
+        return self._assemble(self.dk_d * rhoEt, self.dm_d * rhoEt)
+
+    def dof_coords(self):
+        """Node coordinates for geometric nested dissection (``SpLuOperator(coords=..., dof_per_node=...)``)."""
+        return self.X, self.dof
+
+    def device_call_fused(self, WA, WB, V, cA, cB):
+        """cA * sum_k WA_k^T (dK/drho_e) V_k + cB * sum_k WB_k^T (dM/drho_e) V_k per element (device), both terms in one
+        pass of eigd_stored_quadform over the gathered V."""
+        V2, WA2, WB2 = _cols(V), _cols(WA), _cols(WB)
+        for t in (WA2, WB2):
+            if t is not None and t.shape != V2.shape:
+                raise ValueError("WA / WB must have the shape of V")
+        terms = [(W, U, c, float(s)) for W, U, c, s in ((WA2, self.K0_d, self.dk_d, cA), (WB2, self.M0_d, self.dm_d, cB))
+                 if W is not None]
+        shard = self.sharding
+        lo, hi = (0, self.nelems) if shard is None or shard.world == 1 else shard.my_range(self.nelems)
+        out = D.zeros(hi - lo)
+        if hi > lo and terms:
+            ne2 = self.NE * self.NE
+            (W1, U1, c1, s1), second = terms[0], terms[1] if len(terms) == 2 else None
+            W2, F1, d1, s2 = second if second is not None else (None, None, None, 1.0)
+            rng = lambda t, w: None if t is None else t[lo * w:hi * w]          # noqa: E731  element-range views
+            _lib.check(_lib.load().eigd_stored_quadform(hi - lo, self.NE, _ptr(self.dofmap_d[lo:hi]), _ptr(rng(U1, ne2)), None,
+                                                        _ptr(rng(c1, 1)), None, _ptr(W1), _ptr(V2), V2.shape[1], V2.stride(0),
+                                                        _ptr(out), _ptr(rng(F1, ne2)), _ptr(rng(d1, 1)), _ptr(W2), s1, s2),
+                       "stored_quadform")
+            if second is None and s1 != 1.0:
+                out.mul_(s1)
+        if hi - lo == self.nelems:
+            return out
+        return shard.allgather_ranges(out, self.nelems)              # element-range shard + one all-gather (dist.py)
+
+    def scatter_to_nodes(self, evals, scale=0.125):
+        """rho_b[v] = scale * sum_{e ni v} evals[e]: the transpose of the 8-node element mean."""
         ev = to_dev(evals)
         out = D.empty(self.nnodes)
         D.node_gather(self.nptr_d, self.nelem_d, ev, scale, out)
@@ -353,11 +500,11 @@ class BucklingQ4Problem:
         rhoE_d = self.base.set_density(rho=rho, rhoE=rhoE)
         lib = _lib.load()
         s = self._scratch
-        _lib.check(lib.eigd_q4_material(self.lawG, self.nelems, None, _ptr(rhoE_d), self._parG, None, _ptr(self.kg_d),
+        _lib.check(lib.eigd_q4_material(self.lawG, self.nelems, 4, None, _ptr(rhoE_d), self._parG, None, _ptr(self.kg_d),
                                         _ptr(s), _ptr(self.dkg_d), _ptr(s)), "q4_material")
         if self.lawG == 2:      # the reference differentiates the RAMP law of G with q + 1 (:336)
             tmp = D.empty(self.nelems)
-            _lib.check(lib.eigd_q4_material(self.lawG, self.nelems, None, _ptr(rhoE_d), self._pardG, None, _ptr(tmp),
+            _lib.check(lib.eigd_q4_material(self.lawG, self.nelems, 4, None, _ptr(rhoE_d), self._pardG, None, _ptr(tmp),
                                             _ptr(s), _ptr(self.dkg_d), _ptr(s)), "q4_material")
         return rhoE_d
 
@@ -426,6 +573,9 @@ class NodeFilter:
         self.dvmap = None if dvmap is None else np.asarray(dvmap, dtype=np.int64)
         self.offset_d = None
         if ftype == "helmholtz":
+            if self.X.shape[1] != 2:
+                raise ValueError("the Helmholtz filter is built on the Q4 mesh; it is not available for %d-D coordinates"
+                                 % self.X.shape[1])
             self._init_helmholtz(conn, r0, num_design_vars)
             return
         tree = spatial.cKDTree(self.X)

@@ -201,7 +201,8 @@ class ShellProblem:
         U1, U3 = (self.E1_d, self.E3_d) if which == "A" else (self.F1_d, self.F3_d)
         oute = D.empty(self.nelems)
         _lib.check(_lib.load().eigd_stored_quadform(self.nelems, self.NE, _ptr(self.dofmap_d), _ptr(U1), _ptr(U3), _ptr(self.one_d),
-                                                    _ptr(self.dt3_d), _ptr(W2), _ptr(V2), V2.shape[1], V2.stride(0), _ptr(oute)),
+                                                    _ptr(self.dt3_d), _ptr(W2), _ptr(V2), V2.shape[1], V2.stride(0), _ptr(oute),
+                                                    None, None, None, 1.0, 1.0),
                    "stored_quadform")
         out = D.empty(self.ncomp)
         _lib.check(_lib.load().eigd_segment_sum(self.ncomp, _ptr(self.seg_ptr_d), _ptr(self.perm_d), _ptr(oute), 1.0 / self.scale,

@@ -119,13 +119,25 @@ class _Q4Analysis(_EigenAnalysis):
                  eig_atol=1e-5, adjoint_method="sibk", adjoint_options=None, deriv_type="tensor", seed=0, **material):
         self.fltr = fltr
         self.conn, self.X = np.asarray(conn), np.asarray(X)
-        super().__init__(fe.Q4Problem(self.conn, self.X, self.kind, **material), N, m, solver_type, tol, rtol, eig_atol,
-                         adjoint_method, adjoint_options, deriv_type, seed)
+        super().__init__(self._make_problem(**material), N, m, solver_type, tol, rtol, eig_atol, adjoint_method,
+                         adjoint_options, deriv_type, seed)
         self.nelems, self.nnodes, self.nvars = self.prob.nelems, self.prob.nnodes, self.prob.ndof
         self.sigma, self.Ntarget = sigma, Ntarget
         self.x = 0.95 * np.ones(self.fltr.num_design_vars)      # thermal.py:71, natural_frequency.py:75
         self.profile.update(nnodes=self.nnodes, nelems=self.nelems, solver_type=solver_type,
                             adjoint_method=self.adjoint_method, N=N)
+
+    def _make_problem(self, **material):
+        return fe.Q4Problem(self.conn, self.X, self.kind, **material)
+
+    def _rigid_count(self, lam0):
+        """How many of the computed modes ``lam0`` (ascending) are rigid-body modes."""
+        return self.nrigid
+
+    def _keep_flexible(self, lam0):
+        """``self.keep``: the modes the driver reports, len(lam0) - nrigid of them, after the rigid ones."""
+        r = self._rigid_count(lam0)
+        self.keep = slice(r, r + len(lam0) - self.nrigid)
 
     # ---- forward ------------------------------------------------------------------------------
     def solve_eigenvalue_problem(self, store=False):
@@ -143,7 +155,8 @@ class _Q4Analysis(_EigenAnalysis):
         lam = self._eigensolve(K, M, self.sigma, t1)
         self.lam0 = np.asarray(lam)
         self.Q0 = self.eig_solver._Phi_d                                   # (n, N + nrigid) device
-        return self.lam0[self.nrigid:], self.Q0[:, self.nrigid:]
+        self._keep_flexible(self.lam0)
+        return self.lam0[self.keep], self.Q0[:, self.keep]
 
     def initialize(self, store=False, x=None):
         if x is not None:
@@ -181,7 +194,8 @@ class _Q4Analysis(_EigenAnalysis):
         self._new_eig_solver(self.N + self.nrigid, lanczos=dict(Ntarget=self.Ntarget))
         lam, Phi = self.eig_solver.solve((K, Kt), (M, Mt), self.factor, self.sigma)
         self.lam0, self.Q0 = np.asarray(lam), np.asarray(Phi)               # complex host arrays
-        self.lam, self.Q = self.lam0[self.nrigid:], self.Q0[:, self.nrigid:]
+        self._keep_flexible(self.lam0)
+        self.lam, self.Q = self.lam0[self.keep], self.Q0[:, self.keep]
         self.N = len(self.lam)
         return
 
@@ -190,7 +204,7 @@ class _Q4Analysis(_EigenAnalysis):
         self.rhoEb = D.zeros(self.nelems)
         self.lamb = np.zeros(self.N)
         self.Q0b = D.zeros(self.nvars, self.N + self.nrigid)
-        self.Qb = self.Q0b[:, self.nrigid:]
+        self.Qb = self.Q0b[:, self.keep]
 
     # ---- reverse ------------------------------------------------------------------------------
     def _eigenvector_seeds(self):
@@ -198,8 +212,8 @@ class _Q4Analysis(_EigenAnalysis):
 
     def _total_derivative(self, psi0, corr_data):
         self.psi0 = psi0
-        self.psi = psi0[:, self.nrigid:]
-        nr = self.nrigid
+        self.psi = psi0[:, self.keep]
+        nr = self.keep.start
         if nr:                                                            # natural_frequency.py:484-494
             data0 = {}
             for i, items in corr_data.items():
@@ -207,8 +221,8 @@ class _Q4Analysis(_EigenAnalysis):
                 if i >= nr and keep:
                     data0[i] = keep
             corr_data = data0
-        lamb0 = np.zeros(self.N + nr)
-        lamb0[nr:] = self.lamb
+        lamb0 = np.zeros(self.N + self.nrigid)
+        lamb0[self.keep] = self.lamb
         self.eig_solver.add_total_derivative(lamb0, self.Q0b, psi0, self.prob.dAdx, self.prob.dBdx, self.rhoEb,
                                              adj_corr_data=corr_data, deriv_type=self.deriv_type)
         rhob = self.prob.scatter_to_nodes(self.rhoEb)
@@ -306,6 +320,31 @@ class NaturalFrequencyAnalysis(_Q4Analysis):
         return float(np.sum(val**2))
 
 
+class NaturalFrequency3DAnalysis(NaturalFrequencyAnalysis):
+    """The natural-frequency problem of ``NaturalFrequencyAnalysis`` on a free 3-D solid of trilinear hexahedra
+    (``fe.H8Problem``): N + 6 modes computed with sigma < 0 and the six rigid-body modes (three translations, three
+    rotations) dropped.  Same forward and reverse pipeline and objective helpers; the 2-D node-set helpers are not
+    offered."""
+
+    nrigid = 6
+
+    def _make_problem(self, **material):
+        return fe.H8Problem(self.conn, self.X, **material)
+
+    def _rigid_count(self, lam0):
+        """The leading modes with lambda ~ 0.  IRAM returns all six copies of the six-fold zero eigenvalue; single-vector
+        Lanczos (BasicLanczos) resolves only some of them from one start vector, and the rest of its N + 6 Ritz pairs
+        are flexible modes, so the rigid ones are counted by value, not assumed."""
+        lam = np.abs(np.asarray(lam0).real)
+        return int(min(self.nrigid, np.count_nonzero(lam < 1e-8 * lam.max())))
+
+    def get_point_coefficients(self, name):
+        raise NotImplementedError("node-set point coefficients are defined for the 2-D model only")
+
+    def add_point_derivative(self, name, x0b, xcoefb):
+        raise NotImplementedError("node-set point derivatives are defined for the 2-D model only")
+
+
 class MinFreqOpt:
     """KS-aggregated minimum natural frequency of the structure with a point mass attached at each node set in turn
     (examples/natural_frequency.py ``MinFreqOpt`` :693-803).  For node set s with modal coefficients c (3 x N) the
@@ -314,6 +353,9 @@ class MinFreqOpt:
     eigensolve and the adjoint of ``topo``."""
 
     def __init__(self, topo, ks_param=1.0, fixed_mass=1.0):
+        if isinstance(topo, NaturalFrequency3DAnalysis):
+            raise ValueError("MinFreqOpt attaches point masses to the node sets of the 2-D model; it is not offered for "
+                             "the 3-D solid")
         self.topo, self.ks_param, self.fixed_mass = topo, ks_param, fixed_mass
         self.ks_min = 0.0
         self.node_sets = topo.node_sets
@@ -434,6 +476,15 @@ def make_natural_frequency_model(nx=128, ny=64, Lx=1.0, Ly=1.0, rfact=4.0, N=10,
     model = NaturalFrequencyAnalysis(fltr, conn, X, N=N, **kwargs)
     model.node_sets, model.element_sets = node_sets, element_sets
     return model
+
+
+def make_natural_frequency_3d_model(nx, ny, nz, Lx=2.0, Ly=1.0, Lz=1.0, rfact=4.0, **kwargs):
+    """Free nx x ny x nz hexahedral box (``fe.hex_mesh``), one design variable per node, conic filter of radius
+    rfact * Ly / ny on the 3-D nodes.  The largest box one 180 GB B200 factors is about 80 x 40 x 40 (408k DOF): the
+    factor keeps every front resident (DESIGN.md section 8b)."""
+    conn, X = fe.hex_mesh(nx, ny, nz, Lx, Ly, Lz)
+    fltr = fe.NodeFilter(conn, X, r0=rfact * (Ly / ny))
+    return NaturalFrequency3DAnalysis(fltr, conn, X, **kwargs)
 
 
 # ------------------------------------------------------------------------------------------

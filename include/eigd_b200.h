@@ -177,14 +177,19 @@ int eigd_lanczos_extend(eigd_factor* f, int n, const int* d_b_indptr, const int*
  *      does on the host in reference examples/crm.py:122-142 (assembleMatType) and :331-355 (addMatDVSensInnerProduct,
  *      the per-mode "vector" derivative form).  Element matrices K_e = c1[e] E1_e + c3[e] E3_e, ne x ne row-major,
  *      ne element dofs.  Assembly is gather-form through the (element, a, b) -> CSR source lists of
- *      eigd_q4_assemble; a second matrix on the same pattern (F1, F3, d1, d3 -> vals2) is optional (NULL). ---- */
+ *      eigd_q4_assemble; a second matrix on the same pattern (F1, F3, d1, d3 -> vals2) is optional (NULL), and so
+ *      are the t^3 terms (E3, c3, F3, d3 all NULL: K_e = c1[e] E1_e, the H8 solid). ---- */
 int eigd_stored_assemble(int64_t nnz, const int64_t* d_src_ptr, const int64_t* d_src, int ne, const double* d_E1,
                          const double* d_E3, const double* d_c1, const double* d_c3, double* d_vals, const double* d_F1,
                          const double* d_F3, const double* d_d1, const double* d_d3, double* d_vals2);
 /* out[e] = sum_k W[dof(e,:), k]^T (c1[e] E1_e + c3[e] E3_e) V[dof(e,:), k]; dofmap (nelems x ne, -1 = constrained);
- * W, V row-major (n, N) with leading dimension ld; ne in {8, 24} */
+ * W, V row-major (n, N) with leading dimension ld; ne in {8, 24}; E3 and c3 may both be NULL.  With a second term
+ * (F1, d1, W2 non-NULL; W2 shares the layout of W and V) both are evaluated in the same pass over V:
+ *   out[e] = s1 * sum_k W_k^T (c1[e] E1_e + c3[e] E3_e) V_k + s2 * sum_k W2_k^T (d1[e] F1_e) V_k
+ * (s1, s2 are ignored without it). */
 int eigd_stored_quadform(int nelems, int ne, const int* d_dofmap, const double* d_E1, const double* d_E3, const double* d_c1,
-                         const double* d_c3, const double* d_W, const double* d_V, int N, int64_t ld, double* d_out);
+                         const double* d_c3, const double* d_W, const double* d_V, int N, int64_t ld, double* d_out,
+                         const double* d_F1, const double* d_d1, const double* d_W2, double s1, double s2);
 /* out[c] = scale * sum_{i in [seg_ptr[c], seg_ptr[c+1])} x[perm[i]] (perm NULL: identity): warp-shuffle segmented sum */
 int eigd_segment_sum(int nseg, const int* d_seg_ptr, const int* d_perm, const double* d_x, double scale, double* d_out);
 
@@ -221,12 +226,19 @@ int eigd_q4_assemble(int kind, int nelems, const int* d_conn, const double* d_xy
 int eigd_q4_quadforms(int kind, int nelems, const int* d_conn, const double* d_xy, const double* d_cmat6,
                       const double* d_WA, const double* d_WB, const double* d_V, int N, int ldw,
                       const double* d_dk, const double* d_dm, double sA, double sB, double* d_out);
-/* Element density rhoE[e] = 1/4 sum_a rho[conn[e,a]] (d_conn NULL: d_rho is already per element) and the
+/* Element density rhoE[e] = 1/npe sum_a rho[conn[e,a]], npe = 4 (Q4) or 8 (H8) nodes per element (d_conn NULL:
+ * d_rho is already per element) and the
  * penalised material factors / derivatives of the examples (thermal.py:132,175-188,198,236-244;
  * natural_frequency.py:140-143,198-201,219-220).  law 0 thermal SIMP, 1 structural SIMP, 2 RAMP;
  * par4 = {p or q, k0, c0, beta or rho0} (host).  Any output may be NULL. */
-int eigd_q4_material(int law, int nelems, const int* d_conn, const double* d_rho, const double* par4,
+int eigd_q4_material(int law, int nelems, int npe, const int* d_conn, const double* d_rho, const double* par4,
                      double* d_rhoE, double* d_ks, double* d_ms, double* d_dk, double* d_dm);
+/* ---- 3-D solid (csrc/h8.cu): unit element matrices of the trilinear hexahedron on the 2x2x2 Gauss rule, once per
+ *      mesh.  conn (nelems, 8): nodes 0-3 counter-clockwise on the zeta = -1 face, 4-7 above them; X (nnodes, 3).
+ *      K0, M0: (nelems, 24, 24) row-major, dof order node-major (u_x, u_y, u_z);
+ *      K0_e = sum_q detJ B^T C(E, nu) B, M0_e = density sum_q detJ (N N^T (x) I_3). */
+int eigd_h8_element_matrices(int nelems, const int* d_conn, const double* d_X, double E, double nu, double density,
+                             double* d_K0, double* d_M0);
 /* node_out[v] = scale * sum_{e in adj(v)} e_vals[e]   (gather form of np.add.at, thermal.py:612-615) */
 int eigd_node_gather(int nnodes, const int* d_nptr, const int* d_nelem, const double* d_evals, double scale, double* d_out);
 

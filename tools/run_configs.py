@@ -3,6 +3,7 @@
     python tools/run_configs.py c3 [--nx 352 --ny 704 --modes 20]     buckling, ~497k DOF, 20 modes
     python tools/run_configs.py c5 [--designs 8]                      design sweep, 202k-DOF natural-frequency mesh
     python tools/run_configs.py c4 [--nx 408 --ny 408 --modes 20 --fd]   1M-DOF synthetic shell (6 dof/node), crm.py driver
+    python tools/run_configs.py h8 [--nx 64 --ny 32 --nz 32 --modes 10 --fd]   free 3-D solid of hexahedra (3 dof/node)
 
 Each prints one JSON line: stage times (CUDA-synchronised wall clock of the driver's own timers, as the
 reference examples report them), solve counts, factor statistics, and size-independent acceptance checks
@@ -215,12 +216,101 @@ def run_nf(args, tag):
     return out
 
 
+def gpu_card():
+    """Name and power limit of the GPU the numbers were measured on."""
+    import subprocess
+    try:
+        return subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader", "-i",
+                               os.environ.get("LOCAL_RANK", "0")], capture_output=True, text=True, timeout=60).stdout.strip()
+    except (OSError, subprocess.SubprocessError) as exc:
+        return "unavailable: %s" % exc
+
+
+def run_h8(args):
+    """Free nx x ny x nz box of hexahedra (NaturalFrequency3DAnalysis): N flexible modes + 6 rigid-body modes about
+    sigma = -10, IRAM + sibk with the Lanczos guess, tensor derivative, f = sum_i (phi_i . w_i)^2 as the seed."""
+    from eigd_b200 import device as D, topo as T
+    D.init()
+    out = {"config": "H8 free solid nx=%d ny=%d nz=%d" % (args.nx, args.ny, args.nz), "N": args.modes, "gpu": gpu_card()}
+    t0 = now()
+    model = T.make_natural_frequency_3d_model(args.nx, args.ny, args.nz, N=args.modes, m=60, sigma=-10.0, solver_type="IRAM",
+                                              adjoint_method="sibk", adjoint_options={"lanczos_guess": True}, rtol=1e-10,
+                                              deriv_type="tensor")
+    out.update(n=int(model.nvars), nnz=int(model.prob.nnz), host_setup_s=now() - t0)
+    w_d = D.to_device(np.random.default_rng(99).normal(size=(model.nvars, args.modes)))
+    x0 = np.random.default_rng(0).uniform(0.3, 1.0, model.fltr.num_design_vars)
+    reps = []
+    for rep in range(args.reps):
+        l0 = D.launch_count()
+        ta = now()
+        with warnings.catch_warnings():
+            warnings.simplefilter("ignore")
+            model.initialize(x=x0)
+        model.initialize_adjoint()
+        f = model.add_modal_function_derivative(w_d)
+        model.finalize_adjoint()
+        tb = now()
+        p = model.profile
+        reps.append({"wall_s": tb - ta, "assembly_s": p["matrix assembly time"], "eig_s": p["eigenvalue solve time"],
+                     "adjoint_s": p["adjoint solution time"], "dfdx_s": p["total derivative time"],
+                     "time_to_gradient_s": model.time_to_gradient(), "eig_solves": p["solve preconditioner count"],
+                     "adjoint_solves": p["adjoint preconditioner count"], "launches": D.launch_count() - l0,
+                     "symbolic_s": p.get("symbolic analysis time")})
+    out["reps"] = reps
+    out["factorisation_s"] = _time_factorisation(model)
+    out["lam_first"] = [float(v) for v in model.lam[:3]]
+    out["rigid_lam"] = [float(v) for v in model.lam0[:6]]
+    out["factor_info"] = model.factor.info
+    out["symbolic"] = model.symbolic[0].stats()
+    res, _ = residuals(model, model.K, model.M, model.lam, model.Q, "normal")      # flexible modes: the rigid ones have
+    _, orth = residuals(model, model.K, model.M, model.lam0, model.Q0, "normal")     # lambda ~ 0, their relative residual is 0/0
+    out["eigen_residual_max"] = res
+    out["orthonormality_defect"] = orth
+    ar, ao = model.eig_solver.eval_adjoint_residual_norm(model.Q0b, model.psi0, b_ortho=True)
+    rhs = float(model.Q0b.norm(dim=0).max().item())
+    out["adjoint_residual_over_rtol_rhs"] = float(np.max(ar)) / (1e-10 * rhs)
+    assert out["adjoint_residual_over_rtol_rhs"] < 50.0 and orth < 1e-10, (out["adjoint_residual_over_rtol_rhs"], orth)
+    assert res < 1e-8, res
+    out["objective"] = f
+    xb = model.xb.cpu().numpy().copy()
+    out["xb_norm"] = float(np.linalg.norm(xb))
+    if args.fd:
+        pert = np.random.default_rng(3).uniform(-1.0, 1.0, x0.shape)
+        h = 1e-5
+        vals = []
+        for sgn in (1.0, -1.0):
+            with warnings.catch_warnings():
+                warnings.simplefilter("ignore")
+                model.initialize(x=x0 + sgn * h * pert)
+            vals.append(float(np.sum(D.col_dot(model.Q, w_d).cpu().numpy() ** 2)))
+        fd = (vals[0] - vals[1]) / (2 * h)
+        out["fd_directional"] = fd
+        out["adjoint_directional"] = float(xb @ pert)
+        out["fd_rel_err"] = abs(fd - float(xb @ pert)) / abs(fd)
+    out["gpu_after"] = gpu_card()
+    return out
+
+
+def _time_factorisation(model, reps=3):
+    """Numeric LDL^T of the last design's K - sigma M, alone (the driver's eigensolve time includes it): the driver's
+    factor refactored in place on the same values, device-synchronised, every repetition."""
+    from eigd_b200 import device as D
+    vals = D.axpby(1.0, model.K.data, -float(model.sigma), model.M.data)
+    times = []
+    for _ in range(reps):
+        t0 = now()
+        model.factor.lu.numeric(vals, model.symbolic[1])
+        times.append(now() - t0)
+    return times
+
+
 if __name__ == "__main__":
     ap = argparse.ArgumentParser()
-    ap.add_argument("config", choices=["c3", "c4", "c4plate", "c5"])
+    ap.add_argument("config", choices=["c3", "c4", "c4plate", "c5", "h8"])
     ap.add_argument("--fd", action="store_true", help="c4: add the finite-difference check of the gradient")
     ap.add_argument("--nx", type=int, default=None)
     ap.add_argument("--ny", type=int, default=None)
+    ap.add_argument("--nz", type=int, default=None, help="h8: elements along z")
     ap.add_argument("--modes", type=int, default=None)
     ap.add_argument("--designs", type=int, default=None)
     ap.add_argument("--reps", type=int, default=3)
@@ -231,6 +321,9 @@ if __name__ == "__main__":
     elif a.config == "c5":
         a.nx, a.ny, a.modes, a.designs = a.nx or 448, a.ny or 224, a.modes or 6, a.designs or 8
         res = run_nf(a, "C5 design sweep")
+    elif a.config == "h8":
+        a.nx, a.ny, a.nz, a.modes = a.nx or 64, a.ny or 32, a.nz or 32, a.modes or 10
+        res = run_h8(a)
     elif a.config == "c4":
         a.nx, a.ny, a.modes = a.nx or 408, a.ny or 408, a.modes or 20
         res = run_c4(a)
