@@ -69,8 +69,8 @@ h8_element_matrices_kernel(int nelems, const int* __restrict__ conn, const doubl
 extern "C" int eigd_h8_element_matrices(int nelems, const int* d_conn, const double* d_X, double E, double nu, double density,
                                         double* d_K0, double* d_M0) {
   if (nelems <= 0) return 0;
-  if (!(nu > -1.0 && nu < 0.5)) { eigd_set_error("h8_element_matrices: Poisson ratio %g outside (-1, 0.5)", nu); return 1; }
-  const H8C c = {E * nu / ((1.0 + nu) * (1.0 - 2.0 * nu)), E / (2.0 * (1.0 + nu))};
+  H8C c;
+  if (!h8_isotropic(E, nu, c, "h8_element_matrices")) return 1;
   const int grid = (int)(((int64_t)nelems * 32 + 255) / 256);
   EIGD_LAUNCH(h8_element_matrices_kernel, grid, 256, 0, nelems, d_conn, d_X, c, density, d_K0, d_M0);
   EIGD_CHECK_LAUNCH();

@@ -67,6 +67,17 @@ struct H8C {
   double lam, mu;
 };
 
+// Lame constants of (E, nu) on the host; false (error set, prefixed with `what`) for nu outside (-1, 0.5).
+// Include common.cuh first.
+inline bool h8_isotropic(double E, double nu, H8C& c, const char* what) {
+  if (!(nu > -1.0 && nu < 0.5)) {
+    eigd_set_error("%s: Poisson ratio %g outside (-1, 0.5)", what, nu);
+    return false;
+  }
+  c = {E * nu / ((1.0 + nu) * (1.0 - 2.0 * nu)), E / (2.0 * (1.0 + nu))};
+  return true;
+}
+
 // s = C e
 __device__ __forceinline__ void h8_c_mul(const H8C& c, const double e[6], double s[6]) {
   const double tr = c.lam * (e[0] + e[1] + e[2]);

@@ -796,6 +796,29 @@ def q4_dof_gather(nptr, nelem, nlocal, due, out):
     return out
 
 
+def h8_stress_stiffness(conn, X, E, nu, kg, dofmap, u, stress, G0):
+    """Element stresses kg C B_q u_e (``stress`` (nelems, 8, 6) or None) and the unit stress stiffness G0 (nelems * 576)
+    of the H8 solid; ``u`` is read through ``dofmap`` (nelems, 24), -1 = constrained."""
+    check(_lib.load().eigd_h8_stress_stiffness(conn.shape[0], _ptr(conn), _ptr(X), float(E), float(nu), _ptr(kg), _ptr(dofmap),
+                                               _ptr(u), _ptr(stress), _ptr(G0)), "h8_stress_stiffness")
+    return G0
+
+
+def h8_gderiv_u(conn, X, E, nu, kg, dofmap, W, V, due):
+    """due (nelems, 24): the element terms of d/du sum_k w_k^T G(u) v_k (W, V: (n, N) row-major, read through dofmap)."""
+    if W.stride(1) != 1 or V.stride(1) != 1 or W.stride(0) != V.stride(0) or W.shape != V.shape:
+        raise ValueError("W and V must share one row-major layout")
+    check(_lib.load().eigd_h8_gderiv_u(conn.shape[0], _ptr(conn), _ptr(X), float(E), float(nu), _ptr(kg), _ptr(dofmap), _ptr(W),
+                                       _ptr(V), V.shape[1], V.stride(0), _ptr(due)), "h8_gderiv_u")
+    return due
+
+
+def h8_dof_gather(nptr, nelem, nlocal, due, out):
+    check(_lib.load().eigd_h8_dof_gather(out.numel() // 3, _ptr(nptr), _ptr(nelem), _ptr(nlocal), _ptr(due), _ptr(out)),
+          "h8_dof_gather")
+    return out
+
+
 def expand_rows(idx, red, nfull):
     """full[idx[i], :] = red[i, :], zeros elsewhere (examples/buckling.py full_vector)."""
     r2 = _as2d(red)

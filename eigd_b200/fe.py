@@ -407,51 +407,45 @@ class _BucklingCallback(_SensitivityCallback):
     """dAdu / dAdx / dBdx of examples/buckling.py:924-979 as device operators on REDUCED (n_r, N) operands."""
 
     def device_call(self, Wr, Vr):
-        pr = self.parent
-        W, V = pr.full_vector(Wr), pr.full_vector(Vr)
-        W2 = W if W.dim() == 2 else W.unsqueeze(1)
-        V2 = V if V.dim() == 2 else V.unsqueeze(1)
-        if self.which == "dGdu":
-            due = D.empty(pr.nelems, 8)
-            D.q4_gderiv(pr.conn_d, pr.xy_d, pr.cmat6_d, W2, V2, pr.kg_d, pr.dkg_d, pr.u_d, 1.0, None, due)
-            return D.q4_dof_gather(pr.nptr_d, pr.nelem_d, pr.nlocal_d, due, D.empty(pr.ndof))
-        out = D.zeros(pr.nelems)
-        if self.which == "dGdx":
-            D.q4_gderiv(pr.conn_d, pr.xy_d, pr.cmat6_d, W2, V2, pr.kg_d, pr.dkg_d, pr.u_d, 1.0, out, None)
-        else:                                                                     # dKdx
-            D.q4_quadforms(1, pr.conn_d, pr.xy_d, pr.cmat6_d, W2, None, V2, pr.base.dk_d, pr.base.dm_d, 1.0, 0.0, out)
-        return out
+        return self.parent.sensitivity(self.which, Wr, Vr)
 
 
-class BucklingQ4Problem:
-    """Plane-stress Q4 column of examples/buckling.py in HBM: K(x) with Dirichlet rows removed, the fundamental
-    path K_r u_r = f_r, the stress stiffness G(u, x) and the three sensitivity callbacks.
+def node_local_index(conn):
+    """For every (node, element) pair of ``node_adjacency`` order: the node's local index inside the element."""
+    conn = np.asarray(conn, dtype=np.int64)
+    nelems, npe = conn.shape
+    e = np.repeat(np.arange(nelems, dtype=np.int64), npe)
+    loc = np.tile(np.arange(npe, dtype=np.int64), nelems)
+    return loc[np.lexsort((e, conn.ravel()))].astype(np.int32)
 
-    Element-level outputs stay per element (the node scatter ``np.add.at ... *0.25`` of :212-216, :337-341 is
-    linear and is applied once at the end by the driver).  Reference: examples/buckling.py:152-343, 499-518.
-    """
 
-    def __init__(self, conn, X, bcs, forces, E=1.0, nu=0.3, density=1.0, p=3.0, q=5.0, rho0_K=1e-6, rho0_G=1e-9,
-                 ptype_K="simp", ptype_G="simp"):
+class _BucklingProblem:
+    """What the Q4 and H8 buckling problems share around their element problem ``base`` (``Q4Problem`` /
+    ``H8Problem``, which owns the mesh, K law and element density): Dirichlet conditions and loads on ``dof`` components
+    per node, the reduced pattern and its source lists, the G material law, the Dirichlet maps, the fundamental path
+    and the three sensitivity callbacks (``sensitivity`` of the subclass)."""
+
+    def _setup(self, base, bcs, forces, p, q, density, rho0_G, ptype_G):
         dev = D.dev()
-        self.base = Q4Problem(conn, X, "plane_stress", E=E, nu=nu, density=density, p=p, rho0_K=rho0_K,
-                              ptype_K=ptype_K, q=q)
-        b = self.base
+        self.base = b = base
         self.conn, self.X = b.conn, b.X
-        self.nelems, self.nnodes, self.ndof = b.nelems, b.nnodes, b.ndof
-        self.conn_d, self.xy_d, self.cmat6_d = b.conn_d, b.xy_d, b.cmat6_d
-        self.nptr_d, self.nelem_d = b.nptr_d, b.nelem_d
-        # Dirichlet conditions and loads (:120-150)
+        self.nelems, self.nnodes, self.ndof, self.dof = b.nelems, b.nnodes, b.ndof, b.dof
+        self.conn_d, self.nptr_d, self.nelem_d = b.conn_d, b.nptr_d, b.nelem_d
+        # Dirichlet conditions {node: [components]} and loads {node: [f_0, .., f_dof-1]} (:120-150)
+        dof = self.dof
         fixed = np.zeros(self.ndof, dtype=bool)
-        for node, uv in bcs.items():
-            for index in uv:
-                fixed[2 * int(node) + int(index)] = True
+        for node, comps in bcs.items():
+            for index in comps:
+                if not 0 <= int(index) < dof:
+                    raise ValueError("boundary condition on component %r of node %r: %d components per node"
+                                     % (index, node, dof))
+                fixed[dof * int(node) + int(index)] = True
         self.reduced = np.nonzero(~fixed)[0]
         self.nred = len(self.reduced)
         self.f = np.zeros(self.ndof)
         for node, fv in forces.items():
-            self.f[2 * int(node)] += fv[0]
-            self.f[2 * int(node) + 1] += fv[1]
+            for j in range(dof):
+                self.f[dof * int(node) + j] += fv[j]
         src_ptr, src = to_host_i64(b.src_ptr_d), to_host_i64(b.src_d)
         self.indptr, self.indices, r_src_ptr, r_src = reduced_structure(b.indptr, b.indices, src_ptr, src, self.reduced,
                                                                         self.ndof)
@@ -463,11 +457,7 @@ class BucklingQ4Problem:
         self.reduced_d = torch.as_tensor(self.reduced.astype(np.int32), device=dev)
         self.fr_d = to_dev(self.f[self.reduced])
         # local index of every node inside each adjacent element (dof gather of :318-320)
-        e = np.repeat(np.arange(self.nelems, dtype=np.int64), 4)
-        v = self.conn.ravel()
-        loc = np.tile(np.arange(4, dtype=np.int64), self.nelems)
-        order = np.lexsort((e, v))
-        self.nlocal_d = torch.as_tensor(loc[order].astype(np.int32), device=dev)
+        self.nlocal_d = torch.as_tensor(node_local_index(self.conn), device=dev)
         # G material law (:231-234) and the derivative the reference applies to it (:333-336)
         if ptype_G == "simp":
             self.lawG, parG, pardG = 1, [p, 1.0, density, rho0_G], [p, 1.0, density, rho0_G]
@@ -493,20 +483,46 @@ class BucklingQ4Problem:
 
     def dof_coords(self):
         """Per-dof coordinates of the reduced system for geometric nested dissection."""
-        return self.X[self.reduced // 2], 1
+        return self.X[self.reduced // self.dof], 1
 
     # ---- material ------------------------------------------------------------------------------------
     def set_density(self, rho=None, rhoE=None):
         rhoE_d = self.base.set_density(rho=rho, rhoE=rhoE)
         lib = _lib.load()
-        s = self._scratch
-        _lib.check(lib.eigd_q4_material(self.lawG, self.nelems, 4, None, _ptr(rhoE_d), self._parG, None, _ptr(self.kg_d),
+        s, npe = self._scratch, self.base.npe
+        _lib.check(lib.eigd_q4_material(self.lawG, self.nelems, npe, None, _ptr(rhoE_d), self._parG, None, _ptr(self.kg_d),
                                         _ptr(s), _ptr(self.dkg_d), _ptr(s)), "q4_material")
         if self.lawG == 2:      # the reference differentiates the RAMP law of G with q + 1 (:336)
             tmp = D.empty(self.nelems)
-            _lib.check(lib.eigd_q4_material(self.lawG, self.nelems, 4, None, _ptr(rhoE_d), self._pardG, None, _ptr(tmp),
+            _lib.check(lib.eigd_q4_material(self.lawG, self.nelems, npe, None, _ptr(rhoE_d), self._pardG, None, _ptr(tmp),
                                             _ptr(s), _ptr(self.dkg_d), _ptr(s)), "q4_material")
         return rhoE_d
+
+    def set_displacement(self, ur_d):
+        """u = full_vector(u_r): the fundamental path the stress stiffness is linearised about (:561-562)."""
+        self.ur_d = ur_d
+        self.u_d = self.full_vector(ur_d)
+        return self.u_d
+
+    def scatter_to_nodes(self, evals, scale=None):
+        """rho_b[v] = scale * sum_{e ni v} evals[e]; default scale 1 / (nodes per element), the transpose of the element
+        mean."""
+        return self.base.scatter_to_nodes(evals, 1.0 / self.base.npe if scale is None else scale)
+
+
+class BucklingQ4Problem(_BucklingProblem):
+    """Plane-stress Q4 column of examples/buckling.py in HBM: K(x) with Dirichlet rows removed, the fundamental
+    path K_r u_r = f_r, the stress stiffness G(u, x) and the three sensitivity callbacks.
+
+    Element-level outputs stay per element (the node scatter ``np.add.at ... *0.25`` of :212-216, :337-341 is
+    linear and is applied once at the end by the driver).  Reference: examples/buckling.py:152-343, 499-518.
+    """
+
+    def __init__(self, conn, X, bcs, forces, E=1.0, nu=0.3, density=1.0, p=3.0, q=5.0, rho0_K=1e-6, rho0_G=1e-9,
+                 ptype_K="simp", ptype_G="simp"):
+        base = Q4Problem(conn, X, "plane_stress", E=E, nu=nu, density=density, p=p, rho0_K=rho0_K, ptype_K=ptype_K, q=q)
+        self._setup(base, bcs, forces, p, q, density, rho0_G, ptype_G)
+        self.xy_d, self.cmat6_d = base.xy_d, base.cmat6_d
 
     # ---- assembly -------------------------------------------------------------------------------------
     def assemble_K(self):
@@ -516,11 +532,6 @@ class BucklingQ4Problem:
         Kv, Mv = D.empty(self.nnz), D.empty(self.nnz)
         D.q4_assemble(1, self.conn_d, self.xy_d, b.ks_d, b.ms_d, self.cmat6_d, self.src_ptr_d, self.src_d, self.nnz, Kv, Mv)
         return D.CsrDevice(self.indptr_d, self.indices_d, Kv, (self.nred, self.nred))
-
-    def set_displacement(self, ur_d):
-        """u = full_vector(u_r): the fundamental path the stress stiffness is linearised about (:561-562)."""
-        self.u_d = self.full_vector(ur_d)
-        return self.u_d
 
     def assemble_G(self):
         """G_r(u, rho) = reduce_matrix(get_stress_stiffness_matrix(rhoE, u)) (:220-255)."""
@@ -538,8 +549,90 @@ class BucklingQ4Problem:
                        b.dk_d, b.dm_d, 1.0, 0.0, out)
         return out
 
-    def scatter_to_nodes(self, evals, scale=0.25):
-        return self.base.scatter_to_nodes(evals, scale)
+    # ---- sensitivities --------------------------------------------------------------------------------
+    def sensitivity(self, which, Wr, Vr):
+        """dGdu (full dof vector), dGdx or dKdx (per element) of sum_k w_k^T (.) v_k for reduced (n_r, N) W, V."""
+        W, V = self.full_vector(Wr), self.full_vector(Vr)
+        W2 = W if W.dim() == 2 else W.unsqueeze(1)
+        V2 = V if V.dim() == 2 else V.unsqueeze(1)
+        if which == "dGdu":
+            due = D.empty(self.nelems, 8)
+            D.q4_gderiv(self.conn_d, self.xy_d, self.cmat6_d, W2, V2, self.kg_d, self.dkg_d, self.u_d, 1.0, None, due)
+            return D.q4_dof_gather(self.nptr_d, self.nelem_d, self.nlocal_d, due, D.empty(self.ndof))
+        out = D.zeros(self.nelems)
+        if which == "dGdx":
+            D.q4_gderiv(self.conn_d, self.xy_d, self.cmat6_d, W2, V2, self.kg_d, self.dkg_d, self.u_d, 1.0, out, None)
+        else:                                                                     # dKdx
+            D.q4_quadforms(1, self.conn_d, self.xy_d, self.cmat6_d, W2, None, V2, self.base.dk_d, self.base.dm_d, 1.0, 0.0,
+                           out)
+        return out
+
+
+class BucklingH8Problem(_BucklingProblem):
+    """Linearised buckling of a 3-D isotropic solid on trilinear hexahedra, with the interface of ``BucklingQ4Problem``:
+    K_r(x) with the Dirichlet rows removed, the fundamental path K_r u_r = f_r, the stress stiffness G_r(u, x) and the
+    three sensitivity callbacks.  ``bcs`` is {node: [components 0..2]}, ``forces`` {node: [fx, fy, fz]}.
+
+    K_e = s(rho_e) K0_e as in ``H8Problem`` (whose unit matrices it uses), G_e = kg(rho_e) G0_e(u) with the G law of
+    ``BucklingQ4Problem``.  Per design, eigd_h8_stress_stiffness writes the unit stress stiffness G0_e of the current
+    fundamental path (24 x 24 per element, the layout of K0: 4.6 KB per element), so the assembly of G_r and dG/dx are
+    the stored-matrix kernels, as K_r and dK/dx are.  The reduced operands are read through a reduced element dofmap
+    (-1 on clamped dofs): no expansion to full vectors."""
+
+    def __init__(self, conn, X, bcs, forces, E=1.0, nu=0.3, density=1.0, p=3.0, q=5.0, rho0_K=1e-6, rho0_G=1e-9,
+                 ptype_K="simp", ptype_G="simp"):
+        base = H8Problem(conn, X, E=E, nu=nu, density=density, p=p, rho0_K=rho0_K, ptype_K=ptype_K, q=q)
+        self._setup(base, bcs, forces, p, q, density, rho0_G, ptype_G)
+        self.E, self.nu = float(E), float(nu)
+        self.X_d = base.X_d
+        f2r = np.full(self.ndof, -1, dtype=np.int64)
+        f2r[self.reduced] = np.arange(self.nred)
+        self.dofmap_r_d = torch.as_tensor(f2r[base.var].astype(np.int32), device=D.dev())
+        self.G0_d = D.empty(self.nelems * H8Problem.NE ** 2)
+        self.stress_d = D.empty(self.nelems, 8, 6)          # kg C B_q u_e at the 8 Gauss points of every element
+
+    def _assemble(self, E1, c1):
+        vals = D.empty(self.nnz)
+        _lib.check(_lib.load().eigd_stored_assemble(self.nnz, _ptr(self.src_ptr_d), _ptr(self.src_d), H8Problem.NE, _ptr(E1),
+                                                    None, _ptr(c1), None, _ptr(vals), None, None, None, None, None),
+                   "stored_assemble")
+        return D.CsrDevice(self.indptr_d, self.indices_d, vals, (self.nred, self.nred))
+
+    def _quadform(self, dofmap, E1, c1, W, V):
+        W2, V2 = _cols(W), _cols(V)
+        if W2.shape != V2.shape:
+            raise ValueError("W and V must have the same shape")
+        out = D.zeros(self.nelems)
+        _lib.check(_lib.load().eigd_stored_quadform(self.nelems, H8Problem.NE, _ptr(dofmap), _ptr(E1), None, _ptr(c1), None,
+                                                    _ptr(W2), _ptr(V2), V2.shape[1], V2.stride(0), _ptr(out), None, None,
+                                                    None, 1.0, 0.0), "stored_quadform")
+        return out
+
+    def assemble_K(self):
+        """K_r(rho), gathered directly through the reduced source lists."""
+        return self._assemble(self.base.K0_d, self.base.ks_d)
+
+    def assemble_G(self):
+        """G_r(u, rho) about the displacement of ``set_displacement``: element stresses and G0 of this path, then
+        the gather-form assembly with the coefficients kg."""
+        D.h8_stress_stiffness(self.conn_d, self.X_d, self.E, self.nu, self.kg_d, self.dofmap_r_d, self.ur_d, self.stress_d,
+                              self.G0_d)
+        return self._assemble(self.G0_d, self.kg_d)
+
+    def dK_single(self, psi_full, u_full):
+        """psi^T (dK/drho_e) u per element for one pair of full vectors."""
+        return self._quadform(self.base.dofmap_d, self.base.K0_d, self.base.dk_d, psi_full, u_full)
+
+    def sensitivity(self, which, Wr, Vr):
+        """dGdu (full dof vector), dGdx or dKdx (per element) of sum_k w_k^T (.) v_k for reduced (n_r, N) W, V."""
+        if which == "dGdu":
+            W2, V2 = _cols(Wr), _cols(Vr)
+            due = D.h8_gderiv_u(self.conn_d, self.X_d, self.E, self.nu, self.kg_d, self.dofmap_r_d, W2, V2,
+                                D.empty(self.nelems, H8Problem.NE))
+            return D.h8_dof_gather(self.nptr_d, self.nelem_d, self.nlocal_d, due, D.empty(self.ndof))
+        if which == "dGdx":
+            return self._quadform(self.dofmap_r_d, self.G0_d, self.dkg_d, Wr, Vr)
+        return self._quadform(self.dofmap_r_d, self.base.K0_d, self.base.dk_d, Wr, Vr)
 
 
 def _contig1(t):

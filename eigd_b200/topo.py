@@ -505,8 +505,8 @@ class BucklingTopologyAnalysis(_EigenAnalysis):
         self.fltr = fltr
         self.pivoting = pivoting          # of the shifted factor K_r + sigma G_r (SpLuOperator); K_r alone is SPD
         self.conn, self.X = np.asarray(conn), np.asarray(X)
-        prob = fe.BucklingQ4Problem(self.conn, self.X, bcs, forces, E=E, nu=nu, density=density, p=float(p), q=float(q),
-                                    rho0_K=rho0_K, rho0_G=rho0_G, ptype_K=ptype_K.lower(), ptype_G=ptype_G.lower())
+        prob = self._make_problem(bcs, forces, E=E, nu=nu, density=density, p=float(p), q=float(q), rho0_K=rho0_K,
+                                  rho0_G=rho0_G, ptype_K=ptype_K.lower(), ptype_G=ptype_G.lower())
         super().__init__(prob, N, m, solver_type, tol, rtol, eig_atol, adjoint_method, adjoint_options, deriv_type, seed)
         self.nelems, self.nnodes, self.nvars = self.prob.nelems, self.prob.nnodes, self.prob.ndof
         self.reduced, self.f = self.prob.reduced, self.prob.f
@@ -516,6 +516,9 @@ class BucklingTopologyAnalysis(_EigenAnalysis):
         self.x = 0.5 * np.ones(self.fltr.num_design_vars)                 # buckling.py:81
         self.profile.update(nnodes=self.nnodes, nelems=self.nelems, solver_type=solver_type,
                             adjoint_method=self.adjoint_method, N=N)
+
+    def _make_problem(self, bcs, forces, **material):
+        return fe.BucklingQ4Problem(self.conn, self.X, bcs, forces, **material)
 
     # ---- forward (:548-640, 811-838) ----------------------------------------------------------------
     def solve_eigenvalue_problem(self, store=False):
@@ -688,3 +691,48 @@ def make_buckling_model(nx=64, ny=128, Lx=1.0, Ly=2.0, rfact=4.0, N=10, shear_fo
     conn, X, dvmap, ndv, bcs, forces = domain_compressed_column(nx=nx, ny=ny, Lx=Lx, Ly=Ly, shear_force=shear_force)
     fltr = fe.NodeFilter(conn, X, r0=rfact * (Lx / nx), dvmap=dvmap, num_design_vars=ndv)
     return BucklingTopologyAnalysis(fltr, conn, X, bcs=bcs, forces=forces, N=N, **kwargs)
+
+
+class BucklingTopology3DAnalysis(BucklingTopologyAnalysis):
+    """The linearised buckling problem of ``BucklingTopologyAnalysis`` on a 3-D solid of trilinear hexahedra
+    (``fe.BucklingH8Problem``), with the same forward and reverse pipeline and objectives.
+
+    Each design keeps two factors on one symbolic analysis, K_r (for the fundamental-path adjoint) and K_r + sigma G_r,
+    each with its own front workspace.  The previous design's factors, and the eigensolver that references them, are
+    dropped before the next design is factored, so the peak is two front workspaces rather than three."""
+
+    def _make_problem(self, bcs, forces, **material):
+        return fe.BucklingH8Problem(self.conn, self.X, bcs, forces, **material)
+
+    def solve_eigenvalue_problem(self, store=False):
+        self.factor = self.Kfact = self.eig_solver = None
+        return super().solve_eigenvalue_problem(store)
+
+
+def domain_compressed_column_3d(nx, ny, nz, Lx, Ly, Lz):
+    """Column along z on ``fe.hex_mesh(nx, ny, nz, Lx, Ly, Lz)``, the 3-D counterpart of ``domain_compressed_column``:
+    base face (z = 0) clamped, a compressive load P = 3e-4 in -z spread evenly over a central patch of the top face of
+    (2 ceil(nx / 30) + 1) x (2 ceil(ny / 30) + 1) nodes.  Returns conn, X, bcs {node: [0, 1, 2]} and forces
+    {node: [0, 0, -P / patch nodes]}."""
+    conn, X = fe.hex_mesh(nx, ny, nz, Lx, Ly, Lz)
+    nodes = np.arange((nx + 1) * (ny + 1) * (nz + 1), dtype=np.int64).reshape(nx + 1, ny + 1, nz + 1)
+    bcs = {int(v): [0, 1, 2] for v in nodes[:, :, 0].ravel()}
+    P = 3e-4
+    ox, oy = int(np.ceil(nx / 30)), int(np.ceil(ny / 30))
+    patch = nodes[nx // 2 - ox:nx // 2 + ox + 1, ny // 2 - oy:ny // 2 + oy + 1, nz].ravel()
+    forces = {int(v): [0.0, 0.0, -P / len(patch)] for v in patch}
+    return conn, X, bcs, forces
+
+
+def make_buckling_3d_model(nx=32, ny=24, nz=128, Lx=1.0, Ly=0.75, Lz=4.0, rfact=4.0, N=10, **kwargs):
+    """``domain_compressed_column_3d`` with one design variable per node and a conic filter of radius rfact * Lx / nx.
+    The default cross-section is rectangular: a square column has pairs of equal buckling loads, where eigenvector
+    derivatives are undefined.  The load makes the first load factors O(1): on a coarse 4 x 3 x 16 mesh at x = 0.5 the
+    Euler modes about the weak and strong axes are at about 2.4 and 4.0; finer meshes add modes near the loaded patch
+    from about 2.5 up (32 x 24 x 128, x ~ U(0.3, 0.7): 8 load factors below 3).  The default sigma = 3 lies inside
+    the spectrum, so K_r + sigma G_r is indefinite.  As in the 2-D driver the eigensolver returns the N load factors
+    nearest sigma in the buckling shift-invert transform, which ranks a lambda < sigma below every lambda > sigma
+    when lambda < sigma / 2.  At 32 x 24 x 128 each factor's fronts take 44 GB (DESIGN.md section 8b)."""
+    conn, X, bcs, forces = domain_compressed_column_3d(nx, ny, nz, Lx, Ly, Lz)
+    fltr = fe.NodeFilter(conn, X, r0=rfact * (Lx / nx))
+    return BucklingTopology3DAnalysis(fltr, conn, X, bcs=bcs, forces=forces, N=N, **kwargs)

@@ -264,6 +264,20 @@ int eigd_q4_gderiv(int nelems, const int* d_conn, const double* d_xy, const doub
 /* dfdu[2v + d] = sum_{e around v} due[e][2 local + d] (gather form of np.add.at, :318-320) */
 int eigd_q4_dof_gather(int nnodes, const int* d_nptr, const int* d_nelem, const int* d_nlocal, const double* d_due,
                        double* d_out);
+/* ---- linearised buckling of the 3-D solid (csrc/h8_buckling.cu), H8 elements as eigd_h8_element_matrices.
+ *      dofmap (nelems, 24): element dof (node-major u_x, u_y, u_z) -> row of u, W and V; -1 = constrained (zero).
+ *      Voigt order (xx, yy, zz, yz, xz, xy), engineering shear; C = C(E, nu) of K0. ---- */
+/* per design: stress[e][q][6] = kg[e] C B_q u_e (NULL: not written) and the unit stress stiffness
+ * G0[e] (24 x 24 row-major) = [delta_ij sum_q detJ_q gradN_a^T S_q gradN_b], S_q the 3 x 3 form of C B_q u_e */
+int eigd_h8_stress_stiffness(int nelems, const int* d_conn, const double* d_X, double E, double nu, const double* d_kg,
+                             const int* d_dofmap, const double* d_u, double* d_stress, double* d_G0);
+/* due[e][24] = kg[e] sum_q detJ_q B_q^T C h_q, h_q = sum_k sum_i Voigt(grad w_{i,k} (x) grad v_{i,k}) with both shear
+ * products: d/du_e of sum_k w_k^T G(u) v_k.  W, V row-major with leading dimension ld, N columns. */
+int eigd_h8_gderiv_u(int nelems, const int* d_conn, const double* d_X, double E, double nu, const double* d_kg,
+                     const int* d_dofmap, const double* d_W, const double* d_V, int N, int64_t ld, double* d_due);
+/* out[3v + i] = sum_{e around v} due[e][3 local + i] (gather form, as eigd_q4_dof_gather) */
+int eigd_h8_dof_gather(int nnodes, const int* d_nptr, const int* d_nelem, const int* d_nlocal, const double* d_due,
+                       double* d_out);
 /* full[idx[i], :] = red[i, :] and red[i, :] = full[idx[i], :], k columns, row-major */
 int eigd_expand_rows(int64_t nr, int k, const int* d_idx, const double* d_red, double* d_full);
 int eigd_reduce_rows(int64_t nr, int k, const int* d_idx, const double* d_full, double* d_red);

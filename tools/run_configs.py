@@ -4,6 +4,7 @@
     python tools/run_configs.py c5 [--designs 8]                      design sweep, 202k-DOF natural-frequency mesh
     python tools/run_configs.py c4 [--nx 408 --ny 408 --modes 20 --fd]   1M-DOF synthetic shell (6 dof/node), crm.py driver
     python tools/run_configs.py h8 [--nx 64 --ny 32 --nz 32 --modes 10 --fd]   free 3-D solid of hexahedra (3 dof/node)
+    python tools/run_configs.py h8buck [--nx 32 --ny 24 --nz 128 --modes 10 --fd]   buckling of a clamped 3-D column
 
 Each prints one JSON line: stage times (CUDA-synchronised wall clock of the driver's own timers, as the
 reference examples report them), solve counts, factor statistics, and size-independent acceptance checks
@@ -291,6 +292,91 @@ def run_h8(args):
     return out
 
 
+def run_h8buck(args):
+    """Clamped 3-D column of hexahedra (BucklingTopology3DAnalysis, make_buckling_3d_model): N load factors about
+    sigma = 3 (indefinite shifted factor), IRAM + sibk with the Lanczos guess, tensor derivative, the tanh eigenvector
+    aggregate at the dof of largest |phi_1| as the objective, including the fundamental-path adjoint."""
+    import torch
+    from eigd_b200 import device as D, topo as T
+    D.init()
+    out = {"config": "H8 buckling column nx=%d ny=%d nz=%d" % (args.nx, args.ny, args.nz), "N": args.modes, "gpu": gpu_card()}
+    t0 = now()
+    model = T.make_buckling_3d_model(args.nx, args.ny, args.nz, N=args.modes, m=60, solver_type="IRAM", adjoint_method="sibk",
+                                     adjoint_options={"lanczos_guess": True}, rtol=1e-10, deriv_type="tensor")
+    out.update(n=int(model.prob.nred), nnz=int(model.prob.nnz), sigma=float(model.sigma), host_setup_s=now() - t0)
+    x0 = np.random.default_rng(0).uniform(0.3, 0.7, model.fltr.num_design_vars)       # first load factor below sigma
+    torch.cuda.reset_peak_memory_stats()
+    reps = []
+    for rep in range(args.reps):
+        l0 = D.launch_count()
+        ta = now()
+        with warnings.catch_warnings():
+            warnings.simplefilter("ignore")
+            model.initialize(x=x0)
+        model.initialize_adjoint()
+        if rep == 0:
+            node = int(np.argmax(np.abs(model.prob.full_vector(model.Qr[:, 0].contiguous()).cpu().numpy())))
+        h = model.add_eigenvector_aggregate_derivative(1.0, 100.0, node, mode="tanh")
+        model.finalize_adjoint()
+        tb = now()
+        p = model.profile
+        reps.append({"wall_s": tb - ta, "assembly_s": p["matrix assembly time"], "eig_s": p["eigenvalue solve time"],
+                     "adjoint_s": p["adjoint solution time"], "dfdx_s": p["total derivative time"],
+                     "time_to_gradient_s": model.time_to_gradient(), "eig_solves": p["solve preconditioner count"],
+                     "adjoint_solves": p["adjoint preconditioner count"], "launches": D.launch_count() - l0,
+                     "symbolic_s": p.get("symbolic analysis time")})
+    out["reps"] = reps
+    out["peak_device_bytes"] = int(torch.cuda.max_memory_allocated())
+    amap = model.symbolic[1]
+    shifted = D.axpby(1.0, model.Kr.data, float(model.sigma), model.Gr.data)
+    out["factorisation_s"] = {"K_r": _time_numeric(model.Kfact.lu, model.Kr.data, amap),
+                              "K_r + sigma G_r": _time_numeric(model.factor.lu, shifted, amap)}
+    out["BLF"] = [float(v) for v in model.BLF]
+    out["factor_info"] = {"K_r": model.Kfact.info, "K_r + sigma G_r": model.factor.info}
+    out["refine_steps"] = model.factor.refine
+    out["probe_residual_unrefined"] = model.factor._probe_residual()
+    out["symbolic"] = model.symbolic[0].stats()
+    res, orth = residuals(model, model.Gr, model.Kr, model.BLF, model.Qr, "buckling")
+    out["eigen_residual_max"] = res
+    out["orthonormality_defect"] = orth
+    ar, ao = model.eig_solver.eval_adjoint_residual_norm(model.Qrb, model.psir, b_ortho=True)
+    rhs = float(model.Qrb.norm(dim=0).max().item())
+    out["adjoint_residual_over_rtol_rhs"] = float(np.max(ar)) / (1e-10 * rhs)
+    assert out["adjoint_residual_over_rtol_rhs"] < 50.0, out["adjoint_residual_over_rtol_rhs"]
+    assert res < 1e-8 and orth < 1e-10, (res, orth)
+    assert out["factor_info"]["K_r + sigma G_r"]["negative_pivots"] > 0, out["factor_info"]
+    out["aggregate_h"] = h
+    xb = model.xb.cpu().numpy().copy()
+    out["xb_norm"] = float(np.linalg.norm(xb))
+    if args.fd:
+        pert = np.random.default_rng(3).uniform(-1.0, 1.0, x0.shape)
+        step = 1e-5
+        vals = []
+        for sgn in (1.0, -1.0):
+            with warnings.catch_warnings():
+                warnings.simplefilter("ignore")
+                model.initialize(x=x0 + sgn * step * pert)
+            vals.append(model.get_eigenvector_aggregate(100.0, node, mode="tanh"))
+        fd = (vals[0] - vals[1]) / (2 * step)
+        out["fd_directional"] = fd
+        out["adjoint_directional"] = float(xb @ pert)
+        out["fd_rel_err"] = abs(fd - float(xb @ pert)) / abs(fd)
+        assert out["fd_rel_err"] < 1e-5, out["fd_rel_err"]
+        out["peak_device_bytes_with_fd"] = int(torch.cuda.max_memory_allocated())
+    out["gpu_after"] = gpu_card()
+    return out
+
+
+def _time_numeric(lu, vals, amap, reps=3):
+    """Numeric LDL^T of ``vals`` alone, refactored in place in the factor ``lu``, device-synchronised, every repetition."""
+    times = []
+    for _ in range(reps):
+        t0 = now()
+        lu.numeric(vals, amap)
+        times.append(now() - t0)
+    return times
+
+
 def _time_factorisation(model, reps=3):
     """Numeric LDL^T of the last design's K - sigma M, alone (the driver's eigensolve time includes it): the driver's
     factor refactored in place on the same values, device-synchronised, every repetition."""
@@ -306,11 +392,11 @@ def _time_factorisation(model, reps=3):
 
 if __name__ == "__main__":
     ap = argparse.ArgumentParser()
-    ap.add_argument("config", choices=["c3", "c4", "c4plate", "c5", "h8"])
+    ap.add_argument("config", choices=["c3", "c4", "c4plate", "c5", "h8", "h8buck"])
     ap.add_argument("--fd", action="store_true", help="c4: add the finite-difference check of the gradient")
     ap.add_argument("--nx", type=int, default=None)
     ap.add_argument("--ny", type=int, default=None)
-    ap.add_argument("--nz", type=int, default=None, help="h8: elements along z")
+    ap.add_argument("--nz", type=int, default=None, help="h8, h8buck: elements along z")
     ap.add_argument("--modes", type=int, default=None)
     ap.add_argument("--designs", type=int, default=None)
     ap.add_argument("--reps", type=int, default=3)
@@ -324,6 +410,9 @@ if __name__ == "__main__":
     elif a.config == "h8":
         a.nx, a.ny, a.nz, a.modes = a.nx or 64, a.ny or 32, a.nz or 32, a.modes or 10
         res = run_h8(a)
+    elif a.config == "h8buck":
+        a.nx, a.ny, a.nz, a.modes = a.nx or 32, a.ny or 24, a.nz or 128, a.modes or 10
+        res = run_h8buck(a)
     elif a.config == "c4":
         a.nx, a.ny, a.modes = a.nx or 408, a.ny or 408, a.modes or 20
         res = run_c4(a)
