@@ -41,8 +41,11 @@ SIGNATURES = {
     "eigd_factor_create": (c_int, [c_ptr, c_int, c_ptr]),
     "eigd_factor_workspace_bytes": (c_i64, [c_ptr, c_int]),
     "eigd_factor_create_in": (c_int, [c_ptr, c_int, c_ptr, c_i64, c_ptr]),
+    "eigd_factor_workspace_bytes_fronts": (c_i64, [c_ptr, c_int, c_int]),
+    "eigd_factor_create_in_fronts": (c_int, [c_ptr, c_int, c_int, c_ptr, c_i64, c_ptr]),
     "eigd_factor_destroy": (None, [c_ptr]),
     "eigd_factor_numeric": (c_int, [c_ptr, c_i64, c_ptr, c_ptr]),
+    "eigd_factor_numeric_pool": (c_int, [c_ptr, c_i64, c_ptr, c_ptr, c_ptr, c_ptr, c_i64]),
     "eigd_factor_info": (c_int, [c_ptr, c_ptr]),
     "eigd_factor_set_pivoting": (c_int, [c_ptr, c_int]),
     "eigd_factor_pivot_counts": (c_int, [c_ptr, c_ptr]),

@@ -6,7 +6,9 @@
 // Data layout in HBM
 //   fronts : one dense column-major f x f block per supernode (lower triangle used);
 //            columns [0, ncols) hold L (unit diagonal implied, D on the diagonal), the
-//            trailing (f-ncols)^2 block is the contribution passed to the parent.
+//            trailing (f-ncols)^2 block is the contribution passed to the parent.  Resident (front_off, in the
+//            factor's workspace for its life) or pooled (pool_off, in a pool the caller lends to one numeric call;
+//            a front is live from its own level through its parent's, see pool_layout in symbolic.cpp).
 //   linv   : explicit inverses of the 32x32 unit-lower diagonal blocks of every L11 (used by the
 //            panel solves of the factorisation); with restricted Bunch-Kaufman pivoting the inverses of
 //            the dense diagonal blocks M (diag_factor_bk_kernel).
@@ -45,12 +47,94 @@ static void free_symdev(void* p) {
   free_solve_plan_dev(h);
   for (void* a : h->allocs) cudaFree(a);
   if (h->tasks) cudaFree(h->tasks);
+  if (h->pool_tasks) cudaFree(h->pool_tasks);
   delete h;
 }
 
 inline int tri_tiles(int m, int tile) {
   int t = (m + tile - 1) / tile;
   return t * (t + 1) / 2;
+}
+
+static void push_launch(std::vector<int2>& tasks, std::vector<Launch>& plan, int kind, int kb, int64_t off) {
+  int count = (int)((int64_t)tasks.size() - off);
+  if (count > 0) plan.push_back({kind, kb, off, count});
+}
+
+// extend-add into the fronts of level l (one launch per sibling rank), then the pivot-block chain of its fronts
+static void push_level_tasks(const eigd_symbolic* S, int l, std::vector<int2>& tasks, std::vector<Launch>& plan) {
+  const int* sn = S->level_sn.data() + S->level_ptr[l];
+  int cnt = S->level_ptr[l + 1] - S->level_ptr[l];
+  // extend-add: one launch per sibling rank so that no two tasks touch the same parent
+  int maxrank = 0;
+  for (int i = 0; i < cnt; ++i) maxrank = std::max(maxrank, S->child_ptr[sn[i] + 1] - S->child_ptr[sn[i]]);
+  for (int r = 0; r < maxrank; ++r) {
+    int64_t off = (int64_t)tasks.size();
+    for (int i = 0; i < cnt; ++i) {
+      int p = sn[i];
+      if (S->child_ptr[p] + r >= S->child_ptr[p + 1]) continue;
+      int c = S->child_idx[S->child_ptr[p] + r];
+      int nt = tri_tiles(sn_nbelow(S, c), EA_TILE);
+      for (int t = 0; t < nt; ++t) tasks.push_back(make_int2(c, t));
+    }
+    push_launch(tasks, plan, 0, r, off);
+  }
+  int maxsteps = 0;
+  for (int i = 0; i < cnt; ++i) maxsteps = std::max(maxsteps, (sn_ncols(S, sn[i]) + NB - 1) / NB);
+  for (int kb = 0; kb < maxsteps; ++kb) {
+    int64_t off = (int64_t)tasks.size();
+    for (int i = 0; i < cnt; ++i)
+      if (sn_ncols(S, sn[i]) > kb * NB) tasks.push_back(make_int2(sn[i], 0));
+    push_launch(tasks, plan, 1, kb, off);
+    off = (int64_t)tasks.size();
+    for (int i = 0; i < cnt; ++i) {
+      int k = sn[i], nc = sn_ncols(S, k), f = sn_fsize(S, k);
+      if (nc <= kb * NB) continue;
+      int r0 = std::min(nc, (kb + 1) * NB);
+      int nt = (f - r0 + TRSM_ROWS - 1) / TRSM_ROWS;
+      for (int t = 0; t < nt; ++t) tasks.push_back(make_int2(k, t));
+    }
+    push_launch(tasks, plan, 2, kb, off);
+    off = (int64_t)tasks.size();
+    for (int i = 0; i < cnt; ++i) {
+      int k = sn[i], nc = sn_ncols(S, k), f = sn_fsize(S, k);
+      if (nc <= kb * NB) continue;
+      int r0 = std::min(nc, (kb + 1) * NB);
+      int nt = tri_tiles(f - r0, UPD_TILE);
+      for (int t = 0; t < nt; ++t) tasks.push_back(make_int2(k, t));
+    }
+    push_launch(tasks, plan, 3, kb, off);
+  }
+}
+
+// full inverses of the pivot blocks (recursive doubling) and the solve panels of the fronts sn[0 .. cnt)
+static void push_panel_tasks(const eigd_symbolic* S, const int* sn, int cnt, std::vector<int2>& tasks,
+                             std::vector<Launch>& plan) {
+  int64_t off = (int64_t)tasks.size();
+  int maxcols = 0;
+  for (int i = 0; i < cnt; ++i) {
+    tasks.push_back(make_int2(sn[i], 0));
+    maxcols = std::max(maxcols, sn_ncols(S, sn[i]));
+  }
+  push_launch(tasks, plan, 4, 0, off);
+  for (int stage = 0, hb = NB; hb < maxcols; ++stage, hb *= 2) {
+    off = (int64_t)tasks.size();
+    for (int i = 0; i < cnt; ++i) {
+      int k = sn[i], nc = sn_ncols(S, k);
+      for (int q = 0; (2 * q + 1) * hb < nc; ++q) {
+        int hh = std::min(hb, nc - (2 * q + 1) * hb);
+        for (int ti = 0; ti * NB < hh; ++ti)
+          for (int tj = 0; tj * NB < hb; ++tj) tasks.push_back(make_int2(k, q * 64 + ti * 8 + tj));
+      }
+    }
+    int64_t end = (int64_t)tasks.size();
+    push_launch(tasks, plan, 5, stage, off);       // T = C A^-1
+    if (end > off) plan.push_back({6, stage, off, (int)(end - off)});   // X21 = -B^-1 T (same tasks)
+  }
+  off = (int64_t)tasks.size();
+  for (int i = 0; i < cnt; ++i)
+    for (int t = 0; t * NB < sn_fsize(S, sn[i]); ++t) tasks.push_back(make_int2(sn[i], t));
+  push_launch(tasks, plan, 7, 0, off);
 }
 
 int build_symdev(eigd_symbolic* S) {
@@ -92,85 +176,44 @@ int build_symdev(eigd_symbolic* S) {
 
   // ---- task lists ---------------------------------------------------------------------
   std::vector<int2> tasks;
-  auto push_launch = [&](std::vector<Launch>& plan, int kind, int kb, int64_t off) {
-    int count = (int)((int64_t)tasks.size() - off);
-    if (count > 0) plan.push_back({kind, kb, off, count});
-  };
-  // rank of each child among its siblings
-  std::vector<int> rank(ns, 0);
-  for (int p = 0; p < ns; ++p)
-    for (int q = S->child_ptr[p]; q < S->child_ptr[p + 1]; ++q) rank[S->child_idx[q]] = q - S->child_ptr[p];
-  for (int l = 0; l < S->nlevels; ++l) {
-    const int* sn = S->level_sn.data() + S->level_ptr[l];
-    int cnt = S->level_ptr[l + 1] - S->level_ptr[l];
-    // extend-add: one launch per sibling rank so that no two tasks touch the same parent
-    int maxrank = 0;
-    for (int i = 0; i < cnt; ++i) maxrank = std::max(maxrank, S->child_ptr[sn[i] + 1] - S->child_ptr[sn[i]]);
-    for (int r = 0; r < maxrank; ++r) {
-      int64_t off = (int64_t)tasks.size();
-      for (int i = 0; i < cnt; ++i) {
-        int p = sn[i];
-        if (S->child_ptr[p] + r >= S->child_ptr[p + 1]) continue;
-        int c = S->child_idx[S->child_ptr[p] + r];
-        int nt = tri_tiles(sn_nbelow(S, c), EA_TILE);
-        for (int t = 0; t < nt; ++t) tasks.push_back(make_int2(c, t));
-      }
-      push_launch(h->factor_plan, 0, r, off);
-    }
-    int maxsteps = 0;
-    for (int i = 0; i < cnt; ++i) maxsteps = std::max(maxsteps, (sn_ncols(S, sn[i]) + NB - 1) / NB);
-    for (int kb = 0; kb < maxsteps; ++kb) {
-      int64_t off = (int64_t)tasks.size();
-      for (int i = 0; i < cnt; ++i)
-        if (sn_ncols(S, sn[i]) > kb * NB) tasks.push_back(make_int2(sn[i], 0));
-      push_launch(h->factor_plan, 1, kb, off);
-      off = (int64_t)tasks.size();
-      for (int i = 0; i < cnt; ++i) {
-        int k = sn[i], nc = sn_ncols(S, k), f = sn_fsize(S, k);
-        if (nc <= kb * NB) continue;
-        int r0 = std::min(nc, (kb + 1) * NB);
-        int nt = (f - r0 + TRSM_ROWS - 1) / TRSM_ROWS;
-        for (int t = 0; t < nt; ++t) tasks.push_back(make_int2(k, t));
-      }
-      push_launch(h->factor_plan, 2, kb, off);
-      off = (int64_t)tasks.size();
-      for (int i = 0; i < cnt; ++i) {
-        int k = sn[i], nc = sn_ncols(S, k), f = sn_fsize(S, k);
-        if (nc <= kb * NB) continue;
-        int r0 = std::min(nc, (kb + 1) * NB);
-        int nt = tri_tiles(f - r0, UPD_TILE);
-        for (int t = 0; t < nt; ++t) tasks.push_back(make_int2(k, t));
-      }
-      push_launch(h->factor_plan, 3, kb, off);
-    }
-  }
-  // ---- after the last level: full inverses of the pivot blocks and the solve panels (all fronts at once)
-  {
-    int64_t off = (int64_t)tasks.size();
-    for (int k = 0; k < ns; ++k) tasks.push_back(make_int2(k, 0));
-    push_launch(h->factor_plan, 4, 0, off);
-    for (int stage = 0, hb = NB; hb < S->maxcols; ++stage, hb *= 2) {
-      off = (int64_t)tasks.size();
-      for (int k = 0; k < ns; ++k) {
-        int nc = sn_ncols(S, k);
-        for (int q = 0; (2 * q + 1) * hb < nc; ++q) {
-          int hh = std::min(hb, nc - (2 * q + 1) * hb);
-          for (int ti = 0; ti * NB < hh; ++ti)
-            for (int tj = 0; tj * NB < hb; ++tj) tasks.push_back(make_int2(k, q * 64 + ti * 8 + tj));
-        }
-      }
-      int64_t end = (int64_t)tasks.size();
-      push_launch(h->factor_plan, 5, stage, off);       // T = C A^-1
-      if (end > off) h->factor_plan.push_back({6, stage, off, (int)(end - off)});   // X21 = -B^-1 T (same tasks)
-    }
-    off = (int64_t)tasks.size();
-    for (int k = 0; k < ns; ++k)
-      for (int t = 0; t * NB < sn_fsize(S, k); ++t) tasks.push_back(make_int2(k, t));
-    push_launch(h->factor_plan, 7, 0, off);
-  }
+  std::vector<int> all(ns);
+  for (int k = 0; k < ns; ++k) all[k] = k;
+  for (int l = 0; l < S->nlevels; ++l) push_level_tasks(S, l, tasks, h->factor_plan);
+  // after the last level: full inverses of the pivot blocks and the solve panels (all fronts at once)
+  push_panel_tasks(S, all.data(), ns, tasks, h->factor_plan);
   EIGD_CUDA(cudaMalloc((void**)&h->tasks, std::max<size_t>(tasks.size(), 1) * sizeof(int2)));
   EIGD_CUDA(cudaMemcpy(h->tasks, tasks.data(), tasks.size() * sizeof(int2), cudaMemcpyHostToDevice));
   return build_solve_plan_dev(S, h);
+}
+
+// The plan of the pooled front mode, built on first use: per level, the fronts of the level are zeroed in the pool and
+// receive their matrix entries (kind 8), take their children's contributions, are factorised, and leave their pivot-
+// block inverses and solve panels before any front of a later level can reuse their memory.  Same kernels and the
+// same per-front arithmetic as factor_plan; the fronts are addressed through pool_off instead of front_off.
+int build_pool_plan(eigd_symbolic* S) {
+  int rc = build_symdev(S);
+  if (rc) return rc;
+  auto* h = (SymDevHolder*)S->dev;
+  if (h->pool_tasks) return 0;
+  if (S->maxfront > 46340) { eigd_set_error("pooled fronts: a front of %d rows is wider than the 32-bit slot index allows", S->maxfront); return 4; }
+  rc = upload(h, S->pool_off, &h->pool_off);
+  if (rc) return rc;
+  std::vector<int2> tasks;
+  for (int l = 0; l < S->nlevels; ++l) {
+    const int* sn = S->level_sn.data() + S->level_ptr[l];
+    int cnt = S->level_ptr[l + 1] - S->level_ptr[l];
+    int64_t off = (int64_t)tasks.size();
+    for (int i = 0; i < cnt; ++i) {
+      int64_t f = sn_fsize(S, sn[i]);
+      for (int64_t t = 0; t * POOL_CHUNK < f * f; ++t) tasks.push_back(make_int2(sn[i], (int)t));
+    }
+    push_launch(tasks, h->pool_plan, 8, 0, off);
+    push_level_tasks(S, l, tasks, h->pool_plan);
+    push_panel_tasks(S, sn, cnt, tasks, h->pool_plan);
+  }
+  EIGD_CUDA(cudaMalloc((void**)&h->pool_tasks, std::max<size_t>(tasks.size(), 1) * sizeof(int2)));
+  EIGD_CUDA(cudaMemcpy(h->pool_tasks, tasks.data(), tasks.size() * sizeof(int2), cudaMemcpyHostToDevice));
+  return 0;
 }
 
 namespace {
@@ -224,6 +267,39 @@ __global__ void scatter_values_kernel(int64_t nnz, const double* __restrict__ va
   for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < nnz; e += (int64_t)gridDim.x * blockDim.x) {
     int64_t m = map[e];
     if (m >= 0) fronts[m] = vals[e];
+  }
+}
+
+// Pooled fronts: chunk tk.y (POOL_CHUNK doubles) of front tk.x is zeroed, then receives the matrix entries whose slots
+// fall in it: ent[seg[s] .. seg[s + 1]) are (CSR index, slot in the front) pairs sorted by slot.  One CTA owns the
+// chunk, so the zero stores and the entry stores need no atomics, only one block barrier between them.  Front offsets
+// are multiples of 32 doubles and chunks start at multiples of POOL_CHUNK: the 16-byte zero stores are aligned.
+__global__ void __launch_bounds__(256)
+front_assemble_kernel(SymDev d, const int2* __restrict__ tasks, const double* __restrict__ vals,
+                      const int64_t* __restrict__ seg, const int2* __restrict__ ent, double* __restrict__ pool) {
+  __shared__ int64_t range[2];
+  const int2 tk = tasks[blockIdx.x];
+  const int s = tk.x;
+  const int64_t f = (d.sn_first[s + 1] - d.sn_first[s]) + (d.sn_rowptr[s + 1] - d.sn_rowptr[s]);
+  const int64_t lo = (int64_t)tk.y * POOL_CHUNK, hi = min(f * f, lo + POOL_CHUNK);
+  double* F = pool + d.front_off[s];
+  double2* Z = reinterpret_cast<double2*>(F + lo);
+  const int nz2 = (int)((hi - lo) >> 1);
+  for (int i = threadIdx.x; i < nz2; i += blockDim.x) Z[i] = make_double2(0.0, 0.0);
+  if (((hi - lo) & 1) && threadIdx.x == 0) F[hi - 1] = 0.0;
+  if (threadIdx.x < 2) {                    // first entry with slot >= lo (thread 0) / >= hi (thread 1)
+    const int64_t key = threadIdx.x ? hi : lo;
+    int64_t a = seg[s], b = seg[s + 1];
+    while (a < b) {
+      const int64_t m = (a + b) >> 1;
+      if (ent[m].y < key) a = m + 1; else b = m;
+    }
+    range[threadIdx.x] = a;
+  }
+  __syncthreads();
+  for (int64_t e = range[0] + threadIdx.x; e < range[1]; e += blockDim.x) {
+    const int2 v = ent[e];
+    F[v.y] = vals[v.x];
   }
 }
 
@@ -815,10 +891,10 @@ static inline int64_t align256(int64_t b) { return (b + 255) / 256 * 256; }
 
 // sizes (bytes, 256-aligned) of the device arrays of a factor, in carving order
 constexpr int NARR = 16;
-static void factor_layout(const eigd_symbolic* s, const SymDevHolder* h, int max_rhs, int64_t sz[NARR]) {
+static void factor_layout(const eigd_symbolic* s, const SymDevHolder* h, int max_rhs, bool pooled, int64_t sz[NARR]) {
   int64_t nfront = s->front_off[s->nsuper], sumf = s->w_off[s->nsuper];
   int kc = std::min(max_rhs, 16);                      // the solve processes at most 16 columns per sweep
-  sz[0] = align256(nfront * 8);                        // fronts
+  sz[0] = pooled ? 0 : align256(nfront * 8);           // fronts (pooled: borrowed per numeric call)
   sz[1] = align256(h->linv_total * 8);                 // linv
   sz[2] = align256(h->xinv_total * 8);                 // xinv
   sz[3] = align256(h->xinv_total * 8);                 // xtmp
@@ -836,26 +912,38 @@ static void factor_layout(const eigd_symbolic* s, const SymDevHolder* h, int max
   sz[15] = 0;
 }
 
-extern "C" int64_t eigd_factor_workspace_bytes(eigd_symbolic* s, int max_rhs) {
-  if (build_symdev(s)) return -1;
+static bool fronts_mode_ok(int fronts) {
+  if (fronts == 0 || fronts == 1) return true;
+  eigd_set_error("factor: fronts mode %d (0 resident, 1 pooled)", fronts);
+  return false;
+}
+
+extern "C" int64_t eigd_factor_workspace_bytes_fronts(eigd_symbolic* s, int max_rhs, int fronts) {
+  if (!fronts_mode_ok(fronts) || build_symdev(s)) return -1;
   int64_t sz[NARR], tot = 0;
-  factor_layout(s, (SymDevHolder*)s->dev, std::max(1, max_rhs), sz);
+  factor_layout(s, (SymDevHolder*)s->dev, std::max(1, max_rhs), fronts == 1, sz);
   for (int i = 0; i < NARR; ++i) tot += sz[i];
   return tot + 256;
 }
 
+extern "C" int64_t eigd_factor_workspace_bytes(eigd_symbolic* s, int max_rhs) {
+  return eigd_factor_workspace_bytes_fronts(s, max_rhs, 0);
+}
+
 // d_workspace == NULL: the library allocates (cudaMalloc) and owns the arrays; otherwise they are carved
 // out of the caller's buffer (a torch tensor: the caching allocator then recycles it between factors)
-extern "C" int eigd_factor_create_in(eigd_symbolic* s, int max_rhs, void* d_workspace, int64_t workspace_bytes,
-                                     eigd_factor** out) {
-  int rc = build_symdev(s);
+extern "C" int eigd_factor_create_in_fronts(eigd_symbolic* s, int max_rhs, int fronts, void* d_workspace,
+                                            int64_t workspace_bytes, eigd_factor** out) {
+  if (!fronts_mode_ok(fronts)) return 1;
+  int rc = fronts == 1 ? build_pool_plan(s) : build_symdev(s);
   if (rc) return rc;
   auto* f = new eigd_factor();
   f->sym = s;
   f->h = (SymDevHolder*)s->dev;
   f->max_rhs = std::max(1, max_rhs);
+  f->pooled = fronts == 1;
   int64_t sz[NARR], tot = 0;
-  factor_layout(s, f->h, f->max_rhs, sz);
+  factor_layout(s, f->h, f->max_rhs, f->pooled, sz);
   for (int i = 0; i < NARR; ++i) tot += sz[i];
   char* base = nullptr;
   if (d_workspace) {
@@ -874,7 +962,7 @@ extern "C" int eigd_factor_create_in(eigd_symbolic* s, int max_rhs, void* d_work
   f->base = base;
   f->bytes = tot;
   char* p = base;
-  f->fronts = (double*)p; p += sz[0];
+  f->fronts = f->pooled ? nullptr : (double*)p; p += sz[0];
   f->linv = (double*)p; p += sz[1];
   f->xinv = (double*)p; p += sz[2];
   f->xtmp = (double*)p; p += sz[3];
@@ -900,6 +988,11 @@ extern "C" int eigd_factor_create_in(eigd_symbolic* s, int max_rhs, void* d_work
   return 0;
 }
 
+extern "C" int eigd_factor_create_in(eigd_symbolic* s, int max_rhs, void* d_workspace, int64_t workspace_bytes,
+                                     eigd_factor** out) {
+  return eigd_factor_create_in_fronts(s, max_rhs, 0, d_workspace, workspace_bytes, out);
+}
+
 extern "C" int eigd_factor_create(eigd_symbolic* s, int max_rhs, eigd_factor** out) {
   return eigd_factor_create_in(s, max_rhs, nullptr, 0, out);
 }
@@ -912,48 +1005,40 @@ extern "C" void eigd_factor_destroy(eigd_factor* f) {
 
 extern "C" int64_t eigd_factor_bytes(const eigd_factor* f) { return f->bytes; }
 
-extern "C" int eigd_factor_numeric(eigd_factor* f, int64_t nnz, const double* d_vals, const int64_t* d_map) {
+// The launches of a factor plan.  d: the device symbolic data with front_off pointing at the fronts' layout
+// (front_off for resident fronts, pool_off for pooled ones); vals / seg / ent: the inputs of kind 8 (pooled only).
+static int run_factor_plan(eigd_factor* f, const std::vector<Launch>& plan, const int2* tasks, const SymDev& d,
+                           double* fronts, const double* vals, const int64_t* seg, const int2* ent) {
   eigd_symbolic* s = f->sym;
-  SymDevHolder* h = f->h;
-  int64_t nfront = s->front_off[s->nsuper];
-  EIGD_CUDA(cudaMemsetAsync(f->fronts, 0, (size_t)nfront * 8, g_eigd_stream));
-  EIGD_CUDA(cudaMemsetAsync(f->amax, 0, 8, g_eigd_stream));
-  EIGD_CUDA(cudaMemsetAsync(f->info, 0, f->pivoting ? 40 : 32, g_eigd_stream));
-  EIGD_CUDA(cudaMemsetAsync(f->xinv, 0, (size_t)std::max<int64_t>(h->xinv_total, 1) * 8, g_eigd_stream));
-  int g = (int)std::min<int64_t>((nnz + 255) / 256, 148 * 16);
-  if (g < 1) g = 1;
-  EIGD_LAUNCH(absmax_kernel, g, 256, 0, nnz, d_vals, f->amax);
-  EIGD_CHECK_LAUNCH();
-  EIGD_LAUNCH(scatter_values_kernel, g, 256, 0, nnz, d_vals, d_map, f->fronts);
-  EIGD_CHECK_LAUNCH();
   // developer profiling (EIGD_FACTOR_PROF=1): device time per launch kind, synchronising after every launch
   static int prof = -1;
   if (prof < 0) { const char* e = getenv("EIGD_FACTOR_PROF"); prof = e ? atoi(e) : 0; }
-  double kind_ms[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-  int kind_n[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+  double kind_ms[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+  int kind_n[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
   cudaEvent_t pe0 = nullptr, pe1 = nullptr;
   if (prof) { cudaEventCreate(&pe0); cudaEventCreate(&pe1); }
-  for (const Launch& L : h->factor_plan) {
-    const int2* t = h->tasks + L.off;
+  for (const Launch& L : plan) {
+    const int2* t = tasks + L.off;
     if (prof) cudaEventRecord(pe0, g_eigd_stream);
     switch (L.kind) {
-      case 0: EIGD_LAUNCH(extend_add_kernel, L.count, 256, 0, h->d, t, f->fronts); break;
+      case 0: EIGD_LAUNCH(extend_add_kernel, L.count, 256, 0, d, t, fronts); break;
       case 1:
-        if (f->pivoting) EIGD_LAUNCH(diag_factor_bk_kernel, L.count, 256, 0, h->d, t, L.kb, f->fronts, f->linv, f->dval, f->dinv, f->amax, f->piv_tol, f->info);
-        else EIGD_LAUNCH(diag_factor_kernel, L.count, 256, 0, h->d, t, L.kb, f->fronts, f->linv, f->dval, f->dinv, f->amax, f->piv_tol, f->info);
+        if (f->pivoting) EIGD_LAUNCH(diag_factor_bk_kernel, L.count, 256, 0, d, t, L.kb, fronts, f->linv, f->dval, f->dinv, f->amax, f->piv_tol, f->info);
+        else EIGD_LAUNCH(diag_factor_kernel, L.count, 256, 0, d, t, L.kb, fronts, f->linv, f->dval, f->dinv, f->amax, f->piv_tol, f->info);
         break;
       case 2:
-        if (f->pivoting) EIGD_LAUNCH(trsm_kernel<true>, L.count, TRSM_ROWS, 0, h->d, t, L.kb, f->fronts, f->linv, f->dinv);
-        else EIGD_LAUNCH(trsm_kernel<false>, L.count, TRSM_ROWS, 0, h->d, t, L.kb, f->fronts, f->linv, f->dinv);
+        if (f->pivoting) EIGD_LAUNCH(trsm_kernel<true>, L.count, TRSM_ROWS, 0, d, t, L.kb, fronts, f->linv, f->dinv);
+        else EIGD_LAUNCH(trsm_kernel<false>, L.count, TRSM_ROWS, 0, d, t, L.kb, fronts, f->linv, f->dinv);
         break;
-      case 3: EIGD_LAUNCH(trailing_update_kernel, L.count, 256, 0, h->d, t, L.kb, f->fronts, f->dval); break;
+      case 3: EIGD_LAUNCH(trailing_update_kernel, L.count, 256, 0, d, t, L.kb, fronts, f->dval); break;
       case 4:
-        if (f->pivoting) EIGD_LAUNCH(inverse_init_kernel<true>, L.count, 256, 0, h->d, t, f->linv, f->xinv);
-        else EIGD_LAUNCH(inverse_init_kernel<false>, L.count, 256, 0, h->d, t, f->linv, f->xinv);
+        if (f->pivoting) EIGD_LAUNCH(inverse_init_kernel<true>, L.count, 256, 0, d, t, f->linv, f->xinv);
+        else EIGD_LAUNCH(inverse_init_kernel<false>, L.count, 256, 0, d, t, f->linv, f->xinv);
         break;
-      case 5: EIGD_LAUNCH(inverse_ca_kernel, L.count, 256, 0, h->d, t, NB << L.kb, f->fronts, f->xinv, f->xtmp); break;
-      case 6: EIGD_LAUNCH(inverse_bt_kernel, L.count, 256, 0, h->d, t, NB << L.kb, f->xinv, f->xtmp); break;
-      case 7: EIGD_LAUNCH(panel_build_kernel, L.count, 256, 0, h->d, t, f->fronts, f->xinv, f->sfwd, f->sbwd); break;
+      case 5: EIGD_LAUNCH(inverse_ca_kernel, L.count, 256, 0, d, t, NB << L.kb, fronts, f->xinv, f->xtmp); break;
+      case 6: EIGD_LAUNCH(inverse_bt_kernel, L.count, 256, 0, d, t, NB << L.kb, f->xinv, f->xtmp); break;
+      case 7: EIGD_LAUNCH(panel_build_kernel, L.count, 256, 0, d, t, fronts, f->xinv, f->sfwd, f->sbwd); break;
+      case 8: EIGD_LAUNCH(front_assemble_kernel, L.count, 256, 0, d, t, vals, seg, ent, fronts); break;
       default: break;
     }
     EIGD_CHECK_LAUNCH();
@@ -962,19 +1047,65 @@ extern "C" int eigd_factor_numeric(eigd_factor* f, int64_t nnz, const double* d_
       cudaEventSynchronize(pe1);
       float ms = 0.f;
       cudaEventElapsedTime(&ms, pe0, pe1);
-      kind_ms[L.kind & 7] += ms;
-      kind_n[L.kind & 7]++;
+      kind_ms[L.kind] += ms;
+      kind_n[L.kind]++;
     }
   }
   if (prof) {
-    static const char* names[8] = {"extend_add", "diag_factor", "trsm", "trailing_update", "inverse_init", "inverse_ca", "inverse_bt", "panel_build"};
-    fprintf(stderr, "[factor prof] n=%d levels=%d:", s->n, s->nlevels);
-    for (int k = 0; k < 8; ++k) fprintf(stderr, " %s %.3f ms / %d;", names[k], kind_ms[k], kind_n[k]);
+    static const char* names[9] = {"extend_add", "diag_factor", "trsm", "trailing_update", "inverse_init", "inverse_ca",
+                                   "inverse_bt", "panel_build", "front_assemble"};
+    fprintf(stderr, "[factor prof] n=%d levels=%d%s:", s->n, s->nlevels, f->pooled ? " pooled" : "");
+    for (int k = 0; k < (f->pooled ? 9 : 8); ++k) fprintf(stderr, " %s %.3f ms / %d;", names[k], kind_ms[k], kind_n[k]);
     fprintf(stderr, "\n");
     cudaEventDestroy(pe0);
     cudaEventDestroy(pe1);
   }
   return 0;
+}
+
+// the per-call set-up both modes share: pivot statistics, |A|max for the pivot threshold, zeroed full inverses
+static int numeric_begin(eigd_factor* f, int64_t nnz, const double* d_vals, int* grid) {
+  EIGD_CUDA(cudaMemsetAsync(f->amax, 0, 8, g_eigd_stream));
+  EIGD_CUDA(cudaMemsetAsync(f->info, 0, f->pivoting ? 40 : 32, g_eigd_stream));
+  EIGD_CUDA(cudaMemsetAsync(f->xinv, 0, (size_t)std::max<int64_t>(f->h->xinv_total, 1) * 8, g_eigd_stream));
+  int g = (int)std::min<int64_t>((nnz + 255) / 256, 148 * 16);
+  if (g < 1) g = 1;
+  EIGD_LAUNCH(absmax_kernel, g, 256, 0, nnz, d_vals, f->amax);
+  EIGD_CHECK_LAUNCH();
+  *grid = g;
+  return 0;
+}
+
+extern "C" int eigd_factor_numeric(eigd_factor* f, int64_t nnz, const double* d_vals, const int64_t* d_map) {
+  if (f->pooled) { eigd_set_error("factor_numeric: this factor has pooled fronts; use eigd_factor_numeric_pool"); return 1; }
+  eigd_symbolic* s = f->sym;
+  SymDevHolder* h = f->h;
+  int64_t nfront = s->front_off[s->nsuper];
+  EIGD_CUDA(cudaMemsetAsync(f->fronts, 0, (size_t)nfront * 8, g_eigd_stream));
+  int g = 0, rc = numeric_begin(f, nnz, d_vals, &g);
+  if (rc) return rc;
+  EIGD_LAUNCH(scatter_values_kernel, g, 256, 0, nnz, d_vals, d_map, f->fronts);
+  EIGD_CHECK_LAUNCH();
+  return run_factor_plan(f, h->factor_plan, h->tasks, h->d, f->fronts, nullptr, nullptr, nullptr);
+}
+
+extern "C" int eigd_factor_numeric_pool(eigd_factor* f, int64_t nnz, const double* d_vals, const int64_t* d_seg,
+                                        const int* d_ent, void* d_pool, int64_t pool_bytes) {
+  if (!f->pooled) { eigd_set_error("factor_numeric_pool: this factor has resident fronts; use eigd_factor_numeric"); return 1; }
+  eigd_symbolic* s = f->sym;
+  SymDevHolder* h = f->h;
+  const int64_t need = s->pool_doubles * 8;
+  if (!d_pool || pool_bytes < need) {
+    eigd_set_error("factor_numeric_pool: front pool of %lld bytes, the fronts need %lld (eigd_symbolic_query(s, 10) doubles)",
+                   (long long)pool_bytes, (long long)need);
+    return 3;
+  }
+  if ((uintptr_t)d_pool % 256) { eigd_set_error("factor_numeric_pool: the front pool must be 256-byte aligned"); return 3; }
+  int g = 0, rc = numeric_begin(f, nnz, d_vals, &g);
+  if (rc) return rc;
+  SymDev d = h->d;
+  d.front_off = h->pool_off;
+  return run_factor_plan(f, h->pool_plan, h->pool_tasks, d, (double*)d_pool, d_vals, d_seg, (const int2*)d_ent);
 }
 
 // ---- FP64 tensor-pipe peak of this GPU, measured: every warp of every SM issues independent DMMA chains on register

@@ -11,6 +11,7 @@ constexpr int NB = 32;        // pivot block width
 constexpr int TRSM_ROWS = 128;
 constexpr int UPD_TILE = 64;
 constexpr int EA_TILE = 32;
+constexpr int POOL_CHUNK = 16384;   // doubles of a front zeroed and assembled by one CTA (pooled fronts)
 
 struct SymDev {
   int n, nsuper;
@@ -30,7 +31,8 @@ struct SymDev {
 };
 
 struct Launch {
-  int kind;      // 0 extend-add, 1 diag, 2 trsm, 3 update, 4 inverse-init, 5 inverse GEMM (C A^-1), 6 inverse GEMM (-B^-1 T), 7 panel build
+  int kind;      // 0 extend-add, 1 diag, 2 trsm, 3 update, 4 inverse-init, 5 inverse GEMM (C A^-1), 6 inverse GEMM (-B^-1 T),
+                 // 7 panel build, 8 zero + assemble fronts (pooled fronts)
   int kb;        // pivot block index (kinds 1-3) / doubling stage (kinds 5, 6)
   int64_t off;   // offset into the task array (int2 entries)
   int count;
@@ -59,13 +61,18 @@ struct SymDevHolder {
   int64_t xinv_total = 0;     // full nc x nc inverses of the unit-lower pivot blocks
   int64_t panel_total = 0;    // sum f * nc
   SolvePlanDev solve;
+  // pooled fronts (build_pool_plan, on first use)
+  int64_t* pool_off = nullptr;        // device copy of eigd_symbolic::pool_off
+  int2* pool_tasks = nullptr;
+  std::vector<Launch> pool_plan;
 };
 
 struct eigd_factor {
   eigd_symbolic* sym = nullptr;
   SymDevHolder* h = nullptr;
   int max_rhs = 1;
-  double* fronts = nullptr;   // f x f frontal matrices (factorisation workspace)
+  double* fronts = nullptr;   // f x f frontal matrices (factorisation workspace); NULL with pooled fronts
+  bool pooled = false;        // fronts borrowed per eigd_factor_numeric_pool call (pool_off layout) instead of resident
   double* linv = nullptr;     // inverses of the 32x32 unit-lower diagonal blocks (pivoted: of the dense blocks M, see
                               // diag_factor_bk_kernel)
   double* xinv = nullptr;     // full inverse of every L11 (nc x nc, column-major)
@@ -99,5 +106,6 @@ struct eigd_factor {
 };
 
 int build_symdev(eigd_symbolic* S);
+int build_pool_plan(eigd_symbolic* S);
 int build_solve_plan_dev(eigd_symbolic* S, SymDevHolder* h);
 void free_solve_plan_dev(SymDevHolder* h);

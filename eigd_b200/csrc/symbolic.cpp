@@ -14,6 +14,8 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
+#include <map>
+#include <set>
 #include <numeric>
 #include <string>
 
@@ -471,6 +473,57 @@ static std::vector<int> postorder(int n, const std::vector<int>& parent) {
 
 }  // namespace
 
+// Offsets of the fronts in the pooled front workspace.  Front k is live from its own level (assembly, factorisation,
+// inverse and solve panels) through its parent's level (extend-add of its contribution block); a root only at its own
+// level.  Fronts are placed level by level, best fit (smallest free block that holds the front, lowest offset among
+// equals) after the fronts whose last level has passed are released, so no two fronts live at the same level share
+// memory; in particular a child and its parent never do.  Sizes are rounded up to 256 bytes.
+static void pool_layout(eigd_symbolic* S) {
+  const int ns = S->nsuper;
+  S->pool_off.assign(ns, 0);
+  std::vector<std::vector<int>> dies(S->nlevels + 1);   // fronts released before level l + 1
+  for (int k = 0; k < ns; ++k) {
+    int p = S->sn_parent[k];
+    dies[p >= 0 ? S->sn_level[p] : S->sn_level[k]].push_back(k);
+  }
+  std::map<int64_t, int64_t> free_at;                    // offset -> size of every free block below the top
+  std::set<std::pair<int64_t, int64_t>> by_size;         // (size, offset) of the same blocks
+  int64_t top = 0, peak = 0;
+  auto size_of = [&](int k) { int64_t f = sn_fsize(S, k); return (f * f + 31) / 32 * 32; };
+  auto release = [&](int64_t off, int64_t sz) {
+    auto nx = free_at.lower_bound(off);
+    if (nx != free_at.end() && nx->first == off + sz) { sz += nx->second; by_size.erase({nx->second, nx->first}); nx = free_at.erase(nx); }
+    if (nx != free_at.begin()) {
+      auto pv = std::prev(nx);
+      if (pv->first + pv->second == off) { off = pv->first; sz += pv->second; by_size.erase({pv->second, pv->first}); free_at.erase(pv); }
+    }
+    if (off + sz == top) { top = off; return; }          // the block reaches the top: the used region shrinks
+    free_at[off] = sz;
+    by_size.insert({sz, off});
+  };
+  for (int l = 0; l < S->nlevels; ++l) {
+    if (l > 0)
+      for (int k : dies[l - 1]) release(S->pool_off[k], size_of(k));
+    for (int q = S->level_ptr[l]; q < S->level_ptr[l + 1]; ++q) {
+      const int k = S->level_sn[q];
+      const int64_t sz = size_of(k);
+      auto it = by_size.lower_bound({sz, INT64_MIN});
+      if (it == by_size.end()) {
+        S->pool_off[k] = top;
+        top += sz;
+        peak = std::max(peak, top);
+        continue;
+      }
+      const int64_t off = it->second, bsz = it->first;
+      by_size.erase(it);
+      free_at.erase(off);
+      S->pool_off[k] = off;
+      if (bsz > sz) { free_at[off + sz] = bsz - sz; by_size.insert({bsz - sz, off + sz}); }
+    }
+  }
+  S->pool_doubles = peak;
+}
+
 extern "C" int eigd_symbolic_create(int n, const int* indptr, const int* indices, const double* coords,
                                     int dim, int dof_per_node, const int* opts, eigd_symbolic** out) {
   if (n <= 0 || !indptr || !indices || !out) { eigd_set_error("symbolic_create: bad arguments"); return 1; }
@@ -706,6 +759,7 @@ extern "C" int eigd_symbolic_create(int n, const int* indptr, const int* indices
     std::vector<int> pos(S->level_ptr.begin(), S->level_ptr.end() - 1);
     for (int k = 0; k < ns; ++k) S->level_sn[pos[S->sn_level[k]]++] = k;
   }
+  pool_layout(S);
   *out = S;
   return 0;
 }
@@ -728,6 +782,7 @@ extern "C" int64_t eigd_symbolic_query(const eigd_symbolic* s, int what) {
     case 7: return s->maxcols;
     case 8: return s->flops;
     case 9: return s->exact_nnzL;
+    case 10: return s->pool_doubles;
     default: return -1;
   }
 }
@@ -753,6 +808,7 @@ extern "C" int64_t eigd_symbolic_get(const eigd_symbolic* s, int which, int64_t*
     case 9: return copy_out(s->colcount, out, cap);
     case 10: return copy_out(s->level_ptr, out, cap);
     case 11: return copy_out(s->level_sn, out, cap);
+    case 12: return copy_out(s->pool_off, out, cap);
     default: return -1;
   }
 }

@@ -20,6 +20,8 @@ struct eigd_symbolic {
   std::vector<int> sn_parent;       // supernodal elimination tree
   std::vector<int> sn_level;        // height above the leaves
   std::vector<int64_t> front_off;   // nsuper+1, offsets (doubles) of the f x f fronts
+  std::vector<int64_t> pool_off;    // nsuper, offsets (doubles) of the fronts in the pooled front workspace
+  int64_t pool_doubles = 0;         // size of that workspace
   std::vector<int64_t> w_off;       // nsuper+1, prefix sum of front sizes
   std::vector<int> child_ptr, child_idx;  // children of each supernode (ascending)
   int nlevels = 0;

@@ -467,6 +467,7 @@ _SYM_NAMES = ["perm", "parent", "sn_first", "sn_rowptr", "sn_rows", "sn_parent",
               "front_off", "rel", "colcount", "level_ptr", "level_sn"]
 _QUERY = {"n": 0, "nsuper": 1, "nlevels": 2, "nnzL": 3, "front_doubles": 4, "sum_front": 5,
           "max_front": 6, "max_cols": 7, "flops": 8, "exact_nnzL": 9}
+_QUERY_MORE = {"pool_doubles": 10}      # answered by ``query``, not listed by ``stats``
 
 
 class Symbolic:
@@ -503,7 +504,7 @@ class Symbolic:
             pass
 
     def query(self, name):
-        return int(_lib.load().eigd_symbolic_query(self.handle, _QUERY[name]))
+        return int(_lib.load().eigd_symbolic_query(self.handle, _QUERY[name] if name in _QUERY else _QUERY_MORE[name]))
 
     def stats(self):
         return {k: self.query(k) for k in _QUERY}
@@ -518,6 +519,34 @@ class Symbolic:
 
     def arrays(self):
         return {nm: self.get(nm) for nm in _SYM_NAMES}
+
+    def pool_offsets(self):
+        """Offset (doubles) of every front in the pooled front workspace of ``query("pool_doubles")`` doubles."""
+        lib = _lib.load()
+        cnt = lib.eigd_symbolic_get(self.handle, 12, None, 0)
+        out = np.zeros(cnt, dtype=np.int64)
+        lib.eigd_symbolic_get(self.handle, 12, out.ctypes.data_as(ctypes.c_void_p), cnt)
+        return out
+
+    def pool_scatter(self, d_map):
+        """The entry lists of the pooled factorisation (eigd_factor_numeric_pool) for the assembly map ``d_map``: (seg,
+        ent), ent an (m, 2) int32 device tensor of (CSR index, slot inside its front) grouped by front and sorted by slot,
+        seg the int64 start of every front's group.  Built once per map and kept with it."""
+        cached = getattr(self, "_pool_scatter", None)
+        if cached is not None and cached[0] is d_map:
+            return cached[1], cached[2]
+        d = dev()
+        slots, idx = torch.sort(d_map)
+        keep = slots >= 0                                  # -1: the strict upper triangle of the CSR
+        slots, idx = slots[keep], idx[keep]
+        if not hasattr(self, "_front_off_d"):
+            self._front_off_d = torch.as_tensor(self.get("front_off"), device=d)
+        fo = self._front_off_d
+        seg = torch.searchsorted(slots, fo)
+        front = torch.searchsorted(fo, slots, right=True) - 1
+        ent = torch.stack([idx.to(torch.int32), (slots - fo[front]).to(torch.int32)], dim=1).contiguous()
+        self._pool_scatter = (d_map, seg, ent)
+        return seg, ent
 
     def assembly_map_host(self, indptr=None, indices=None):
         ip = self._indptr if indptr is None else np.ascontiguousarray(indptr, dtype=np.int32)
@@ -588,6 +617,13 @@ class PatternCache:
 
 
 PIVOTING_MODES = ("static", "bunch-kaufman")
+FRONTS_MODES = ("resident", "pooled")
+
+
+def check_fronts(fronts, who="fronts"):
+    if fronts not in FRONTS_MODES:
+        raise ValueError("%s must be one of %s, not %r" % (who, FRONTS_MODES, fronts))
+    return fronts
 
 
 class Factor:
@@ -595,24 +631,33 @@ class Factor:
 
     pivoting: "static" (no pivot search; a pivot below 1e-11 max|A| is perturbed to +-that threshold) or
     "bunch-kaufman" (restricted Bunch-Kaufman 1x1 / 2x2 pivoting inside every 32-column pivot block, for indefinite
-    matrices with tiny or zero diagonal entries; pivots that are still tiny are perturbed and counted as well)."""
+    matrices with tiny or zero diagonal entries; pivots that are still tiny are perturbed and counted as well).
 
-    def __init__(self, symbolic, max_rhs=32, pivoting="static"):
+    fronts: "resident" (one dense front per supernode kept in the factor's workspace for its whole life) or "pooled"
+    (the workspace holds no fronts; ``numeric`` borrows a pool of ``symbolic.query("pool_doubles")`` doubles from
+    torch's caching allocator for the duration of the call, laid out by front lifetimes, so it is many times smaller
+    and factors of one pattern take turns on it).  Both give the same factor bit for bit; "pooled" launches the
+    inverse and panel kernels once per tree level instead of once, which costs time on small models."""
+
+    def __init__(self, symbolic, max_rhs=32, pivoting="static", fronts="resident"):
         if pivoting not in PIVOTING_MODES:
             raise ValueError("pivoting must be one of %s, not %r" % (PIVOTING_MODES, pivoting))
+        check_fronts(fronts)
         dev()
         self.sym = symbolic
         self.n = symbolic.n
         h = ctypes.c_void_p()
         lib = _lib.load()
-        nbytes = int(lib.eigd_factor_workspace_bytes(symbolic.handle, int(max_rhs)))
+        mode = FRONTS_MODES.index(fronts)
+        nbytes = int(lib.eigd_factor_workspace_bytes_fronts(symbolic.handle, int(max_rhs), mode))
         if nbytes < 0:
             check(1, "factor_workspace_bytes")
         # torch owns the memory: the caching allocator recycles it when this factor is dropped
         self._workspace = torch.empty(nbytes, dtype=torch.uint8, device=dev())
-        check(lib.eigd_factor_create_in(symbolic.handle, int(max_rhs), _ptr(self._workspace), nbytes, ctypes.byref(h)),
-              "factor_create_in")
+        check(lib.eigd_factor_create_in_fronts(symbolic.handle, int(max_rhs), mode, _ptr(self._workspace), nbytes,
+                                               ctypes.byref(h)), "factor_create_in")
         self.handle = h
+        self.fronts = fronts
         self.max_rhs = int(max_rhs)
         self.pivoting = pivoting
         self.refine, self._refine_mat, self._refine_work, self._refine_cols = 0, None, None, 0
@@ -630,9 +675,20 @@ class Factor:
     def numeric(self, d_vals, d_map):
         tok = Timeline.begin("factor")
         l0 = launch_count()
-        check(_lib.load().eigd_factor_numeric(self.handle, d_vals.numel(), _ptr(_chk(d_vals)), _ptr(d_map)), "factor_numeric")
+        if self.fronts == "resident":
+            check(_lib.load().eigd_factor_numeric(self.handle, d_vals.numel(), _ptr(_chk(d_vals)), _ptr(d_map)), "factor_numeric")
+        else:
+            seg, ent = self.sym.pool_scatter(d_map)
+            pool = torch.empty(self.pool_bytes(), dtype=torch.uint8, device=dev())
+            check(_lib.load().eigd_factor_numeric_pool(self.handle, d_vals.numel(), _ptr(_chk(d_vals)), _ptr(seg), _ptr(ent),
+                                                       _ptr(pool), pool.numel()), "factor_numeric_pool")
+            del pool            # back to the caching allocator, stream-ordered after the kernels just queued
         Timeline.end(tok, 0, launch_count() - l0)
         return self
+
+    def pool_bytes(self):
+        """Bytes of the front pool a pooled ``numeric`` borrows (0 for resident fronts)."""
+        return 8 * self.sym.query("pool_doubles") if self.fronts == "pooled" else 0
 
     def solve_bytes(self, k):
         """Algorithmic bytes of one forward+backward sweep with k right-hand sides (SURVEY.md 8d):

@@ -107,13 +107,17 @@ class SpLuOperator:
     1e-11 max|A| is perturbed to +-that threshold and the solves are refined) or ``"bunch-kaufman"`` (restricted
     Bunch-Kaufman 1x1 / 2x2 pivoting inside every 32-column pivot block: for indefinite shifts with zero or tiny
     diagonal entries, e.g. saddle-point operators or a shift close to an eigenvalue).  ``info`` reports the pivot
-    statistics either way; the probe / refinement policy is the same for both.
+    statistics either way; the probe / refinement policy is the same for both.  ``fronts`` chooses the memory of the
+    factorisation's dense fronts (``device.Factor``): ``"resident"`` (default) keeps them in the factor,
+    ``"pooled"`` borrows a much smaller lifetime-ordered pool for each factorisation only; the factor is the same.
     """
 
     @_public
-    def __init__(self, mat, coords=None, dof_per_node=1, symbolic=None, refine=None, max_rhs=32, pivoting="static"):
+    def __init__(self, mat, coords=None, dof_per_node=1, symbolic=None, refine=None, max_rhs=32, pivoting="static",
+                 fronts="resident"):
         if pivoting not in D.PIVOTING_MODES:
             raise ValueError("SpLuOperator: pivoting must be one of %s, not %r" % (D.PIVOTING_MODES, pivoting))
+        D.check_fronts(fronts, "SpLuOperator: fronts")
         self.tangent = None
         if isinstance(mat, D.CsrDevice):
             csr = mat
@@ -155,7 +159,7 @@ class SpLuOperator:
         elif isinstance(symbolic, D.Symbolic):
             symbolic = (symbolic, symbolic.assembly_map_device(csr.indptr, csr.indices))
         self.symbolic, self._amap = symbolic
-        self.lu = D.Factor(self.symbolic, max_rhs=max_rhs, pivoting=pivoting).numeric(csr.data, self._amap)
+        self.lu = D.Factor(self.symbolic, max_rhs=max_rhs, pivoting=pivoting, fronts=fronts).numeric(csr.data, self._amap)
         # The factorisation is now queued on the device.  Its pivot statistics (inertia, perturbed pivots) and the choice
         # of the refinement depth need a read-back, i.e. a wait for the whole factorisation: that is deferred to the first
         # use (``info`` / ``refine`` / the first solve), so that the caller's next host-side steps -- typically the

@@ -215,8 +215,9 @@ class ShellModalAnalysis(_EigenAnalysis):
     modal-compliance objective with f[1::6] = 1 (:267-293), per-mode "vector" total derivative (:357-370)."""
 
     def __init__(self, prob, N=10, m=None, omega0=10.0, solver_type="IRAM", tol=1e-14, rtol=1e-10, eig_atol=1e-5,
-                 adjoint_method="sibk", adjoint_options=None, deriv_type="vector", seed=0):
-        super().__init__(prob, N, m, solver_type, tol, rtol, eig_atol, adjoint_method, adjoint_options, deriv_type, seed)
+                 adjoint_method="sibk", adjoint_options=None, deriv_type="vector", seed=0, fronts="resident"):
+        super().__init__(prob, N, m, solver_type, tol, rtol, eig_atol, adjoint_method, adjoint_options, deriv_type, seed,
+                         fronts)
         self.omega0 = omega0
         self.x = np.ones(prob.ncomp)                       # crm.py: t = 0.01, scale 100
         f = np.zeros(prob.ndof_full)
@@ -242,7 +243,7 @@ class ShellModalAnalysis(_EigenAnalysis):
         vals = D.axpby(1.0, self.Kr.data, -float(sigma), self.Mr.data)
         if self._symbolic_once(self.Kr) is not None:
             t1 = _now()                                    # the eigensolve time excludes the analysis
-        self.factor = SpLuOperator(self.Kr.with_values(vals), symbolic=self.symbolic)
+        self.factor = SpLuOperator(self.Kr.with_values(vals), symbolic=self.symbolic, fronts=self.fronts)
         self._new_eig_solver(self.N)
         self.lam = np.asarray(self._eigensolve(self.Kr, self.Mr, sigma, t1))
         self.Q = self.eig_solver._Phi_d

@@ -36,8 +36,10 @@ class _EigenAnalysis:
     ``finalize_adjoint`` here, with the driver's eigenvector seeds (``_eigenvector_seeds``) and total derivative
     (``_total_derivative``)."""
 
-    def __init__(self, prob, N, m, solver_type, tol, rtol, eig_atol, adjoint_method, adjoint_options, deriv_type, seed):
+    def __init__(self, prob, N, m, solver_type, tol, rtol, eig_atol, adjoint_method, adjoint_options, deriv_type, seed,
+                 fronts="resident"):
         self.prob = prob
+        self.fronts = D.check_fronts(fronts)      # front memory of every factor the driver builds (SpLuOperator)
         self.N, self.m = N, m
         self.solver_type, self.tol, self.rtol, self.eig_atol = solver_type, tol, rtol, eig_atol
         if adjoint_method == "shift-invert":          # the examples' historical alias (thermal.py:37)
@@ -116,11 +118,12 @@ class _Q4Analysis(_EigenAnalysis):
     nrigid = 0            # leading modes computed but dropped (rigid-body modes of the free structure)
 
     def __init__(self, fltr, conn, X, sigma, N=10, m=None, Ntarget=None, solver_type="IRAM", tol=0.0, rtol=1e-10,
-                 eig_atol=1e-5, adjoint_method="sibk", adjoint_options=None, deriv_type="tensor", seed=0, **material):
+                 eig_atol=1e-5, adjoint_method="sibk", adjoint_options=None, deriv_type="tensor", seed=0, fronts="resident",
+                 **material):
         self.fltr = fltr
         self.conn, self.X = np.asarray(conn), np.asarray(X)
         super().__init__(self._make_problem(**material), N, m, solver_type, tol, rtol, eig_atol, adjoint_method,
-                         adjoint_options, deriv_type, seed)
+                         adjoint_options, deriv_type, seed, fronts)
         self.nelems, self.nnodes, self.nvars = self.prob.nelems, self.prob.nnodes, self.prob.ndof
         self.sigma, self.Ntarget = sigma, Ntarget
         self.x = 0.95 * np.ones(self.fltr.num_design_vars)      # thermal.py:71, natural_frequency.py:75
@@ -148,7 +151,7 @@ class _Q4Analysis(_EigenAnalysis):
         shifted = K.with_values(D.axpby(1.0, K.data, -float(self.sigma), M.data))    # K - sigma M on the shared pattern
         if self._symbolic_once(K) is not None:
             t1 = _now()                                                   # the eigensolve time excludes the analysis
-        self.factor = SpLuOperator(shifted, symbolic=self.symbolic)
+        self.factor = SpLuOperator(shifted, symbolic=self.symbolic, fronts=self.fronts)
         self.K, self.M = K, M
         self._new_eig_solver(self.N + self.nrigid, iram=dict(tol=self.tol), lanczos=dict(Ntarget=self.Ntarget))
         self.prob.sharding = self.sharding
@@ -187,7 +190,7 @@ class _Q4Analysis(_EigenAnalysis):
         Kt, Mt = self.prob.assemble_tangent(rho_t)
         self._symbolic_once(K)
         shifted = K.with_values(D.axpby(1.0, K.data, -float(self.sigma), M.data))
-        self.factor = SpLuOperator(shifted, symbolic=self.symbolic)
+        self.factor = SpLuOperator(shifted, symbolic=self.symbolic, fronts=self.fronts)
         self.factor.tangent = K.with_values(D.axpby(1.0, Kt.data, -float(self.sigma), Mt.data))
         self.factor.dtype = np.dtype(np.complex128)
         self.K, self.M = K, M
@@ -480,8 +483,9 @@ def make_natural_frequency_model(nx=128, ny=64, Lx=1.0, Ly=1.0, rfact=4.0, N=10,
 
 def make_natural_frequency_3d_model(nx, ny, nz, Lx=2.0, Ly=1.0, Lz=1.0, rfact=4.0, **kwargs):
     """Free nx x ny x nz hexahedral box (``fe.hex_mesh``), one design variable per node, conic filter of radius
-    rfact * Ly / ny on the 3-D nodes.  The largest box one 180 GB B200 factors is about 80 x 40 x 40 (408k DOF): the
-    factor keeps every front resident (DESIGN.md section 8b)."""
+    rfact * Ly / ny on the 3-D nodes.  With the default resident fronts the largest box one 180 GB B200 factors is
+    about 80 x 40 x 40 (408k DOF); ``fronts="pooled"`` (forwarded through ``kwargs``) borrows a lifetime-ordered front
+    pool per factorisation instead, which takes 96 x 48 x 48 (699k DOF) (DESIGN.md section 8b)."""
     conn, X = fe.hex_mesh(nx, ny, nz, Lx, Ly, Lz)
     fltr = fe.NodeFilter(conn, X, r0=rfact * (Ly / ny))
     return NaturalFrequency3DAnalysis(fltr, conn, X, **kwargs)
@@ -501,13 +505,14 @@ class BucklingTopologyAnalysis(_EigenAnalysis):
     def __init__(self, fltr, conn, X, bcs, forces={}, E=1.0, nu=0.3, ptype_K="simp", ptype_M="simp", ptype_G="simp",
                  rho0_K=1e-6, rho0_M=1e-9, rho0_G=1e-9, p=3.0, q=5.0, density=1.0, sigma=3.0, N=10, m=None,
                  solver_type="IRAM", tol=0.0, rtol=1e-10, eig_atol=1e-5, adjoint_method="shift-invert",
-                 adjoint_options=None, cost=1, deriv_type="tensor", seed=0, pivoting="static"):
+                 adjoint_options=None, cost=1, deriv_type="tensor", seed=0, pivoting="static", fronts="resident"):
         self.fltr = fltr
         self.pivoting = pivoting          # of the shifted factor K_r + sigma G_r (SpLuOperator); K_r alone is SPD
         self.conn, self.X = np.asarray(conn), np.asarray(X)
         prob = self._make_problem(bcs, forces, E=E, nu=nu, density=density, p=float(p), q=float(q), rho0_K=rho0_K,
                                   rho0_G=rho0_G, ptype_K=ptype_K.lower(), ptype_G=ptype_G.lower())
-        super().__init__(prob, N, m, solver_type, tol, rtol, eig_atol, adjoint_method, adjoint_options, deriv_type, seed)
+        super().__init__(prob, N, m, solver_type, tol, rtol, eig_atol, adjoint_method, adjoint_options, deriv_type, seed,
+                         fronts)
         self.nelems, self.nnodes, self.nvars = self.prob.nelems, self.prob.nnodes, self.prob.ndof
         self.reduced, self.f = self.prob.reduced, self.prob.f
         self.E, self.nu, self.p, self.q, self.density = E, nu, p, q, density
@@ -525,14 +530,14 @@ class BucklingTopologyAnalysis(_EigenAnalysis):
         t0 = _now()
         Kr = self.prob.assemble_K()
         t0 += self._symbolic_once(Kr) or 0.0                              # the assembly time excludes the analysis
-        self.Kfact = SpLuOperator(Kr, symbolic=self.symbolic, max_rhs=1)  # fundamental path K_r u_r = f_r
+        self.Kfact = SpLuOperator(Kr, symbolic=self.symbolic, max_rhs=1, fronts=self.fronts)  # fundamental path K_r u_r = f_r
         ur = self.Kfact.solve_dev(self.prob.fr_d)
         self.u_d = self.prob.set_displacement(ur)
         Gr = self.prob.assemble_G()
         t1 = _now()
         self.profile["matrix assembly time"] = t1 - t0
         vals = D.axpby(1.0, Kr.data, float(self.sigma), Gr.data)          # K_r + sigma G_r on the shared pattern
-        self.factor = SpLuOperator(Kr.with_values(vals), symbolic=self.symbolic, pivoting=self.pivoting)
+        self.factor = SpLuOperator(Kr.with_values(vals), symbolic=self.symbolic, pivoting=self.pivoting, fronts=self.fronts)
         self.Kr, self.Gr = Kr, Gr
         self._new_eig_solver(self.N, iram=dict(mode="buckling"), lanczos=dict(mode="buckling"))
         if self.solver_type == "IRAM":
@@ -697,9 +702,11 @@ class BucklingTopology3DAnalysis(BucklingTopologyAnalysis):
     """The linearised buckling problem of ``BucklingTopologyAnalysis`` on a 3-D solid of trilinear hexahedra
     (``fe.BucklingH8Problem``), with the same forward and reverse pipeline and objectives.
 
-    Each design keeps two factors on one symbolic analysis, K_r (for the fundamental-path adjoint) and K_r + sigma G_r,
-    each with its own front workspace.  The previous design's factors, and the eigensolver that references them, are
-    dropped before the next design is factored, so the peak is two front workspaces rather than three."""
+    Each design keeps two factors on one symbolic analysis, K_r (for the fundamental-path adjoint) and K_r + sigma G_r.
+    With resident fronts (the default) each keeps its own front workspace; the previous design's factors, and the
+    eigensolver that references them, are dropped before the next design is factored, so the peak is two front
+    workspaces rather than three.  With ``fronts="pooled"`` neither keeps fronts: both factorisations borrow one
+    lifetime-ordered pool in turn."""
 
     def _make_problem(self, bcs, forces, **material):
         return fe.BucklingH8Problem(self.conn, self.X, bcs, forces, **material)
@@ -732,7 +739,8 @@ def make_buckling_3d_model(nx=32, ny=24, nz=128, Lx=1.0, Ly=0.75, Lz=4.0, rfact=
     from about 2.5 up (32 x 24 x 128, x ~ U(0.3, 0.7): 8 load factors below 3).  The default sigma = 3 lies inside
     the spectrum, so K_r + sigma G_r is indefinite.  As in the 2-D driver the eigensolver returns the N load factors
     nearest sigma in the buckling shift-invert transform, which ranks a lambda < sigma below every lambda > sigma
-    when lambda < sigma / 2.  At 32 x 24 x 128 each factor's fronts take 44 GB (DESIGN.md section 8b)."""
+    when lambda < sigma / 2.  At 32 x 24 x 128 each factor's resident fronts take 44 GB (DESIGN.md section 8b);
+    ``fronts="pooled"`` (forwarded through ``kwargs``) replaces them by one shared pool."""
     conn, X, bcs, forces = domain_compressed_column_3d(nx, ny, nz, Lx, Ly, Lz)
     fltr = fe.NodeFilter(conn, X, r0=rfact * (Lx / nx))
     return BucklingTopology3DAnalysis(fltr, conn, X, bcs=bcs, forces=forces, N=N, **kwargs)

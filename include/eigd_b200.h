@@ -87,12 +87,15 @@ int eigd_symbolic_create(int n, const int* indptr, const int* indices,
 void eigd_symbolic_destroy(eigd_symbolic* s);
 /* scalar queries: what = 0 n, 1 nsuper, 2 nlevels, 3 nnz(L) (strict lower, dense fronts),
  * 4 front storage doubles, 5 sum of front sizes, 6 max front size, 7 max supernode cols,
- * 8 flops of the factorisation, 9 nnz of exact (unrelaxed) L */
+ * 8 flops of the factorisation, 9 nnz of exact (unrelaxed) L, 10 doubles of the pooled front workspace
+ * (eigd_factor_numeric_pool) */
 int64_t eigd_symbolic_query(const eigd_symbolic* s, int what);
 /* array getters (host copies): which = 0 perm[n] (new->old), 1 etree parent[n], 2 sn_first[nsuper+1],
  * 3 sn_rowptr[nsuper+1], 4 sn_rows[...], 5 sn_parent[nsuper], 6 sn_level[nsuper],
  * 7 front_off[nsuper+1], 8 rel[...] (aligned with sn_rows), 9 colcount[n], 10 level_ptr[nlevels+1],
- * 11 level_sn[nsuper].  Returns the element count; copies min(count, cap) int64 values. */
+ * 11 level_sn[nsuper], 12 pool_off[nsuper] (offset of every front in the pooled front workspace: front k is live
+ * from level sn_level[k] through sn_level[sn_parent[k]], and fronts live at one level never overlap).
+ * Returns the element count; copies min(count, cap) int64 values. */
 int64_t eigd_symbolic_get(const eigd_symbolic* s, int which, int64_t* out, int64_t cap);
 /* assembly map nz -> slot in front storage (or -1), computed by host code */
 int eigd_symbolic_assembly_map_host(const eigd_symbolic* s, int n, const int* indptr, const int* indices, int64_t* out_map);
@@ -116,13 +119,27 @@ int eigd_factor_create(eigd_symbolic* s, int max_rhs, eigd_factor** out);
  * bytes (a torch tensor, so that the caching allocator recycles it: no cudaMalloc / cudaFree per design) */
 int64_t eigd_factor_workspace_bytes(eigd_symbolic* s, int max_rhs);
 int eigd_factor_create_in(eigd_symbolic* s, int max_rhs, void* d_workspace, int64_t workspace_bytes, eigd_factor** out);
+/* the same two with a choice of front memory: fronts = 0 resident (as above: one f x f front per supernode in the
+ * workspace, kept for the factor's life), 1 pooled (no fronts in the workspace: every eigd_factor_numeric_pool call
+ * borrows a pool of eigd_symbolic_query(s, 10) doubles from the caller, so factors can take turns on one pool).  The
+ * factor is the same bit for bit in both modes.  Any other mode fails. */
+int64_t eigd_factor_workspace_bytes_fronts(eigd_symbolic* s, int max_rhs, int fronts);
+int eigd_factor_create_in_fronts(eigd_symbolic* s, int max_rhs, int fronts, void* d_workspace, int64_t workspace_bytes,
+                                 eigd_factor** out);
 void eigd_factor_destroy(eigd_factor* f);
 /* measured FP64 tensor-pipe (DMMA, mma.sync.m8n8k4.f64) peak of the current device in TFLOP/s: register-resident
  * micro-benchmark on all SMs, best of `reps` launches of `iters` x 8 MMAs per warp (denominator of bench.py's
  * roofline_fp64_tensor) */
 int eigd_dmma_peak(int iters, int reps, double* tflops_out);
-/* numeric factorisation from device CSR values + device assembly map */
+/* numeric factorisation from device CSR values + device assembly map (resident fronts only) */
 int eigd_factor_numeric(eigd_factor* f, int64_t nnz, const double* d_vals, const int64_t* d_map);
+/* the same for a factor with pooled fronts.  d_ent: int32 pairs (CSR index p, slot of entry p inside its front,
+ * i.e. assembly map[p] - front_off[k]) of every mapped entry, grouped by front and sorted by slot inside a front;
+ * d_seg[nsuper + 1] (int64): the pairs of front k are d_ent[2 d_seg[k] .. 2 d_seg[k + 1]).  d_pool: a 256-byte
+ * aligned device buffer of pool_bytes >= 8 * eigd_symbolic_query(s, 10) bytes, used only until the kernels queued by
+ * this call have run (returns 3 when it is smaller). */
+int eigd_factor_numeric_pool(eigd_factor* f, int64_t nnz, const double* d_vals, const int64_t* d_seg, const int* d_ent,
+                             void* d_pool, int64_t pool_bytes);
 /* info[0] = #negative pivots (inertia), info[1] = #perturbed pivots, info[2] = #non-finite */
 int eigd_factor_info(eigd_factor* f, int64_t* info3);
 /* pivoting of the following eigd_factor_numeric calls: 0 = static (default; tiny pivots perturbed to +-1e-11 max|A|),

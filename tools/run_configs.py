@@ -6,6 +6,9 @@
     python tools/run_configs.py h8 [--nx 64 --ny 32 --nz 32 --modes 10 --fd]   free 3-D solid of hexahedra (3 dof/node)
     python tools/run_configs.py h8buck [--nx 32 --ny 24 --nz 128 --modes 10 --fd]   buckling of a clamped 3-D column
 
+h8 and h8buck take --fronts resident|pooled (the front memory of the factors) and report, for either mode, the pool
+size, the persistent bytes of the factors, torch's peak allocated device memory and the factorisation time.
+
 Each prints one JSON line: stage times (CUDA-synchronised wall clock of the driver's own timers, as the
 reference examples report them), solve counts, factor statistics, and size-independent acceptance checks
 (eigen-residuals, B-orthonormality, adjoint residual of the converged psi) -- the reference cannot be run at
@@ -230,14 +233,16 @@ def gpu_card():
 def run_h8(args):
     """Free nx x ny x nz box of hexahedra (NaturalFrequency3DAnalysis): N flexible modes + 6 rigid-body modes about
     sigma = -10, IRAM + sibk with the Lanczos guess, tensor derivative, f = sum_i (phi_i . w_i)^2 as the seed."""
+    import torch
     from eigd_b200 import device as D, topo as T
     D.init()
     out = {"config": "H8 free solid nx=%d ny=%d nz=%d" % (args.nx, args.ny, args.nz), "N": args.modes, "gpu": gpu_card()}
     t0 = now()
     model = T.make_natural_frequency_3d_model(args.nx, args.ny, args.nz, N=args.modes, m=60, sigma=-10.0, solver_type="IRAM",
                                               adjoint_method="sibk", adjoint_options={"lanczos_guess": True}, rtol=1e-10,
-                                              deriv_type="tensor")
-    out.update(n=int(model.nvars), nnz=int(model.prob.nnz), host_setup_s=now() - t0)
+                                              deriv_type="tensor", fronts=args.fronts)
+    out.update(n=int(model.nvars), nnz=int(model.prob.nnz), fronts=args.fronts, host_setup_s=now() - t0)
+    torch.cuda.reset_peak_memory_stats()
     w_d = D.to_device(np.random.default_rng(99).normal(size=(model.nvars, args.modes)))
     x0 = np.random.default_rng(0).uniform(0.3, 1.0, model.fltr.num_design_vars)
     reps = []
@@ -258,7 +263,9 @@ def run_h8(args):
                      "adjoint_solves": p["adjoint preconditioner count"], "launches": D.launch_count() - l0,
                      "symbolic_s": p.get("symbolic analysis time")})
     out["reps"] = reps
+    out["peak_device_bytes"] = int(torch.cuda.max_memory_allocated())
     out["factorisation_s"] = _time_factorisation(model)
+    out["memory"] = _factor_memory(model, [model.factor])
     out["lam_first"] = [float(v) for v in model.lam[:3]]
     out["rigid_lam"] = [float(v) for v in model.lam0[:6]]
     out["factor_info"] = model.factor.info
@@ -302,8 +309,10 @@ def run_h8buck(args):
     out = {"config": "H8 buckling column nx=%d ny=%d nz=%d" % (args.nx, args.ny, args.nz), "N": args.modes, "gpu": gpu_card()}
     t0 = now()
     model = T.make_buckling_3d_model(args.nx, args.ny, args.nz, N=args.modes, m=60, solver_type="IRAM", adjoint_method="sibk",
-                                     adjoint_options={"lanczos_guess": True}, rtol=1e-10, deriv_type="tensor")
-    out.update(n=int(model.prob.nred), nnz=int(model.prob.nnz), sigma=float(model.sigma), host_setup_s=now() - t0)
+                                     adjoint_options={"lanczos_guess": True}, rtol=1e-10, deriv_type="tensor",
+                                     fronts=args.fronts)
+    out.update(n=int(model.prob.nred), nnz=int(model.prob.nnz), sigma=float(model.sigma), fronts=args.fronts,
+               host_setup_s=now() - t0)
     x0 = np.random.default_rng(0).uniform(0.3, 0.7, model.fltr.num_design_vars)       # first load factor below sigma
     torch.cuda.reset_peak_memory_stats()
     reps = []
@@ -332,6 +341,7 @@ def run_h8buck(args):
     out["factorisation_s"] = {"K_r": _time_numeric(model.Kfact.lu, model.Kr.data, amap),
                               "K_r + sigma G_r": _time_numeric(model.factor.lu, shifted, amap)}
     out["BLF"] = [float(v) for v in model.BLF]
+    out["memory"] = _factor_memory(model, [model.Kfact, model.factor])
     out["factor_info"] = {"K_r": model.Kfact.info, "K_r + sigma G_r": model.factor.info}
     out["refine_steps"] = model.factor.refine
     out["probe_residual_unrefined"] = model.factor._probe_residual()
@@ -367,6 +377,14 @@ def run_h8buck(args):
     return out
 
 
+def _factor_memory(model, ops):
+    """Front memory of the driver's factors: the pool a pooled factorisation borrows (0 resident), the resident fronts
+    of one factor, and the bytes every factor keeps for its life (its workspace: fronts included when resident)."""
+    sym = model.symbolic[0]
+    return {"pool_bytes": ops[0].lu.pool_bytes(), "resident_front_bytes": 8 * sym.query("front_doubles"),
+            "pool_doubles": sym.query("pool_doubles"), "factor_bytes": [op.lu.nbytes() for op in ops]}
+
+
 def _time_numeric(lu, vals, amap, reps=3):
     """Numeric LDL^T of ``vals`` alone, refactored in place in the factor ``lu``, device-synchronised, every repetition."""
     times = []
@@ -400,6 +418,7 @@ if __name__ == "__main__":
     ap.add_argument("--modes", type=int, default=None)
     ap.add_argument("--designs", type=int, default=None)
     ap.add_argument("--reps", type=int, default=3)
+    ap.add_argument("--fronts", choices=["resident", "pooled"], default="resident", help="h8, h8buck: front memory of the factors")
     a = ap.parse_args()
     if a.config == "c3":
         a.nx, a.ny, a.modes = a.nx or 352, a.ny or 704, a.modes or 20
