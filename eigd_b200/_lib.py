@@ -75,13 +75,12 @@ SIGNATURES = {
     "eigd_h8_element_matrices": (c_int, [c_int, c_ptr, c_ptr, c_dbl, c_dbl, c_dbl, c_ptr, c_ptr]),
     "eigd_h8_stress_stiffness": (c_int, [c_int, c_ptr, c_ptr, c_dbl, c_dbl, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr]),
     "eigd_h8_gderiv_u": (c_int, [c_int, c_ptr, c_ptr, c_dbl, c_dbl, c_ptr, c_ptr, c_ptr, c_ptr, c_int, c_i64, c_ptr]),
-    "eigd_h8_dof_gather": (c_int, [c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr]),
     "eigd_node_gather": (c_int, [c_int, c_ptr, c_ptr, c_ptr, c_dbl, c_ptr]),
+    "eigd_dof_gather": (c_int, [c_int, c_int, c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr]),
     "eigd_filter_project": (c_int, [c_int, c_dbl, c_dbl, c_ptr, c_ptr, c_ptr]),
     "eigd_q4_stress": (c_int, [c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr]),
     "eigd_q4_assemble_geometric": (c_int, [c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_ptr]),
     "eigd_q4_gderiv": (c_int, [c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_int, c_int, c_ptr, c_ptr, c_ptr, c_dbl, c_ptr, c_ptr]),
-    "eigd_q4_dof_gather": (c_int, [c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr]),
     "eigd_expand_rows": (c_int, [c_i64, c_int, c_ptr, c_ptr, c_ptr]),
     "eigd_reduce_rows": (c_int, [c_i64, c_int, c_ptr, c_ptr, c_ptr]),
 }

@@ -161,21 +161,6 @@ q4_gderiv_kernel(int nelems, const int* __restrict__ conn, const double* __restr
   }
 }
 
-// dfdu[2 v + d] = sum over the elements e around node v of due[e][2 local(v, e) + d]  (np.add.at, :318-320)
-__global__ void q4_dof_gather_kernel(int nnodes, const int* __restrict__ nptr, const int* __restrict__ nelem,
-                                     const int* __restrict__ nlocal, const double* __restrict__ due, double* __restrict__ out) {
-  int v = blockIdx.x * blockDim.x + threadIdx.x;
-  if (v >= nnodes) return;
-  double s0 = 0.0, s1 = 0.0;
-  for (int p = nptr[v]; p < nptr[v + 1]; ++p) {
-    const double* d = due + (int64_t)nelem[p] * 8 + 2 * nlocal[p];
-    s0 += d[0];
-    s1 += d[1];
-  }
-  out[2 * v] = s0;
-  out[2 * v + 1] = s1;
-}
-
 // full[idx[i], :] = red[i, :]   (full_vector, :506-511; the rest of `full` must be zero)
 __global__ void expand_rows_kernel(int64_t nr, int k, const int* __restrict__ idx, const double* __restrict__ red,
                                    double* __restrict__ full) {
@@ -223,14 +208,6 @@ extern "C" int eigd_q4_gderiv(int nelems, const int* d_conn, const double* d_xy,
   int grid = (int)(((int64_t)nelems * G + 255) / 256);
   EIGD_LAUNCH((q4_gderiv_kernel<G>), grid, 256, 0, nelems, d_conn, d_xy, d_cmat6, d_W, d_V, N, ldw, d_ks, d_dks, d_u, sx,
               d_out_rho, d_due);
-  EIGD_CHECK_LAUNCH();
-  return 0;
-}
-
-extern "C" int eigd_q4_dof_gather(int nnodes, const int* d_nptr, const int* d_nelem, const int* d_nlocal, const double* d_due,
-                                  double* d_out) {
-  if (nnodes <= 0) return 0;
-  EIGD_LAUNCH(q4_dof_gather_kernel, (nnodes + 255) / 256, 256, 0, nnodes, d_nptr, d_nelem, d_nlocal, d_due, d_out);
   EIGD_CHECK_LAUNCH();
   return 0;
 }

@@ -1,6 +1,7 @@
 // Q4 element kernels: per-element bilinear forms w_e^T (dK_e/ds) v_e, w_e^T (dM_e/dm) v_e summed
 // over modes (warp-shuffle segmented reduction, one lane group per element), gather-form
-// assembly of K and M through the (element, a, b) -> CSR map, and the element -> node gather.
+// assembly of K and M through the (element, a, b) -> CSR map, the element -> node gather and the element -> dof gather
+// of the buckling problems.
 //
 // Replaces the numpy einsum callbacks of the reference examples:
 //   thermal      examples/thermal.py:126-148 (K), :150-190 (dK), :192-214 (M), :216-246 (dM)
@@ -151,6 +152,25 @@ __global__ void node_gather_kernel(int nnodes, const int* __restrict__ nptr, con
   out[v] = scale * s;
 }
 
+// out[NC v + i] = sum over the elements e around node v of due[e][NC local(v, e) + i], due (nelems, npe * NC): the
+// gather form of the dof scatter np.add.at (examples/buckling.py:318-320), deterministic and without atomics
+template <int NC>
+__global__ void dof_gather_kernel(int nnodes, int npe, const int* __restrict__ nptr, const int* __restrict__ nelem,
+                                  const int* __restrict__ nlocal, const double* __restrict__ due, double* __restrict__ out) {
+  const int v = blockIdx.x * blockDim.x + threadIdx.x;
+  if (v >= nnodes) return;
+  double s[NC];
+#pragma unroll
+  for (int i = 0; i < NC; ++i) s[i] = 0.0;
+  for (int p = nptr[v]; p < nptr[v + 1]; ++p) {
+    const double* d = due + (int64_t)nelem[p] * (npe * NC) + NC * nlocal[p];
+#pragma unroll
+    for (int i = 0; i < NC; ++i) s[i] += d[i];
+  }
+#pragma unroll
+  for (int i = 0; i < NC; ++i) out[NC * (int64_t)v + i] = s[i];
+}
+
 }  // namespace
 
 extern "C" int eigd_q4_assemble(int kind, int nelems, const int* d_conn, const double* d_xy, const double* d_ks,
@@ -183,6 +203,17 @@ extern "C" int eigd_node_gather(int nnodes, const int* d_nptr, const int* d_nele
                                 double* d_out) {
   if (nnodes <= 0) return 0;
   EIGD_LAUNCH(node_gather_kernel, (nnodes + 255) / 256, 256, 0, nnodes, d_nptr, d_nelem, d_evals, scale, d_out);
+  EIGD_CHECK_LAUNCH();
+  return 0;
+}
+
+extern "C" int eigd_dof_gather(int nnodes, int ncomp, int npe, const int* d_nptr, const int* d_nelem, const int* d_nlocal,
+                               const double* d_due, double* d_out) {
+  if (nnodes <= 0) return 0;
+  const int grid = (nnodes + 255) / 256;
+  if (ncomp == 2) EIGD_LAUNCH(dof_gather_kernel<2>, grid, 256, 0, nnodes, npe, d_nptr, d_nelem, d_nlocal, d_due, d_out);
+  else if (ncomp == 3) EIGD_LAUNCH(dof_gather_kernel<3>, grid, 256, 0, nnodes, npe, d_nptr, d_nelem, d_nlocal, d_due, d_out);
+  else { eigd_set_error("dof_gather: %d components per node not instantiated (2: Q4 plane stress, 3: H8)", ncomp); return 1; }
   EIGD_CHECK_LAUNCH();
   return 0;
 }

@@ -169,24 +169,6 @@ h8_gderiv_u_kernel(int nelems, const int* __restrict__ conn, const double* __res
   for (int i = 0; i < 3; ++i) due[e * 24 + 3 * a + i] = kge * de[i];
 }
 
-// out[3 v + i] = sum over the elements e around node v of due[e][3 local(v, e) + i]: the gather form of the dof
-// scatter, deterministic and without atomics (q4_dof_gather_kernel with three components)
-__global__ void h8_dof_gather_kernel(int nnodes, const int* __restrict__ nptr, const int* __restrict__ nelem,
-                                     const int* __restrict__ nlocal, const double* __restrict__ due, double* __restrict__ out) {
-  const int v = blockIdx.x * blockDim.x + threadIdx.x;
-  if (v >= nnodes) return;
-  double s0 = 0.0, s1 = 0.0, s2 = 0.0;
-  for (int p = nptr[v]; p < nptr[v + 1]; ++p) {
-    const double* d = due + (int64_t)nelem[p] * 24 + 3 * nlocal[p];
-    s0 += d[0];
-    s1 += d[1];
-    s2 += d[2];
-  }
-  out[3 * (int64_t)v] = s0;
-  out[3 * (int64_t)v + 1] = s1;
-  out[3 * (int64_t)v + 2] = s2;
-}
-
 }  // namespace
 
 extern "C" int eigd_h8_stress_stiffness(int nelems, const int* d_conn, const double* d_X, double E, double nu,
@@ -209,14 +191,6 @@ extern "C" int eigd_h8_gderiv_u(int nelems, const int* d_conn, const double* d_X
   if (!h8_isotropic(E, nu, c, "h8_gderiv_u")) return 1;
   const int grid = (int)(((int64_t)nelems * 32 + 255) / 256);
   EIGD_LAUNCH(h8_gderiv_u_kernel, grid, 256, 0, nelems, d_conn, d_X, c, d_kg, d_dofmap, d_W, d_V, N, ld, d_due);
-  EIGD_CHECK_LAUNCH();
-  return 0;
-}
-
-extern "C" int eigd_h8_dof_gather(int nnodes, const int* d_nptr, const int* d_nelem, const int* d_nlocal, const double* d_due,
-                                  double* d_out) {
-  if (nnodes <= 0) return 0;
-  EIGD_LAUNCH(h8_dof_gather_kernel, (nnodes + 255) / 256, 256, 0, nnodes, d_nptr, d_nelem, d_nlocal, d_due, d_out);
   EIGD_CHECK_LAUNCH();
   return 0;
 }

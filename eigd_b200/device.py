@@ -817,8 +817,76 @@ def q4_assemble(kind, conn, xy, ks, ms, cmat6, src_ptr, src, nnz, Kvals, Mvals):
                                        _ptr(src_ptr), _ptr(src), int(nnz), _ptr(Kvals), _ptr(Mvals)), "q4_assemble")
 
 
+def element_material(law, par, rho, conn=None, rhoE=None, ks=None, ms=None, dk=None, dm=None):
+    """Penalised material factors ks, ms and their derivatives dk, dm of law 0 / 1 / 2 with the four parameters ``par``
+    (eigd_q4_material), of the element densities: the mean of the nodal ``rho`` over the element's nodes (``conn``
+    (nelems, npe), mean written to ``rhoE``) or, without ``conn``, ``rho`` itself.  Outputs left None are not written."""
+    nelems, npe = (conn.shape[0], conn.shape[1]) if conn is not None else (rho.numel(), 4)     # npe unread without conn
+    par4 = (ctypes.c_double * 4)(*[float(v) for v in par])
+    check(_lib.load().eigd_q4_material(int(law), nelems, npe, _ptr(conn), _ptr(rho), par4, _ptr(rhoE), _ptr(ks), _ptr(ms),
+                                       _ptr(dk), _ptr(dm)), "q4_material")
+
+
 def node_gather(nptr, nelem, evals, scale, out):
     check(_lib.load().eigd_node_gather(out.numel(), _ptr(nptr), _ptr(nelem), _ptr(evals), float(scale), _ptr(out)), "node_gather")
+    return out
+
+
+def dof_gather(nptr, nelem, nlocal, due, out):
+    """out[c v + i] = sum over the elements e around node v of due[e, c nlocal + i]: the element terms due (nelems,
+    npe * c) gathered to the c = out.numel() / nnodes components of every node."""
+    nnodes = nptr.numel() - 1
+    ncomp = out.numel() // nnodes
+    check(_lib.load().eigd_dof_gather(nnodes, ncomp, due.shape[1] // ncomp, _ptr(nptr), _ptr(nelem), _ptr(nlocal), _ptr(due),
+                                      _ptr(out)), "dof_gather")
+    return out
+
+
+def filter_project(rho, beta, eta, g=None):
+    """tanh projection of the filtered density ``rho``, or with ``g`` the gradient g * d(projection)/d(rho)."""
+    out = empty(rho.shape[0])
+    check(_lib.load().eigd_filter_project(rho.shape[0], float(beta), float(eta), _ptr(rho), _ptr(g), _ptr(out)),
+          "filter_project")
+    return out
+
+
+# ------------------------------------------------------------------------------------------
+# stored unit element matrices (csrc/stored_fe.cu, csrc/h8.cu)
+# ------------------------------------------------------------------------------------------
+def h8_element_matrices(conn, X, E, nu, density, K0, M0):
+    """Unit stiffness and mass matrices K0, M0 (nelems * 576 each) of the H8 elements ``conn`` (nelems, 8)."""
+    check(_lib.load().eigd_h8_element_matrices(conn.shape[0], _ptr(conn), _ptr(X), float(E), float(nu), float(density),
+                                               _ptr(K0), _ptr(M0)), "h8_element_matrices")
+
+
+def stored_assemble(src_ptr, src, ne, E1, c1, vals, E3=None, c3=None, F1=None, d1=None, vals2=None, F3=None, d3=None):
+    """vals = CSR values of the elements c1[e] E1_e (+ c3[e] E3_e) through the (element, a, b) source lists; with
+    ``vals2``, the second matrix d1[e] F1_e (+ d3[e] F3_e) on the same pattern in the same pass."""
+    check(_lib.load().eigd_stored_assemble(src_ptr.numel() - 1, _ptr(src_ptr), _ptr(src), int(ne), _ptr(E1), _ptr(E3), _ptr(c1),
+                                           _ptr(c3), _ptr(vals), _ptr(F1), _ptr(F3), _ptr(d1), _ptr(d3), _ptr(vals2)),
+          "stored_assemble")
+    return vals
+
+
+def stored_quadform(dofmap, E1, c1, W, V, out, E3=None, c3=None, F1=None, d1=None, W2=None, s1=1.0, s2=1.0):
+    """out[e] = sum_k W_k^T (c1[e] E1_e + c3[e] E3_e) V_k over the element dofs ``dofmap`` (nelems, ne); with the second
+    term, s1 * that + s2 * sum_k W2_k^T (d1[e] F1_e) V_k (eigd_stored_quadform).  W, W2, V: (n, N) row-major."""
+    ld = V.stride(0)
+    for t in (W, W2):
+        if t is not None and (t.shape != V.shape or t.stride(0) != ld or t.stride(1) != 1):
+            raise ValueError("W / W2 must have the shape and row-major layout of V")
+    if V.stride(1) != 1:
+        raise ValueError("V must be row-major")
+    check(_lib.load().eigd_stored_quadform(dofmap.shape[0], dofmap.shape[1], _ptr(dofmap), _ptr(E1), _ptr(E3), _ptr(c1), _ptr(c3),
+                                           _ptr(W), _ptr(V), V.shape[1], ld, _ptr(out), _ptr(F1), _ptr(d1), _ptr(W2), float(s1),
+                                           float(s2)), "stored_quadform")
+    return out
+
+
+def segment_sum(seg_ptr, perm, x, scale, out):
+    """out[c] = scale * sum of x[perm[i]] over the segment [seg_ptr[c], seg_ptr[c + 1])."""
+    check(_lib.load().eigd_segment_sum(seg_ptr.numel() - 1, _ptr(seg_ptr), _ptr(perm), _ptr(x), float(scale), _ptr(out)),
+          "segment_sum")
     return out
 
 
@@ -846,12 +914,6 @@ def q4_gderiv(conn, xy, cmat6, W, V, ks, dks, u, sx, out_rho=None, due=None):
           "q4_gderiv")
 
 
-def q4_dof_gather(nptr, nelem, nlocal, due, out):
-    check(_lib.load().eigd_q4_dof_gather(out.numel() // 2, _ptr(nptr), _ptr(nelem), _ptr(nlocal), _ptr(due), _ptr(out)),
-          "q4_dof_gather")
-    return out
-
-
 def h8_stress_stiffness(conn, X, E, nu, kg, dofmap, u, stress, G0):
     """Element stresses kg C B_q u_e (``stress`` (nelems, 8, 6) or None) and the unit stress stiffness G0 (nelems * 576)
     of the H8 solid; ``u`` is read through ``dofmap`` (nelems, 24), -1 = constrained."""
@@ -867,12 +929,6 @@ def h8_gderiv_u(conn, X, E, nu, kg, dofmap, W, V, due):
     check(_lib.load().eigd_h8_gderiv_u(conn.shape[0], _ptr(conn), _ptr(X), float(E), float(nu), _ptr(kg), _ptr(dofmap), _ptr(W),
                                        _ptr(V), V.shape[1], V.stride(0), _ptr(due)), "h8_gderiv_u")
     return due
-
-
-def h8_dof_gather(nptr, nelem, nlocal, due, out):
-    check(_lib.load().eigd_h8_dof_gather(out.numel() // 3, _ptr(nptr), _ptr(nelem), _ptr(nlocal), _ptr(due), _ptr(out)),
-          "h8_dof_gather")
-    return out
 
 
 def expand_rows(idx, red, nfull):

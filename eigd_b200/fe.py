@@ -14,15 +14,11 @@ Mirrors (paths relative to the reference root):
   node scatter              examples/thermal.py:612-615
   node filter               examples/node_filter.py:61-88 (construction), :164-217 (apply / gradient)
 """
-import ctypes
-
 import numpy as np
 import torch
 
-from . import _lib
 from . import device as D
-from ._hostdev import is_dev, to_dev, to_host, like_input
-from .device import _ptr
+from ._hostdev import to_dev, like_input
 
 
 def grid_mesh(nx, ny, Lx=1.0, Ly=1.0):
@@ -98,6 +94,49 @@ def node_adjacency(conn, nnodes):
     return np.cumsum(nptr).astype(np.int32), e[order].astype(np.int32)
 
 
+class AssemblyPattern:
+    """The CSR pattern of assembled K/M matrices (``assembly_structure``) and, for every non-zero, the list of its
+    (element, a, b) sources: ``indptr``, ``indices`` on the host, all four arrays in HBM.  The host copies of the source
+    lists are not kept; ``reduced`` downloads them when it needs them."""
+
+    def __init__(self, indptr, indices, src_ptr, src):
+        dev = D.dev()
+        self.indptr, self.indices = indptr, indices
+        self.nnz = len(indices)
+        self.shape = (len(indptr) - 1, len(indptr) - 1)
+        self.indptr_d = torch.as_tensor(indptr, device=dev)
+        self.indices_d = torch.as_tensor(indices, device=dev)
+        self.src_ptr_d = torch.as_tensor(src_ptr, device=dev)
+        self.src_d = torch.as_tensor(src, device=dev)
+
+    def csr(self, vals):
+        """The matrix with values ``vals`` (device, (nnz,)) on this pattern."""
+        return D.CsrDevice(self.indptr_d, self.indices_d, vals, self.shape)
+
+    def reduced(self, reduced):
+        """The pattern of ``matrix[reduced, :][:, reduced]`` (``reduced_structure``)."""
+        return AssemblyPattern(*reduced_structure(self.indptr, self.indices, to_host_i64(self.src_ptr_d),
+                                                  to_host_i64(self.src_d), reduced, self.shape[0]))
+
+
+def _penalty_law(name, ptype, p, q, c0, rho0):
+    """Law and parameters of eigd_q4_material for the structural penalisation ``ptype`` ("simp": rho^p + rho0, "ramp":
+    rho/(1+q(1-rho)) + rho0), mass factor c0 rho; ``name`` is the option the error message names."""
+    if ptype == "simp":
+        return 1, np.array([p, 1.0, c0, rho0])
+    if ptype == "ramp":
+        return 2, np.array([q, 1.0, c0, rho0])
+    raise ValueError("unknown %s %r" % (name, ptype))
+
+
+def _cols(t):
+    """(n,) or (n, N) device operand -> contiguous (n, N)."""
+    if t is None:
+        return None
+    t = t if t.dim() == 2 else t.unsqueeze(1)
+    return t if t.is_contiguous() else t.contiguous()
+
+
 class _SensitivityCallback:
     """A reference sensitivity callback such as ``dAdx(w, v)``: ``which`` of the operators of ``parent``, called with
     host or device operands; subclasses give its device form ``device_call(W, V)``."""
@@ -120,36 +159,90 @@ class _Half(_SensitivityCallback):
         return self.parent.device_call_fused(None, W, V, 0.0, 1.0)
 
 
-class _ElementMaterial:
-    """Nodal density -> element density (the mean over the element's ``npe`` nodes) and the penalised material factors
-    ks, ms and their derivatives dk, dm (eigd_q4_material), for the problems with one density per element."""
+class _ElementModel:
+    """What the models with one density per element share: the mesh and its dof numbering, the assembly pattern, node
+    adjacency, nodal density -> element density (the mean over the element's ``npe`` nodes) -> penalised material
+    factors ks, ms and their derivatives dk, dm (eigd_q4_material with ``law``, ``par``), the assembly of K, M and of
+    their tangent, and the element-range sharding of the fused sensitivities.  Subclasses give the element kernels:
+    ``_assemble_values(ck, cm)`` and ``_quadforms(lo, hi, WA, WB, V, cA, cB)`` on the elements [lo, hi)."""
 
-    npe = 4
+    def _setup(self, conn, X, nnodes, dof, law, par):
+        dev = D.dev()
+        self.conn, self.X = conn, X
+        self.nelems, self.nnodes, self.dof = conn.shape[0], nnodes, dof
+        self.ndof = dof * nnodes
+        self.var = element_dofs(conn, dof)
+        self.pattern = AssemblyPattern(*assembly_structure(self.var, self.ndof))
+        self.indptr, self.indices, self.nnz = self.pattern.indptr, self.pattern.indices, self.pattern.nnz
+        nptr, nelem = node_adjacency(conn, nnodes)
+        self.conn_d = torch.as_tensor(conn.astype(np.int32), device=dev)
+        self.nptr_d = torch.as_tensor(nptr, device=dev)
+        self.nelem_d = torch.as_tensor(nelem, device=dev)
+        self.law, self.par = law, par
+        self.rhoE_d = D.empty(self.nelems)
+        self.ks_d, self.ms_d = D.empty(self.nelems), D.empty(self.nelems)
+        self.dk_d, self.dm_d = D.empty(self.nelems), D.empty(self.nelems)
+        self.sharding = None          # dist.ModeSharding: element-range shards of the df/dx reduction
+        self.dAdx, self.dBdx = _Half(self, "A"), _Half(self, "B")
+        self.dAdx.fused_with, self.dBdx.fused_with = self.dBdx, self.dAdx
 
+    # ---- material -------------------------------------------------------------------------------
     def set_density(self, rho=None, rhoE=None):
         """Nodal density rho (filtered design) -> element density + material factors, or set the
         element densities directly."""
-        lib = _lib.load()
+        out = dict(ks=self.ks_d, ms=self.ms_d, dk=self.dk_d, dm=self.dm_d)
         if rhoE is not None:
             self.rhoE_d.copy_(to_dev(rhoE))
-            _lib.check(lib.eigd_q4_material(self.law, self.nelems, self.npe, None, _ptr(self.rhoE_d), self._par_c, None,
-                                            _ptr(self.ks_d), _ptr(self.ms_d), _ptr(self.dk_d), _ptr(self.dm_d)), "q4_material")
+            D.element_material(self.law, self.par, self.rhoE_d, **out)
         else:
-            rho_d = to_dev(rho)
-            _lib.check(lib.eigd_q4_material(self.law, self.nelems, self.npe, _ptr(self.conn_d), _ptr(rho_d), self._par_c,
-                                            _ptr(self.rhoE_d), _ptr(self.ks_d), _ptr(self.ms_d), _ptr(self.dk_d),
-                                            _ptr(self.dm_d)), "q4_material")
+            D.element_material(self.law, self.par, to_dev(rho), conn=self.conn_d, rhoE=self.rhoE_d, **out)
         return self.rhoE_d
 
     def _element_mean(self, rho_t):
-        """Element mean of the nodal vector ``rho_t`` (the material outputs of this call are scratch)."""
-        rhoEt, s1, s2, s3, s4 = (D.empty(self.nelems) for _ in range(5))
-        _lib.check(_lib.load().eigd_q4_material(self.law, self.nelems, self.npe, _ptr(self.conn_d), _ptr(to_dev(rho_t)),
-                                                self._par_c, _ptr(rhoEt), _ptr(s1), _ptr(s2), _ptr(s3), _ptr(s4)), "q4_material")
+        """Element mean of the nodal vector ``rho_t``."""
+        rhoEt = D.empty(self.nelems)
+        D.element_material(self.law, self.par, to_dev(rho_t), conn=self.conn_d, rhoE=rhoEt)
         return rhoEt
 
+    # ---- assembly -------------------------------------------------------------------------------
+    def assemble(self):
+        """K(rho), M(rho) as CsrDevice sharing one pattern (values computed in gather form)."""
+        Kv, Mv = self._assemble_values(self.ks_d, self.ms_d)
+        return self.pattern.csr(Kv), self.pattern.csr(Mv)
 
-class Q4Problem(_ElementMaterial):
+    def assemble_tangent(self, rho_t):
+        """Directional derivative of (K, M) along the nodal density direction ``rho_t`` (device, (nnodes,)), on the same
+        pattern: the assembly with the material factors replaced by (dk/drho_e) rho_e', (dm/drho_e) rho_e'.
+        Used by the dual-number (complex-step) mode of the drivers."""
+        rhoEt = self._element_mean(rho_t)
+        Kv, Mv = self._assemble_values(self.dk_d * rhoEt, self.dm_d * rhoEt)
+        return self.pattern.csr(Kv), self.pattern.csr(Mv)
+
+    def dof_coords(self):
+        """Node coordinates for geometric nested dissection (``SpLuOperator(coords=..., dof_per_node=...)``)."""
+        return self.X, self.dof
+
+    # ---- sensitivities ----------------------------------------------------------------------------
+    def device_call_fused(self, WA, WB, V, cA, cB):
+        """cA * sum_k WA_k^T (dK/drho_e) V_k + cB * sum_k WB_k^T (dM/drho_e) V_k per element (device).  With
+        ``sharding``, every rank evaluates its element range and one all-gather joins them (dist.py)."""
+        args = (_cols(WA), _cols(WB), _cols(V), float(cA), float(cB))
+        shard = self.sharding
+        if shard is None or shard.world == 1:
+            return self._quadforms(0, self.nelems, *args)
+        lo, hi = shard.my_range(self.nelems)
+        return shard.allgather_ranges(self._quadforms(lo, hi, *args), self.nelems)
+
+    def scatter_to_nodes(self, evals, scale=None):
+        """rho_b[v] = scale * sum_{e ni v} evals[e] (examples/thermal.py:612-615); default scale 1 / npe, the transpose
+        of the element mean."""
+        ev = to_dev(evals)
+        out = D.empty(self.nnodes)
+        D.node_gather(self.nptr_d, self.nelem_d, ev, 1.0 / self.npe if scale is None else scale, out)
+        return like_input(out, evals)
+
+
+class Q4Problem(_ElementModel):
     """Thermal (1 DOF/node) or plane-stress (2 DOF/node) Q4 model with its operators in HBM.
 
     kind "thermal": K_e = kappa(rho_e) sum_q detJ Be^T Be, M_e = c(rho_e) sum_q detJ N N^T
@@ -160,117 +253,39 @@ class Q4Problem(_ElementMaterial):
       (examples/natural_frequency.py:83-86,140-155,219-231).
     """
 
+    npe = 4
+
     def __init__(self, conn, X, kind="thermal", E=1.0, nu=0.3, kappa=1.0, density=1.0, heat_capacity=1.0, p=3.0,
                  beta=1e-6, rho0_K=1e-6, ptype_K="simp", q=5.0):
         if kind not in ("thermal", "plane_stress"):
             raise ValueError("unknown kind %r" % kind)
-        dev = D.dev()
         self.kind = kind
         self.kid = 0 if kind == "thermal" else 1
-        self.conn = np.asarray(conn, dtype=np.int64)
-        self.X = np.asarray(X, dtype=np.float64)
-        self.nelems = self.conn.shape[0]
-        self.nnodes = int(self.conn.max()) + 1
-        self.dof = 1 if kind == "thermal" else 2
-        self.ndof = self.dof * self.nnodes
-        self.var = element_dofs(self.conn, self.dof)
-        self.indptr, self.indices, src_ptr, src = assembly_structure(self.var, self.ndof)
-        self.nnz = len(self.indices)
-        nptr, nelem = node_adjacency(self.conn, self.nnodes)
+        conn = np.asarray(conn, dtype=np.int64)
         if kind == "thermal":
-            self.law, self.par = 0, np.array([p, kappa, heat_capacity * density, beta])
-        elif ptype_K == "simp":
-            self.law, self.par = 1, np.array([p, 1.0, density, rho0_K])
-        elif ptype_K == "ramp":
-            self.law, self.par = 2, np.array([q, 1.0, density, rho0_K])
+            law, par = 0, np.array([p, kappa, heat_capacity * density, beta])
         else:
-            raise ValueError("unknown ptype_K %r" % ptype_K)
+            law, par = _penalty_law("ptype_K", ptype_K, p, q, density, rho0_K)
+        self._setup(conn, np.asarray(X, dtype=np.float64), int(conn.max()) + 1, 1 if kind == "thermal" else 2, law, par)
         C0 = E * np.array([[1.0, nu, 0.0], [nu, 1.0, 0.0], [0.0, 0.0, 0.5 * (1.0 - nu)]]) / (1.0 - nu**2)
         self.C0 = C0
-        # ---- device mirrors -------------------------------------------------------------
-        self.conn_d = torch.as_tensor(self.conn.astype(np.int32), device=dev)
         self.xy_d = to_dev(self.X)
         self.cmat6_d = to_dev(np.array([C0[0, 0], C0[0, 1], C0[0, 2], C0[1, 1], C0[1, 2], C0[2, 2]]))
-        self.indptr_d = torch.as_tensor(self.indptr, device=dev)
-        self.indices_d = torch.as_tensor(self.indices, device=dev)
-        self.src_ptr_d = torch.as_tensor(src_ptr, device=dev)
-        self.src_d = torch.as_tensor(src, device=dev)
-        self.nptr_d = torch.as_tensor(nptr, device=dev)
-        self.nelem_d = torch.as_tensor(nelem, device=dev)
-        self.rhoE_d = D.empty(self.nelems)
-        self.ks_d, self.ms_d = D.empty(self.nelems), D.empty(self.nelems)
-        self.dk_d, self.dm_d = D.empty(self.nelems), D.empty(self.nelems)
-        self._par_c = (ctypes.c_double * 4)(*[float(v) for v in self.par])
-        self.sharding = None          # dist.ModeSharding: element-range shards of the df/dx reduction
-        self.dAdx, self.dBdx = _Half(self, "A"), _Half(self, "B")
-        self.dAdx.fused_with, self.dBdx.fused_with = self.dBdx, self.dAdx
 
-    # ---- material (set_density: _ElementMaterial) -----------------------------------------------
-    def assemble_tangent(self, rho_t):
-        """Directional derivative of (K, M) along the nodal density direction ``rho_t`` (device, (nnodes,)), on the same
-        pattern: the assembly kernel with the material factors replaced by (dk/drho_e) rho_e', (dm/drho_e) rho_e'.
-        Used by the dual-number (complex-step) mode of the drivers."""
-        rhoEt = self._element_mean(rho_t)
-        kt, mt = self.dk_d * rhoEt, self.dm_d * rhoEt
+    def _assemble_values(self, ck, cm):
+        p = self.pattern
         Kv, Mv = D.empty(self.nnz), D.empty(self.nnz)
-        D.q4_assemble(self.kid, self.conn_d, self.xy_d, kt, mt, self.cmat6_d, self.src_ptr_d, self.src_d, self.nnz, Kv, Mv)
-        shape = (self.ndof, self.ndof)
-        return (D.CsrDevice(self.indptr_d, self.indices_d, Kv, shape), D.CsrDevice(self.indptr_d, self.indices_d, Mv, shape))
+        D.q4_assemble(self.kid, self.conn_d, self.xy_d, ck, cm, self.cmat6_d, p.src_ptr_d, p.src_d, self.nnz, Kv, Mv)
+        return Kv, Mv
 
-    # ---- assembly -------------------------------------------------------------------------------
-    def assemble(self):
-        """K(rho), M(rho) as CsrDevice sharing one pattern (values computed in gather form)."""
-        Kv, Mv = D.empty(self.nnz), D.empty(self.nnz)
-        D.q4_assemble(self.kid, self.conn_d, self.xy_d, self.ks_d, self.ms_d, self.cmat6_d, self.src_ptr_d, self.src_d,
-                      self.nnz, Kv, Mv)
-        shape = (self.ndof, self.ndof)
-        K = D.CsrDevice(self.indptr_d, self.indices_d, Kv, shape)
-        M = D.CsrDevice(self.indptr_d, self.indices_d, Mv, shape)
-        return K, M
-
-    def dof_coords(self):
-        """Node coordinates for geometric nested dissection (``SpLuOperator(coords=..., dof_per_node=...)``)."""
-        return self.X, self.dof
-
-    # ---- sensitivities ----------------------------------------------------------------------------
-    def device_call_fused(self, WA, WB, V, cA, cB):
-        """cA * sum_k WA_k^T (dK/drho_e) V_k + cB * sum_k WB_k^T (dM/drho_e) V_k per element (device)."""
-        V2 = V if V.dim() == 2 else V.unsqueeze(1)
-        WA2 = None if WA is None else (WA if WA.dim() == 2 else WA.unsqueeze(1))
-        WB2 = None if WB is None else (WB if WB.dim() == 2 else WB.unsqueeze(1))
-        V2 = V2 if V2.is_contiguous() else V2.contiguous()
-        WA2 = None if WA2 is None else (WA2 if WA2.is_contiguous() else WA2.contiguous())
-        WB2 = None if WB2 is None else (WB2 if WB2.is_contiguous() else WB2.contiguous())
-        shard = self.sharding
-        if shard is None or shard.world == 1:
-            out = D.zeros(self.nelems)
-            D.q4_quadforms(self.kid, self.conn_d, self.xy_d, self.cmat6_d, WA2, WB2, V2, self.dk_d, self.dm_d,
-                           float(cA), -float(cB), out)
-            return out
-        lo, hi = shard.my_range(self.nelems)                  # element-range shard + one all-gather (dist.py)
-        part = D.zeros(hi - lo)
-        if hi > lo:
-            D.q4_quadforms(self.kid, self.conn_d[lo:hi], self.xy_d, self.cmat6_d, WA2, WB2, V2, self.dk_d[lo:hi],
-                           self.dm_d[lo:hi], float(cA), -float(cB), part)
-        return shard.allgather_ranges(part, self.nelems)
-
-    def scatter_to_nodes(self, evals, scale=0.25):
-        """rho_b[v] = scale * sum_{e ni v} evals[e] (examples/thermal.py:612-615)."""
-        ev = to_dev(evals)
-        out = D.empty(self.nnodes)
-        D.node_gather(self.nptr_d, self.nelem_d, ev, scale, out)
-        return like_input(out, evals)
+    def _quadforms(self, lo, hi, WA, WB, V, cA, cB):
+        out = D.zeros(hi - lo)
+        D.q4_quadforms(self.kid, self.conn_d[lo:hi], self.xy_d, self.cmat6_d, WA, WB, V, self.dk_d[lo:hi], self.dm_d[lo:hi],
+                       cA, -cB, out)
+        return out
 
 
-def _cols(t):
-    """(n,) or (n, N) device operand -> contiguous (n, N)."""
-    if t is None:
-        return None
-    t = t if t.dim() == 2 else t.unsqueeze(1)
-    return t if t.is_contiguous() else t.contiguous()
-
-
-class H8Problem(_ElementMaterial):
+class H8Problem(_ElementModel):
     """Free 3-D isotropic solid on trilinear hexahedra (3 DOF/node) with its operators in HBM.
 
     K_e = s(rho_e) K0_e, M_e = rho_e M0_e with s = rho^p + rho0_K (SIMP) or rho/(1+q(1-rho)) + rho0_K (RAMP), the laws
@@ -283,104 +298,38 @@ class H8Problem(_ElementMaterial):
     NE = 24
 
     def __init__(self, conn, X, E=1.0, nu=0.3, density=1.0, p=3.0, rho0_K=1e-6, ptype_K="simp", q=5.0):
-        dev = D.dev()
-        self.conn = np.asarray(conn, dtype=np.int64)
-        self.X = np.asarray(X, dtype=np.float64)
-        if self.conn.ndim != 2 or self.conn.shape[1] != 8 or self.X.ndim != 2 or self.X.shape[1] != 3:
+        conn = np.asarray(conn, dtype=np.int64)
+        X = np.asarray(X, dtype=np.float64)
+        if conn.ndim != 2 or conn.shape[1] != 8 or X.ndim != 2 or X.shape[1] != 3:
             raise ValueError("H8Problem needs conn (nelems, 8) and X (nnodes, 3)")
-        self.nelems = self.conn.shape[0]
-        self.nnodes = self.X.shape[0]
-        self.dof = 3
-        self.ndof = 3 * self.nnodes
-        self.var = element_dofs(self.conn, 3)
-        self.indptr, self.indices, src_ptr, src = assembly_structure(self.var, self.ndof)
-        self.nnz = len(self.indices)
-        nptr, nelem = node_adjacency(self.conn, self.nnodes)
-        if ptype_K == "simp":
-            self.law, self.par = 1, np.array([p, 1.0, 1.0, rho0_K])
-        elif ptype_K == "ramp":
-            self.law, self.par = 2, np.array([q, 1.0, 1.0, rho0_K])
-        else:
-            raise ValueError("unknown ptype_K %r" % ptype_K)
-        self._par_c = (ctypes.c_double * 4)(*[float(v) for v in self.par])
-        # ---- device mirrors -------------------------------------------------------------
-        self.conn_d = torch.as_tensor(self.conn.astype(np.int32), device=dev)
+        self._setup(conn, X, X.shape[0], 3, *_penalty_law("ptype_K", ptype_K, p, q, 1.0, rho0_K))
         self.X_d = to_dev(np.ascontiguousarray(self.X))
-        self.dofmap_d = torch.as_tensor(self.var.astype(np.int32), device=dev)
-        self.indptr_d = torch.as_tensor(self.indptr, device=dev)
-        self.indices_d = torch.as_tensor(self.indices, device=dev)
-        self.src_ptr_d = torch.as_tensor(src_ptr, device=dev)
-        self.src_d = torch.as_tensor(src, device=dev)
-        del src_ptr, src
-        self.nptr_d = torch.as_tensor(nptr, device=dev)
-        self.nelem_d = torch.as_tensor(nelem, device=dev)
+        self.dofmap_d = torch.as_tensor(self.var.astype(np.int32), device=D.dev())
         ne2 = self.NE * self.NE
         self.K0_d, self.M0_d = D.empty(self.nelems * ne2), D.empty(self.nelems * ne2)
-        _lib.check(_lib.load().eigd_h8_element_matrices(self.nelems, _ptr(self.conn_d), _ptr(self.X_d), float(E), float(nu),
-                                                        float(density), _ptr(self.K0_d), _ptr(self.M0_d)), "h8_element_matrices")
-        self.rhoE_d = D.empty(self.nelems)
-        self.ks_d, self.ms_d = D.empty(self.nelems), D.empty(self.nelems)
-        self.dk_d, self.dm_d = D.empty(self.nelems), D.empty(self.nelems)
-        self.sharding = None          # dist.ModeSharding: element-range shards of the df/dx reduction
-        self.dAdx, self.dBdx = _Half(self, "A"), _Half(self, "B")
-        self.dAdx.fused_with, self.dBdx.fused_with = self.dBdx, self.dAdx
+        D.h8_element_matrices(self.conn_d, self.X_d, E, nu, density, self.K0_d, self.M0_d)
 
-    def _assemble(self, ck, cm):
+    def _assemble_values(self, ck, cm):
+        p = self.pattern
         Kv, Mv = D.empty(self.nnz), D.empty(self.nnz)
-        _lib.check(_lib.load().eigd_stored_assemble(self.nnz, _ptr(self.src_ptr_d), _ptr(self.src_d), self.NE, _ptr(self.K0_d),
-                                                    None, _ptr(ck), None, _ptr(Kv), _ptr(self.M0_d), None, _ptr(cm), None,
-                                                    _ptr(Mv)), "stored_assemble")
-        shape = (self.ndof, self.ndof)
-        return (D.CsrDevice(self.indptr_d, self.indices_d, Kv, shape), D.CsrDevice(self.indptr_d, self.indices_d, Mv, shape))
+        D.stored_assemble(p.src_ptr_d, p.src_d, self.NE, self.K0_d, ck, Kv, F1=self.M0_d, d1=cm, vals2=Mv)
+        return Kv, Mv
 
-    def assemble(self):
-        """K(rho), M(rho) as CsrDevice sharing one pattern."""
-        return self._assemble(self.ks_d, self.ms_d)
-
-    def assemble_tangent(self, rho_t):
-        """Directional derivative of (K, M) along the nodal density direction ``rho_t`` (device, (nnodes,)): the same
-        assembly with the coefficients (dk/drho_e) rho_e', (dm/drho_e) rho_e'.  Used by the dual-number mode of the
-        drivers."""
-        rhoEt = self._element_mean(rho_t)
-        return self._assemble(self.dk_d * rhoEt, self.dm_d * rhoEt)
-
-    def dof_coords(self):
-        """Node coordinates for geometric nested dissection (``SpLuOperator(coords=..., dof_per_node=...)``)."""
-        return self.X, self.dof
-
-    def device_call_fused(self, WA, WB, V, cA, cB):
-        """cA * sum_k WA_k^T (dK/drho_e) V_k + cB * sum_k WB_k^T (dM/drho_e) V_k per element (device), both terms in one
-        pass of eigd_stored_quadform over the gathered V."""
-        V2, WA2, WB2 = _cols(V), _cols(WA), _cols(WB)
-        for t in (WA2, WB2):
-            if t is not None and t.shape != V2.shape:
-                raise ValueError("WA / WB must have the shape of V")
-        terms = [(W, U, c, float(s)) for W, U, c, s in ((WA2, self.K0_d, self.dk_d, cA), (WB2, self.M0_d, self.dm_d, cB))
-                 if W is not None]
-        shard = self.sharding
-        lo, hi = (0, self.nelems) if shard is None or shard.world == 1 else shard.my_range(self.nelems)
+    def _quadforms(self, lo, hi, WA, WB, V, cA, cB):
+        """Both terms in one pass of eigd_stored_quadform over the gathered V."""
+        ne2 = self.NE * self.NE
+        terms = [(W, U[lo * ne2:hi * ne2], c[lo:hi], s)
+                 for W, U, c, s in ((WA, self.K0_d, self.dk_d, cA), (WB, self.M0_d, self.dm_d, cB)) if W is not None]
+        (W1, U1, c1, s1), second = terms[0], terms[1:]
         out = D.zeros(hi - lo)
-        if hi > lo and terms:
-            ne2 = self.NE * self.NE
-            (W1, U1, c1, s1), second = terms[0], terms[1] if len(terms) == 2 else None
-            W2, F1, d1, s2 = second if second is not None else (None, None, None, 1.0)
-            rng = lambda t, w: None if t is None else t[lo * w:hi * w]          # noqa: E731  element-range views
-            _lib.check(_lib.load().eigd_stored_quadform(hi - lo, self.NE, _ptr(self.dofmap_d[lo:hi]), _ptr(rng(U1, ne2)), None,
-                                                        _ptr(rng(c1, 1)), None, _ptr(W1), _ptr(V2), V2.shape[1], V2.stride(0),
-                                                        _ptr(out), _ptr(rng(F1, ne2)), _ptr(rng(d1, 1)), _ptr(W2), s1, s2),
-                       "stored_quadform")
-            if second is None and s1 != 1.0:
+        if second:
+            W2, F1, d1, s2 = second[0]
+            D.stored_quadform(self.dofmap_d[lo:hi], U1, c1, W1, V, out, F1=F1, d1=d1, W2=W2, s1=s1, s2=s2)
+        else:
+            D.stored_quadform(self.dofmap_d[lo:hi], U1, c1, W1, V, out)
+            if s1 != 1.0:
                 out.mul_(s1)
-        if hi - lo == self.nelems:
-            return out
-        return shard.allgather_ranges(out, self.nelems)              # element-range shard + one all-gather (dist.py)
-
-    def scatter_to_nodes(self, evals, scale=0.125):
-        """rho_b[v] = scale * sum_{e ni v} evals[e]: the transpose of the 8-node element mean."""
-        ev = to_dev(evals)
-        out = D.empty(self.nnodes)
-        D.node_gather(self.nptr_d, self.nelem_d, ev, scale, out)
-        return like_input(out, evals)
+        return out
 
 
 def reduced_structure(indptr, indices, src_ptr, src, reduced, ndof):
@@ -446,29 +395,16 @@ class _BucklingProblem:
         for node, fv in forces.items():
             for j in range(dof):
                 self.f[dof * int(node) + j] += fv[j]
-        src_ptr, src = to_host_i64(b.src_ptr_d), to_host_i64(b.src_d)
-        self.indptr, self.indices, r_src_ptr, r_src = reduced_structure(b.indptr, b.indices, src_ptr, src, self.reduced,
-                                                                        self.ndof)
-        self.nnz = len(self.indices)
-        self.indptr_d = torch.as_tensor(self.indptr, device=dev)
-        self.indices_d = torch.as_tensor(self.indices, device=dev)
-        self.src_ptr_d = torch.as_tensor(r_src_ptr, device=dev)
-        self.src_d = torch.as_tensor(r_src, device=dev)
+        self.pattern = b.pattern.reduced(self.reduced)
+        self.indptr, self.indices, self.nnz = self.pattern.indptr, self.pattern.indices, self.pattern.nnz
         self.reduced_d = torch.as_tensor(self.reduced.astype(np.int32), device=dev)
         self.fr_d = to_dev(self.f[self.reduced])
         # local index of every node inside each adjacent element (dof gather of :318-320)
         self.nlocal_d = torch.as_tensor(node_local_index(self.conn), device=dev)
-        # G material law (:231-234) and the derivative the reference applies to it (:333-336)
-        if ptype_G == "simp":
-            self.lawG, parG, pardG = 1, [p, 1.0, density, rho0_G], [p, 1.0, density, rho0_G]
-        elif ptype_G == "ramp":
-            self.lawG, parG, pardG = 2, [q, 1.0, density, rho0_G], [q + 1.0, 1.0, density, rho0_G]
-        else:
-            raise ValueError("unknown ptype_G %r" % ptype_G)
-        self._parG = (ctypes.c_double * 4)(*[float(t) for t in parG])
-        self._pardG = (ctypes.c_double * 4)(*[float(t) for t in pardG])
+        # G material law (:231-234) and the RAMP parameters the reference differentiates it with (:333-336)
+        self.lawG, self._parG = _penalty_law("ptype_G", ptype_G, p, q, density, rho0_G)
+        self._pardG = [q + 1.0, 1.0, density, rho0_G]
         self.kg_d, self.dkg_d = D.empty(self.nelems), D.empty(self.nelems)
-        self._scratch = D.empty(self.nelems)
         self.u_d = None
         self.dGdu = _BucklingCallback(self, "dGdu")
         self.dGdx = _BucklingCallback(self, "dGdx")
@@ -488,14 +424,9 @@ class _BucklingProblem:
     # ---- material ------------------------------------------------------------------------------------
     def set_density(self, rho=None, rhoE=None):
         rhoE_d = self.base.set_density(rho=rho, rhoE=rhoE)
-        lib = _lib.load()
-        s, npe = self._scratch, self.base.npe
-        _lib.check(lib.eigd_q4_material(self.lawG, self.nelems, npe, None, _ptr(rhoE_d), self._parG, None, _ptr(self.kg_d),
-                                        _ptr(s), _ptr(self.dkg_d), _ptr(s)), "q4_material")
+        D.element_material(self.lawG, self._parG, rhoE_d, ks=self.kg_d, dk=self.dkg_d)
         if self.lawG == 2:      # the reference differentiates the RAMP law of G with q + 1 (:336)
-            tmp = D.empty(self.nelems)
-            _lib.check(lib.eigd_q4_material(self.lawG, self.nelems, npe, None, _ptr(rhoE_d), self._pardG, None, _ptr(tmp),
-                                            _ptr(s), _ptr(self.dkg_d), _ptr(s)), "q4_material")
+            D.element_material(self.lawG, self._pardG, rhoE_d, dk=self.dkg_d)
         return rhoE_d
 
     def set_displacement(self, ur_d):
@@ -507,7 +438,7 @@ class _BucklingProblem:
     def scatter_to_nodes(self, evals, scale=None):
         """rho_b[v] = scale * sum_{e ni v} evals[e]; default scale 1 / (nodes per element), the transpose of the element
         mean."""
-        return self.base.scatter_to_nodes(evals, 1.0 / self.base.npe if scale is None else scale)
+        return self.base.scatter_to_nodes(evals, scale)
 
 
 class BucklingQ4Problem(_BucklingProblem):
@@ -528,18 +459,19 @@ class BucklingQ4Problem(_BucklingProblem):
     def assemble_K(self):
         """K_r(rho) = reduce_matrix(get_stiffness_matrix(rhoE)) (:152-176, 505-510), values gathered directly
         through the reduced source lists."""
-        b = self.base
-        Kv, Mv = D.empty(self.nnz), D.empty(self.nnz)
-        D.q4_assemble(1, self.conn_d, self.xy_d, b.ks_d, b.ms_d, self.cmat6_d, self.src_ptr_d, self.src_d, self.nnz, Kv, Mv)
-        return D.CsrDevice(self.indptr_d, self.indices_d, Kv, (self.nred, self.nred))
+        b, p = self.base, self.pattern
+        Kv = D.empty(self.nnz)
+        D.q4_assemble(1, self.conn_d, self.xy_d, b.ks_d, b.ms_d, self.cmat6_d, p.src_ptr_d, p.src_d, self.nnz, Kv, None)
+        return p.csr(Kv)
 
     def assemble_G(self):
         """G_r(u, rho) = reduce_matrix(get_stress_stiffness_matrix(rhoE, u)) (:220-255)."""
+        p = self.pattern
         sdet = D.empty(self.nelems, 4, 3)
         D.q4_stress(self.conn_d, self.xy_d, self.cmat6_d, self.kg_d, self.u_d, sdet)
         Gv = D.empty(self.nnz)
-        D.q4_assemble_geometric(self.conn_d, self.xy_d, sdet, self.src_ptr_d, self.src_d, self.nnz, Gv)
-        return D.CsrDevice(self.indptr_d, self.indices_d, Gv, (self.nred, self.nred))
+        D.q4_assemble_geometric(self.conn_d, self.xy_d, sdet, p.src_ptr_d, p.src_d, self.nnz, Gv)
+        return p.csr(Gv)
 
     def dK_single(self, psi_full, u_full):
         """psi^T (dK/drho_e) u per element for one pair of full vectors (:178-218 before the node scatter)."""
@@ -552,13 +484,11 @@ class BucklingQ4Problem(_BucklingProblem):
     # ---- sensitivities --------------------------------------------------------------------------------
     def sensitivity(self, which, Wr, Vr):
         """dGdu (full dof vector), dGdx or dKdx (per element) of sum_k w_k^T (.) v_k for reduced (n_r, N) W, V."""
-        W, V = self.full_vector(Wr), self.full_vector(Vr)
-        W2 = W if W.dim() == 2 else W.unsqueeze(1)
-        V2 = V if V.dim() == 2 else V.unsqueeze(1)
+        W2, V2 = _cols(self.full_vector(Wr)), _cols(self.full_vector(Vr))
         if which == "dGdu":
             due = D.empty(self.nelems, 8)
             D.q4_gderiv(self.conn_d, self.xy_d, self.cmat6_d, W2, V2, self.kg_d, self.dkg_d, self.u_d, 1.0, None, due)
-            return D.q4_dof_gather(self.nptr_d, self.nelem_d, self.nlocal_d, due, D.empty(self.ndof))
+            return D.dof_gather(self.nptr_d, self.nelem_d, self.nlocal_d, due, D.empty(self.ndof))
         out = D.zeros(self.nelems)
         if which == "dGdx":
             D.q4_gderiv(self.conn_d, self.xy_d, self.cmat6_d, W2, V2, self.kg_d, self.dkg_d, self.u_d, 1.0, out, None)
@@ -592,21 +522,11 @@ class BucklingH8Problem(_BucklingProblem):
         self.stress_d = D.empty(self.nelems, 8, 6)          # kg C B_q u_e at the 8 Gauss points of every element
 
     def _assemble(self, E1, c1):
-        vals = D.empty(self.nnz)
-        _lib.check(_lib.load().eigd_stored_assemble(self.nnz, _ptr(self.src_ptr_d), _ptr(self.src_d), H8Problem.NE, _ptr(E1),
-                                                    None, _ptr(c1), None, _ptr(vals), None, None, None, None, None),
-                   "stored_assemble")
-        return D.CsrDevice(self.indptr_d, self.indices_d, vals, (self.nred, self.nred))
+        p = self.pattern
+        return p.csr(D.stored_assemble(p.src_ptr_d, p.src_d, H8Problem.NE, E1, c1, D.empty(self.nnz)))
 
     def _quadform(self, dofmap, E1, c1, W, V):
-        W2, V2 = _cols(W), _cols(V)
-        if W2.shape != V2.shape:
-            raise ValueError("W and V must have the same shape")
-        out = D.zeros(self.nelems)
-        _lib.check(_lib.load().eigd_stored_quadform(self.nelems, H8Problem.NE, _ptr(dofmap), _ptr(E1), None, _ptr(c1), None,
-                                                    _ptr(W2), _ptr(V2), V2.shape[1], V2.stride(0), _ptr(out), None, None,
-                                                    None, 1.0, 0.0), "stored_quadform")
-        return out
+        return D.stored_quadform(dofmap, E1, c1, _cols(W), _cols(V), D.zeros(self.nelems))
 
     def assemble_K(self):
         """K_r(rho), gathered directly through the reduced source lists."""
@@ -629,7 +549,7 @@ class BucklingH8Problem(_BucklingProblem):
             W2, V2 = _cols(Wr), _cols(Vr)
             due = D.h8_gderiv_u(self.conn_d, self.X_d, self.E, self.nu, self.kg_d, self.dofmap_r_d, W2, V2,
                                 D.empty(self.nelems, H8Problem.NE))
-            return D.h8_dof_gather(self.nptr_d, self.nelem_d, self.nlocal_d, due, D.empty(self.ndof))
+            return D.dof_gather(self.nptr_d, self.nelem_d, self.nlocal_d, due, D.empty(self.ndof))
         if which == "dGdx":
             return self._quadform(self.dofmap_r_d, self.G0_d, self.dkg_d, Wr, Vr)
         return self._quadform(self.dofmap_r_d, self.base.K0_d, self.base.dk_d, Wr, Vr)
@@ -740,10 +660,7 @@ class NodeFilter:
         return rho
 
     def _project(self, rho, g=None):
-        out = D.empty(rho.shape[0])
-        _lib.check(_lib.load().eigd_filter_project(rho.shape[0], self.beta, self.eta, _ptr(rho), _ptr(g), _ptr(out)),
-                   "filter_project")
-        return out
+        return D.filter_project(rho, self.beta, self.eta, g)
 
     def apply_tangent(self, x, xt):
         """Directional derivative of ``apply`` at x along xt (dual-number mode of the drivers)."""

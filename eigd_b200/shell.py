@@ -22,11 +22,9 @@ sensitivities w^T (dK/dt_c) v per component with one warp per element and a warp
 import numpy as np
 import torch
 
-from . import _lib
 from . import device as D
 from . import fe
 from ._hostdev import to_dev, to_host, small_to_dev
-from .device import _ptr
 from .eigenvector_derivatives import SpLuOperator, add_eig_total_derivative
 from .topo import _EigenAnalysis, _now
 
@@ -141,11 +139,10 @@ class ShellProblem:
         self.reduced = (self.free_nodes[:, None] * 6 + np.arange(6)[None, :]).ravel()     # crm.py self.dof
         self.ndof = len(self.reduced)
         var = fe.element_dofs(self.conn, 6)                                          # (nelems, 24) full dofs
-        indptr, indices, src_ptr, src = fe.assembly_structure(var, self.ndof_full)
-        self.indptr, self.indices, r_src_ptr, r_src = fe.reduced_structure(indptr, indices, src_ptr, src, self.reduced,
-                                                                           self.ndof_full)
-        del indptr, indices, src_ptr, src
-        self.nnz = len(self.indices)
+        # only the reduced pattern goes to HBM: the full one is reduced on the host
+        self.pattern = fe.AssemblyPattern(*fe.reduced_structure(*fe.assembly_structure(var, self.ndof_full), self.reduced,
+                                                                self.ndof_full))
+        self.indptr, self.indices, self.nnz = self.pattern.indptr, self.pattern.indices, self.pattern.nnz
         f2r = np.full(self.ndof_full, -1, dtype=np.int64)
         f2r[self.reduced] = np.arange(self.ndof)
         self.dofmap = f2r[var].astype(np.int32)                                      # -1 = clamped
@@ -155,10 +152,6 @@ class ShellProblem:
         self.E1_d, self.E3_d = to_dev(E1.reshape(-1)), to_dev(E3.reshape(-1))
         self.F1_d, self.F3_d = to_dev(F1.reshape(-1)), to_dev(F3.reshape(-1))
         del E1, E3, F1, F3
-        self.indptr_d = torch.as_tensor(self.indptr, device=dev)
-        self.indices_d = torch.as_tensor(self.indices, device=dev)
-        self.src_ptr_d = torch.as_tensor(r_src_ptr, device=dev)
-        self.src_d = torch.as_tensor(r_src, device=dev)
         self.dofmap_d = torch.as_tensor(self.dofmap, device=dev)
         # elements sorted by component: segments of the per-component reduction
         order = np.argsort(self.comp, kind="stable")
@@ -185,29 +178,18 @@ class ShellProblem:
 
     def assemble(self):
         """K(t), M(t) as CsrDevice sharing one pattern (reduced system)."""
+        p = self.pattern
         Kv, Mv = D.empty(self.nnz), D.empty(self.nnz)
-        _lib.check(_lib.load().eigd_stored_assemble(self.nnz, _ptr(self.src_ptr_d), _ptr(self.src_d), self.NE, _ptr(self.E1_d),
-                                                    _ptr(self.E3_d), _ptr(self.t_d), _ptr(self.t3_d), _ptr(Kv), _ptr(self.F1_d),
-                                                    _ptr(self.F3_d), _ptr(self.t_d), _ptr(self.t3_d), _ptr(Mv)), "stored_assemble")
-        shape = (self.ndof, self.ndof)
-        return (D.CsrDevice(self.indptr_d, self.indices_d, Kv, shape), D.CsrDevice(self.indptr_d, self.indices_d, Mv, shape))
+        D.stored_assemble(p.src_ptr_d, p.src_d, self.NE, self.E1_d, self.t_d, Kv, E3=self.E3_d, c3=self.t3_d, F1=self.F1_d,
+                          d1=self.t_d, vals2=Mv, F3=self.F3_d, d3=self.t3_d)
+        return p.csr(Kv), p.csr(Mv)
 
     def _sensitivity(self, which, W, V):
         """d/dx_c of W^T A(x) V summed over the columns: (ncomp,) device vector."""
-        W2 = W if W.dim() == 2 else W.unsqueeze(1)
-        V2 = V if V.dim() == 2 else V.unsqueeze(1)
-        W2 = W2 if W2.is_contiguous() else W2.contiguous()
-        V2 = V2 if V2.is_contiguous() else V2.contiguous()
         U1, U3 = (self.E1_d, self.E3_d) if which == "A" else (self.F1_d, self.F3_d)
-        oute = D.empty(self.nelems)
-        _lib.check(_lib.load().eigd_stored_quadform(self.nelems, self.NE, _ptr(self.dofmap_d), _ptr(U1), _ptr(U3), _ptr(self.one_d),
-                                                    _ptr(self.dt3_d), _ptr(W2), _ptr(V2), V2.shape[1], V2.stride(0), _ptr(oute),
-                                                    None, None, None, 1.0, 1.0),
-                   "stored_quadform")
-        out = D.empty(self.ncomp)
-        _lib.check(_lib.load().eigd_segment_sum(self.ncomp, _ptr(self.seg_ptr_d), _ptr(self.perm_d), _ptr(oute), 1.0 / self.scale,
-                                                _ptr(out)), "segment_sum")
-        return out
+        oute = D.stored_quadform(self.dofmap_d, U1, self.one_d, fe._cols(W), fe._cols(V), D.empty(self.nelems), E3=U3,
+                                 c3=self.dt3_d)
+        return D.segment_sum(self.seg_ptr_d, self.perm_d, oute, 1.0 / self.scale, D.empty(self.ncomp))
 
 
 class ShellModalAnalysis(_EigenAnalysis):

@@ -258,6 +258,11 @@ int eigd_h8_element_matrices(int nelems, const int* d_conn, const double* d_X, d
                              double* d_K0, double* d_M0);
 /* node_out[v] = scale * sum_{e in adj(v)} e_vals[e]   (gather form of np.add.at, thermal.py:612-615) */
 int eigd_node_gather(int nnodes, const int* d_nptr, const int* d_nelem, const double* d_evals, double scale, double* d_out);
+/* out[ncomp v + i] = sum_{e around v} due[e][ncomp local + i], due (nelems, npe * ncomp), local = d_nlocal (the node's
+ * index inside each adjacent element): the dof scatter np.add.at of examples/buckling.py:318-320 in gather form, for
+ * the element terms of eigd_q4_gderiv (ncomp 2, npe 4) and eigd_h8_gderiv_u (ncomp 3, npe 8) */
+int eigd_dof_gather(int nnodes, int ncomp, int npe, const int* d_nptr, const int* d_nelem, const int* d_nlocal,
+                    const double* d_due, double* d_out);
 
 /* tanh projection of the filtered density (examples/node_filter.py:174-181) and its gradient factor (:193-203):
  * d_g == NULL: out = projected rho; otherwise out = g * d(projection)/d(rho) evaluated at the UNPROJECTED rho */
@@ -278,9 +283,6 @@ int eigd_q4_assemble_geometric(int nelems, const int* d_conn, const double* d_xy
 int eigd_q4_gderiv(int nelems, const int* d_conn, const double* d_xy, const double* d_cmat6, const double* d_W,
                    const double* d_V, int N, int ldw, const double* d_ks, const double* d_dks, const double* d_u,
                    double sx, double* d_out_rho, double* d_due);
-/* dfdu[2v + d] = sum_{e around v} due[e][2 local + d] (gather form of np.add.at, :318-320) */
-int eigd_q4_dof_gather(int nnodes, const int* d_nptr, const int* d_nelem, const int* d_nlocal, const double* d_due,
-                       double* d_out);
 /* ---- linearised buckling of the 3-D solid (csrc/h8_buckling.cu), H8 elements as eigd_h8_element_matrices.
  *      dofmap (nelems, 24): element dof (node-major u_x, u_y, u_z) -> row of u, W and V; -1 = constrained (zero).
  *      Voigt order (xx, yy, zz, yz, xz, xy), engineering shear; C = C(E, nu) of K0. ---- */
@@ -292,9 +294,6 @@ int eigd_h8_stress_stiffness(int nelems, const int* d_conn, const double* d_X, d
  * products: d/du_e of sum_k w_k^T G(u) v_k.  W, V row-major with leading dimension ld, N columns. */
 int eigd_h8_gderiv_u(int nelems, const int* d_conn, const double* d_X, double E, double nu, const double* d_kg,
                      const int* d_dofmap, const double* d_W, const double* d_V, int N, int64_t ld, double* d_due);
-/* out[3v + i] = sum_{e around v} due[e][3 local + i] (gather form, as eigd_q4_dof_gather) */
-int eigd_h8_dof_gather(int nnodes, const int* d_nptr, const int* d_nelem, const int* d_nlocal, const double* d_due,
-                       double* d_out);
 /* full[idx[i], :] = red[i, :] and red[i, :] = full[idx[i], :], k columns, row-major */
 int eigd_expand_rows(int64_t nr, int k, const int* d_idx, const double* d_red, double* d_full);
 int eigd_reduce_rows(int64_t nr, int k, const int* d_idx, const double* d_full, double* d_red);

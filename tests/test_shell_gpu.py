@@ -59,6 +59,18 @@ def test_shell_assembly_and_sensitivities_vs_oracle(setup):
     assert rel(tens, sum(orc.dK(g["x"], W[:, k], V[:, k]) for k in range(5))) < 1e-12
 
 
+def test_shell_sensitivity_rejects_mismatched_columns(setup):
+    """W and V with different column counts are refused: the kernel reads W with V's leading dimension."""
+    from eigd_b200 import device as D
+    g, model, orc = setup
+    p = model.prob
+    p.set_design(g["x"])
+    rng = np.random.default_rng(1)
+    W, V = D.to_device(rng.normal(size=(p.ndof, 6))), D.to_device(rng.normal(size=(p.ndof, 5)))
+    with pytest.raises(ValueError):
+        p.dAdx.device_call(W, V)
+
+
 def test_shell_driver_vs_reference_solvers(setup):
     g, model, orc = setup
     model.set_design_vars(g["x"])
