@@ -5,7 +5,13 @@
 //   K0_e = sum_q detJ B^T C B                      (isotropic elasticity, E and nu)
 //   M0_e = density sum_q detJ (N N^T (x) I_3)      (consistent mass)
 //
-// dof order node-major (u_x, u_y, u_z), as fe.element_dofs(conn, 3).  Element: h8_element.cuh.
+// dof order node-major (u_x, u_y, u_z), as fe.element_dofs(conn, 3).  The scalar (heat conduction) element has one
+// dof per node and the 8 x 8 unit matrices
+//
+//   K0_e = sum_q detJ grad N_a . grad N_b          (conductivity 1)
+//   M0_e = sum_q detJ N_a N_b                      (heat capacity 1: the scalar block of the solid's M0 at density 1)
+//
+// Element: h8_element.cuh.
 #include "common.cuh"
 #include "h8_element.cuh"
 #include "../../include/eigd_b200.h"
@@ -64,6 +70,45 @@ h8_element_matrices_kernel(int nelems, const int* __restrict__ conn, const doubl
   }
 }
 
+// Four elements per warp: lane l is node a = l & 7 of element 4 warp + l / 8 and owns column a of both matrices; the
+// values of node an of the same element come from lane an of its 8-lane group.  The shuffles run on the full mask, so
+// the lanes past the last element work on element nelems - 1 and skip the store.  M0 accumulates in the order of mc in
+// h8_element_matrices_kernel (Gauss points 0..7, one fma each), so it equals the scalar block of the solid's M0 at
+// density 1 bit for bit.  Row r of an element is written by its 8 lanes at once (64 contiguous bytes).
+__global__ void __launch_bounds__(256)
+h8_thermal_element_matrices_kernel(int nelems, const int* __restrict__ conn, const double* __restrict__ X,
+                                   double* __restrict__ K0, double* __restrict__ M0) {
+  const int64_t eg = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 3;
+  const bool store = eg < nelems;
+  const int64_t e = store ? eg : nelems - 1;
+  const int a = threadIdx.x & 7;
+  const H8Node nd = h8_gather(conn, X, e, a);
+  double kc[8], mc[8];
+#pragma unroll
+  for (int i = 0; i < 8; ++i) kc[i] = mc[i] = 0.0;
+#pragma unroll 1
+  for (int q = 0; q < 8; ++q) {
+    double N, Nx, Ny, Nz;
+    const double det = h8_point(nd, a, q, N, Nx, Ny, Nz);
+#pragma unroll
+    for (int an = 0; an < 8; ++an) {
+      const double na = __shfl_sync(0xffffffffu, N, an, 8), nxa = __shfl_sync(0xffffffffu, Nx, an, 8);
+      const double nya = __shfl_sync(0xffffffffu, Ny, an, 8), nza = __shfl_sync(0xffffffffu, Nz, an, 8);
+      const double t = fma(nza, Nz, fma(nya, Ny, nxa * Nx));
+      kc[an] = fma(det, t, kc[an]);
+      mc[an] = fma(det, na * N, mc[an]);
+    }
+  }
+  if (!store) return;
+  double* k = K0 + e * 64 + a;
+  double* m = M0 + e * 64 + a;
+#pragma unroll
+  for (int r = 0; r < 8; ++r) {
+    k[r * 8] = kc[r];
+    m[r * 8] = mc[r];
+  }
+}
+
 }  // namespace
 
 extern "C" int eigd_h8_element_matrices(int nelems, const int* d_conn, const double* d_X, double E, double nu, double density,
@@ -73,6 +118,14 @@ extern "C" int eigd_h8_element_matrices(int nelems, const int* d_conn, const dou
   if (!h8_isotropic(E, nu, c, "h8_element_matrices")) return 1;
   const int grid = (int)(((int64_t)nelems * 32 + 255) / 256);
   EIGD_LAUNCH(h8_element_matrices_kernel, grid, 256, 0, nelems, d_conn, d_X, c, density, d_K0, d_M0);
+  EIGD_CHECK_LAUNCH();
+  return 0;
+}
+
+extern "C" int eigd_h8_thermal_element_matrices(int nelems, const int* d_conn, const double* d_X, double* d_K0, double* d_M0) {
+  if (nelems <= 0) return 0;
+  const int grid = (int)(((int64_t)nelems * 8 + 255) / 256);
+  EIGD_LAUNCH(h8_thermal_element_matrices_kernel, grid, 256, 0, nelems, d_conn, d_X, d_K0, d_M0);
   EIGD_CHECK_LAUNCH();
   return 0;
 }

@@ -859,6 +859,12 @@ def h8_element_matrices(conn, X, E, nu, density, K0, M0):
                                                _ptr(K0), _ptr(M0)), "h8_element_matrices")
 
 
+def h8_thermal_element_matrices(conn, X, K0, M0):
+    """Unit conductivity and capacity matrices K0, M0 (nelems * 64 each) of the scalar H8 elements ``conn`` (nelems, 8)."""
+    check(_lib.load().eigd_h8_thermal_element_matrices(conn.shape[0], _ptr(conn), _ptr(X), _ptr(K0), _ptr(M0)),
+          "h8_thermal_element_matrices")
+
+
 def stored_assemble(src_ptr, src, ne, E1, c1, vals, E3=None, c3=None, F1=None, d1=None, vals2=None, F3=None, d3=None):
     """vals = CSR values of the elements c1[e] E1_e (+ c3[e] E3_e) through the (element, a, b) source lists; with
     ``vals2``, the second matrix d1[e] F1_e (+ d3[e] F3_e) on the same pattern in the same pass."""

@@ -1,4 +1,5 @@
-"""Device-side finite-element operators for the Q4 problems of the reference examples and the H8 solid.
+"""Device-side finite-element operators for the Q4 problems of the reference examples, the H8 solid and H8 heat
+conduction.
 
 Host part (numpy, runs once per mesh): mesh numbering, DOF maps, the CSR pattern of K/M and the
 integer assembly maps (element, a, b) -> CSR non-zero, node -> element adjacency, the conic
@@ -285,29 +286,23 @@ class Q4Problem(_ElementModel):
         return out
 
 
-class H8Problem(_ElementModel):
-    """Free 3-D isotropic solid on trilinear hexahedra (3 DOF/node) with its operators in HBM.
+class _StoredMatrixModel(_ElementModel):
+    """Element models whose unit element matrices are computed once per mesh and stay resident: ``K0_d``, ``M0_d``
+    (nelems * NE * NE each, row-major) and the element dof map ``dofmap_d`` (nelems, NE).  Per design, assembly and
+    the sensitivities are the stored-matrix kernels (eigd_stored_assemble, eigd_stored_quadform)."""
 
-    K_e = s(rho_e) K0_e, M_e = rho_e M0_e with s = rho^p + rho0_K (SIMP) or rho/(1+q(1-rho)) + rho0_K (RAMP), the laws
-    of the plane-stress ``Q4Problem``; rho_e is the mean of the 8 nodal densities.  The unit matrices
-    K0_e = sum_q detJ B^T C B and M0_e = density sum_q detJ (N N^T (x) I_3) (2x2x2 Gauss) are computed once per mesh on
-    the device (eigd_h8_element_matrices, 9.2 KB per element) and stay resident; per design, assembly and the
-    sensitivities are the stored-matrix kernels (eigd_stored_assemble, eigd_stored_quadform)."""
-
-    npe = 8
-    NE = 24
-
-    def __init__(self, conn, X, E=1.0, nu=0.3, density=1.0, p=3.0, rho0_K=1e-6, ptype_K="simp", q=5.0):
+    def _setup_hex(self, conn, X, dof, law, par):
+        """``_setup`` on a hexahedral mesh, conn (nelems, 8) and X (nnodes, 3) (ValueError otherwise), the element dof
+        map and room for K0, M0, which the subclass's element kernel fills."""
         conn = np.asarray(conn, dtype=np.int64)
         X = np.asarray(X, dtype=np.float64)
         if conn.ndim != 2 or conn.shape[1] != 8 or X.ndim != 2 or X.shape[1] != 3:
-            raise ValueError("H8Problem needs conn (nelems, 8) and X (nnodes, 3)")
-        self._setup(conn, X, X.shape[0], 3, *_penalty_law("ptype_K", ptype_K, p, q, 1.0, rho0_K))
+            raise ValueError("%s needs conn (nelems, 8) and X (nnodes, 3)" % type(self).__name__)
+        self._setup(conn, X, X.shape[0], dof, law, par)
         self.X_d = to_dev(np.ascontiguousarray(self.X))
         self.dofmap_d = torch.as_tensor(self.var.astype(np.int32), device=D.dev())
         ne2 = self.NE * self.NE
         self.K0_d, self.M0_d = D.empty(self.nelems * ne2), D.empty(self.nelems * ne2)
-        D.h8_element_matrices(self.conn_d, self.X_d, E, nu, density, self.K0_d, self.M0_d)
 
     def _assemble_values(self, ck, cm):
         p = self.pattern
@@ -330,6 +325,40 @@ class H8Problem(_ElementModel):
             if s1 != 1.0:
                 out.mul_(s1)
         return out
+
+
+class H8Problem(_StoredMatrixModel):
+    """Free 3-D isotropic solid on trilinear hexahedra (3 DOF/node) with its operators in HBM.
+
+    K_e = s(rho_e) K0_e, M_e = rho_e M0_e with s = rho^p + rho0_K (SIMP) or rho/(1+q(1-rho)) + rho0_K (RAMP), the laws
+    of the plane-stress ``Q4Problem``; rho_e is the mean of the 8 nodal densities.  The unit matrices
+    K0_e = sum_q detJ B^T C B and M0_e = density sum_q detJ (N N^T (x) I_3) (2x2x2 Gauss) are computed once per mesh on
+    the device (eigd_h8_element_matrices, 9.2 KB per element) and stay resident; per design, assembly and the
+    sensitivities are the stored-matrix kernels (eigd_stored_assemble, eigd_stored_quadform)."""
+
+    npe = 8
+    NE = 24
+
+    def __init__(self, conn, X, E=1.0, nu=0.3, density=1.0, p=3.0, rho0_K=1e-6, ptype_K="simp", q=5.0):
+        self._setup_hex(conn, X, 3, *_penalty_law("ptype_K", ptype_K, p, q, 1.0, rho0_K))
+        D.h8_element_matrices(self.conn_d, self.X_d, E, nu, density, self.K0_d, self.M0_d)
+
+
+class H8ThermalProblem(_StoredMatrixModel):
+    """Heat conduction on trilinear hexahedra (1 DOF/node), the 3-D counterpart of ``Q4Problem(kind="thermal")``.
+
+    K_e = kappa(rho_e) K0_e, M_e = c(rho_e) M0_e with the thermal law of ``Q4Problem``: kappa = kappa0((1-beta) rho^p
+    + beta), c = heat_capacity * density * ((1-beta) rho + beta); rho_e is the mean of the 8 nodal densities.  The unit
+    matrices K0_e = sum_q detJ grad N grad N^T and M0_e = sum_q detJ N N^T (2x2x2 Gauss) are computed once per mesh on
+    the device (eigd_h8_thermal_element_matrices, 1 KB per element for the pair) and stay resident; per design, assembly
+    and the sensitivities are the stored-matrix kernels, as for ``H8Problem``."""
+
+    npe = 8
+    NE = 8
+
+    def __init__(self, conn, X, kappa=1.0, density=1.0, heat_capacity=1.0, p=3.0, beta=1e-6):
+        self._setup_hex(conn, X, 1, 0, np.array([p, kappa, heat_capacity * density, beta]))
+        D.h8_thermal_element_matrices(self.conn_d, self.X_d, self.K0_d, self.M0_d)
 
 
 def reduced_structure(indptr, indices, src_ptr, src, reduced, ndof):
@@ -567,7 +596,9 @@ class NodeFilter:
     """Conic node filter F[i, j] ~ max(0, r0 - |X_i - X_j|), rows normalised to 1
     (examples/node_filter.py:61-88), applied on the device as CSR products (:164-217).
     Spatial filter with optional design-variable map (the symmetric column of examples/buckling.py:1331-1344)
-    and optional tanh projection (``projection=True``, ``beta``, ``eta``)."""
+    and optional tanh projection (``projection=True``, ``beta``, ``eta``).  ``ftype="helmholtz"`` is the PDE filter
+    (``_init_helmholtz``) on a Q4 mesh (2-D coordinates) or a hexahedral mesh (3-D coordinates); in 3-D it replaces the
+    conic filter's pair search and its two CSR operators by one scalar LDL^T of the mesh, factored once."""
 
     ftype = "spatial"
 
@@ -586,9 +617,6 @@ class NodeFilter:
         self.dvmap = None if dvmap is None else np.asarray(dvmap, dtype=np.int64)
         self.offset_d = None
         if ftype == "helmholtz":
-            if self.X.shape[1] != 2:
-                raise ValueError("the Helmholtz filter is built on the Q4 mesh; it is not available for %d-D coordinates"
-                                 % self.X.shape[1])
             self._init_helmholtz(conn, r0, num_design_vars)
             return
         tree = spatial.cKDTree(self.X)
@@ -622,16 +650,29 @@ class NodeFilter:
 
     def _init_helmholtz(self, conn, r0, num_design_vars):
         """Helmholtz (PDE) filter of examples/node_filter.py:90-162: rho = A^-1 (B x) with A = r0^2 int grad N . grad N +
-        int N N and B = int N N on the Q4 mesh.  A and B are the unit-material thermal stiffness / capacity matrices of
-        ``Q4Problem`` (assembled by the same gather kernel), A is factored once by the GPU LDL^T (the reference uses
-        scipy's ``factorized``) and applied to one right-hand side per call."""
+        int N N and B = int N N on the element mesh: Q4 for 2-D coordinates with 4-node ``conn``, trilinear hexahedra for
+        3-D coordinates with 8-node ``conn``.  A and B are the unit-material conductivity / capacity matrices of
+        ``Q4Problem(kind="thermal")`` or ``H8ThermalProblem`` (assembled by the same kernels), A is factored once by the
+        GPU LDL^T (the reference uses scipy's ``factorized``) and applied to one right-hand side per call."""
         from .eigenvector_derivatives import SpLuOperator
-        prob = Q4Problem(conn, self.X, "thermal", kappa=1.0, density=1.0, heat_capacity=1.0, p=1.0, beta=0.0)
+        conn = np.asarray(conn, dtype=np.int64)
+        dim, npe = self.X.shape[1] if self.X.ndim == 2 else 0, conn.shape[1] if conn.ndim == 2 else 0
+        fronts = "resident"
+        if (dim, npe) == (2, 4):
+            prob = Q4Problem(conn, self.X, "thermal", kappa=1.0, density=1.0, heat_capacity=1.0, p=1.0, beta=0.0)
+        elif (dim, npe) == (3, 8):
+            prob = H8ThermalProblem(conn, self.X, p=1.0, beta=0.0)
+            # A is factored once and only solved with afterwards, so a pooled factor keeps no dense fronts for the
+            # filter's life (17 GB at 80 x 64 x 48 hexahedra); it is bitwise the resident factor.
+            fronts = "pooled"
+        else:
+            raise ValueError("the Helmholtz filter needs 2-D coordinates with 4-node (Q4) conn or 3-D coordinates with "
+                             "8-node (H8) conn; got %d-D coordinates with %d-node conn" % (dim, npe))
         prob.set_density(rhoE=np.ones(prob.nelems))
         K, M = prob.assemble()
         self._hB = M
         vals = D.axpby(float(r0) ** 2, K.data, 1.0, M.data)
-        self._hA = SpLuOperator(K.with_values(vals), coords=self.X, dof_per_node=1, max_rhs=1)
+        self._hA = SpLuOperator(K.with_values(vals), coords=self.X, dof_per_node=1, max_rhs=1, fronts=fronts)
         self._hprob = prob
         if self.dvmap is None:
             self.num_design_vars = self.nnodes

@@ -256,6 +256,10 @@ int eigd_q4_material(int law, int nelems, int npe, const int* d_conn, const doub
  *      K0_e = sum_q detJ B^T C(E, nu) B, M0_e = density sum_q detJ (N N^T (x) I_3). */
 int eigd_h8_element_matrices(int nelems, const int* d_conn, const double* d_X, double E, double nu, double density,
                              double* d_K0, double* d_M0);
+/* Scalar (heat conduction) H8, one dof per node in node order (fe.element_dofs(conn, 1)), same element and rule:
+ * K0, M0 (nelems, 8, 8) row-major, K0_e = sum_q detJ grad N_a . grad N_b, M0_e = sum_q detJ N_a N_b (unit material;
+ * M0 is bitwise the scalar block of eigd_h8_element_matrices' M0 at density 1). */
+int eigd_h8_thermal_element_matrices(int nelems, const int* d_conn, const double* d_X, double* d_K0, double* d_M0);
 /* node_out[v] = scale * sum_{e in adj(v)} e_vals[e]   (gather form of np.add.at, thermal.py:612-615) */
 int eigd_node_gather(int nnodes, const int* d_nptr, const int* d_nelem, const double* d_evals, double scale, double* d_out);
 /* out[ncomp v + i] = sum_{e around v} due[e][ncomp local + i], due (nelems, npe * ncomp), local = d_nlocal (the node's

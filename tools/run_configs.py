@@ -5,9 +5,12 @@
     python tools/run_configs.py c4 [--nx 408 --ny 408 --modes 20 --fd]   1M-DOF synthetic shell (6 dof/node), crm.py driver
     python tools/run_configs.py h8 [--nx 64 --ny 32 --nz 32 --modes 10 --fd]   free 3-D solid of hexahedra (3 dof/node)
     python tools/run_configs.py h8buck [--nx 32 --ny 24 --nz 128 --modes 10 --fd]   buckling of a clamped 3-D column
+    python tools/run_configs.py h8thermal [--nx 80 --ny 64 --nz 48 --modes 10 --ftype spatial|helmholtz --fd]
+                                                                       heat conduction in an insulated 3-D box (1 dof/node)
 
-h8 and h8buck take --fronts resident|pooled (the front memory of the factors) and report, for either mode, the pool
-size, the persistent bytes of the factors, torch's peak allocated device memory and the factorisation time.
+h8, h8buck and h8thermal take --fronts resident|pooled (the front memory of the factors) and report, for either mode,
+the pool size, the persistent bytes of the factors, torch's peak allocated device memory and the factorisation time.
+h8thermal also reports the set-up time, device memory and per-design time (apply + apply_gradient) of its filter.
 
 Each prints one JSON line: stage times (CUDA-synchronised wall clock of the driver's own timers, as the
 reference examples report them), solve counts, factor statistics, and size-independent acceptance checks
@@ -377,6 +380,100 @@ def run_h8buck(args):
     return out
 
 
+def run_h8thermal(args):
+    """Insulated nx x ny x nz box of hexahedra (ThermalTopology3DAnalysis; mesh, filter radius and driver of
+    make_thermal_3d_model, built step by step so that the filter is timed alone): N modes about sigma = -0.1, mode 0
+    the zero mode, IRAM + sibk with the Lanczos guess, tensor derivative, thermal compliance against the seeded uniform
+    heat vector of bench.py as the objective, conic or Helmholtz filter (--ftype)."""
+    import torch
+    from eigd_b200 import device as D, fe, topo as T
+    D.init()
+    Lx, Ly, Lz = 1.0, 0.8, 0.6
+    out = {"config": "H8 thermal box nx=%d ny=%d nz=%d" % (args.nx, args.ny, args.nz), "N": args.modes,
+           "ftype": args.ftype, "gpu": gpu_card()}
+    t0 = time.perf_counter()
+    conn, X = fe.hex_mesh(args.nx, args.ny, args.nz, Lx, Ly, Lz)
+    t_mesh = time.perf_counter() - t0
+    m0 = torch.cuda.memory_allocated()
+    t0 = now()
+    fltr = fe.NodeFilter(conn, X, r0=4.0 * Ly / args.ny, ftype=args.ftype)
+    filt = {"host_setup_s": now() - t0, "device_bytes": int(torch.cuda.memory_allocated() - m0)}
+    if args.ftype == "spatial":
+        filt["nnz_F"] = int(fltr.F.nnz)
+    else:
+        filt.update(factor_bytes=fltr._hA.lu.nbytes(), pool_bytes=fltr._hA.lu.pool_bytes(),
+                    symbolic=fltr._hA.lu.sym.stats())
+    t0 = now()
+    model = T.ThermalTopology3DAnalysis(fltr, conn, X, N=args.modes, m=60, sigma=-0.1, solver_type="IRAM",
+                                        adjoint_method="sibk", adjoint_options={"lanczos_guess": True}, rtol=1e-10,
+                                        deriv_type="tensor", fronts=args.fronts)
+    out.update(n=int(model.nvars), nnz=int(model.prob.nnz), fronts=args.fronts, mesh_s=t_mesh,
+               host_setup_s=now() - t0, filter=filt)
+    torch.cuda.reset_peak_memory_stats()
+    x0 = np.random.default_rng(0).uniform(0.3, 1.0, model.fltr.num_design_vars)     # bench.py X_SEED, VEC_SEED
+    vec_d = D.to_device(np.random.default_rng(12345).uniform(size=model.nnodes))
+    reps = []
+    for rep in range(args.reps):
+        l0 = D.launch_count()
+        ta = now()
+        with warnings.catch_warnings():
+            warnings.simplefilter("ignore")
+            model.initialize(x=x0)
+        model.initialize_adjoint()
+        model.add_thermal_compliance_derivative(1.0, vec_d)
+        model.finalize_adjoint()
+        tb = now()
+        p = model.profile
+        reps.append({"wall_s": tb - ta, "assembly_s": p["matrix assembly time"], "eig_s": p["eigenvalue solve time"],
+                     "adjoint_s": p["adjoint solution time"], "dfdx_s": p["total derivative time"],
+                     "time_to_gradient_s": model.time_to_gradient(), "eig_solves": p["solve preconditioner count"],
+                     "adjoint_solves": p["adjoint preconditioner count"], "launches": D.launch_count() - l0,
+                     "symbolic_s": p.get("symbolic analysis time")})
+    out["reps"] = reps
+    out["peak_device_bytes"] = int(torch.cuda.max_memory_allocated())
+    out["factorisation_s"] = _time_factorisation(model)
+    out["memory"] = _factor_memory(model, [model.factor])
+    x_d, g_d = D.to_device(x0), D.to_device(np.random.default_rng(2).normal(size=model.nnodes))
+    filt["apply_plus_gradient_s"] = []
+    for _ in range(5):
+        t0 = now()
+        fltr.apply(x_d)
+        fltr.apply_gradient(g_d, x_d)
+        filt["apply_plus_gradient_s"].append(now() - t0)
+    out["lam_first"] = [float(v) for v in model.lam[:4]]
+    out["factor_info"] = model.factor.info
+    out["symbolic"] = model.symbolic[0].stats()
+    # nonzero modes only: mode 0 has lambda = 0 (the constant temperature), its relative residual is 0/0
+    res, _ = residuals(model, model.K, model.M, model.lam[1:], model.Q[:, 1:].contiguous(), "normal")
+    _, orth = residuals(model, model.K, model.M, model.lam, model.Q.contiguous(), "normal")
+    out["eigen_residual_max"] = res
+    out["orthonormality_defect"] = orth
+    ar, ao = model.eig_solver.eval_adjoint_residual_norm(model.Q0b, model.psi0, b_ortho=True)
+    rhs = float(model.Q0b.norm(dim=0).max().item())
+    out["adjoint_residual_over_rtol_rhs"] = float(np.max(ar)) / (1e-10 * rhs)
+    assert out["adjoint_residual_over_rtol_rhs"] < 50.0 and orth < 1e-10, (out["adjoint_residual_over_rtol_rhs"], orth)
+    assert res < 1e-8, res
+    out["objective"] = model.get_thermal_compliance(vec_d)
+    xb = model.xb.cpu().numpy().copy()
+    out["xb_norm"] = float(np.linalg.norm(xb))
+    if args.fd:
+        pert = np.random.default_rng(3).uniform(-1.0, 1.0, x0.shape)
+        h = 1e-5
+        vals = []
+        for sgn in (1.0, -1.0):
+            with warnings.catch_warnings():
+                warnings.simplefilter("ignore")
+                model.initialize(x=x0 + sgn * h * pert)
+            vals.append(model.get_thermal_compliance(vec_d))
+        fd = (vals[0] - vals[1]) / (2 * h)
+        out["fd_directional"] = fd
+        out["adjoint_directional"] = float(xb @ pert)
+        out["fd_rel_err"] = abs(fd - float(xb @ pert)) / abs(fd)
+        out["peak_device_bytes_with_fd"] = int(torch.cuda.max_memory_allocated())
+    out["gpu_after"] = gpu_card()
+    return out
+
+
 def _factor_memory(model, ops):
     """Front memory of the driver's factors: the pool a pooled factorisation borrows (0 resident), the resident fronts
     of one factor, and the bytes every factor keeps for its life (its workspace: fronts included when resident)."""
@@ -410,15 +507,17 @@ def _time_factorisation(model, reps=3):
 
 if __name__ == "__main__":
     ap = argparse.ArgumentParser()
-    ap.add_argument("config", choices=["c3", "c4", "c4plate", "c5", "h8", "h8buck"])
+    ap.add_argument("config", choices=["c3", "c4", "c4plate", "c5", "h8", "h8buck", "h8thermal"])
     ap.add_argument("--fd", action="store_true", help="c4: add the finite-difference check of the gradient")
     ap.add_argument("--nx", type=int, default=None)
     ap.add_argument("--ny", type=int, default=None)
-    ap.add_argument("--nz", type=int, default=None, help="h8, h8buck: elements along z")
+    ap.add_argument("--nz", type=int, default=None, help="h8, h8buck, h8thermal: elements along z")
     ap.add_argument("--modes", type=int, default=None)
     ap.add_argument("--designs", type=int, default=None)
     ap.add_argument("--reps", type=int, default=3)
-    ap.add_argument("--fronts", choices=["resident", "pooled"], default="resident", help="h8, h8buck: front memory of the factors")
+    ap.add_argument("--fronts", choices=["resident", "pooled"], default="resident",
+                    help="h8, h8buck, h8thermal: front memory of the factors")
+    ap.add_argument("--ftype", choices=["spatial", "helmholtz"], default="spatial", help="h8thermal: filter type")
     a = ap.parse_args()
     if a.config == "c3":
         a.nx, a.ny, a.modes = a.nx or 352, a.ny or 704, a.modes or 20
@@ -432,6 +531,9 @@ if __name__ == "__main__":
     elif a.config == "h8buck":
         a.nx, a.ny, a.nz, a.modes = a.nx or 32, a.ny or 24, a.nz or 128, a.modes or 10
         res = run_h8buck(a)
+    elif a.config == "h8thermal":
+        a.nx, a.ny, a.nz, a.modes = a.nx or 80, a.ny or 64, a.nz or 48, a.modes or 10
+        res = run_h8thermal(a)
     elif a.config == "c4":
         a.nx, a.ny, a.modes = a.nx or 408, a.ny or 408, a.modes or 20
         res = run_c4(a)
