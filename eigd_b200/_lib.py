@@ -74,6 +74,8 @@ SIGNATURES = {
     "eigd_q4_material": (c_int, [c_int, c_int, c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr]),
     "eigd_h8_element_matrices": (c_int, [c_int, c_ptr, c_ptr, c_dbl, c_dbl, c_dbl, c_ptr, c_ptr]),
     "eigd_h8_thermal_element_matrices": (c_int, [c_int, c_ptr, c_ptr, c_ptr, c_ptr]),
+    "eigd_t10_element_matrices": (c_int, [c_int, c_ptr, c_ptr, c_dbl, c_dbl, c_dbl, c_ptr, c_ptr]),
+    "eigd_t10_thermal_element_matrices": (c_int, [c_int, c_ptr, c_ptr, c_ptr, c_ptr]),
     "eigd_h8_stress_stiffness": (c_int, [c_int, c_ptr, c_ptr, c_dbl, c_dbl, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr]),
     "eigd_h8_gderiv_u": (c_int, [c_int, c_ptr, c_ptr, c_dbl, c_dbl, c_ptr, c_ptr, c_ptr, c_ptr, c_int, c_i64, c_ptr]),
     "eigd_node_gather": (c_int, [c_int, c_ptr, c_ptr, c_ptr, c_dbl, c_ptr]),

@@ -246,7 +246,7 @@ extern "C" int eigd_filter_project(int n, double beta, double eta, const double*
 
 // ---- element density and material interpolation ----------------------------------------------
 // rhoE[e] = 1/npe sum_a rho[conn[e, a]]        (examples/thermal.py:348-353, natural_frequency.py:399-404)
-//   npe = 4 (Q4) or 8 (H8) nodes per element
+//   npe = 4 (Q4), 8 (H8) or 10 (T10) nodes per element
 // law 0 (thermal.py:132,198,175-188,236-244): ks = k0((1-b) r^p + b), ms = c0((1-b) r + b)
 // law 1 (natural_frequency.py:140-143,219-220 "simp"): ks = r^p + r0, ms = c0 r
 // law 2 (RAMP, natural_frequency.py:142-143): ks = r/(1+q(1-r)) + r0, ms = c0 r
@@ -263,8 +263,11 @@ __global__ void q4_material_kernel(int law, int nelems, int npe, const int* __re
     const int* c = conn + (int64_t)npe * e;
     if (npe == 4)
       r = 0.25 * (rho[c[0]] + rho[c[1]] + rho[c[2]] + rho[c[3]]);
-    else
+    else if (npe == 8)
       r = 0.125 * (rho[c[0]] + rho[c[1]] + rho[c[2]] + rho[c[3]] + rho[c[4]] + rho[c[5]] + rho[c[6]] + rho[c[7]]);
+    else
+      r = 0.1 * (rho[c[0]] + rho[c[1]] + rho[c[2]] + rho[c[3]] + rho[c[4]] + rho[c[5]] + rho[c[6]] + rho[c[7]] + rho[c[8]] +
+                 rho[c[9]]);
     if (rhoE) rhoE[e] = r;
   } else {
     r = rho[e];
@@ -298,7 +301,10 @@ extern "C" int eigd_q4_material(int law, int nelems, int npe, const int* d_conn,
                                 double* d_rhoE, double* d_ks, double* d_ms, double* d_dk, double* d_dm) {
   if (nelems <= 0) return 0;
   if (law < 0 || law > 2) { eigd_set_error("q4_material: unknown law %d", law); return 1; }
-  if (npe != 4 && npe != 8) { eigd_set_error("q4_material: %d nodes per element (4: Q4, 8: H8)", npe); return 1; }
+  if (npe != 4 && npe != 8 && npe != 10) {
+    eigd_set_error("q4_material: %d nodes per element (4: Q4, 8: H8, 10: T10)", npe);
+    return 1;
+  }
   EIGD_LAUNCH(q4_material_kernel, (nelems + 255) / 256, 256, 0, law, nelems, npe, d_conn, d_rho, par4[0], par4[1], par4[2],
               par4[3], d_rhoE, d_ks, d_ms, d_dk, d_dm);
   EIGD_CHECK_LAUNCH();

@@ -3,7 +3,7 @@
 // design coefficients:  K_e = c1[e] E1_e + c3[e] E3_e  (flat shell: membrane + transverse shear ~ t, bending ~ t^3;
 // mass: translation ~ t, rotary inertia ~ t^3).  With 180 GB of HBM the unit matrices of a 1M-DOF shell model
 // (167k elements x 576 x 4 arrays = 3 GB) simply stay resident; per design only the coefficients change.  The H8
-// solid (h8.cu) uses them with one term per matrix: K_e = ks[e] K0_e, M_e = ms[e] M0_e.
+// and T10 elements (h8.cu, t10.cu) use them with one term per matrix: K_e = ks[e] K0_e, M_e = ms[e] M0_e.
 //
 // Replaces, for the CRM-like driver (reference examples/crm.py:122-142, 331-355), what TACS does on the host:
 //   assembleMatType(STIFFNESS_MATRIX / MASS_MATRIX)            -> eigd_stored_assemble (gather form, no atomics)
@@ -166,7 +166,12 @@ extern "C" int eigd_stored_quadform(int nelems, int ne, const int* d_dofmap, con
   switch (ne) {
     case 24: stored_quadform_launch<24>(grid, t3, two, nelems, d_dofmap, d_E1, d_E3, d_c1, d_c3, d_W, d_V, N, ld, d_out, d_F1, d_d1, d_W2, s1, s2); break;
     case 8: stored_quadform_launch<8>(grid, t3, two, nelems, d_dofmap, d_E1, d_E3, d_c1, d_c3, d_W, d_V, N, ld, d_out, d_F1, d_d1, d_W2, s1, s2); break;
-    default: eigd_set_error("stored_quadform: element size %d not instantiated (24: shell Q4 and H8, 8: membrane Q4)", ne); return 7;
+    case 30: stored_quadform_launch<30>(grid, t3, two, nelems, d_dofmap, d_E1, d_E3, d_c1, d_c3, d_W, d_V, N, ld, d_out, d_F1, d_d1, d_W2, s1, s2); break;
+    case 10: stored_quadform_launch<10>(grid, t3, two, nelems, d_dofmap, d_E1, d_E3, d_c1, d_c3, d_W, d_V, N, ld, d_out, d_F1, d_d1, d_W2, s1, s2); break;
+    default:
+      eigd_set_error("stored_quadform: element size %d not instantiated (24: shell Q4 and H8, 8: membrane Q4 and scalar H8, "
+                     "30: T10, 10: scalar T10)", ne);
+      return 7;
   }
   EIGD_CHECK_LAUNCH();
   return 0;

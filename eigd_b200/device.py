@@ -851,7 +851,7 @@ def filter_project(rho, beta, eta, g=None):
 
 
 # ------------------------------------------------------------------------------------------
-# stored unit element matrices (csrc/stored_fe.cu, csrc/h8.cu)
+# stored unit element matrices (csrc/stored_fe.cu, csrc/h8.cu, csrc/t10.cu)
 # ------------------------------------------------------------------------------------------
 def h8_element_matrices(conn, X, E, nu, density, K0, M0):
     """Unit stiffness and mass matrices K0, M0 (nelems * 576 each) of the H8 elements ``conn`` (nelems, 8)."""
@@ -863,6 +863,19 @@ def h8_thermal_element_matrices(conn, X, K0, M0):
     """Unit conductivity and capacity matrices K0, M0 (nelems * 64 each) of the scalar H8 elements ``conn`` (nelems, 8)."""
     check(_lib.load().eigd_h8_thermal_element_matrices(conn.shape[0], _ptr(conn), _ptr(X), _ptr(K0), _ptr(M0)),
           "h8_thermal_element_matrices")
+
+
+def t10_element_matrices(conn, X, E, nu, density, K0, M0):
+    """Unit stiffness and mass matrices K0, M0 (nelems * 900 each) of the T10 elements ``conn`` (nelems, 10)."""
+    check(_lib.load().eigd_t10_element_matrices(conn.shape[0], _ptr(conn), _ptr(X), float(E), float(nu), float(density),
+                                                _ptr(K0), _ptr(M0)), "t10_element_matrices")
+
+
+def t10_thermal_element_matrices(conn, X, K0, M0):
+    """Unit conductivity and capacity matrices K0, M0 (nelems * 100 each) of the scalar T10 elements ``conn``
+    (nelems, 10)."""
+    check(_lib.load().eigd_t10_thermal_element_matrices(conn.shape[0], _ptr(conn), _ptr(X), _ptr(K0), _ptr(M0)),
+          "t10_thermal_element_matrices")
 
 
 def stored_assemble(src_ptr, src, ne, E1, c1, vals, E3=None, c3=None, F1=None, d1=None, vals2=None, F3=None, d3=None):

@@ -1,5 +1,5 @@
-"""Device-side finite-element operators for the Q4 problems of the reference examples, the H8 solid and H8 heat
-conduction.
+"""Device-side finite-element operators for the Q4 problems of the reference examples, the 3-D solid and 3-D heat
+conduction on trilinear hexahedra (H8) and quadratic tetrahedra (T10).
 
 Host part (numpy, runs once per mesh): mesh numbering, DOF maps, the CSR pattern of K/M and the
 integer assembly maps (element, a, b) -> CSR non-zero, node -> element adjacency, the conic
@@ -51,6 +51,65 @@ def hex_mesh(nx, ny, nz, Lx=1.0, Ly=1.0, Lz=1.0):
             c = nodes[di:di + nx, dj:dj + ny, dk:dk + nz]
             conn[:, 4 * dk + a] = c.transpose(2, 1, 0).ravel()      # i fastest, then j, then k
     return conn, X
+
+
+# corner pairs of the T10 midside nodes 4-9 (VTK quadratic tetra)
+TET10_EDGES = ((0, 1), (1, 2), (2, 0), (0, 3), (1, 3), (2, 3))
+
+
+def tet10_mesh(nx, ny, nz, Lx=1.0, Ly=1.0, Lz=1.0):
+    """Structured T10 mesh of a box: nx x ny x nz cubes, each split into 6 tetrahedra around its main diagonal (the
+    Kuhn split, conforming across cubes), with quadratic 10-node elements in VTK order.  The nodes are exactly the
+    (2nx+1)(2ny+1)(2nz+1) points of the half-step lattice, numbered and placed as ``hex_mesh(2nx, 2ny, 2nz, ...)`` does,
+    so that T10 and H8 models on the same nodes can be compared at equal DOF.  Element 6 c + t is tetrahedron t of cube
+    c = i + nx*(j + ny*k); corner volumes are positive.  Returns conn (nelems, 10) and X (nnodes, 3)."""
+    _, X = hex_mesh(2 * nx, 2 * ny, 2 * nz, Lx, Ly, Lz)
+    cube = np.stack([a.transpose(2, 1, 0).ravel() for a in np.meshgrid(np.arange(nx), np.arange(ny), np.arange(nz),
+                                                                        indexing="ij")], axis=1)   # i fastest
+    unit = np.eye(3, dtype=np.int64)
+    conn = np.empty((nx * ny * nz, 6, 10), dtype=np.int64)
+    ny2, nz2 = 2 * ny + 1, 2 * nz + 1
+    # the path (0,0,0) -> +e_a -> +e_b -> (1,1,1) of every axis order (a, b, c); odd orders have negative volume and
+    # get corners 1 and 2 swapped
+    for t, (order, odd) in enumerate((((0, 1, 2), 0), ((1, 2, 0), 0), ((2, 0, 1), 0),
+                                      ((0, 2, 1), 1), ((2, 1, 0), 1), ((1, 0, 2), 1))):
+        v1 = unit[order[0]]
+        corners = [np.zeros(3, dtype=np.int64), v1, v1 + unit[order[1]], np.ones(3, dtype=np.int64)]
+        if odd:
+            corners[1], corners[2] = corners[2], corners[1]
+        offsets = [2 * c for c in corners] + [corners[a] + corners[b] for a, b in TET10_EDGES]   # half-step lattice
+        for a, off in enumerate(offsets):
+            L = 2 * cube + off[None, :]
+            conn[:, t, a] = (L[:, 0] * ny2 + L[:, 1]) * nz2 + L[:, 2]
+    return conn.reshape(-1, 10), X
+
+
+def tet10_from_tet4(conn4, X):
+    """Quadratic tetrahedra from a linear tetrahedral mesh (conn4 (nelems, 4), X (nnodes, 3)), such as one a mesher
+    writes: each edge gets one midside node at its midpoint, numbered after the corner nodes in the order of the sorted
+    edge list.  Negatively oriented elements are flipped (corners 1 and 2 swapped); degenerate elements
+    (|6 V| <= 1e-12 (longest edge)^3) raise ValueError.  Returns conn (nelems, 10) and X (nnodes + nedges, 3)."""
+    conn4 = np.array(conn4, dtype=np.int64)
+    X = np.asarray(X, dtype=np.float64)
+    if conn4.ndim != 2 or conn4.shape[1] != 4 or X.ndim != 2 or X.shape[1] != 3:
+        raise ValueError("tet10_from_tet4 needs conn (nelems, 4) and X (nnodes, 3)")
+    xe = X[conn4]
+    d = xe[:, 1:] - xe[:, :1]
+    vol6 = np.einsum("ei,ei->e", d[:, 0], np.cross(d[:, 1], d[:, 2]))
+    lmax = np.max([np.linalg.norm(xe[:, a] - xe[:, b], axis=1) for a, b in TET10_EDGES], axis=0)
+    bad = np.abs(vol6) <= 1e-12 * lmax ** 3
+    if bad.any():
+        raise ValueError("tet10_from_tet4: %d degenerate element(s), the first is element %d"
+                         % (bad.sum(), np.nonzero(bad)[0][0]))
+    neg = vol6 < 0
+    conn4[neg, 1], conn4[neg, 2] = conn4[neg, 2], conn4[neg, 1].copy()
+    nn = np.int64(X.shape[0])
+    ends = np.stack([conn4[:, [a, b]] for a, b in TET10_EDGES], axis=1)           # (nelems, 6, 2)
+    key = ends.min(axis=2) * nn + ends.max(axis=2)
+    ukey, inv = np.unique(key.ravel(), return_inverse=True)
+    Xm = 0.5 * (X[ukey // nn] + X[ukey % nn])
+    conn = np.concatenate([conn4, nn + inv.reshape(-1, 6)], axis=1)
+    return conn, np.concatenate([X, Xm], axis=0)
 
 
 def element_dofs(conn, dof):
@@ -304,6 +363,19 @@ class _StoredMatrixModel(_ElementModel):
         ne2 = self.NE * self.NE
         self.K0_d, self.M0_d = D.empty(self.nelems * ne2), D.empty(self.nelems * ne2)
 
+    def _setup_tet(self, conn, X, dof, law, par):
+        """``_setup`` on a quadratic tetrahedral mesh, conn (nelems, 10) and X (nnodes, 3) (ValueError otherwise), the
+        element dof map and room for K0, M0, which the subclass's element kernel fills."""
+        conn = np.asarray(conn, dtype=np.int64)
+        X = np.asarray(X, dtype=np.float64)
+        if conn.ndim != 2 or conn.shape[1] != 10 or X.ndim != 2 or X.shape[1] != 3:
+            raise ValueError("%s needs conn (nelems, 10) and X (nnodes, 3)" % type(self).__name__)
+        self._setup(conn, X, X.shape[0], dof, law, par)
+        self.X_d = to_dev(np.ascontiguousarray(self.X))
+        self.dofmap_d = torch.as_tensor(self.var.astype(np.int32), device=D.dev())
+        ne2 = self.NE * self.NE
+        self.K0_d, self.M0_d = D.empty(self.nelems * ne2), D.empty(self.nelems * ne2)
+
     def _assemble_values(self, ck, cm):
         p = self.pattern
         Kv, Mv = D.empty(self.nnz), D.empty(self.nnz)
@@ -359,6 +431,35 @@ class H8ThermalProblem(_StoredMatrixModel):
     def __init__(self, conn, X, kappa=1.0, density=1.0, heat_capacity=1.0, p=3.0, beta=1e-6):
         self._setup_hex(conn, X, 1, 0, np.array([p, kappa, heat_capacity * density, beta]))
         D.h8_thermal_element_matrices(self.conn_d, self.X_d, self.K0_d, self.M0_d)
+
+
+class T10Problem(_StoredMatrixModel):
+    """Free 3-D isotropic solid on quadratic tetrahedra (T10, 3 DOF/node), with the material laws and interface of
+    ``H8Problem``: K_e = s(rho_e) K0_e, M_e = rho_e M0_e, rho_e the mean of the 10 nodal densities.  The unit matrices
+    K0_e = sum_q w_q detJ B^T C B and M0_e = density sum_q w_q detJ (N N^T (x) I_3) (14-point degree-5 rule) are
+    computed once per mesh on the device (eigd_t10_element_matrices, 14.4 KB per element for the pair) and stay
+    resident; per design, assembly and the sensitivities are the stored-matrix kernels.  Node order: ``tet10_mesh``."""
+
+    npe = 10
+    NE = 30
+
+    def __init__(self, conn, X, E=1.0, nu=0.3, density=1.0, p=3.0, rho0_K=1e-6, ptype_K="simp", q=5.0):
+        self._setup_tet(conn, X, 3, *_penalty_law("ptype_K", ptype_K, p, q, 1.0, rho0_K))
+        D.t10_element_matrices(self.conn_d, self.X_d, E, nu, density, self.K0_d, self.M0_d)
+
+
+class T10ThermalProblem(_StoredMatrixModel):
+    """Heat conduction on quadratic tetrahedra (1 DOF/node), with the thermal law and interface of
+    ``H8ThermalProblem``; rho_e is the mean of the 10 nodal densities.  The unit matrices K0_e = sum_q w_q detJ
+    grad N grad N^T and M0_e = sum_q w_q detJ N N^T are computed once per mesh on the device
+    (eigd_t10_thermal_element_matrices, 1.6 KB per element for the pair) and stay resident."""
+
+    npe = 10
+    NE = 10
+
+    def __init__(self, conn, X, kappa=1.0, density=1.0, heat_capacity=1.0, p=3.0, beta=1e-6):
+        self._setup_tet(conn, X, 1, 0, np.array([p, kappa, heat_capacity * density, beta]))
+        D.t10_thermal_element_matrices(self.conn_d, self.X_d, self.K0_d, self.M0_d)
 
 
 def reduced_structure(indptr, indices, src_ptr, src, reduced, ndof):
@@ -597,7 +698,7 @@ class NodeFilter:
     (examples/node_filter.py:61-88), applied on the device as CSR products (:164-217).
     Spatial filter with optional design-variable map (the symmetric column of examples/buckling.py:1331-1344)
     and optional tanh projection (``projection=True``, ``beta``, ``eta``).  ``ftype="helmholtz"`` is the PDE filter
-    (``_init_helmholtz``) on a Q4 mesh (2-D coordinates) or a hexahedral mesh (3-D coordinates); in 3-D it replaces the
+    (``_init_helmholtz``) on a Q4 mesh (2-D coordinates) or a hexahedral or T10 mesh (3-D coordinates); in 3-D it replaces the
     conic filter's pair search and its two CSR operators by one scalar LDL^T of the mesh, factored once."""
 
     ftype = "spatial"
@@ -650,9 +751,10 @@ class NodeFilter:
 
     def _init_helmholtz(self, conn, r0, num_design_vars):
         """Helmholtz (PDE) filter of examples/node_filter.py:90-162: rho = A^-1 (B x) with A = r0^2 int grad N . grad N +
-        int N N and B = int N N on the element mesh: Q4 for 2-D coordinates with 4-node ``conn``, trilinear hexahedra for
-        3-D coordinates with 8-node ``conn``.  A and B are the unit-material conductivity / capacity matrices of
-        ``Q4Problem(kind="thermal")`` or ``H8ThermalProblem`` (assembled by the same kernels), A is factored once by the
+        int N N and B = int N N on the element mesh: Q4 for 2-D coordinates with 4-node ``conn``, trilinear hexahedra or
+        quadratic tetrahedra for 3-D coordinates with 8- or 10-node ``conn``.  A and B are the unit-material conductivity
+        / capacity matrices of ``Q4Problem(kind="thermal")``, ``H8ThermalProblem`` or ``T10ThermalProblem`` (assembled
+        by the same kernels), A is factored once by the
         GPU LDL^T (the reference uses scipy's ``factorized``) and applied to one right-hand side per call."""
         from .eigenvector_derivatives import SpLuOperator
         conn = np.asarray(conn, dtype=np.int64)
@@ -660,14 +762,14 @@ class NodeFilter:
         fronts = "resident"
         if (dim, npe) == (2, 4):
             prob = Q4Problem(conn, self.X, "thermal", kappa=1.0, density=1.0, heat_capacity=1.0, p=1.0, beta=0.0)
-        elif (dim, npe) == (3, 8):
-            prob = H8ThermalProblem(conn, self.X, p=1.0, beta=0.0)
+        elif (dim, npe) in ((3, 8), (3, 10)):
+            prob = (H8ThermalProblem if npe == 8 else T10ThermalProblem)(conn, self.X, p=1.0, beta=0.0)
             # A is factored once and only solved with afterwards, so a pooled factor keeps no dense fronts for the
             # filter's life (17 GB at 80 x 64 x 48 hexahedra); it is bitwise the resident factor.
             fronts = "pooled"
         else:
             raise ValueError("the Helmholtz filter needs 2-D coordinates with 4-node (Q4) conn or 3-D coordinates with "
-                             "8-node (H8) conn; got %d-D coordinates with %d-node conn" % (dim, npe))
+                             "8-node (H8) or 10-node (T10) conn; got %d-D coordinates with %d-node conn" % (dim, npe))
         prob.set_density(rhoE=np.ones(prob.nelems))
         K, M = prob.assemble()
         self._hB = M

@@ -272,6 +272,14 @@ class ThermalTopology3DAnalysis(ThermalTopologyAnalysis):
         return fe.H8ThermalProblem(self.conn, self.X, **material)
 
 
+class ThermalTopologyTetAnalysis(ThermalTopologyAnalysis):
+    """The heat-conduction problem of ``ThermalTopologyAnalysis`` on a 3-D body of quadratic tetrahedra
+    (``fe.T10ThermalProblem``, conn (nelems, 10)): everything else as ``ThermalTopology3DAnalysis``."""
+
+    def _make_problem(self, **material):
+        return fe.T10ThermalProblem(self.conn, self.X, **material)
+
+
 class NaturalFrequencyAnalysis(_Q4Analysis):
     """examples/natural_frequency.py ``TopologyAnalysis``: free plane-stress structure, N + 3 modes
     computed with sigma < 0 and the three rigid-body modes dropped (:348, :383-384, :457-458)."""
@@ -355,6 +363,14 @@ class NaturalFrequency3DAnalysis(NaturalFrequencyAnalysis):
 
     def add_point_derivative(self, name, x0b, xcoefb):
         raise NotImplementedError("node-set point derivatives are defined for the 2-D model only")
+
+
+class NaturalFrequencyTetAnalysis(NaturalFrequency3DAnalysis):
+    """The natural-frequency problem of ``NaturalFrequency3DAnalysis`` on a free 3-D solid of quadratic tetrahedra
+    (``fe.T10Problem``, conn (nelems, 10)): six rigid-body modes dropped, same pipeline and objective helpers."""
+
+    def _make_problem(self, **material):
+        return fe.T10Problem(self.conn, self.X, **material)
 
 
 class MinFreqOpt:
@@ -450,6 +466,17 @@ def make_thermal_3d_model(nx=80, ny=64, nz=48, Lx=1.0, Ly=0.8, Lz=0.6, rfact=4.0
     return ThermalTopology3DAnalysis(fltr, conn, X, **kwargs)
 
 
+def make_thermal_tet_model(nx=40, ny=32, nz=24, Lx=1.0, Ly=0.8, Lz=0.6, rfact=4.0, ftype="spatial", **kwargs):
+    """Insulated box of nx x ny x nz cubes, 6 quadratic tetrahedra each (``fe.tet10_mesh``), of
+    ``ThermalTopologyTetAnalysis``, one design variable per node.  Its nodes are those of
+    ``make_thermal_3d_model(2 nx, 2 ny, 2 nz)``: the default has the 257 985 DOF of the H8 default, and the filter
+    radius, rfact times the node spacing Ly / (2 ny), is the H8 model's on the same lattice.  Conic
+    (``ftype="spatial"``) or Helmholtz (``"helmholtz"``) filter; ``fronts=`` and the solver options go to the driver."""
+    conn, X = fe.tet10_mesh(nx, ny, nz, Lx, Ly, Lz)
+    fltr = fe.NodeFilter(conn, X, r0=rfact * (Ly / (2 * ny)), ftype=ftype)
+    return ThermalTopologyTetAnalysis(fltr, conn, X, **kwargs)
+
+
 def natural_frequency_design_map(nx, ny, rfact=4.0, Mx=3, My=3, ns=2):
     """Design-variable map, node sets and element sets of examples/natural_frequency.py ``make_model`` (:896-954):
     Mx x My patches of non-design material (dvmap = -1, the filter treats them as x = 1) and a four-fold mirror
@@ -513,6 +540,17 @@ def make_natural_frequency_3d_model(nx, ny, nz, Lx=2.0, Ly=1.0, Lz=1.0, rfact=4.
     conn, X = fe.hex_mesh(nx, ny, nz, Lx, Ly, Lz)
     fltr = fe.NodeFilter(conn, X, r0=rfact * (Ly / ny))
     return NaturalFrequency3DAnalysis(fltr, conn, X, **kwargs)
+
+
+def make_natural_frequency_tet_model(nx=32, ny=16, nz=16, Lx=2.0, Ly=1.0, Lz=1.0, rfact=4.0, **kwargs):
+    """Free box of nx x ny x nz cubes, 6 quadratic tetrahedra each (``fe.tet10_mesh``), of
+    ``NaturalFrequencyTetAnalysis``, one design variable per node, conic filter of radius rfact times the node spacing
+    Ly / (2 ny).  Its nodes are those of ``make_natural_frequency_3d_model(2 nx, 2 ny, 2 nz)``: the default has the
+    212 355 DOF of the H8 64 x 32 x 32 box and the same filter radius.  ``fronts=`` and the solver options go to the
+    driver."""
+    conn, X = fe.tet10_mesh(nx, ny, nz, Lx, Ly, Lz)
+    fltr = fe.NodeFilter(conn, X, r0=rfact * (Ly / (2 * ny)))
+    return NaturalFrequencyTetAnalysis(fltr, conn, X, **kwargs)
 
 
 # ------------------------------------------------------------------------------------------

@@ -243,7 +243,7 @@ int eigd_q4_assemble(int kind, int nelems, const int* d_conn, const double* d_xy
 int eigd_q4_quadforms(int kind, int nelems, const int* d_conn, const double* d_xy, const double* d_cmat6,
                       const double* d_WA, const double* d_WB, const double* d_V, int N, int ldw,
                       const double* d_dk, const double* d_dm, double sA, double sB, double* d_out);
-/* Element density rhoE[e] = 1/npe sum_a rho[conn[e,a]], npe = 4 (Q4) or 8 (H8) nodes per element (d_conn NULL:
+/* Element density rhoE[e] = 1/npe sum_a rho[conn[e,a]], npe = 4 (Q4), 8 (H8) or 10 (T10) nodes per element (d_conn NULL:
  * d_rho is already per element) and the
  * penalised material factors / derivatives of the examples (thermal.py:132,175-188,198,236-244;
  * natural_frequency.py:140-143,198-201,219-220).  law 0 thermal SIMP, 1 structural SIMP, 2 RAMP;
@@ -260,6 +260,16 @@ int eigd_h8_element_matrices(int nelems, const int* d_conn, const double* d_X, d
  * K0, M0 (nelems, 8, 8) row-major, K0_e = sum_q detJ grad N_a . grad N_b, M0_e = sum_q detJ N_a N_b (unit material;
  * M0 is bitwise the scalar block of eigd_h8_element_matrices' M0 at density 1). */
 int eigd_h8_thermal_element_matrices(int nelems, const int* d_conn, const double* d_X, double* d_K0, double* d_M0);
+/* ---- quadratic tetrahedra (csrc/t10.cu): unit element matrices on the 14-point degree-5 rule, once per mesh.
+ *      conn (nelems, 10), VTK quadratic-tetra order: corners 0-3 (positive volume), then the midside nodes of the edges
+ *      (0,1), (1,2), (2,0), (0,3), (1,3), (2,3); X (nnodes, 3).  Solid: K0, M0 (nelems, 30, 30) row-major, dof order
+ *      node-major (u_x, u_y, u_z); K0_e = sum_q w_q detJ B^T C(E, nu) B, M0_e = density sum_q w_q detJ (N N^T (x) I_3). */
+int eigd_t10_element_matrices(int nelems, const int* d_conn, const double* d_X, double E, double nu, double density,
+                              double* d_K0, double* d_M0);
+/* Scalar (heat conduction) T10, one dof per node in node order: K0, M0 (nelems, 10, 10) row-major,
+ * K0_e = sum_q w_q detJ grad N_a . grad N_b, M0_e = sum_q w_q detJ N_a N_b (M0 is bitwise the scalar block of
+ * eigd_t10_element_matrices' M0 at density 1). */
+int eigd_t10_thermal_element_matrices(int nelems, const int* d_conn, const double* d_X, double* d_K0, double* d_M0);
 /* node_out[v] = scale * sum_{e in adj(v)} e_vals[e]   (gather form of np.add.at, thermal.py:612-615) */
 int eigd_node_gather(int nnodes, const int* d_nptr, const int* d_nelem, const double* d_evals, double scale, double* d_out);
 /* out[ncomp v + i] = sum_{e around v} due[e][ncomp local + i], due (nelems, npe * ncomp), local = d_nlocal (the node's

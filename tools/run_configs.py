@@ -7,10 +7,18 @@
     python tools/run_configs.py h8buck [--nx 32 --ny 24 --nz 128 --modes 10 --fd]   buckling of a clamped 3-D column
     python tools/run_configs.py h8thermal [--nx 80 --ny 64 --nz 48 --modes 10 --ftype spatial|helmholtz --fd]
                                                                        heat conduction in an insulated 3-D box (1 dof/node)
+    python tools/run_configs.py t10 [--nx 32 --ny 16 --nz 16 --modes 10 --fd]   the h8 solid on quadratic tetrahedra
+    python tools/run_configs.py t10thermal [--nx 40 --ny 32 --nz 24 --modes 10 --ftype spatial|helmholtz --fd]
+                                                                       the h8thermal box on quadratic tetrahedra
+
+t10 and t10thermal count cubes of 6 tetrahedra (fe.tet10_mesh): their nodes, DOF and filter radius are those of h8 and
+h8thermal at twice the element counts (the defaults 64 x 32 x 32 and 80 x 64 x 48).
 
 h8, h8buck and h8thermal take --fronts resident|pooled (the front memory of the factors) and report, for either mode,
 the pool size, the persistent bytes of the factors, torch's peak allocated device memory and the factorisation time.
 h8thermal also reports the set-up time, device memory and per-design time (apply + apply_gradient) of its filter.
+All four of h8, h8thermal, t10 and t10thermal report the time and bytes of the unit element matrices (the element kernel
+alone, into fresh buffers) and the time of one fused df/dx call (stored_quadform on the last adjoint's operands).
 
 Each prints one JSON line: stage times (CUDA-synchronised wall clock of the driver's own timers, as the
 reference examples report them), solve counts, factor statistics, and size-independent acceptance checks
@@ -233,17 +241,51 @@ def gpu_card():
         return "unavailable: %s" % exc
 
 
+def _element_setup(prob, reps=3):
+    """The element kernel that fills the model's unit matrices, rerun into fresh buffers (device-synchronised, every
+    repetition), and the bytes of the resident pair."""
+    import torch
+    from eigd_b200 import device as D, fe
+    K0, M0 = torch.empty_like(prob.K0_d), torch.empty_like(prob.M0_d)
+    solid = {fe.H8Problem: D.h8_element_matrices, fe.T10Problem: D.t10_element_matrices}
+    scalar = {fe.H8ThermalProblem: D.h8_thermal_element_matrices, fe.T10ThermalProblem: D.t10_thermal_element_matrices}
+    times = []
+    for _ in range(reps):
+        t0 = now()
+        if type(prob) in solid:
+            solid[type(prob)](prob.conn_d, prob.X_d, 1.0, 0.3, 1.0, K0, M0)
+        else:
+            scalar[type(prob)](prob.conn_d, prob.X_d, K0, M0)
+        times.append(now() - t0)
+    return {"kernel_s": times, "bytes": int(prob.K0_d.numel() + prob.M0_d.numel()) * 8, "NE": prob.NE,
+            "nelems": int(prob.nelems)}
+
+
+def _dfdx_kernel(model, reps=5):
+    """One fused df/dx call (both terms, stored_quadform over N + nrigid columns) on the last adjoint's operands,
+    device-synchronised, every repetition."""
+    times = []
+    for _ in range(reps):
+        t0 = now()
+        model.prob.device_call_fused(model.psi0, model.psi0, model.Q0, 1.0, -1.0)
+        times.append(now() - t0)
+    return times
+
+
 def run_h8(args):
-    """Free nx x ny x nz box of hexahedra (NaturalFrequency3DAnalysis): N flexible modes + 6 rigid-body modes about
-    sigma = -10, IRAM + sibk with the Lanczos guess, tensor derivative, f = sum_i (phi_i . w_i)^2 as the seed."""
+    """Free nx x ny x nz box of hexahedra (NaturalFrequency3DAnalysis), or with ``args.config == "t10"`` of
+    nx x ny x nz cubes of quadratic tetrahedra (NaturalFrequencyTetAnalysis): N flexible modes + 6 rigid-body modes
+    about sigma = -10, IRAM + sibk with the Lanczos guess, tensor derivative, f = sum_i (phi_i . w_i)^2 as the seed."""
     import torch
     from eigd_b200 import device as D, topo as T
     D.init()
-    out = {"config": "H8 free solid nx=%d ny=%d nz=%d" % (args.nx, args.ny, args.nz), "N": args.modes, "gpu": gpu_card()}
+    tet = args.config == "t10"
+    out = {"config": "%s free solid nx=%d ny=%d nz=%d" % ("T10" if tet else "H8", args.nx, args.ny, args.nz),
+           "N": args.modes, "gpu": gpu_card()}
     t0 = now()
-    model = T.make_natural_frequency_3d_model(args.nx, args.ny, args.nz, N=args.modes, m=60, sigma=-10.0, solver_type="IRAM",
-                                              adjoint_method="sibk", adjoint_options={"lanczos_guess": True}, rtol=1e-10,
-                                              deriv_type="tensor", fronts=args.fronts)
+    make = T.make_natural_frequency_tet_model if tet else T.make_natural_frequency_3d_model
+    model = make(args.nx, args.ny, args.nz, N=args.modes, m=60, sigma=-10.0, solver_type="IRAM", adjoint_method="sibk",
+                 adjoint_options={"lanczos_guess": True}, rtol=1e-10, deriv_type="tensor", fronts=args.fronts)
     out.update(n=int(model.nvars), nnz=int(model.prob.nnz), fronts=args.fronts, host_setup_s=now() - t0)
     torch.cuda.reset_peak_memory_stats()
     w_d = D.to_device(np.random.default_rng(99).normal(size=(model.nvars, args.modes)))
@@ -269,6 +311,8 @@ def run_h8(args):
     out["peak_device_bytes"] = int(torch.cuda.max_memory_allocated())
     out["factorisation_s"] = _time_factorisation(model)
     out["memory"] = _factor_memory(model, [model.factor])
+    out["element_matrices"] = _element_setup(model.prob)
+    out["dfdx_kernel_s"] = _dfdx_kernel(model)
     out["lam_first"] = [float(v) for v in model.lam[:3]]
     out["rigid_lam"] = [float(v) for v in model.lam0[:6]]
     out["factor_info"] = model.factor.info
@@ -382,21 +426,24 @@ def run_h8buck(args):
 
 def run_h8thermal(args):
     """Insulated nx x ny x nz box of hexahedra (ThermalTopology3DAnalysis; mesh, filter radius and driver of
-    make_thermal_3d_model, built step by step so that the filter is timed alone): N modes about sigma = -0.1, mode 0
-    the zero mode, IRAM + sibk with the Lanczos guess, tensor derivative, thermal compliance against the seeded uniform
-    heat vector of bench.py as the objective, conic or Helmholtz filter (--ftype)."""
+    make_thermal_3d_model, built step by step so that the filter is timed alone), or with ``args.config ==
+    "t10thermal"`` of nx x ny x nz cubes of quadratic tetrahedra (ThermalTopologyTetAnalysis, make_thermal_tet_model):
+    N modes about sigma = -0.1, mode 0 the zero mode, IRAM + sibk with the Lanczos guess, tensor derivative, thermal
+    compliance against the seeded uniform heat vector of bench.py as the objective, conic or Helmholtz filter
+    (--ftype)."""
     import torch
     from eigd_b200 import device as D, fe, topo as T
     D.init()
+    tet = args.config == "t10thermal"
     Lx, Ly, Lz = 1.0, 0.8, 0.6
-    out = {"config": "H8 thermal box nx=%d ny=%d nz=%d" % (args.nx, args.ny, args.nz), "N": args.modes,
-           "ftype": args.ftype, "gpu": gpu_card()}
+    out = {"config": "%s thermal box nx=%d ny=%d nz=%d" % ("T10" if tet else "H8", args.nx, args.ny, args.nz),
+           "N": args.modes, "ftype": args.ftype, "gpu": gpu_card()}
     t0 = time.perf_counter()
-    conn, X = fe.hex_mesh(args.nx, args.ny, args.nz, Lx, Ly, Lz)
+    conn, X = (fe.tet10_mesh if tet else fe.hex_mesh)(args.nx, args.ny, args.nz, Lx, Ly, Lz)
     t_mesh = time.perf_counter() - t0
     m0 = torch.cuda.memory_allocated()
     t0 = now()
-    fltr = fe.NodeFilter(conn, X, r0=4.0 * Ly / args.ny, ftype=args.ftype)
+    fltr = fe.NodeFilter(conn, X, r0=4.0 * Ly / ((2 if tet else 1) * args.ny), ftype=args.ftype)
     filt = {"host_setup_s": now() - t0, "device_bytes": int(torch.cuda.memory_allocated() - m0)}
     if args.ftype == "spatial":
         filt["nnz_F"] = int(fltr.F.nnz)
@@ -404,9 +451,9 @@ def run_h8thermal(args):
         filt.update(factor_bytes=fltr._hA.lu.nbytes(), pool_bytes=fltr._hA.lu.pool_bytes(),
                     symbolic=fltr._hA.lu.sym.stats())
     t0 = now()
-    model = T.ThermalTopology3DAnalysis(fltr, conn, X, N=args.modes, m=60, sigma=-0.1, solver_type="IRAM",
-                                        adjoint_method="sibk", adjoint_options={"lanczos_guess": True}, rtol=1e-10,
-                                        deriv_type="tensor", fronts=args.fronts)
+    model = (T.ThermalTopologyTetAnalysis if tet else T.ThermalTopology3DAnalysis)(
+        fltr, conn, X, N=args.modes, m=60, sigma=-0.1, solver_type="IRAM", adjoint_method="sibk",
+        adjoint_options={"lanczos_guess": True}, rtol=1e-10, deriv_type="tensor", fronts=args.fronts)
     out.update(n=int(model.nvars), nnz=int(model.prob.nnz), fronts=args.fronts, mesh_s=t_mesh,
                host_setup_s=now() - t0, filter=filt)
     torch.cuda.reset_peak_memory_stats()
@@ -433,6 +480,8 @@ def run_h8thermal(args):
     out["peak_device_bytes"] = int(torch.cuda.max_memory_allocated())
     out["factorisation_s"] = _time_factorisation(model)
     out["memory"] = _factor_memory(model, [model.factor])
+    out["element_matrices"] = _element_setup(model.prob)
+    out["dfdx_kernel_s"] = _dfdx_kernel(model)
     x_d, g_d = D.to_device(x0), D.to_device(np.random.default_rng(2).normal(size=model.nnodes))
     filt["apply_plus_gradient_s"] = []
     for _ in range(5):
@@ -507,17 +556,17 @@ def _time_factorisation(model, reps=3):
 
 if __name__ == "__main__":
     ap = argparse.ArgumentParser()
-    ap.add_argument("config", choices=["c3", "c4", "c4plate", "c5", "h8", "h8buck", "h8thermal"])
+    ap.add_argument("config", choices=["c3", "c4", "c4plate", "c5", "h8", "h8buck", "h8thermal", "t10", "t10thermal"])
     ap.add_argument("--fd", action="store_true", help="c4: add the finite-difference check of the gradient")
     ap.add_argument("--nx", type=int, default=None)
     ap.add_argument("--ny", type=int, default=None)
-    ap.add_argument("--nz", type=int, default=None, help="h8, h8buck, h8thermal: elements along z")
+    ap.add_argument("--nz", type=int, default=None, help="h8, h8buck, h8thermal, t10, t10thermal: elements (cubes) along z")
     ap.add_argument("--modes", type=int, default=None)
     ap.add_argument("--designs", type=int, default=None)
     ap.add_argument("--reps", type=int, default=3)
     ap.add_argument("--fronts", choices=["resident", "pooled"], default="resident",
-                    help="h8, h8buck, h8thermal: front memory of the factors")
-    ap.add_argument("--ftype", choices=["spatial", "helmholtz"], default="spatial", help="h8thermal: filter type")
+                    help="h8, h8buck, h8thermal, t10, t10thermal: front memory of the factors")
+    ap.add_argument("--ftype", choices=["spatial", "helmholtz"], default="spatial", help="h8thermal, t10thermal: filter type")
     a = ap.parse_args()
     if a.config == "c3":
         a.nx, a.ny, a.modes = a.nx or 352, a.ny or 704, a.modes or 20
@@ -533,6 +582,12 @@ if __name__ == "__main__":
         res = run_h8buck(a)
     elif a.config == "h8thermal":
         a.nx, a.ny, a.nz, a.modes = a.nx or 80, a.ny or 64, a.nz or 48, a.modes or 10
+        res = run_h8thermal(a)
+    elif a.config == "t10":
+        a.nx, a.ny, a.nz, a.modes = a.nx or 32, a.ny or 16, a.nz or 16, a.modes or 10
+        res = run_h8(a)
+    elif a.config == "t10thermal":
+        a.nx, a.ny, a.nz, a.modes = a.nx or 40, a.ny or 32, a.nz or 24, a.modes or 10
         res = run_h8thermal(a)
     elif a.config == "c4":
         a.nx, a.ny, a.modes = a.nx or 408, a.ny or 408, a.modes or 20
